@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload stencil27|rmat] [--format csr|tjds] [--variant ...] [--no-secondary]
+                    [--dump-outputs DIR]
 
 Default (N=1): BASELINE.json configs[2], the HBM-roofline run the metric is quoted on --
 27-point stencil on a 369^3 grid (50 243 409 rows, 1 349 232 625 nnz, fp64), CSR, one SpMV per step.
@@ -23,10 +24,16 @@ TJDS atomic / deterministic (configs[4]), each with its own parity check against
 
 `--impl reference` times the reference's own CPU loop (oracle/_ref when it was built, else the
 oracle port) on a bounded sample of the same workload; `config.workload` names the sample it actually ran.
+
+`--dump-outputs DIR` writes the y of the last timed step of every configuration the run times to DIR/<name>.npy
+(float64): `y.npy` for the headline, `y_<secondary name>.npy` for the others.  A y longer than its row budget (2^22
+rows for the headline, 2^19 for each secondary: under 64 MB in all) is written as a sample of rows drawn with a fixed
+seed.  The inputs are seeded too, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
 import os
+import re
 import sys
 import threading
 import time
@@ -69,7 +76,18 @@ def parse_args():
     p.add_argument("--secondary-steps", type=int, default=8)
     p.add_argument("--secondary-scale", type=int, default=26, help="R-MAT scale of the secondary configurations")
     p.add_argument("--no-tune", action="store_true", help="N>1: keep the default exchange scheme (no warm-up tuning)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", help="write the y of the last timed step of every configuration to "
+                   "DIR/<name>.npy (float64, a seeded sample of rows when y is large)")
+    args = p.parse_args()
+    for name in ("steps", "secondary_steps", "cpu_iters"):
+        if getattr(args, name) < 1:
+            p.error("--%s must be at least 1" % name.replace("_", "-"))
+    if args.warmup < 0:
+        p.error("--warmup must not be negative")
+    if args.dump_outputs and args.format == "tjds" and args.gpus > 1 and args.exchange == "none":
+        # without the reduce-scatter every rank holds a partial sum over its columns, no rank holds rows of y
+        p.error("--dump-outputs with --format tjds at --gpus > 1 needs an exchange (not --exchange none)")
+    return args
 
 
 # --------------------------------------------------------------------------------------- helpers
@@ -139,6 +157,28 @@ def tjds_bytes(rows, cols, nnz, ndiag):
     return 12 * nnz + 4 * (ndiag + 1) + 8 * cols + 8 * rows
 
 
+DUMP_ROWS = 1 << 22            # --dump-outputs: rows of the headline y (32 MB of float64)
+DUMP_ROWS_SECONDARY = 1 << 19  # rows of each of the 7 secondary y (4 MB each)
+
+
+def dump_rows(rows, limit):
+    """The rows of a y that --dump-outputs writes: all of them up to `limit`, else at most `limit` rows drawn with a
+    fixed seed, ascending (the same rows for the same arguments in every run)."""
+    if rows <= limit:
+        return np.arange(rows)
+    return np.unique(np.random.default_rng(0).integers(0, rows, limit))
+
+
+def output_name(config_name):
+    """File name of a secondary configuration's y: "R-MAT scale 26 CSR" -> "y_r_mat_scale_26_csr"."""
+    return "y_" + re.sub(r"[^0-9a-z]+", "_", config_name.lower()).strip("_")
+
+
+def save_output(args, name, values):
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    np.save(os.path.join(args.dump_outputs, name + ".npy"), np.asarray(values, np.float64))
+
+
 # --------------------------------------------------------------------------------------- CPU arm
 def stencil_coo_numpy(g):
     """27-point stencil COO on a g^3 grid, (row,col)-sorted, {26,-1} values -- numpy only (no engine).  Built plane by
@@ -197,24 +237,24 @@ def cpu_reference_run(args, iters, drop=0):
         # matrices without empty rows, i.e. the stencil
         if oracle.ref_available() and args.workload == "stencil27":
             kind = "reference"
-            _, ms = oracle.ref_csr_compute(coo, m, iters)
+            y, ms = oracle.ref_csr_compute(coo, m, iters)
             what = "oracle/_ref/libsmvp_ref.so: the unmodified smvp_csr_compute (main-cli.c:325), its own clock_gettime bracket"
         else:
             kind = "port"
             rp, ci, va = oracle.csr_build(coo, m, n)
-            _, ms = oracle.csr_mult_timed(rp, ci, va, np.ones(n), iters)
+            y, ms = oracle.csr_mult_timed(rp, ci, va, np.ones(n), iters)
             what = "oracle/smvp_oracle.c: oracle_csr_mult_timed (restatement of main-cli.c:402-420)"
     else:
         kind = "port"  # the reference's TJDS build is O(nnz*N) (main-cli.c:894-904): not runnable at this size
         t = oracle.tjds_build(coo, m, n)
         nbytes = tjds_bytes(m, n, nnz, t.ndiag)
-        _, ms = oracle.tjds_mult_timed(t, np.ones(n), iters)
+        y, ms = oracle.tjds_mult_timed(t, np.ones(n), iters)
         what = "oracle/smvp_oracle.c: oracle_tjds_mult_timed (restatement of main-cli.c:1004-1024, all diagonals)"
     ms = np.asarray(ms)[drop:]
     avg_ms = float(ms.mean())
     res = {"value": nbytes / (avg_ms * 1e-3) / 1e9, "unit": UNIT, "cores": 1, "kind": kind,
            "sample": sample + "; " + what, "gflops": 2 * nnz / (avg_ms * 1e-3) / 1e9, "ms_per_step": avg_ms,
-           "min_ms": float(ms.min()), "rows": m, "nnz": nnz, "x_bytes": 8 * n}
+           "min_ms": float(ms.min()), "rows": m, "nnz": nnz, "x_bytes": 8 * n, "y": y}
     if args.format == "csr" and not args.no_all_cores:
         # NOT the reference (it is single-threaded): its loop over nnz-balanced row blocks on every core of the box,
         # same sample, so the 1-thread figure can be put in proportion.  Reported beside it, never instead of it.
@@ -233,9 +273,10 @@ def run_reference_arm(args):
     if rank != 0:
         return
     t0 = time.time()
-    iters = max(1, args.steps)
     # warm-up iterations are part of the same call; the first `warmup` timings are dropped
-    res = cpu_reference_run(args, iters + args.warmup, drop=args.warmup)
+    res = cpu_reference_run(args, args.steps + args.warmup, drop=args.warmup)
+    if args.dump_outputs:
+        save_output(args, "y", res["y"][dump_rows(len(res["y"]), DUMP_ROWS)])
     # config.workload names what THIS arm ran: a bounded sample, not the GPU arm's full-size matrix (the reference's
     # builder cannot run at that size: stack VLA main-cli.c:1426, and one CPU pass over it would take seconds)
     cfg = workload_config(args, None)
@@ -339,6 +380,29 @@ def timed_steps(ctx, op, steps, warmup, sample_clocks=True):
     return {"ms_per_step": total_max / steps, "kern_ms_local": kern_ms, "kern_ms_max": kern_max, "launches": int(launches),
             "kern_ms_min": float(per_step.min()), "kern_ms_median": float(np.median(per_step)),
             "clocks": sampler.result() if sampler else None}
+
+
+def dump_output(ctx, args, name, op, limit):
+    """--dump-outputs: the y of op's last step (call it before anything else runs op), the rows of dump_rows(M, limit)
+    gathered from the ranks that hold them, written by rank 0."""
+    if not args.dump_outputs:
+        return
+    torch = ctx.torch
+    if isinstance(op, ctx.sdist.ColBlockTjds):  # rank g holds the g-th of `world` equal slices of the padded y
+        per = op.Mp // ctx.world
+        row0 = ctx.rank * per
+        held = op.last_y()[:max(0, min(per, op.M - row0))]
+    else:
+        row0 = op.r0
+        held = op.last_y()[op.r0:op.r1]
+    idx = torch.from_numpy(dump_rows(op.M, limit)).to("cuda")
+    mine = (idx >= row0) & (idx < row0 + held.numel())
+    vals = torch.full(idx.shape, float("-inf"), dtype=torch.float64, device="cuda")
+    vals[mine] = held[idx[mine] - row0]
+    if ctx.world > 1:
+        ctx.dist.all_reduce(vals, op=ctx.dist.ReduceOp.MAX)  # every row is held by exactly one rank
+    if ctx.rank == 0:
+        save_output(args, name, vals.cpu().numpy())
 
 
 def block_checksums(torch, y, bounds):
@@ -502,12 +566,14 @@ def run_secondary(ctx, args, stencil_gen, y_stencil_csr, x_stencil):
     tjds_variants = (("atomic", eng.TJDS_ATOMIC), ("deterministic", eng.TJDS_DETERMINISTIC),
                      ("deterministic_fast", eng.TJDS_DETERMINISTIC_FAST))
     for vname, variant in tjds_variants:
+        name = "stencil %d^3 TJDS %s" % (args.grid, vname)
         op = sdist.ColBlockTjds(eng, stencil_gen, ctx.rank, ctx.world, variant, exchange=exch_tjds)
         op.set_x(x_stencil, ctx.stream)
         t = timed_steps(ctx, op, steps, 3)
+        dump_output(ctx, args, output_name(name), op, DUMP_ROWS_SECONDARY)
         parity = check_tjds_parity(ctx, op, y_stencil_csr, variant != eng.TJDS_ATOMIC)
-        record("stencil 369^3 TJDS %s" % vname if args.grid == 369 else "stencil %d^3 TJDS %s" % (args.grid, vname),
-               "configs[2]", op, t, parity, {"ndiag": op.ndiag, "tjds_plan": dict(zip(("skewed_walk", "det_route"), op.T.plan()))})
+        record(name, "configs[2]", op, t, parity,
+               {"ndiag": op.ndiag, "tjds_plan": dict(zip(("skewed_walk", "det_route"), op.T.plan()))})
         op.free()
         del op
     del y_stencil_csr
@@ -525,19 +591,23 @@ def run_secondary(ctx, args, stencil_gen, y_stencil_csr, x_stencil):
     if ctx.world > 1 and exch == "pipeline" and not args.no_tune:
         tuning = op.tune_pipeline(ctx.stream)
     t = timed_steps(ctx, op, steps, 3)
+    name = "R-MAT scale %d CSR" % scale
+    dump_output(ctx, args, output_name(name), op, DUMP_ROWS_SECONDARY)
     parity = check_csr_parity(ctx, op, x)
     y_csr = op.last_y().clone() if ctx.world > 1 else op.y_full.clone()
-    record("R-MAT scale %d CSR" % scale, "configs[3]", op, t, parity,
+    record(name, "configs[3]", op, t, parity,
            {"kernel_variant": op.variant_name, "exchange": exch, "exchange_tuning": tuning})
     op.free()
     del op
     torch.cuda.empty_cache()
     for vname, variant in tjds_variants:
+        name = "R-MAT scale %d TJDS %s" % (scale, vname)
         op = sdist.ColBlockTjds(eng, gen, ctx.rank, ctx.world, variant, exchange=exch_tjds)
         op.set_x(x, ctx.stream)
         t = timed_steps(ctx, op, steps, 3)
+        dump_output(ctx, args, output_name(name), op, DUMP_ROWS_SECONDARY)
         parity = check_tjds_parity(ctx, op, y_csr, variant != eng.TJDS_ATOMIC)
-        record("R-MAT scale %d TJDS %s" % (scale, vname), "configs[4]", op, t, parity,
+        record(name, "configs[4]", op, t, parity,
                {"ndiag": op.ndiag, "tjds_plan": dict(zip(("skewed_walk", "det_route"), op.T.plan()))})
         op.free()
         del op
@@ -602,6 +672,7 @@ def run_ours(args):
 
     # ---------------- warm-up, then the timed region: exactly K steps
     t = timed_steps(ctx, op, args.steps, args.warmup)
+    dump_output(ctx, args, "y", op, DUMP_ROWS)
     ms_per_step = t["ms_per_step"]
     value = nbytes / (ms_per_step * 1e-3) / 1e9
 

@@ -1,8 +1,10 @@
 #!/usr/bin/env python3
 """Apply INTEGRATION.md option B to the reference's own main-cli.c and (optionally) build it.
 
-    python integration/apply_dropin.py /root/reference/main-cli.c OUT.c            # splice only
-    python integration/apply_dropin.py --build [REFERENCE_DIR] [OUT_DIR]           # splice + gcc -> OUT_DIR/smvp-toolkit-cli-dropin
+    python integration/apply_dropin.py REFERENCE_DIR/main-cli.c OUT.c              # splice only
+    python integration/apply_dropin.py --build REFERENCE_DIR [OUT_DIR]             # splice + gcc -> OUT_DIR/smvp-toolkit-cli-dropin
+
+REFERENCE_DIR is a checkout of circletile/smvp-toolkit (main-cli.c and mmio/ at its top level).
 
 What changes in the reference's file (nothing else is touched):
   * `#include "smvp_cuda.h"` after `#include "mmio/mmio.h"`;
@@ -88,7 +90,7 @@ def splice(ref_path, out_path):
     return out_path
 
 
-def build(ref_dir="/root/reference", out_dir=None):
+def build(ref_dir, out_dir=None):
     out_dir = out_dir or os.path.join(HERE, "_build")
     os.makedirs(out_dir, exist_ok=True)
     patched = splice(os.path.join(ref_dir, "main-cli.c"), os.path.join(out_dir, "main-cli.dropin.c"))
@@ -105,7 +107,7 @@ def build(ref_dir="/root/reference", out_dir=None):
 
 
 if __name__ == "__main__":
-    if len(sys.argv) >= 2 and sys.argv[1] == "--build":
+    if len(sys.argv) in (3, 4) and sys.argv[1] == "--build":
         print(build(*sys.argv[2:4]))
     elif len(sys.argv) == 3:
         print(splice(sys.argv[1], sys.argv[2]))

@@ -1,24 +1,41 @@
-"""INTEGRATION.md option B, compiled: the reference's OWN main-cli.c with the bodies of smvp_csr_compute
-(/root/reference/main-cli.c:325) and smvp_tjds_compute (:734) replaced by calls into libsmvp_cuda.
-
-CPU part (build container, /root/reference present): integration/apply_dropin.py splices the bodies into a scratch copy
-of the reference's file and gcc builds it against include/smvp_cuda.h -- the drop-in really compiles and binds every
-entry point the brief names.  GPU part: the binary built by __graft_entry__.build() (integration/_build/, shipped to the
-GPU box like oracle/_ref) reproduces the reference's golden CSR reports through the reference's own main(), loader and
-report writer (call sites main-cli.c:1457, :1469)."""
-import glob
+"""INTEGRATION.md option B: integration/apply_dropin.py splices the two bodies of integration/dropin_bodies.c into the
+upstream smvp-toolkit main-cli.c.  The repository holds no line of that file, so the splice is checked on a stand-in:
+a C file with the two functions, taking the parameters the bodies use, and braces hidden in strings, character
+literals and comments."""
 import importlib.util
 import os
 import subprocess
 
-import numpy as np
-import pytest
-
-import util
-
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
-EXE = os.path.join(REPO, "integration", "_build", "smvp-toolkit-cli-dropin")
+
+HEAD = r'''#include <stdio.h>
+#include <stdlib.h>
+#include "mmio/mmio.h"
+#define ANSI_COLOR_RED "\x1b[31m"
+#define ANSI_COLOR_YELLOW "\x1b[33m"
+#define ANSI_COLOR_RESET "\x1b[0m"
+typedef struct { int row, col; double val; } MMRawData;
+struct _time_data_ { double time_total, time_avg, time_stdev, time_min, time_max; double time_each[]; };
+/* double *smvp_csr_compute( in a comment is not a definition */
+'''
+CSR_SIG = "double *smvp_csr_compute(MMRawData *mmImportData, int fInputRows, int fInputNonZeros, int compiter,\n" \
+          "                         struct _time_data_ *csr_time)\n"
+CSR_OLD = r'''{
+    const char *s = "}{\"}"; /* } */
+    char c = '}', d = '\'';
+    // }
+    (void)mmImportData; (void)fInputRows; (void)fInputNonZeros; (void)compiter; (void)csr_time; (void)s; (void)c; (void)d;
+    { return NULL; }
+}'''
+MID = "\n\nstatic int kept(void) { return '{'; }\n\n"
+TJDS_SIG = "double *smvp_tjds_compute(MMRawData *mmImportData, int fInputRows, int fInputColumns, int fInputNonZeros,\n" \
+           "                          int compiter, struct _time_data_ *tjds_time)\n"
+TJDS_OLD = r'''{
+    /* { */
+    (void)mmImportData; (void)fInputRows; (void)fInputColumns; (void)fInputNonZeros; (void)compiter; (void)tjds_time;
+    return NULL;
+}'''
+TAIL = "\n\nint main(void) { return kept() == '}'; }\n"
 
 
 def _apply():
@@ -28,63 +45,21 @@ def _apply():
     return mod
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "main-cli.c")), reason="the reference is only mounted in the build container")
-def test_dropin_splices_and_links(tmp_path):
+def test_splice_replaces_exactly_the_two_bodies_and_compiles(tmp_path):
     mod = _apply()
-    out = mod.splice(os.path.join(REF, "main-cli.c"), str(tmp_path / "main-cli.c"))
+    src = tmp_path / "main-cli.c"
+    src.write_text(HEAD + CSR_SIG + CSR_OLD + MID + TJDS_SIG + TJDS_OLD + TAIL)
+    out = mod.splice(str(src), str(tmp_path / "main-cli.dropin.c"))
     text = open(out).read()
-    ref = open(os.path.join(REF, "main-cli.c")).read()
-    # only the two bodies and one include changed: everything before / between / after them is the reference's text
-    assert '#include "smvp_cuda.h"' in text and "smvp_csr_build(" in text and "smvp_tjds_mult(" in text
-    assert "qsort(mmImportData" not in text.split("double *smvp_csr_compute(")[1].split("void smvp_cisr_coegen(")[0]
-    for keep in ("void smvp_cisr_coegen(", "void generateReportText(", "int main(int argc", "double calcStDevDouble("):
-        assert keep in text
-    assert len(text) < len(ref) - 12000, "the CPU implementations are gone"
-    exe = mod.build(REF, str(tmp_path))
-    und = subprocess.run(["nm", "-D", "--undefined-only", exe], capture_output=True, text=True).stdout
-    for sym in ("smvp_csr_build", "smvp_csr_mult", "smvp_tjds_build", "smvp_tjds_mult", "smvp_time_stats", "smvp_csr_free",
-                "smvp_tjds_free"):
-        assert " U %s" % sym in und, sym
-    assert not os.path.exists(str(tmp_path / "main-cli.dropin.c")), "the spliced copy of the reference's file is not kept"
-
-
-def _close(y, ref, coo):
-    scale = np.abs(coo["val"]).max() if len(coo) else 1.0
-    return np.all(np.abs(y - ref) <= 1e-5 * np.abs(ref) + 1e-12 * scale * 600)
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("name", ["ibm32", "curtis54", "pdp08-pg4", "memplus", "pwt"])
-def test_dropin_reproduces_golden_reports(tmp_path, name):
-    if not os.path.exists(EXE):
-        pytest.skip("integration/_build/smvp-toolkit-cli-dropin not built (needs /root/reference at build time)")
-    m, n, coo = util.load_sample(name)
-    rd = str(tmp_path) + "/"
-    # the reference's own option parser and report writer: -c / -t (its --all-algs runs nothing, U1), -d is mandatory (U2)
-    r = subprocess.run([EXE, "-c", "-n", "7", "-d", rd, util.sample_path(name)], capture_output=True, text=True, cwd=str(tmp_path))
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-    assert "Calculating 7 iterations of SMVP CSR." in r.stdout
-    rep = util.parse_report(glob.glob(str(tmp_path / "smvp-toolbox_report_CSR_*.txt"))[0])
-    assert rep["nnz"] == len(coo) and rep["iters"] == 7 and len(rep["y"]) == m
-    assert rep["min"] <= rep["avg"] <= rep["max"]
-    if (name, "CSR") in util.GOLDEN_REPORTS:
-        gold = util.parse_report(os.path.join(util.GOLDEN, "reports", util.GOLDEN_REPORTS[(name, "CSR")]))
-        if name == "pwt":  # the golden pwt report carries the reference's uninitialised row_ptr[0] in y[0] (U3)
-            assert _close(rep["y"][1:], gold["y"][1:], coo)
-        else:
-            assert _close(rep["y"], gold["y"], coo)
-    # TJDS through the same binary: full product == CSR; with SMVP_DROPIN_REF_COMPAT=1 the shipped truncated product
-    r = subprocess.run([EXE, "-t", "-n", "3", "-d", rd, util.sample_path(name)], capture_output=True, text=True, cwd=str(tmp_path))
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-    rt = util.parse_report(sorted(glob.glob(str(tmp_path / "smvp-toolbox_report_TJDS_*.txt")))[-1])
-    assert _close(rt["y"], rep["y"], coo)
-    if (name, "TJDS") in util.GOLDEN_REPORTS:
-        for f in glob.glob(str(tmp_path / "smvp-toolbox_report_TJDS_*.txt")):
-            os.remove(f)
-        env = dict(os.environ, SMVP_DROPIN_REF_COMPAT="1")
-        r = subprocess.run([EXE, "-t", "-n", "3", "-d", rd, util.sample_path(name)], capture_output=True, text=True,
-                           cwd=str(tmp_path), env=env)
-        assert r.returncode == 0
-        rt = util.parse_report(glob.glob(str(tmp_path / "smvp-toolbox_report_TJDS_*.txt"))[0])
-        gold = util.parse_report(os.path.join(util.GOLDEN, "reports", util.GOLDEN_REPORTS[(name, "TJDS")]))
-        assert _close(rt["y"], gold["y"], coo)
+    inc = '\n#include "smvp_cuda.h" /* smvp_coo has the layout of MMRawData (main-cli.c:42-47) */'
+    assert '#include "mmio/mmio.h"' + inc + "\n" in text
+    want = (HEAD + CSR_SIG + mod.new_body("smvp_csr_compute").rstrip("\n") + MID + TJDS_SIG +
+            mod.new_body("smvp_tjds_compute").rstrip("\n") + TAIL)
+    # everything outside the two bodies is the input's text, plus that one include
+    assert text.replace(inc, "", 1) == want
+    (tmp_path / "mmio").mkdir()
+    (tmp_path / "mmio" / "mmio.h").write_text("")
+    r = subprocess.run(["gcc", "-std=gnu11", "-fsyntax-only", "-I" + os.path.join(REPO, "include"), "-I" + str(tmp_path), out],
+                       capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr
+    assert "smvp_csr_mult(" in text and "smvp_tjds_mult(" in text and "return NULL" not in text
