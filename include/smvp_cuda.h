@@ -167,6 +167,11 @@ typedef struct smvp_csr_info_t
                                  the others (y += ...): a row sum is then taken in two parts -- within 1e-12, not
                                  bit-identical to the one-pass order; -1 = one pass (the default: the split is an
                                  opt-in experiment, SMVP_CSR_SPLIT=1, that loses on R-MAT); 0 = not decided yet   */
+    int32_t row_patterns;     /* multiply plan: P > 0 = every row's column offsets (col - row) are one of P lists of at most
+                                 32 entries (stencils, banded matrices); the merge variant then streams a one-byte pattern id
+                                 per row instead of col_ind and sums each row in the reference's order (y bit-identical to
+                                 main-cli.c:410-416); -1 = not used (more than 256 lists, a longer row, a relabelled handle,
+                                 or SMVP_CSR_PATTERN=0); 0 = not decided yet (decided at the first pass)              */
 } smvp_csr_info_t;
 
 typedef struct smvp_tjds_info_t

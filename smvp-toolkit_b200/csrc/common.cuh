@@ -136,6 +136,10 @@ static inline int bits_for(uint32_t n) // bits needed to represent values in [0,
 
 constexpr int32_t EXP_NONE = (int32_t)0x80808080; // memset(0x80) pattern: "no exponent seen", below any real one
 
+// row-pattern plan (pattern.cu): at most PAT_MAX distinct column-offset lists (ids are one byte), none longer than PAT_LMAX
+constexpr int PAT_MAX = 256;
+constexpr int PAT_LMAX = 32;
+
 } // namespace smvp
 
 // ---------------------------------------------------------------- handles
@@ -177,6 +181,13 @@ struct smvp_csr
     int32_t split_state;
     int32_t ranked_cols; // 1: col_ind already holds popularity ranks (a hot / cold part): the ranked gather hints apply
     smvp_csr *hot, *cold;
+    // row-pattern plan (pattern.cu): 0 undecided, 1 in use, -1 not used.  Row r's k-th nonzero sits in column
+    // r + pat_off[pat_id[r] * PAT_LMAX + k]; the multiply reads pat_id instead of col_ind.
+    int32_t pattern_state;
+    int32_t pattern_count, pattern_maxlen; // distinct patterns, longest pattern
+    uint8_t *pat_id;                       // [rows]
+    int32_t *pat_off;                      // [pattern_count * PAT_LMAX]
+    int32_t *pat_len;                      // [pattern_count]
 };
 namespace smvp
 {
@@ -185,6 +196,8 @@ int csr_relabel_plan(smvp_csr *A, cudaStream_t s);                 // relabel.cu
 int csr_relabel_x(smvp_csr *A, const double *d_x, cudaStream_t s); // relabel.cu
 void csr_relabel_release(smvp_csr *A);                             // relabel.cu
 int csr_split_plan(smvp_csr *A, cudaStream_t s);                   // relabel.cu: after csr_relabel_plan
+int csr_pattern_plan(smvp_csr *A, cudaStream_t s);                // pattern.cu: decides the relabelling first
+void csr_pattern_release(smvp_csr *A);                             // pattern.cu
 void csr_release(smvp_csr *A);                                     // csr_build.cu
 int csr_build_impl(const int32_t *d_row, const int32_t *d_col, const double *d_val, int32_t rows, int32_t cols, int64_t nnz,
                    smvp_csr *A, cudaStream_t s);                   // csr_build.cu

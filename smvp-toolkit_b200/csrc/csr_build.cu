@@ -41,6 +41,7 @@ void csr_release(smvp_csr *A)
     cudaFree(A->d_y);
     csr_pipe_release(A);
     csr_relabel_release(A);
+    csr_pattern_release(A);
     delete A;
 }
 

@@ -922,6 +922,244 @@ static int wmerge_tile_items(int cfg)
     }
 }
 
+// =====================================================================================  PATTERN
+// Handles with the row-pattern plan (pattern.cu): the kernel streams val and one pattern id per row, never col_ind.
+// Row per lane: a warp tile is 32*R consecutive rows, lane l owns rows r0 + l, r0 + 32 + l, ...  The warp stages the
+// tile's val slice and pat_id slice into its own shared-memory ring with TMA bulk copies (evict-first) and never meets a
+// block-wide barrier after the pattern table is loaded.  Row starts inside the tile come from a warp scan of the pattern
+// lengths (one row_ptr entry per tile, not per row).  Step k of a round gathers x[r + off_k]: on the 91 % of rounds whose
+// 32 rows share a pattern that is 32 consecutive doubles, and the offset load is a shared-memory broadcast.  Each row is
+// summed left to right from +0.0, product rounded then added -- the reference loop's order (main-cli.c:410-416), so y
+// is bit-identical to it.  One launch per pass: no row is cut, nothing to stitch.
+template <int R>
+struct PatternShape
+{
+    static constexpr int ROWS = 32 * R;
+    // val slice (16-byte aligned start: up to one extra double at each end) + pat_id slice (16-byte aligned)
+    static int stage_bytes(int maxlen) { return (((ROWS * maxlen + 2) * 8 + 15) / 16 * 16 + ROWS + 32 + 127) & ~127; }
+};
+
+template <int WARPS, int R, int STAGES, int CH, int MINB, bool FANOUT>
+__global__ void __launch_bounds__(WARPS * 32, MINB)
+    csr_pattern_kernel(const int32_t *__restrict__ row_ptr, const double *__restrict__ val, const uint8_t *__restrict__ pat_id,
+                       const int32_t *__restrict__ pat_off, const int32_t *__restrict__ pat_len, int32_t npat, int32_t maxlen,
+                       const double *__restrict__ x, double *__restrict__ y, int32_t row_begin, int32_t row_end,
+                       uint32_t stage_bytes, const __grid_constant__ YFan fan)
+{
+    constexpr int ROWS = PatternShape<R>::ROWS;
+    extern __shared__ __align__(128) unsigned char smem[];
+    __shared__ __align__(8) uint64_t full_bar[WARPS * STAGES];
+    __shared__ int32_t stage_n0[WARPS * STAGES]; // first nonzero of the tile in each stage
+    // pattern table: offsets with row stride maxlen, then the lengths; the stages follow, 128-byte aligned
+    const uint32_t table_bytes = ((uint32_t)npat * (uint32_t)(maxlen + 1) * 4u + 127u) & ~127u;
+    int32_t *s_off = reinterpret_cast<int32_t *>(smem), *s_len = s_off + npat * maxlen;
+    for (int i = threadIdx.x; i < npat * maxlen; i += WARPS * 32)
+        s_off[i] = pat_off[(i / maxlen) * PAT_LMAX + i % maxlen];
+    for (int i = threadIdx.x; i < npat; i += WARPS * 32)
+        s_len[i] = pat_len[i];
+
+    const int lane = threadIdx.x & 31, w = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
+    uint64_t *bars = &full_bar[w * STAGES];
+    const uint32_t base = smem_u32(smem) + table_bytes + (uint32_t)(w * STAGES) * stage_bytes;
+    const uint32_t val_bytes = (stage_bytes - ROWS - 32) & ~15u; // where the pat_id slice starts inside a stage
+    uint64_t policy = 0;
+    if (lane == 0)
+    {
+        for (int s = 0; s < STAGES; s++)
+            mbar_init(&bars[s], 1);
+        fence_mbar_init();
+        policy = l2_evict_first_policy();
+    }
+    __syncthreads(); // the table is complete; from here on the warps are on their own
+
+    const int32_t ntiles = (int32_t)(((int64_t)row_end - row_begin + ROWS - 1) / ROWS);
+    const int32_t warp_stride = (int32_t)gridDim.x * WARPS;
+    // rows [r0, r1) of tile t; lane 0 stages it (n0 = row_ptr[r0], n1 = row_ptr[r1] loaded by the caller)
+    auto issue = [&](int32_t t, int s, int32_t n0, int32_t n1) {
+        const int32_t r0 = row_begin + t * ROWS, r1 = min(r0 + ROWS, row_end);
+        const int32_t va = n0 & ~1, pa = r0 & ~15;
+        const uint32_t vb = n1 > n0 ? (uint32_t)(((n1 + 1) & ~1) - va) * 8u : 0u;
+        const uint32_t pb = (uint32_t)(((r1 + 15) & ~15) - pa);
+        unsigned char *dst = smem + (base - smem_u32(smem)) + (uint32_t)s * stage_bytes;
+        stage_n0[w * STAGES + s] = n0;
+        mbar_expect_tx(&bars[s], vb + pb);
+        if (vb)
+            bulk_g2s(dst, val + va, vb, &bars[s], policy);
+        bulk_g2s(dst + val_bytes, pat_id + pa, pb, &bars[s], policy);
+    };
+    auto bounds = [&](int32_t t, int32_t *n0, int32_t *n1) {
+        const int32_t r0 = row_begin + t * ROWS;
+        *n0 = __ldg(row_ptr + r0);
+        *n1 = __ldg(row_ptr + min(r0 + ROWS, row_end));
+    };
+
+    int32_t t = (int32_t)blockIdx.x * WARPS + w;
+#pragma unroll
+    for (int s = 0; s < STAGES; s++)
+    {
+        const int32_t ts = t + s * warp_stride;
+        if (ts < ntiles)
+        {
+            int32_t n0, n1;
+            bounds(ts, &n0, &n1);
+            if (lane == 0)
+                issue(ts, s, n0, n1);
+        }
+    }
+    __syncwarp();
+    uint32_t phase = 0;
+    int s = 0;
+    while (t < ntiles)
+    {
+        // bounds of the tile this stage takes next: loaded now, used after the walk
+        const int32_t tn = t + STAGES * warp_stride;
+        int32_t nn0 = 0, nn1 = 0;
+        if (tn < ntiles && tn > t)
+            bounds(tn, &nn0, &nn1);
+
+        mbar_wait(&bars[s], (phase >> s) & 1u);
+        phase ^= 1u << s;
+        const int32_t r0 = row_begin + t * ROWS, r1 = min(r0 + ROWS, row_end);
+        const int32_t n0 = stage_n0[w * STAGES + s];
+        const uint32_t sb = base + (uint32_t)s * stage_bytes;
+        const uint32_t sval = sb + 8u * (uint32_t)(n0 - (n0 & ~1)); // nonzero n0
+        const uint32_t spid = sb + val_bytes + (uint32_t)(r0 - (r0 & ~15)); // row r0
+        int32_t done = 0; // nonzeros of the tile before the current round
+#pragma unroll 1
+        for (int i = 0; i < R; i++)
+        {
+            const int32_t rr = 32 * i;
+            if (r0 + rr >= r1)
+                break;
+            const int32_t r = r0 + rr + lane;
+            const bool live = r < r1;
+            int32_t p = 0, len = 0;
+            if (live)
+            {
+                asm volatile("ld.shared.u8 %0, [%1];" : "=r"(p) : "r"(spid + (uint32_t)(rr + lane)));
+                len = s_len[p];
+            }
+            int32_t incl = len; // inclusive scan of the row lengths of the round
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1)
+            {
+                const int32_t v = __shfl_up_sync(0xffffffffu, incl, o);
+                if (lane >= o)
+                    incl += v;
+            }
+            const uint32_t vrow = sval + 8u * (uint32_t)(done + incl - len);
+            const uint32_t orow = smem_u32(s_off) + 4u * (uint32_t)(p * maxlen);
+            done += __shfl_sync(0xffffffffu, incl, 31);
+            const int32_t kmax = __reduce_max_sync(0xffffffffu, len);
+            double sum = 0.0;
+#pragma unroll 1
+            for (int32_t k0 = 0; k0 < kmax; k0 += CH)
+            {
+                // three phases pinned by volatile asm: the offsets, every gather of the chunk (CH loads in flight), the sums
+                int32_t off[CH];
+                double xv[CH];
+#pragma unroll
+                for (int q = 0; q < CH; q++)
+                    off[q] = k0 + q < len ? lds_s32(orow + 4u * (uint32_t)(k0 + q)) : 0;
+#pragma unroll
+                for (int q = 0; q < CH; q++)
+                {
+                    xv[q] = 0.0;
+                    if (k0 + q < len)
+                        xv[q] = ldg_x_pinned(x, r + off[q]);
+                }
+#pragma unroll
+                for (int q = 0; q < CH; q++)
+                    if (k0 + q < len)
+                        sum = __dadd_rn(sum, __dmul_rn(lds_f64(vrow + 8u * (uint32_t)(k0 + q)), xv[q]));
+            }
+            if (live)
+                store_y<FANOUT>(y, fan, r, sum);
+        }
+        // the stage is consumed: refill it with tile tn
+        __syncwarp();
+        if (tn < ntiles && tn > t && lane == 0)
+            issue(tn, s, nn0, nn1);
+        __syncwarp();
+        if (t + warp_stride <= t)
+            break; // 32-bit overflow guard
+        t += warp_stride;
+        s = s + 1 == STAGES ? 0 : s + 1;
+    }
+}
+
+// ---- the instantiations of the pattern kernel: {warps per CTA, rounds of 32 rows per tile, stages per warp, gathers in
+// flight per lane, min CTAs/SM}.  Measured on B200 (tools/sweep_pattern.py, profiles/r03_logs/sweep_pattern.log, stencil
+// 369^3): one stage per warp and 28 warps per SM (0: 1.75 ms, 1: 1.72-1.81 ms) against 2.1-3.2 ms for every
+// configuration with two stages or two rounds per tile -- a 7 KB stage per warp, so resident warps, not staging depth,
+// keep enough gathers in flight.  SMVP_PATTERN_CFG=k picks another one.
+#define SMVP_PATTERN_CFGS(X) \
+    X(0, 4, 1, 1, 14, 7)     \
+    X(1, 4, 1, 1, 9, 8)      \
+    X(2, 4, 1, 2, 9, 4)      \
+    X(3, 4, 1, 2, 14, 4)     \
+    X(4, 4, 2, 1, 9, 4)      \
+    X(5, 8, 1, 2, 9, 2)      \
+    X(6, 4, 2, 2, 9, 2)      \
+    X(7, 2, 1, 2, 9, 7)
+
+static int pick_pattern_cfg() { return env_int_early("SMVP_PATTERN_CFG", 0, 0, 7); }
+
+template <int WARPS, int R, int STAGES, int CH, int MINB, bool FANOUT>
+static int launch_pattern(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fanp, cudaStream_t s, int32_t row_begin,
+                          int32_t row_end)
+{
+    auto kern = csr_pattern_kernel<WARPS, R, STAGES, CH, MINB, FANOUT>;
+    const int maxlen = A->pattern_maxlen > 0 ? A->pattern_maxlen : 1;
+    const int stage = PatternShape<R>::stage_bytes(maxlen);
+    const int table = (A->pattern_count * (maxlen + 1) * 4 + 127) & ~127;
+    const int smem = table + WARPS * STAGES * stage;
+    // the shared memory depends on the matrix (longest pattern, pattern count): occupancy is looked up per size
+    static thread_local int configured_dev = -1, configured_smem = -1, resident = 1;
+    int dev = 0;
+    SMVP_CUDA(cudaGetDevice(&dev));
+    if (configured_dev != dev || configured_smem != smem)
+    {
+        SMVP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        SMVP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kern, WARPS * 32, smem));
+        if (resident < 1)
+            resident = 1;
+        configured_dev = dev;
+        configured_smem = smem;
+    }
+    // persistent grid with a static stride over the tiles: the co-runner headroom works as for the merge kernel
+    static thread_local int env_headroom = -2;
+    if (env_headroom == -2)
+        env_headroom = env_int_early("SMVP_MERGE_HEADROOM", -1, -1, 8);
+    const int headroom = env_headroom >= 0 ? env_headroom : A->merge_headroom;
+    const int res_used = resident - headroom >= 1 ? resident - headroom : 1;
+    int64_t grid = (int64_t)device_props().sms * res_used;
+    const int64_t need = ceil_div64(ceil_div64((int64_t)row_end - row_begin, PatternShape<R>::ROWS), WARPS);
+    if (grid > need)
+        grid = need;
+    if (grid > 0)
+        SMVP_LAUNCH(kern, (unsigned)grid, WARPS * 32, smem, s, A->row_ptr, A->val, A->pat_id, A->pat_off, A->pat_len,
+                    A->pattern_count, maxlen, d_x, d_y, row_begin, row_end, (uint32_t)stage, fanp ? *fanp : YFan());
+    return SMVP_OK;
+}
+
+// rows [row_begin, row_end) of a handle with the row-pattern plan
+static int csr_mult_pattern(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, cudaStream_t s, int32_t row_begin,
+                            int32_t row_end)
+{
+    switch (pick_pattern_cfg())
+    {
+#define X(id, wp, r, st, ch, mb)                                                                        \
+    case id:                                                                                            \
+        return fan ? launch_pattern<wp, r, st, ch, mb, true>(A, d_x, d_y, fan, s, row_begin, row_end) \
+                   : launch_pattern<wp, r, st, ch, mb, false>(A, d_x, d_y, nullptr, s, row_begin, row_end);
+        SMVP_PATTERN_CFGS(X)
+#undef X
+    default:
+        return SMVP_E_ARG;
+    }
+}
+
 // tiles [tile_begin, tile_end) of the plan; (0, -1) = all
 static int csr_mult_merge(smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, cudaStream_t s, int32_t tile_begin = 0,
                           int32_t tile_end = -1, int32_t accum = 0)
@@ -934,6 +1172,9 @@ static int csr_mult_merge(smvp_csr *A, const double *d_x, double *d_y, const YFa
     }
     if (accum && fan)
         return SMVP_E_ARG;
+    // the row-pattern plan serves whole passes (the pipelined host call cuts its ranges on rows: csr_mult_pattern)
+    if (A->pattern_state == 1 && tile_begin == 0 && tile_end < 0 && !accum)
+        return csr_mult_pattern(A, d_x, d_y, fan, s, 0, A->rows);
     const int cfg = pick_merge_cfg(A);
     SMVP_TRY(merge_plan(A, cfg, s));
     if (tile_end < 0)
@@ -1032,7 +1273,7 @@ static int csr_mult_any(smvp_csr *A, const double *d_x, double *d_y, const YFan 
     if (A->rows == 0)
         return SMVP_OK;
     cudaStream_t s = (cudaStream_t)stream;
-    SMVP_TRY(csr_relabel_plan(A, s));
+    SMVP_TRY(csr_pattern_plan(A, s)); // decides the relabelling first
     const double *x = d_x; // NULL: the x last given to smvp_csr_set_x_device
     if (A->relabel_state == 1)
     {
@@ -1061,7 +1302,7 @@ extern "C" int smvp_csr_set_x_device(smvp_csr *A, const double *d_x, void *strea
 {
     if (!A || (A->cols > 0 && !d_x))
         return SMVP_E_ARG;
-    SMVP_TRY(csr_relabel_plan(A, (cudaStream_t)stream));
+    SMVP_TRY(csr_pattern_plan(A, (cudaStream_t)stream)); // decides the relabelling first
     if (A->relabel_state == 1)
         SMVP_TRY(csr_relabel_x(A, d_x, (cudaStream_t)stream));
     A->x_set = d_x;
@@ -1205,18 +1446,24 @@ __global__ void __launch_bounds__(256) col_range_kernel(const int32_t *__restric
     }
 }
 
+// Ranges of a handle with the row-pattern plan are cut on rows (the pattern kernel takes a row range, pipe_tile = pipe_row);
+// pipe_cfg is then PIPE_CFG_PATTERN instead of a merge tile size.
+constexpr int32_t PIPE_CFG_PATTERN = -2;
 static int pipe_plan(smvp_csr *A)
 {
-    SMVP_TRY(merge_plan(A, pick_merge_cfg(A), 0));
+    const bool pat = A->pattern_state == 1;
+    if (!pat)
+        SMVP_TRY(merge_plan(A, pick_merge_cfg(A), 0));
     double rf[PIPE_MAX_RANGES + 1];
     const int NR = pipe_profile(8 * (int64_t)A->rows, pipe_ranges(8 * (int64_t)A->rows), PIPE_MAX_RANGES, rf);
     const char *pe = getenv("SMVP_PIPE_PROFILE");
     const int ramp = pe && pe[0] == 'r' ? 1 : 0;
-    if (A->pipe_cfg == A->merge_cfg && A->pipe_ranges == NR && A->pipe_ramp == ramp)
+    const int32_t key = pat ? PIPE_CFG_PATTERN : A->merge_cfg;
+    if (A->pipe_cfg == key && A->pipe_ranges == NR && A->pipe_ramp == ramp)
         return SMVP_OK;
     A->pipe_ramp = ramp;
-    const int32_t T = A->merge_tiles;
-    const int64_t tile_items = A->merge_cfg;
+    const int32_t T = pat ? 0 : A->merge_tiles;
+    const int64_t tile_items = pat ? 0 : A->merge_cfg;
     int32_t *d_max = nullptr; // per range: {largest, smallest} column index
     int32_t h_max[2 * PIPE_MAX_RANGES];
     for (int c = 0; c < PIPE_MAX_RANGES; c++)
@@ -1226,8 +1473,15 @@ static int pipe_plan(smvp_csr *A)
     }
     SMVP_CUDA(dev_alloc(&d_max, 2 * PIPE_MAX_RANGES));
     cudaError_t e = cudaMemcpy(d_max, h_max, sizeof(h_max), cudaMemcpyHostToDevice);
+    int32_t pat_nz[PIPE_MAX_RANGES + 1]; // pattern plan: first nonzero of each range (row_ptr at its first row)
     for (int c = 0; c <= NR && e == cudaSuccess; c++)
     {
+        if (pat)
+        {
+            A->pipe_tile[c] = A->pipe_row[c] = c == NR ? A->rows : (int32_t)((double)A->rows * rf[c]);
+            e = cudaMemcpy(&pat_nz[c], A->row_ptr + A->pipe_row[c], sizeof(int32_t), cudaMemcpyDeviceToHost);
+            continue;
+        }
         A->pipe_tile[c] = c == NR ? T : (int32_t)((double)T * rf[c]);
         // rows consumed before each boundary tile (tile_row[T] = rows)
         e = cudaMemcpy(&A->pipe_row[c], A->tile_row + A->pipe_tile[c], sizeof(int32_t), cudaMemcpyDeviceToHost);
@@ -1235,8 +1489,8 @@ static int pipe_plan(smvp_csr *A)
     for (int c = 0; c < NR && e == cudaSuccess; c++)
     {
         // nonzeros of the range: merge items before the boundary minus the row ends among them
-        int64_t n0 = (int64_t)A->pipe_tile[c] * tile_items - A->pipe_row[c];
-        int64_t n1 = (int64_t)A->pipe_tile[c + 1] * tile_items - A->pipe_row[c + 1];
+        int64_t n0 = pat ? pat_nz[c] : (int64_t)A->pipe_tile[c] * tile_items - A->pipe_row[c];
+        int64_t n1 = pat ? pat_nz[c + 1] : (int64_t)A->pipe_tile[c + 1] * tile_items - A->pipe_row[c + 1];
         n0 = n0 < A->nnz ? n0 : A->nnz;
         n1 = (c + 1 == NR || n1 > A->nnz) ? A->nnz : n1;
         if (n1 > n0)
@@ -1262,7 +1516,7 @@ static int pipe_plan(smvp_csr *A)
     // nothing below the smallest column index is ever read: the upload starts there (a row block of a banded matrix,
     // the shard of one GPU, reads a window of x, not a prefix).  Rounded down to 512 bytes.
     A->pipe_xlo = need > 0 ? (lowest / 64) * 64 : 0;
-    A->pipe_cfg = A->merge_cfg;
+    A->pipe_cfg = key;
     A->pipe_ranges = NR;
     return SMVP_OK;
 }
@@ -1416,7 +1670,8 @@ static int csr_mult_pipelined(smvp_csr *A, const double *x_host, double *y_host,
         }
         PIPE_CK(cudaEventRecord(R.t0[c], cs));
         if (A->pipe_tile[c + 1] > A->pipe_tile[c] && e == cudaSuccess)
-            rc = csr_mult_merge(A, xm, A->d_y, nullptr, cs, A->pipe_tile[c], A->pipe_tile[c + 1]);
+            rc = A->pattern_state == 1 ? csr_mult_pattern(A, xm, A->d_y, nullptr, cs, A->pipe_row[c], A->pipe_row[c + 1])
+                                       : csr_mult_merge(A, xm, A->d_y, nullptr, cs, A->pipe_tile[c], A->pipe_tile[c + 1]);
         PIPE_CK(cudaEventRecord(R.t1[c], cs));
         if (y_host)
         {
@@ -1502,10 +1757,10 @@ extern "C" int smvp_csr_mult(smvp_csr *A, const double *x_host, double *y_host, 
     int rc = SMVP_OK;
     // plans outside the timed bracket (the reference builds its format before the loop too)
     if (A->rows > 0)
-        rc = csr_relabel_plan(A, 0);
+        rc = csr_pattern_plan(A, 0); // decides the relabelling first
     if (rc == SMVP_OK && pipelined)
         rc = pipe_plan(A);
-    else if (rc == SMVP_OK && merge)
+    else if (rc == SMVP_OK && merge && A->pattern_state != 1)
         rc = merge_plan(A, pick_merge_cfg(A), 0);
     if (rc != SMVP_OK)
         return rc;
@@ -1618,7 +1873,8 @@ extern "C" int smvp_csr_info(const smvp_csr *A, smvp_csr_info_t *out)
     out->launches_per_mult[SMVP_CSR_AUTO] = out->launches_per_mult[out->auto_variant];
     out->x_relabel = A->relabel_state;
     out->x_split = A->split_state;
-    out->launches_per_mult[SMVP_CSR_MERGE] = A->split_state == 1 ? 4 : 2;
+    out->launches_per_mult[SMVP_CSR_MERGE] = A->pattern_state == 1 ? 1 : A->split_state == 1 ? 4 : 2;
     out->launches_per_mult[SMVP_CSR_AUTO] = out->launches_per_mult[out->auto_variant];
+    out->row_patterns = A->pattern_state == 1 ? A->pattern_count : A->pattern_state;
     return SMVP_OK;
 }

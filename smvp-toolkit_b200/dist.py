@@ -343,7 +343,6 @@ class RowBlockCsr:
         self.local_rows_out = self.r1 - self.r0
         resolved = self.A.auto_variant if variant == eng.CSR_AUTO else variant
         self.variant_name = {eng.CSR_VECTOR: "vector", eng.CSR_MERGE: "merge"}[resolved]
-        self.kernel_name = {"vector": "csr_vector_kernel", "merge": "csr_merge_warp_kernel"}[self.variant_name]
         self.x = None
         self._source_desc = source.desc
 
@@ -700,11 +699,22 @@ class RowBlockCsr:
             hy.copy_(self.y_local, non_blocking=True)
             stream.synchronize()
 
+    @property
+    def kernel_name(self):
+        """The kernel a pass runs; the merge variant of a handle with the row-pattern plan runs the pattern kernel
+        (the plan is decided at the first pass, so read this after it)."""
+        if self.variant_name == "vector":
+            return "csr_vector_kernel"
+        return "csr_pattern_kernel" if self.A.row_patterns > 0 else "csr_merge_warp_kernel"
+
     def measured_traffic_bytes(self):
         return _measured_traffic(self.kernel_name)
 
     def plan_desc(self):
         """What the multiply does beyond the plain kernel (decided by the library from the matrix, reported as is)."""
+        if self.variant_name == "merge" and self.A.row_patterns > 0:
+            return ("rows share %d column-offset patterns (smvp_csr_info_t.row_patterns): the kernel streams pattern ids "
+                    "instead of col_ind" % self.A.row_patterns)
         if self.A.x_relabel == 1:
             return ("column space relabelled by popularity (smvp_csr_info_t.x_relabel = 1): the kernels read rank-ordered "
                     "column indices and a permuted copy of x formed ONCE per x by smvp_csr_set_x_device, outside the "

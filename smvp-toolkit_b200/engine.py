@@ -44,7 +44,8 @@ class _CsrInfo(ctypes.Structure):
     _fields_ = [("rows", ctypes.c_int32), ("cols", ctypes.c_int32), ("nnz", ctypes.c_int64),
                 ("max_row_nnz", ctypes.c_int32), ("auto_variant", ctypes.c_int32), ("input_order", ctypes.c_int32),
                 ("bytes_per_mult", ctypes.c_int64), ("device_bytes", ctypes.c_int64),
-                ("launches_per_mult", ctypes.c_int32 * 3), ("x_relabel", ctypes.c_int32), ("x_split", ctypes.c_int32)]
+                ("launches_per_mult", ctypes.c_int32 * 3), ("x_relabel", ctypes.c_int32), ("x_split", ctypes.c_int32),
+                ("row_patterns", ctypes.c_int32)]
 
 
 class _TjdsInfo(ctypes.Structure):
@@ -269,6 +270,13 @@ class CsrMatrix:
         info = _CsrInfo()
         _check(lib().smvp_csr_info(self._h, ctypes.byref(info)), "smvp_csr_info")
         return info.x_split
+
+    @property
+    def row_patterns(self):
+        """P > 0: the merge variant streams one of P row patterns per row instead of col_ind, -1: not used, 0: not decided yet."""
+        info = _CsrInfo()
+        _check(lib().smvp_csr_info(self._h, ctypes.byref(info)), "smvp_csr_info")
+        return info.row_patterns
 
     def mult_device_fanout(self, d_x, y_ptrs, variant=CSR_AUTO, stream=None):
         """y = A x stored into every destination of y_ptrs (device addresses, possibly peer-mapped)."""
