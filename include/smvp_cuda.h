@@ -148,6 +148,31 @@ int smvp_tjds_set_x_device(smvp_tjds *A, const double *d_x, void *stream);
 /* one pass y = A x with the x last given to smvp_tjds_set_x_device; zero-fills y first */
 int smvp_tjds_mult_device(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit, void *stream);
 
+/* ---- transposed product y = A^T x (BiCG, QMR, LSQR and CGNE need it once per iteration; pull-direction graph walks
+ * multiply by A^T).  Two routes, one per format:
+ *   CSR   a second handle holds A^T; every CSR plan (row patterns, relabelling, pipelined host call, fan-out) serves it
+ *         through the ordinary smvp_csr_mult* calls.
+ *   TJDS  the handle itself: TJDS stores A by column, so A^T x is a gather along each column -- no atomics, no second
+ *         copy of the matrix.                                                                                         */
+/* A^T as a new, independent CSR handle, built on the device from A's arrays (A is not modified; free the two in any
+ * order).  Row c of the result lists A's column c in ascending row order, i.e. its arrays are bit-identical to what
+ * smvp_csr_build makes from the COO with rows and columns swapped.  Synchronous, like the builders.  The new handle
+ * starts with every plan undecided and no co-runner headroom.  It holds as much HBM as A, and its build takes about as
+ * much temporary HBM as a build of A from a device COO.                                                            */
+int smvp_csr_transpose(const smvp_csr *A, smvp_csr **out);
+/* one pass y = A^T x: d_x has A->rows entries, d_y A->cols.  Every entry of d_y is written (+0.0 for an empty column).
+ * Deterministic, no atomics.  Column c's terms val * x[row] are taken in ascending row order: columns of at most 32
+ * entries are summed left to right from +0.0 (bit-identical to the sequential transposed loop); longer columns in
+ * chunks of 32 entries, each summed left to right from +0.0, the chunk sums then added left to right from +0.0 -- the
+ * order is a function of the matrix alone.  The first call on a handle may synchronise (plan + scratch: one double per
+ * chunk of a column longer than 32 entries, counted in smvp_tjds_info_t.device_bytes).  A pass is one launch when no
+ * column holds more than 32 entries, two otherwise.  Independent of smvp_tjds_set_x_device and of the row relabelling
+ * of A x; the handle's x and plans stay as they are.                                                              */
+int smvp_tjds_mult_transpose_device(smvp_tjds *A, const double *d_x, double *d_y, void *stream);
+/* the same with host vectors x_host[rows] -> y_host[cols], `iters` timed passes: the -n loop of smvp_tjds_mult (x copied
+ * to the device once and y back once per call; ms_each as there, exact or batched for small matrices)             */
+int smvp_tjds_mult_transpose(smvp_tjds *A, const double *x_host, double *y_host, int iters, double *ms_each);
+
 /* ---- introspection ---- */
 typedef struct smvp_csr_info_t
 {

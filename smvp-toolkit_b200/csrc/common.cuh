@@ -201,6 +201,8 @@ void csr_pattern_release(smvp_csr *A);                             // pattern.cu
 void csr_release(smvp_csr *A);                                     // csr_build.cu
 int csr_build_impl(const int32_t *d_row, const int32_t *d_col, const double *d_val, int32_t rows, int32_t cols, int64_t nnz,
                    smvp_csr *A, cudaStream_t s);                   // csr_build.cu
+// row_of[j] = row of nonzero j, from row_ptr[rows+1] (asynchronous on s)
+int csr_expand_rows(const int32_t *row_ptr, int32_t rows, int64_t nnz, int32_t *row_of, cudaStream_t s); // csr_build.cu
 } // namespace smvp
 
 struct smvp_tjds
@@ -240,6 +242,14 @@ struct smvp_tjds
     int32_t *row_rel;        // [nnz]  rank of row_ind[j]; what the kernels scatter through when in use
     int32_t *row_rank;       // [rows] rank of row r
     double *y_rel;           // [rows] y in rank order (atomic variant)
+    // transposed product y = A^T x (tjds_mult.cu), scratch built at its first call.  Columns longer than TJDS_SEG
+    // (slots [0, tr_nlong)) are summed per segment into tr_part, then combined; tr_nwide of them are longer than
+    // TJDS_SEG^2 entries and are combined by a whole warp.
+    int32_t tr_ready;        // 1 once the scratch below exists
+    int32_t tr_nlong, tr_nwide;
+    uint32_t *tr_seg_off;    // [nseg] first partial of segment g; slot q of segment g writes tr_part[tr_seg_off[g] + q]
+    double *tr_part;         // one partial per (segment, slot) pair of the long columns
+    double *d_xt, *d_yt;     // [rows] / [cols]: scratch of the host-vector entry point
 };
 namespace smvp
 {

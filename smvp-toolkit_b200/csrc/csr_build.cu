@@ -25,6 +25,42 @@ __global__ void __launch_bounds__(256) gather_csr_kernel(const uint32_t *__restr
 
 __global__ void set_last_kernel(int32_t *row_ptr, int32_t rows, int32_t nnz) { row_ptr[rows] = nnz; }
 
+__global__ void __launch_bounds__(256) expand_rows_kernel(const int32_t *__restrict__ row_ptr, int32_t rows, int64_t nnz,
+                                                          int32_t *__restrict__ row_of)
+{
+    // 8 consecutive nonzeros per thread: one binary search for the first, then a walk along row_ptr
+    for (int64_t j0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 8; j0 < nnz; j0 += (int64_t)gridDim.x * blockDim.x * 8)
+    {
+        int32_t lo = 0, hi = rows; // last row with row_ptr[row] <= j0
+        while (hi - lo > 1)
+        {
+            const int32_t mid = lo + ((hi - lo) >> 1);
+            if ((int64_t)__ldg(row_ptr + mid) <= j0)
+                lo = mid;
+            else
+                hi = mid;
+        }
+        int32_t r = lo;
+        const int64_t j1 = j0 + 8 < nnz ? j0 + 8 : nnz;
+        for (int64_t j = j0; j < j1; j++)
+        {
+            while ((int64_t)__ldg(row_ptr + r + 1) <= j)
+                r++;
+            row_of[j] = r;
+        }
+    }
+}
+
+int csr_expand_rows(const int32_t *row_ptr, int32_t rows, int64_t nnz, int32_t *row_of, cudaStream_t s)
+{
+    if (nnz == 0)
+        return SMVP_OK;
+    const int64_t blocks = ceil_div64(nnz, 256 * 8), cap = (int64_t)device_props().sms * 16;
+    SMVP_LAUNCH(expand_rows_kernel, (unsigned)(blocks < cap ? blocks : cap), 256, 0, s, row_ptr, rows, nnz, row_of);
+    SMVP_CUDA(cudaGetLastError());
+    return SMVP_OK;
+}
+
 void csr_release(smvp_csr *A)
 {
     if (!A)
@@ -172,6 +208,39 @@ extern "C" int smvp_csr_build(const smvp_coo *coo, int32_t rows, int32_t cols, i
     cudaFree(d_col);
     cudaFree(d_val);
     return rc;
+}
+
+// A^T from A's arrays: the entries of A, read in its (row, col) order, are the entries of A^T in (col, row) order, so
+// coo_inspect reports ORDER_COL_ROW and the build's stable sort on the row key alone keeps each row of A^T in ascending
+// column order.  A's natural col_ind is read whatever plan A uses (relabelled and split handles keep it).
+extern "C" int smvp_csr_transpose(const smvp_csr *A, smvp_csr **out)
+{
+    if (!out)
+        return SMVP_E_ARG;
+    *out = nullptr;
+    if (!A)
+        return SMVP_E_ARG;
+    smvp_csr *T = new (std::nothrow) smvp_csr();
+    if (!T)
+        return SMVP_E_ALLOC;
+    T->rows = A->cols;
+    T->cols = A->rows;
+    T->nnz = A->nnz;
+    T->merge_cfg = -1;
+    auto body = [&]() -> int {
+        DevTmp row_of;
+        SMVP_CUDA(row_of.alloc<int32_t>(A->nnz));
+        SMVP_TRY(csr_expand_rows(A->row_ptr, A->rows, A->nnz, row_of.as<int32_t>(), 0));
+        return csr_build_impl(A->col_ind, row_of.as<int32_t>(), A->val, T->rows, T->cols, T->nnz, T, 0);
+    };
+    const int rc = body();
+    if (rc != SMVP_OK)
+    {
+        csr_release(T);
+        return rc;
+    }
+    *out = T;
+    return SMVP_OK;
 }
 
 extern "C" void smvp_csr_free(smvp_csr *A) { smvp::csr_release(A); }

@@ -309,32 +309,6 @@ void tjds_relabel_release(smvp_tjds *A)
 // 6.9 ms against 5.33 ms for the one-pass relabelled kernel, which overlaps the cold misses with the hot hits.  So the
 // split stays an opt-in experiment (SMVP_CSR_SPLIT=1), and the R-MAT multiply is gather-rate-bound: the next lever is
 // fewer sector accesses per gather (the hottest few thousand x entries held in shared memory), not less DRAM traffic.
-__global__ void __launch_bounds__(256) expand_rows_kernel(const int32_t *__restrict__ row_ptr, int32_t rows, int64_t nnz,
-                                                          int32_t *__restrict__ row_of)
-{
-    // 8 consecutive nonzeros per thread: one binary search for the first, then a walk along row_ptr
-    for (int64_t j0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 8; j0 < nnz; j0 += (int64_t)gridDim.x * blockDim.x * 8)
-    {
-        int32_t lo = 0, hi = rows; // last row with row_ptr[row] <= j0
-        while (hi - lo > 1)
-        {
-            const int32_t mid = lo + ((hi - lo) >> 1);
-            if ((int64_t)__ldg(row_ptr + mid) <= j0)
-                lo = mid;
-            else
-                hi = mid;
-        }
-        int32_t r = lo;
-        const int64_t j1 = j0 + 8 < nnz ? j0 + 8 : nnz;
-        for (int64_t j = j0; j < j1; j++)
-        {
-            while ((int64_t)__ldg(row_ptr + r + 1) <= j)
-                r++;
-            row_of[j] = r;
-        }
-    }
-}
-
 __global__ void __launch_bounds__(256) split_flag_kernel(const int32_t *__restrict__ col_rel, int64_t nnz, int32_t hot,
                                                          uint32_t *__restrict__ flag)
 {
@@ -397,7 +371,7 @@ int csr_split_plan(smvp_csr *A, cudaStream_t s)
         SMVP_CUDA(row_of.alloc<int32_t>(nnz));
         SMVP_CUDA(pos.alloc<uint32_t>(nnz));
         SMVP_CUDA(total.alloc<uint32_t>(1));
-        SMVP_LAUNCH(expand_rows_kernel, grid, 256, 0, s, (const int32_t *)A->row_ptr, A->rows, nnz, row_of.as<int32_t>());
+        SMVP_TRY(csr_expand_rows(A->row_ptr, A->rows, nnz, row_of.as<int32_t>(), s));
         SMVP_LAUNCH(split_flag_kernel, grid, 256, 0, s, (const int32_t *)A->col_rel, nnz, hot, pos.as<uint32_t>());
         SMVP_TRY(exclusive_scan_u32(pos.as<uint32_t>(), pos.as<uint32_t>(), nnz, total.as<uint32_t>(), s));
         uint32_t nh = 0;

@@ -102,6 +102,10 @@ void tjds_release(smvp_tjds *A)
         cudaEventDestroy(A->x_exp_event);
     cudaFree(A->d_x);
     cudaFree(A->d_y);
+    cudaFree(A->tr_seg_off);
+    cudaFree(A->tr_part);
+    cudaFree(A->d_xt);
+    cudaFree(A->d_yt);
     tjds_relabel_release(A);
     delete A;
 }

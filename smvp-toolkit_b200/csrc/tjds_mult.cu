@@ -555,6 +555,129 @@ __global__ void __launch_bounds__(256) tjds_unrank_y_kernel(const double *__rest
         y[r] = __ldg(y_rel + __ldg(row_rank + r));
 }
 
+// ---- transposed product y = A^T x --------------------------------------------------------------------------------
+// Slot q of every diagonal belongs to column perm[q], and the d-th entry of a column is its d-th by row, so
+//     (A^T x)[perm[q]] = sum_d val[start_pos[d] + q] * x[row_ind[start_pos[d] + q]]
+// is a GATHER along the slot: the streams of tjds_atomic_kernel, no atomics, the terms in ascending row order.  The
+// handle's segment table (tjds_plan) cuts a column into chunks of TJDS_SEG entries; thread (segment g, slot q) sums its
+// chunk left to right from +0.0.  A column of at most TJDS_SEG entries (every column of the 27-point stencil) is done
+// there, bit-identical to the sequential transposed loop, and a pass is one launch.  The chunk sums of a longer column
+// go to tr_part[tr_seg_off[g] + q] (one coalesced store per warp) and tjds_transpose_combine_kernel adds them in
+// segment order.  The table is walked straight whatever walk A x uses: a skewed table only has extra slots past the
+// end of each segment's first diagonal, and those threads find nothing to do.  row_ind is read, never row_rel.
+constexpr int TJDS_TR_UNROLL = 8; // entries whose loads are issued before the first of them is used
+__global__ void __launch_bounds__(256) tjds_transpose_kernel(const int2 *__restrict__ blocks, const int32_t *__restrict__ start_pos,
+                                                             const int32_t *__restrict__ row_ind, const double *__restrict__ val,
+                                                             const int32_t *__restrict__ perm, const double *__restrict__ x,
+                                                             double *__restrict__ y, double *__restrict__ part,
+                                                             const uint32_t *__restrict__ seg_off, int32_t ndiag, int32_t nslots,
+                                                             int32_t cols, int32_t nlong)
+{
+    static_assert(TJDS_SEG % TJDS_TR_UNROLL == 0, "s_sp holds TJDS_SEG + 1 entries");
+    __shared__ int32_t s_sp[TJDS_SEG + 1];
+    // empty columns (slots nslots .. cols-1) get +0.0, spread over the whole grid
+    for (int64_t p = (int64_t)nslots + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < cols; p += (int64_t)gridDim.x * blockDim.x)
+        y[__ldg(perm + p)] = 0.0;
+    const int2 blk = __ldg(blocks + blockIdx.x);
+    const int32_t d_begin = blk.x * TJDS_SEG;
+    const int32_t nd = min(TJDS_SEG, ndiag - d_begin);
+    // entries past the segment's last diagonal repeat its end: such a diagonal is empty
+    if ((int32_t)threadIdx.x <= TJDS_SEG)
+        s_sp[threadIdx.x] = __ldg(start_pos + d_begin + min((int32_t)threadIdx.x, nd));
+    __syncthreads();
+    const int32_t q = blk.y + (int32_t)threadIdx.x;
+    if (q >= s_sp[1] - s_sp[0])
+        return; // the column at this slot ends before the segment (or the slot is past the table's diagonals)
+    double s = 0.0;
+    for (int32_t i0 = 0; i0 < nd; i0 += TJDS_TR_UNROLL)
+    {
+        int32_t r[TJDS_TR_UNROLL];
+        double v[TJDS_TR_UNROLL], xv[TJDS_TR_UNROLL];
+#pragma unroll
+        for (int u = 0; u < TJDS_TR_UNROLL; u++)
+        {
+            const int32_t i = i0 + u, sp = s_sp[i];
+            const bool live = q < s_sp[i + 1] - sp;
+            r[u] = live ? ld_stream_i32(row_ind + sp + q) : -1;
+            v[u] = live ? ld_stream_f64(val + sp + q) : 0.0;
+        }
+#pragma unroll
+        for (int u = 0; u < TJDS_TR_UNROLL; u++)
+            xv[u] = r[u] >= 0 ? __ldg(x + r[u]) : 0.0;
+#pragma unroll
+        for (int u = 0; u < TJDS_TR_UNROLL; u++)
+            if (r[u] >= 0)
+                s = __dadd_rn(s, __dmul_rn(v[u], xv[u]));
+    }
+    if (q >= nlong)
+        y[__ldg(perm + q)] = s; // a column of at most TJDS_SEG entries lives in segment 0 alone
+    else
+        part[(int64_t)__ldg(seg_off + blk.x) + q] = s;
+}
+
+// y[perm[q]] = tr_part partials of long column q added left to right from +0.0, chunk 0 first.  Slots [0, nwide) hold
+// more than TJDS_SEG chunks (a power-law column can hold ~1e6 entries, ~3e4 chunks): a warp loads 32 chunk sums per
+// round, TJDS_TR_ROUNDS rounds ahead, and every lane adds them in order from shuffles (the additions are the serial
+// part, the loads are not).  Slots [nwide, nlong) take one thread each.
+constexpr int TJDS_TR_ROUNDS = 4;
+__global__ void __launch_bounds__(256) tjds_transpose_combine_kernel(const double *__restrict__ part, const uint32_t *__restrict__ seg_off,
+                                                                     const int32_t *__restrict__ slot_len, const int32_t *__restrict__ perm,
+                                                                     int32_t nlong, int32_t nwide, double *__restrict__ y)
+{
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, wide_threads = (int64_t)nwide * 32;
+    if (t < wide_threads)
+    {
+        // whole warps: wide_threads is a multiple of 32
+        const int32_t q = (int32_t)(t >> 5), lane = threadIdx.x & 31;
+        const int32_t nch = (__ldg(slot_len + q) + TJDS_SEG - 1) / TJDS_SEG;
+        double s = 0.0;
+        for (int32_t g0 = 0; g0 < nch; g0 += 32 * TJDS_TR_ROUNDS)
+        {
+            double v[TJDS_TR_ROUNDS];
+#pragma unroll
+            for (int k = 0; k < TJDS_TR_ROUNDS; k++)
+            {
+                const int32_t g = g0 + 32 * k + lane;
+                v[k] = g < nch ? __ldg(part + __ldg(seg_off + g) + q) : 0.0;
+            }
+#pragma unroll
+            for (int k = 0; k < TJDS_TR_ROUNDS; k++)
+#pragma unroll 8
+                for (int l = 0; l < 32; l++)
+                {
+                    const double c = __shfl_sync(0xffffffffu, v[k], l);
+                    if (g0 + 32 * k + l < nch)
+                        s = __dadd_rn(s, c);
+                }
+        }
+        if (lane == 0)
+            y[__ldg(perm + q)] = s;
+        return;
+    }
+    const int64_t qq = (int64_t)nwide + (t - wide_threads);
+    if (qq >= nlong)
+        return;
+    const int32_t q = (int32_t)qq;
+    const int32_t nch = (__ldg(slot_len + q) + TJDS_SEG - 1) / TJDS_SEG;
+    double s = 0.0;
+#pragma unroll 4
+    for (int32_t g = 0; g < nch; g++)
+        s = __dadd_rn(s, __ldg(part + __ldg(seg_off + g) + q));
+    y[__ldg(perm + q)] = s;
+}
+
+// partials segment g holds: the long columns (slots [0, nlong), nlong = length of diagonal TJDS_SEG) in segment 0, the
+// columns that reach its first diagonal in every later one
+__global__ void __launch_bounds__(256) tjds_transpose_count_kernel(const int32_t *__restrict__ start_pos, int32_t nseg,
+                                                                   uint32_t *__restrict__ count)
+{
+    const int32_t g = blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= nseg)
+        return;
+    const int32_t d = g == 0 ? TJDS_SEG : g * TJDS_SEG;
+    count[g] = (uint32_t)(start_pos[d + 1] - start_pos[d]);
+}
+
 // the row indices the kernels scatter through: the relabelled copy when that plan is in use (relabel.cu)
 static inline const int32_t *mult_rows(const smvp_tjds *A) { return A->relabel_state == 1 ? A->row_rel : A->row_ind; }
 
@@ -700,9 +823,110 @@ static int tjds_det_route(smvp_tjds *A)
     return SMVP_OK;
 }
 
+// plan and scratch of the transposed product (once per handle).  Synchronous.
+static int tjds_transpose_prepare(smvp_tjds *A, cudaStream_t s)
+{
+    if (A->tr_ready || A->ndiag == 0)
+        return SMVP_OK;
+    SMVP_TRY(tjds_plan(A, s));
+    if (A->ndiag > TJDS_SEG)
+    {
+        const int32_t nseg = (A->ndiag + TJDS_SEG - 1) / TJDS_SEG;
+        const int32_t wide = TJDS_SEG * TJDS_SEG; // columns longer than this have more than TJDS_SEG chunks
+        int32_t h[4] = {0, 0, 0, 0};
+        SMVP_CUDA(cudaMemcpyAsync(h, A->start_pos + TJDS_SEG, 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+        if (A->ndiag > wide)
+            SMVP_CUDA(cudaMemcpyAsync(h + 2, A->start_pos + wide, 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+        uint32_t *seg_off = nullptr;
+        double *part = nullptr;
+        uint32_t total = 0;
+        auto body = [&]() -> int {
+            DevTmp d_total;
+            SMVP_CUDA(d_total.alloc<uint32_t>(1));
+            SMVP_CUDA(dev_alloc(&seg_off, nseg));
+            SMVP_LAUNCH(tjds_transpose_count_kernel, (unsigned)ceil_div64(nseg, 256), 256, 0, s, (const int32_t *)A->start_pos, nseg,
+                        seg_off);
+            SMVP_TRY(exclusive_scan_u32(seg_off, seg_off, nseg, d_total.as<uint32_t>(), s));
+            SMVP_CUDA(cudaMemcpyAsync(&total, d_total.p, sizeof(total), cudaMemcpyDeviceToHost, s));
+            SMVP_CUDA(cudaStreamSynchronize(s));
+            SMVP_CUDA(cudaGetLastError());
+            SMVP_CUDA(dev_alloc(&part, total));
+            return SMVP_OK;
+        };
+        const int rc = body();
+        if (rc != SMVP_OK)
+        {
+            cudaFree(seg_off);
+            cudaFree(part);
+            return rc;
+        }
+        A->tr_seg_off = seg_off;
+        A->tr_part = part;
+        A->tr_nlong = h[1] - h[0];
+        A->tr_nwide = h[3] - h[2];
+        A->device_bytes += 4 * (int64_t)nseg + 8 * (int64_t)total;
+    }
+    A->tr_ready = 1;
+    return SMVP_OK;
+}
+
+// one transposed pass, asynchronous on s; tjds_transpose_prepare has run and A->cols > 0
+static int tjds_transpose_pass(smvp_tjds *A, const double *d_x, double *d_y, cudaStream_t s)
+{
+    if (A->ndiag == 0)
+    {
+        SMVP_CUDA(cudaMemsetAsync(d_y, 0, sizeof(double) * (size_t)A->cols, s)); // no entries: every column is empty
+        return SMVP_OK;
+    }
+    SMVP_LAUNCH(tjds_transpose_kernel, (unsigned)A->num_seg_blocks, 256, 0, s, (const int2 *)A->seg_blocks, (const int32_t *)A->start_pos,
+                (const int32_t *)A->row_ind, (const double *)A->val, (const int32_t *)A->perm, d_x, d_y, A->tr_part,
+                (const uint32_t *)A->tr_seg_off, A->ndiag, A->nslots, A->cols, A->tr_nlong);
+    if (A->ndiag > TJDS_SEG)
+    {
+        const int64_t threads = 32 * (int64_t)A->tr_nwide + (A->tr_nlong - A->tr_nwide);
+        SMVP_LAUNCH(tjds_transpose_combine_kernel, (unsigned)ceil_div64(threads, 256), 256, 0, s, (const double *)A->tr_part,
+                    (const uint32_t *)A->tr_seg_off, (const int32_t *)A->slot_len, (const int32_t *)A->perm, A->tr_nlong, A->tr_nwide, d_y);
+    }
+    SMVP_CUDA(cudaGetLastError());
+    return SMVP_OK;
+}
+
 } // namespace smvp
 
 using namespace smvp;
+
+extern "C" int smvp_tjds_mult_transpose_device(smvp_tjds *A, const double *d_x, double *d_y, void *stream)
+{
+    if (!A || (A->rows > 0 && !d_x) || (A->cols > 0 && !d_y))
+        return SMVP_E_ARG;
+    if (A->cols == 0)
+        return SMVP_OK;
+    cudaStream_t s = (cudaStream_t)stream;
+    SMVP_TRY(tjds_transpose_prepare(A, s));
+    return tjds_transpose_pass(A, d_x, d_y, s);
+}
+
+extern "C" int smvp_tjds_mult_transpose(smvp_tjds *A, const double *x_host, double *y_host, int iters, double *ms_each)
+{
+    if (!A || iters < 1 || (A->rows > 0 && !x_host) || (A->cols > 0 && !y_host))
+        return SMVP_E_ARG;
+    if (!A->d_xt)
+        SMVP_CUDA(dev_alloc(&A->d_xt, A->rows));
+    if (!A->d_yt)
+        SMVP_CUDA(dev_alloc(&A->d_yt, A->cols));
+    if (A->rows > 0)
+        SMVP_CUDA(cudaMemcpy(A->d_xt, x_host, sizeof(double) * (size_t)A->rows, cudaMemcpyHostToDevice));
+    SMVP_TRY(tjds_transpose_prepare(A, 0));
+    const bool small = (int64_t)A->rows + A->cols + A->nnz < SMVP_SMALL_LOOP_ITEMS;
+    if (A->cols > 0)
+        SMVP_TRY(timed_loop(iters, ms_each, small, [&](cudaStream_t s) { return tjds_transpose_pass(A, A->d_xt, A->d_yt, s); }));
+    else if (ms_each)
+        for (int it = 0; it < iters; it++)
+            ms_each[it] = 0.0;
+    if (A->cols > 0)
+        SMVP_CUDA(cudaMemcpy(y_host, A->d_yt, sizeof(double) * (size_t)A->cols, cudaMemcpyDeviceToHost));
+    return SMVP_OK;
+}
 
 extern "C" int smvp_tjds_set_x_device(smvp_tjds *A, const double *d_x, void *stream)
 {

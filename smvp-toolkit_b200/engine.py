@@ -79,6 +79,9 @@ SIGNATURES = {
     "smvp_csr_mult_device_fanout": (_int, [_vp, _vp, _vp, _int, _int, _vp]),
     "smvp_tjds_set_x_device": (_int, [_vp, _vp, _vp]),
     "smvp_tjds_mult_device": (_int, [_vp, _vp, _int, _i32, _vp]),
+    "smvp_csr_transpose": (_int, [_vp, _pp]),
+    "smvp_tjds_mult_transpose_device": (_int, [_vp, _vp, _vp, _vp]),
+    "smvp_tjds_mult_transpose": (_int, [_vp, _vp, _vp, _int, _vp]),
     "smvp_csr_info": (_int, [_vp, ctypes.POINTER(_CsrInfo)]),
     "smvp_tjds_info": (_int, [_vp, ctypes.POINTER(_TjdsInfo)]),
     "smvp_csr_export": (_int, [_vp, _vp, _vp, _vp]),
@@ -235,6 +238,12 @@ class CsrMatrix:
                "smvp_csr_build_device")
         return cls(h)
 
+    def transpose(self):
+        """A^T as a new, independent CsrMatrix built on the device (smvp_csr_transpose); this matrix is unchanged."""
+        h = ctypes.c_void_p()
+        _check(lib().smvp_csr_transpose(self._h, ctypes.byref(h)), "smvp_csr_transpose")
+        return CsrMatrix(h)
+
     def mult(self, x, iters=1, variant=CSR_AUTO):
         """`iters` timed passes of y = A x with host vectors (smvp_csr_mult). Returns (y, TimeData)."""
         x = np.ascontiguousarray(x, np.float64)
@@ -362,6 +371,22 @@ class TjdsMatrix:
         ms = np.zeros(iters, np.float64)
         _check(lib().smvp_tjds_mult(self._h, _ptr(x), _ptr(y), iters, _ptr(ms), variant, diag_limit), "smvp_tjds_mult")
         return y, TimeData(ms)
+
+    def mult_transpose(self, x, iters=1):
+        """`iters` timed passes of y = A^T x with host vectors (smvp_tjds_mult_transpose): x has `rows` entries, y `cols`.
+        Returns (y, TimeData)."""
+        x = np.ascontiguousarray(x, np.float64)
+        if x.shape != (self.rows,):
+            raise ValueError("x must have %d entries" % self.rows)
+        y = np.zeros(self.cols, np.float64)
+        ms = np.zeros(iters, np.float64)
+        _check(lib().smvp_tjds_mult_transpose(self._h, _ptr(x), _ptr(y), iters, _ptr(ms)), "smvp_tjds_mult_transpose")
+        return y, TimeData(ms)
+
+    def mult_transpose_device(self, d_x, d_y, stream=None):
+        """One pass y = A^T x on device vectors (d_x: `rows` entries, d_y: `cols`)."""
+        _check(lib().smvp_tjds_mult_transpose_device(self._h, _ptr(d_x), _ptr(d_y), _stream(stream)),
+               "smvp_tjds_mult_transpose_device")
 
     def set_x_device(self, d_x, stream=None):
         _check(lib().smvp_tjds_set_x_device(self._h, _ptr(d_x), _stream(stream)), "smvp_tjds_set_x_device")
