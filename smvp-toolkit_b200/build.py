@@ -39,24 +39,6 @@ def _run(cmd):
     return r.stdout + r.stderr
 
 
-def build_alt(name, defines, verbose=False):
-    """A/B builds: lib/libsmvp_cuda_<name>.so with extra -D switches (select it with SMVP_CUDA_LIB=<path>)."""
-    obj = os.path.join(LIB, "obj_" + name)
-    os.makedirs(obj, exist_ok=True)
-    srcs = sorted(f for f in os.listdir(CSRC) if f.endswith(".cu"))
-    objs = [os.path.join(obj, f[:-3] + ".o") for f in srcs]
-    jobs = [[NVCC] + NVCC_FLAGS + ["-D" + d for d in defines] + (["-Xptxas", "-v"] if verbose else []) +
-            ["-c", os.path.join(CSRC, f), "-o", o] for f, o in zip(srcs, objs)]
-    with ThreadPoolExecutor(max_workers=8) as ex:
-        outs = list(ex.map(_run, jobs))
-    if verbose:
-        for o in outs:
-            print(o)
-    so = os.path.join(LIB, "libsmvp_cuda_%s.so" % name)
-    _run([NVCC, "-shared", "-gencode", "arch=compute_100a,code=sm_100a", "-o", so] + objs)
-    return so
-
-
 def build_cuda(force=False, verbose=False):
     os.makedirs(OBJ, exist_ok=True)
     headers = [os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith((".cuh", ".h"))]
@@ -108,8 +90,4 @@ def build_all(force=False, verbose=False):
 
 
 if __name__ == "__main__":
-    if "--alt" in sys.argv:  # python build.py --alt phased SMVP_PHASED_PLAIN=1 [-v]
-        i = sys.argv.index("--alt")
-        print(build_alt(sys.argv[i + 1], [a for a in sys.argv[i + 2:] if "=" in a], verbose="-v" in sys.argv))
-    else:
-        print(build_all(force="--force" in sys.argv, verbose="-v" in sys.argv))
+    print(build_all(force="--force" in sys.argv, verbose="-v" in sys.argv))

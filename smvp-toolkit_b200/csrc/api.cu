@@ -60,10 +60,27 @@ extern "C" int64_t smvp_launch_count(void) { return (int64_t)g_launches.load(); 
 
 namespace smvp
 {
-static int loop_env_int(const char *name, int dflt)
+const char *env_str(const char *name)
 {
     const char *e = getenv(name);
-    return e && e[0] ? atoi(e) : dflt;
+    return e && e[0] ? e : nullptr;
+}
+
+bool env_set(const char *name) { return getenv(name) != nullptr; }
+
+int env_int(const char *name, int dflt, int lo, int hi)
+{
+    const char *e = env_str(name);
+    if (!e)
+        return dflt;
+    const long long v = atoll(e);
+    return v < lo ? lo : (v > hi ? hi : (int)v);
+}
+
+int env_tristate(const char *name)
+{
+    const char *e = env_str(name);
+    return (e && e[0] == '1') ? 1 : (e && e[0] == '0') ? -1 : 0;
 }
 
 int timed_loop(int iters, double *ms_each, bool batched, const std::function<int(cudaStream_t)> &pass,
@@ -71,7 +88,7 @@ int timed_loop(int iters, double *ms_each, bool batched, const std::function<int
 {
     if (iters < 1)
         return SMVP_E_ARG;
-    if (loop_env_int("SMVP_EXACT_ITER_TIMES", 0) == 1 || iters < 4)
+    if (env_int("SMVP_EXACT_ITER_TIMES", 0, INT32_MIN, INT32_MAX) == 1 || iters < 4)
         batched = false;
     cudaEvent_t e0 = nullptr, e1 = nullptr;
     SMVP_CUDA(cudaEventCreate(&e0));
@@ -123,8 +140,7 @@ int timed_loop(int iters, double *ms_each, bool batched, const std::function<int
 
     // ---- the remaining passes: graphs of `batch` passes replayed back to back on a private stream
     const int rest = iters - 1;
-    int batch = loop_env_int("SMVP_LOOP_BATCH", 50);
-    batch = batch < 1 ? 1 : batch;
+    int batch = env_int("SMVP_LOOP_BATCH", 50, 1, INT32_MAX);
     if ((rest + batch - 1) / batch > 1024)
         batch = (rest + 1023) / 1024; // bounds the number of events
     if (batch > rest)

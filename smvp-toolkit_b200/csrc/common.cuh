@@ -7,6 +7,7 @@
 #include <cstdlib>
 #include <functional>
 #include <new>
+#include <type_traits>
 
 #include "../../include/smvp_cuda.h"
 
@@ -44,6 +45,21 @@ int cuda_fail(cudaError_t e, const char *what, const char *file, int line);
     } while (0)
 
 static inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }
+
+// Lifts a run-time flag into a template argument: f(std::true_type()) or f(std::false_type()), so that a launcher names
+// each kernel instantiation once.
+template <typename F>
+static inline int with_flag(bool b, F &&f)
+{
+    return b ? f(std::true_type()) : f(std::false_type());
+}
+
+// ---------------------------------------------------------------- environment (api.cu)
+// The library's only reader of the environment: every SMVP_* switch goes through these (table in INTEGRATION.md).
+const char *env_str(const char *name);                   // the value; NULL when unset or empty
+bool env_set(const char *name);                          // set at all, even to ""
+int env_int(const char *name, int dflt, int lo, int hi); // decimal integer clamped to [lo, hi]; dflt when unset or empty
+int env_tristate(const char *name);                      // 1 for "1...", -1 for "0...", 0 otherwise
 
 // device allocation padded so that 16-byte vector / bulk copies may over-read the tail
 template <typename T>
@@ -196,6 +212,7 @@ int csr_relabel_plan(smvp_csr *A, cudaStream_t s);                 // relabel.cu
 int csr_relabel_x(smvp_csr *A, const double *d_x, cudaStream_t s); // relabel.cu
 void csr_relabel_release(smvp_csr *A);                             // relabel.cu
 int csr_split_plan(smvp_csr *A, cudaStream_t s);                   // relabel.cu: after csr_relabel_plan
+int32_t hot_l2_entries(); // relabel.cu: rank-ordered x entries expected to stay L2-resident (SMVP_HOT_L2)
 int csr_pattern_plan(smvp_csr *A, cudaStream_t s);                // pattern.cu: decides the relabelling first
 void csr_pattern_release(smvp_csr *A);                             // pattern.cu
 void csr_release(smvp_csr *A);                                     // csr_build.cu

@@ -138,8 +138,8 @@ int csr_build_impl(const int32_t *d_row, const int32_t *d_col, const double *d_v
     const double mean = rows > 0 ? (double)nnz / rows : 0.0;
     const bool tiny = nnz < (1 << 20);
     const bool skewed = A->max_row_nnz > 8.0 * (mean + 1.0); // memplus: vector 37 us, merge 13 us per SpMV
-    // long regular rows: measured on dense-band matrices of ~1 B nnz (tools/sweep_vector.py, profiles/r02_logs/
-    // r02_vector_sweep.log): 128 per row -- merge 1.97 ms, vector 2.33 ms; 512 per row -- vector 1.74 ms (7.09 TB/s, 88.6 % of
+    // long regular rows: measured on dense-band matrices of ~1 B nnz (profiles/r02_logs/r02_vector_sweep.log):
+    //: 128 per row -- merge 1.97 ms, vector 2.33 ms; 512 per row -- vector 1.74 ms (7.09 TB/s, 88.6 % of
     // 8 TB/s), merge 2.59 ms (rows that span several warp tiles chain through the fix-up).  The crossover is put at 256.
     const bool regular_long = mean >= 256.0 && A->max_row_nnz <= 4.0 * mean + 32.0;
     A->auto_variant = ((tiny && !skewed) || regular_long) ? SMVP_CSR_VECTOR : SMVP_CSR_MERGE;

@@ -28,15 +28,6 @@
 namespace smvp
 {
 
-static int env_int_early(const char *name, int dflt, int lo, int hi)
-{
-    const char *e = getenv(name);
-    if (!e || !e[0])
-        return dflt;
-    const int v = atoi(e);
-    return v < lo ? lo : (v > hi ? hi : v);
-}
-
 // ------------------------------------------------------------------ PTX helpers
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -81,17 +72,6 @@ __device__ __forceinline__ uint64_t l2_evict_last_policy()
     asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
     return pol;
 }
-__device__ __forceinline__ double ldg_x(const double *p, uint64_t pol)
-{
-#if SMVP_X_EVICT_LAST
-    double v;
-    asm volatile("ld.global.nc.L2::cache_hint.f64 %0, [%1], %2;" : "=d"(v) : "l"(p), "l"(pol));
-    return v;
-#else
-    (void)pol;
-    return __ldg(p);
-#endif
-}
 // x gather of a popularity-relabelled matrix (relabel.cu): the column index IS the popularity rank, so the
 // load can say how long the line deserves to live.  rank < hot_l1: keep in L1; rank < hot_l2: keep in L2
 // (evict-last) while the matrix streams and the cold gathers pass through evict-first and do not allocate in L1.
@@ -130,44 +110,25 @@ __device__ __forceinline__ void bulk_g2s(void *smem_dst, const void *gmem_src, u
                  : "memory");
 }
 
-// Tuning switches, A/B-tested on B200 (profiles/r01_logs/ab_variants.log, stencil 369^3, ms per SpMV):
-//   all off 2.995 | explicit 32-bit ld.shared 2.984 | + warp-uniform fast path for regular tiles 3.13 |
+// Variants A/B-tested on B200 and dropped from the source (profiles/r01_logs/ab_variants.log, stencil 369^3, ms per
+// SpMV): all off 2.995 | explicit 32-bit ld.shared 2.984 | + warp-uniform fast path for regular tiles 3.13 |
 //   + clamped (unpredicated) gathers 3.20 | + early-exit stitch scan 3.26 | all on 3.22
-// i.e. every extra vote / branch costs more than the instructions it saves.  The fast path and the clamped gathers
-// have since been removed from the source; the others stay for future re-tests.
-#ifndef SMVP_ASM_LDS
-#define SMVP_ASM_LDS 1
-#endif
-#ifndef SMVP_SCAN_EXIT
-#define SMVP_SCAN_EXIT 0
-#endif
-#ifndef SMVP_UNIFORM_TILES
-#define SMVP_UNIFORM_TILES 1 // broadcast the warp index / tile coordinates from lane 0 so the bookkeeping lives in uniform registers
-#endif
-#ifndef SMVP_X_EVICT_LAST
-#define SMVP_X_EVICT_LAST 0 // gather x with an L2 evict-last policy: measured 1 % on the stencil, 0 % on R-MAT -> off
-#endif
+// i.e. every extra vote / branch costs more than the instructions it saves.  Only the explicit ld.shared is kept:
+//   early-exit stitch scan (an __any_sync vote per step of the lane-boundary scan): removed.
+//   x gathers with an L2 evict-last policy: measured 1 % on the stencil, 0 % on R-MAT: removed.
 
 // explicit shared-window loads with 32-bit addresses (one register per view instead of a 64-bit generic pointer)
 __device__ __forceinline__ double lds_f64(uint32_t a)
 {
-#if SMVP_ASM_LDS
     double v;
     asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a));
     return v;
-#else
-    return *reinterpret_cast<const double *>(__cvta_shared_to_generic(a));
-#endif
 }
 __device__ __forceinline__ int32_t lds_s32(uint32_t a)
 {
-#if SMVP_ASM_LDS
     int32_t v;
     asm volatile("ld.shared.s32 %0, [%1];" : "=r"(v) : "r"(a));
     return v;
-#else
-    return *reinterpret_cast<const int32_t *>(__cvta_shared_to_generic(a));
-#endif
 }
 
 // ------------------------------------------------------------------ where y goes
@@ -194,28 +155,18 @@ __device__ __forceinline__ void store_y_acc(double *__restrict__ y, const YFan &
     else
         y[row] = accum ? __dadd_rn(y[row], v) : v;
 }
-template <bool FANOUT>
-__device__ __forceinline__ void store_y(double *__restrict__ y, const YFan &fan, int64_t row, double v)
-{
-    if (FANOUT)
-    {
-        for (int k = 0; k < fan.n; k++)
-            fan.p[k][row] = v;
-    }
-    else
-        y[row] = v;
-}
 
 // =====================================================================================  VECTOR
-// WIDE = true : each lane pulls 4 consecutive entries per step with 128-bit loads (long rows).
-// WIDE = false: lane l takes entries l, l+LPR, ... with 8/4-byte loads (short rows).  With only a few rows per warp
-//               the lanes of one request then sit on consecutive entries of consecutive rows, so the x gather of a
-//               banded matrix touches far fewer sectors per request -- the vector kernel is L1-bound on such rows.
-template <int LPR, bool FANOUT, bool WIDE>
+// LPR >= 16 (WIDE): each lane pulls 4 consecutive entries per step with 128-bit loads (long rows).
+// LPR < 16: lane l takes entries l, l+LPR, ... with 8/4-byte loads (short rows).  With only a few rows per warp
+//           the lanes of one request then sit on consecutive entries of consecutive rows, so the x gather of a
+//           banded matrix touches far fewer sectors per request -- the vector kernel is L1-bound on such rows.
+template <int LPR, bool FANOUT>
 __global__ void __launch_bounds__(256) csr_vector_kernel(const int32_t *__restrict__ row_ptr, const int32_t *__restrict__ col_ind,
                                                          const double *__restrict__ val, const double *__restrict__ x,
                                                          double *__restrict__ y, int32_t rows, const __grid_constant__ YFan fan)
 {
+    constexpr bool WIDE = LPR >= 16;
     const int64_t gt = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const int64_t row = gt / LPR;
     const int lane = (int)(gt % LPR);
@@ -269,7 +220,7 @@ __global__ void __launch_bounds__(256) csr_vector_kernel(const int32_t *__restri
     for (int o = LPR / 2; o > 0; o >>= 1)
         sum = __dadd_rn(sum, __shfl_xor_sync(0xffffffffu, sum, o));
     if (row < rows && lane == 0)
-        store_y<FANOUT>(y, fan, row, sum);
+        store_y_acc<FANOUT>(y, fan, row, sum, 0);
 }
 
 // =====================================================================================  TINY LOOP
@@ -320,28 +271,11 @@ static int launch_vector(const smvp_csr *A, const double *d_x, double *d_y, cons
     if (blocks > 0x7fffffffLL)
         return SMVP_E_TOOBIG;
     if (blocks > 0)
-    {
-        const char *we = getenv("SMVP_VECTOR_WIDE"); // tuning hook: force 128-bit (1) or lane-contiguous (0) loads
-        const bool wide = we && we[0] ? we[0] == '1' : LPR >= 16;
-        if (fan)
-        {
-            if (wide)
-                SMVP_LAUNCH((csr_vector_kernel<LPR, true, true>), (unsigned)blocks, 256, 0, s, A->row_ptr, mult_cols(A), A->val, d_x,
-                            d_y, A->rows, *fan);
-            else
-                SMVP_LAUNCH((csr_vector_kernel<LPR, true, false>), (unsigned)blocks, 256, 0, s, A->row_ptr, mult_cols(A), A->val, d_x,
-                            d_y, A->rows, *fan);
-        }
-        else
-        {
-            if (wide)
-                SMVP_LAUNCH((csr_vector_kernel<LPR, false, true>), (unsigned)blocks, 256, 0, s, A->row_ptr, mult_cols(A), A->val, d_x,
-                            d_y, A->rows, YFan());
-            else
-                SMVP_LAUNCH((csr_vector_kernel<LPR, false, false>), (unsigned)blocks, 256, 0, s, A->row_ptr, mult_cols(A), A->val, d_x,
-                            d_y, A->rows, YFan());
-        }
-    }
+        with_flag(fan != nullptr, [&](auto F) {
+            SMVP_LAUNCH((csr_vector_kernel<LPR, decltype(F)::value>), (unsigned)blocks, 256, 0, s, A->row_ptr, mult_cols(A), A->val,
+                        d_x, d_y, A->rows, fan ? *fan : YFan());
+            return SMVP_OK;
+        });
     return SMVP_OK;
 }
 
@@ -392,12 +326,11 @@ __global__ void __launch_bounds__(256) merge_plan_kernel(const int32_t *__restri
     tile_row[t] = merge_rows_before(row_ptr, rows, nnz, d);
 }
 
-template <int THREADS, int IPT, int STAGES>
+template <int THREADS, int IPT>
 struct MergeShape
 {
     static constexpr int TILE = THREADS * IPT;
-    static constexpr int STAGE_BYTES = ((12 * TILE + 128) + 127) & ~127;
-    static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES;
+    static constexpr int SMEM_BYTES = ((12 * TILE + 128) + 127) & ~127; // one stage per warp
 };
 
 struct TileView
@@ -470,11 +403,11 @@ __device__ __forceinline__ void merge_fixup_tile(int32_t t, const int32_t *__res
 
 // ---------------------------------------------------------------------------------------------
 // Warp-autonomous merge-path: the unit of work is a WARP tile of 32*IPT merge items.  Every warp owns
-// its shared-memory stage(s) and its mbarrier, fetches its tiles with its own TMA bulk copies and
+// its shared-memory stage and its mbarrier, fetches its tiles with its own TMA bulk copies and
 // never meets a block-wide barrier: warps of a CTA drift apart freely, so while one waits for HBM
 // or for its x gathers the others walk.  Rows cut by lane boundaries are stitched with a segmented
 // warp scan (__shfl_up_sync), rows cut by tile boundaries by the fix-up kernel -- fixed order, no atomics.
-template <int WARPS, int IPT, int STAGES, int MINB, bool FANOUT, bool RANKED, bool UNI>
+template <int WARPS, int IPT, int MINB, bool FANOUT, bool RANKED, bool UNI>
 __global__ void __launch_bounds__(WARPS * 32, MINB)
     csr_merge_warp_kernel(const int32_t *__restrict__ row_ptr, const int32_t *__restrict__ col_ind, const double *__restrict__ val,
                           const double *__restrict__ x, double *__restrict__ y, const int32_t *__restrict__ tile_row, int32_t rows,
@@ -487,9 +420,9 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
     // of a matrix like memplus that hides the second launch's latency (a pass lasts as long as a launch).
     if (early_dependents)
         asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    // processes tiles [tile_begin, num_tiles): a sub-range lets the host overlap the copy-out of finished rows
-    static_assert(STAGES == 1, "one stage per warp: deeper rings lost to more resident warps in every sweep");
-    using Shape = MergeShape<32, IPT, 1>;
+    // processes tiles [tile_begin, num_tiles): a sub-range lets the host overlap the copy-out of finished rows.
+    // One stage per warp: deeper rings lost to more resident warps in every sweep.
+    using Shape = MergeShape<32, IPT>;
     extern __shared__ __align__(128) unsigned char stage_mem[];
     __shared__ __align__(8) uint64_t full_bar[WARPS];
 
@@ -497,8 +430,8 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
     // anyway, but the broadcast lets the compiler PROVE it and keep the whole tile bookkeeping (and the operands of the
     // bulk copies) in uniform registers instead of electing a lane and converting per copy.  Measured on B200
     // (profiles/r01_logs/diet_bisect.log): stencil configuration 2.78 -> 2.69 ms, but the R-MAT configuration 5.67 ->
-    // 6.39 ms, so it is a per-configuration switch (last column of SMVP_WMERGE_CFGS).
-#define SMVP_BCAST(v) ((UNI && SMVP_UNIFORM_TILES) ? __shfl_sync(0xffffffffu, (v), 0) : (v))
+    // 6.39 ms, so it is a per-configuration choice (MergeStencil::UNI, MergeSkewed::UNI).
+#define SMVP_BCAST(v) (UNI ? __shfl_sync(0xffffffffu, (v), 0) : (v))
     const int lane = threadIdx.x & 31, w = SMVP_BCAST((int)(threadIdx.x >> 5));
     const int64_t total = (int64_t)rows + nnz;
     unsigned char *base = stage_mem + (size_t)w * Shape::SMEM_BYTES;
@@ -512,15 +445,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
     }
     __syncwarp();
 
-#if SMVP_X_EVICT_LAST
-    const uint64_t xpol = l2_evict_last_policy();
-#else
-    const uint64_t xpol = 0;
-#endif
     const uint64_t pol_last = RANKED ? l2_evict_last_policy() : 0, pol_first = RANKED ? l2_evict_first_policy() : 0;
-    auto gather = [&](int32_t c) -> double {
-        return RANKED ? ldg_x_ranked(x, c, hot_l1, hot_l2, pol_last, pol_first) : ldg_x(x + c, xpol);
-    };
     const int32_t warp_stride = (int32_t)gridDim.x * WARPS;
     auto issue = [&](const TileView &v) { // lane 0 only
         mbar_expect_tx(my_bar, v.vb + v.cb + v.rb);
@@ -717,8 +642,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
                 issue(make_tile(cur_r0, cur_r1, tn, Shape::TILE, total));
         }
 
-        // ---- stitch rows cut by lane boundaries: segmented inclusive scan of (carry row, carry sum); stops as
-        // soon as no run of equal keys is longer than the distance already covered
+        // ---- stitch rows cut by lane boundaries: segmented inclusive scan of (carry row, carry sum)
         const int32_t key = i_next; // the row my trailing partial belongs to
         double scan = sum;
 #pragma unroll
@@ -726,10 +650,6 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
         {
             const int32_t pk = __shfl_up_sync(0xffffffffu, key, o);
             const bool take = lane >= o && pk == key;
-#if SMVP_SCAN_EXIT
-            if (!__any_sync(0xffffffffu, take))
-                break;
-#endif
             const double pv = __shfl_up_sync(0xffffffffu, scan, o);
             if (take)
                 scan = __dadd_rn(pv, scan);
@@ -769,33 +689,33 @@ __global__ void __launch_bounds__(256) merge_fixup_kernel(const int32_t *__restr
         merge_fixup_tile<FANOUT>(t, tile_row, head_val, carry_val, y, fan, accum);
 }
 
-// ---- the instantiations AUTO chooses from: {warps per CTA, items per thread, stages per warp, min CTAs/SM}.
-// Measured on B200 (tools/sweep_csr.py; logs under profiles/): shared memory holds 12 B per staged
-// nonzero, so the items per thread bound how many warps an SM can keep busy; single-stage warps at
-// <= 64 registers (32 warps/SM) beat deeper rings, and any register spill halves the throughput.
-static int wmerge_tile_items(int cfg);
-
-static int pick_merge_cfg(const smvp_csr *A)
+// ---- the two instantiations AUTO chooses from (merge_skewed).  Measured on B200 (logs under profiles/, the swept
+// configurations in DESIGN.md §5.2): shared memory holds 12 B per staged nonzero, so the items per thread bound how many
+// warps an SM can keep busy; single-stage warps at <= 64 registers (32 warps/SM) beat deeper rings, and any register
+// spill halves the throughput.
+struct MergeStencil // 14 items per thread (two lanes per 27-point-stencil row), 4 warps per CTA
 {
-    const char *env = getenv("SMVP_MERGE_CFG");
-    if (env && env[0])
-    {
-        const int v = atoi(env);
-        if (wmerge_tile_items(v) > 0)
-            return v;
-    }
+    static constexpr int WARPS = 4, IPT = 14, MINB = 8;
+    static constexpr bool UNI = true;
+};
+struct MergeSkewed // 10 items per thread, 28 warps/SM (R-MAT scale 26: 8.0 ms vs 8.8 ms at 32 warps/SM and 62 registers)
+{
+    static constexpr int WARPS = 2, IPT = 10, MINB = 14;
+    static constexpr bool UNI = false;
+};
+
+// skewed or short rows take MergeSkewed, the others MergeStencil
+static bool merge_skewed(const smvp_csr *A)
+{
     const double mean = A->rows > 0 ? (double)A->nnz / A->rows : 0.0;
-    const bool skewed = A->max_row_nnz > 64.0 * (mean + 1.0);
-    if (skewed || mean < 20.0)
-        return 4; // 10 items per thread, 28 warps/SM (R-MAT scale 26: 8.0 ms vs 8.8 ms at 32 warps/SM and 62 registers)
-    return 2;     // 14 items per thread (two lanes per 27-point-stencil row), 4 warps per CTA
+    return A->max_row_nnz > 64.0 * (mean + 1.0) || mean < 20.0;
 }
 
 constexpr int32_t MERGE_PDL_TILES = 8192; // grids of at most this many warp tiles launch their fix-up early
 
-static int merge_plan(smvp_csr *A, int cfg, cudaStream_t s)
+static int merge_plan(smvp_csr *A, cudaStream_t s)
 {
-    const int32_t tile_items = wmerge_tile_items(cfg);
+    const int32_t tile_items = 32 * (merge_skewed(A) ? MergeSkewed::IPT : MergeStencil::IPT);
     if (A->merge_cfg == tile_items)
         return SMVP_OK;
     cudaFree(A->tile_row);
@@ -819,71 +739,66 @@ static int merge_plan(smvp_csr *A, int cfg, cudaStream_t s)
     return SMVP_OK;
 }
 
-#define SMVP_WMERGE_CFGS(X)    \
-    X(0, 2, 14, 1, 16, true)   \
-    X(1, 2, 10, 1, 16, false)  \
-    X(2, 4, 14, 1, 8, true)    \
-    X(3, 2, 12, 1, 16, true)   \
-    X(4, 2, 10, 1, 14, false)  \
-    X(5, 2, 7, 1, 16, false)   \
-    X(6, 2, 9, 1, 16, false)   \
-    X(7, 4, 14, 1, 9, true)
-
 // how much of the rank-ordered x a relabelled multiply asks L1 / L2 to retain (entries; SMVP_HOT_L1 / SMVP_HOT_L2)
 static void hot_limits(int32_t *l1, int32_t *l2)
 {
-    const char *e1 = getenv("SMVP_HOT_L1"), *e2 = getenv("SMVP_HOT_L2");
-    *l1 = e1 && e1[0] ? atoi(e1) : 8192;     // 64 KB
-    *l2 = e2 && e2[0] ? atoi(e2) : (4 << 20); // 32 MB
+    *l1 = env_int("SMVP_HOT_L1", 8192, 0, INT32_MAX); // 64 KB
+    *l2 = hot_l2_entries();                           // 32 MB
 }
 
-template <int WARPS, int IPT, int STAGES, int MINB, bool FANOUT, bool RANKED, bool UNI>
+// Persistent grid with a static stride over the tiles: the CTAs that fit on the device at once, at most `need`.
+// smvp_csr_set_corunner_headroom / SMVP_MERGE_HEADROOM=k: leave room for k more CTAs per SM.  Every CTA must be resident
+// from the start: a CTA that has to wait for a co-running kernel's CTA to retire (the exchange kernel of the multi-GPU
+// path) begins its full share of tiles late and the pass ends that much later (measured: SpMV 1.34 ms + copy kernel
+// 0.42 ms side by side = 1.78 ms).
+struct Residency // CTAs per SM of one kernel, looked up per device and dynamic shared-memory size
+{
+    int dev = -1, smem = -1, ctas = 1;
+};
+template <typename K>
+static int persistent_grid(K kern, int threads, int smem, int handle_headroom, int64_t need, Residency &res, int64_t *grid)
+{
+    int dev = 0;
+    SMVP_CUDA(cudaGetDevice(&dev));
+    if (res.dev != dev || res.smem != smem)
+    {
+        SMVP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        SMVP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&res.ctas, kern, threads, smem));
+        if (res.ctas < 1)
+            res.ctas = 1;
+        res.dev = dev;
+        res.smem = smem;
+    }
+    static thread_local const int env_headroom = env_int("SMVP_MERGE_HEADROOM", -1, -1, 8);
+    const int headroom = env_headroom >= 0 ? env_headroom : handle_headroom;
+    const int used = res.ctas - headroom >= 1 ? res.ctas - headroom : 1;
+    const int64_t g = (int64_t)device_props().sms * used;
+    *grid = g > need ? need : g;
+    return SMVP_OK;
+}
+
+template <class C, bool FANOUT, bool RANKED>
 static int launch_wmerge(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fanp, cudaStream_t s, int32_t tile_begin,
                          int32_t tile_end, int32_t accum)
 {
-    using Shape = MergeShape<32, IPT, STAGES>;
-    constexpr int SMEM = WARPS * Shape::SMEM_BYTES;
-    auto kern = csr_merge_warp_kernel<WARPS, IPT, STAGES, MINB, FANOUT, RANKED, UNI>;
+    constexpr int SMEM = C::WARPS * MergeShape<32, C::IPT>::SMEM_BYTES;
+    auto kern = csr_merge_warp_kernel<C::WARPS, C::IPT, C::MINB, FANOUT, RANKED, C::UNI>;
     int32_t hot_l1 = 0, hot_l2 = 0;
     if (RANKED)
         hot_limits(&hot_l1, &hot_l2);
     const YFan fan = fanp ? *fanp : YFan();
-    static thread_local int configured_dev = -1;
-    static thread_local int resident = 1;
-    int dev = 0;
-    SMVP_CUDA(cudaGetDevice(&dev));
-    if (configured_dev != dev)
-    {
-        SMVP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
-        SMVP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kern, WARPS * 32, SMEM));
-        if (resident < 1)
-            resident = 1;
-        configured_dev = dev;
-    }
-    // smvp_csr_set_corunner_headroom / SMVP_MERGE_HEADROOM=k: leave room for k more CTAs per SM.  The grid is persistent with a static stride over the
-    // tiles, so every CTA must be resident from the start: a CTA that has to wait for a co-running kernel's CTA to
-    // retire (the exchange kernel of the multi-GPU path) begins its full share of tiles late and the pass ends that much
-    // later (measured: SpMV 1.34 ms + copy kernel 0.42 ms side by side = 1.78 ms).
-    static thread_local int env_headroom = -2;
-    if (env_headroom == -2)
-        env_headroom = env_int_early("SMVP_MERGE_HEADROOM", -1, -1, 8);
-    const int headroom = env_headroom >= 0 ? env_headroom : A->merge_headroom;
-    const int res_used = resident - headroom >= 1 ? resident - headroom : 1;
-    int64_t grid = (int64_t)device_props().sms * res_used;
+    static thread_local Residency res;
     const int32_t ntiles = tile_end - tile_begin;
-    const int64_t need = ceil_div64(ntiles, WARPS);
-    if (grid > need)
-        grid = need;
+    int64_t grid = 0;
+    SMVP_TRY(persistent_grid(kern, C::WARPS * 32, SMEM, A->merge_headroom, ceil_div64(ntiles, C::WARPS), res, &grid));
     if (grid > 0)
     {
         // (a fix-up fused into the kernel -- the last warp of the grid to finish walks the tiles -- was tried for the
         // batched `-n` loop of small matrices: one warp serialises the few hundred tiles of a matrix like memplus,
         // 12.1 us per pass against 5.7 us with the second launch.  Two launches it stays.)
-        static thread_local int pdl_ok = -1; // SMVP_NO_PDL=1 switches the early launch of the fix-up off
-        if (pdl_ok < 0)
-            pdl_ok = getenv("SMVP_NO_PDL") == nullptr ? 1 : 0;
-        const bool early = pdl_ok == 1 && ntiles <= MERGE_PDL_TILES;
-        SMVP_LAUNCH(kern, (unsigned)grid, WARPS * 32, SMEM, s, A->row_ptr, mult_cols(A), A->val, d_x, d_y, A->tile_row, A->rows,
+        static thread_local const bool pdl_ok = !env_set("SMVP_NO_PDL"); // SMVP_NO_PDL: no early launch of the fix-up
+        const bool early = pdl_ok && ntiles <= MERGE_PDL_TILES;
+        SMVP_LAUNCH(kern, (unsigned)grid, C::WARPS * 32, SMEM, s, A->row_ptr, mult_cols(A), A->val, d_x, d_y, A->tile_row, A->rows,
                     A->nnz, tile_begin, tile_end, A->head_val, A->carry_val, fan, hot_l1, hot_l2, early ? 1 : 0, accum);
         if (early)
         {
@@ -906,20 +821,6 @@ static int launch_wmerge(const smvp_csr *A, const double *d_x, double *d_y, cons
                         (const double *)A->head_val, (const double *)A->carry_val, tile_begin, tile_end, d_y, fan, accum);
     }
     return SMVP_OK;
-}
-
-static int wmerge_tile_items(int cfg)
-{
-    switch (cfg)
-    {
-#define X(id, wp, i, st, mb, un) \
-    case id:                     \
-        return 32 * i;
-        SMVP_WMERGE_CFGS(X)
-#undef X
-    default:
-        return 0;
-    }
 }
 
 // =====================================================================================  PATTERN
@@ -1074,7 +975,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
                         sum = __dadd_rn(sum, __dmul_rn(lds_f64(vrow + 8u * (uint32_t)(k0 + q)), xv[q]));
             }
             if (live)
-                store_y<FANOUT>(y, fan, r, sum);
+                store_y_acc<FANOUT>(y, fan, r, sum, 0);
         }
         // the stage is consumed: refill it with tile tn
         __syncwarp();
@@ -1088,76 +989,40 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
     }
 }
 
-// ---- the instantiations of the pattern kernel: {warps per CTA, rounds of 32 rows per tile, stages per warp, gathers in
-// flight per lane, min CTAs/SM}.  Measured on B200 (tools/sweep_pattern.py, profiles/r03_logs/sweep_pattern.log, stencil
-// 369^3): one stage per warp and 28 warps per SM (0: 1.75 ms, 1: 1.72-1.81 ms) against 2.1-3.2 ms for every
+// ---- the pattern kernel's configuration.  Measured on B200 (profiles/r03_logs/sweep_pattern.log, stencil 369^3, the
+// swept configurations in DESIGN.md §5.2): one stage per warp and 28 warps per SM (1.75 ms) against 2.1-3.2 ms for every
 // configuration with two stages or two rounds per tile -- a 7 KB stage per warp, so resident warps, not staging depth,
-// keep enough gathers in flight.  SMVP_PATTERN_CFG=k picks another one.
-#define SMVP_PATTERN_CFGS(X) \
-    X(0, 4, 1, 1, 14, 7)     \
-    X(1, 4, 1, 1, 9, 8)      \
-    X(2, 4, 1, 2, 9, 4)      \
-    X(3, 4, 1, 2, 14, 4)     \
-    X(4, 4, 2, 1, 9, 4)      \
-    X(5, 8, 1, 2, 9, 2)      \
-    X(6, 4, 2, 2, 9, 2)      \
-    X(7, 2, 1, 2, 9, 7)
-
-static int pick_pattern_cfg() { return env_int_early("SMVP_PATTERN_CFG", 0, 0, 7); }
-
-template <int WARPS, int R, int STAGES, int CH, int MINB, bool FANOUT>
-static int launch_pattern(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fanp, cudaStream_t s, int32_t row_begin,
-                          int32_t row_end)
+// keep enough gathers in flight.
+struct PatternCfg
 {
-    auto kern = csr_pattern_kernel<WARPS, R, STAGES, CH, MINB, FANOUT>;
-    const int maxlen = A->pattern_maxlen > 0 ? A->pattern_maxlen : 1;
-    const int stage = PatternShape<R>::stage_bytes(maxlen);
-    const int table = (A->pattern_count * (maxlen + 1) * 4 + 127) & ~127;
-    const int smem = table + WARPS * STAGES * stage;
-    // the shared memory depends on the matrix (longest pattern, pattern count): occupancy is looked up per size
-    static thread_local int configured_dev = -1, configured_smem = -1, resident = 1;
-    int dev = 0;
-    SMVP_CUDA(cudaGetDevice(&dev));
-    if (configured_dev != dev || configured_smem != smem)
-    {
-        SMVP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        SMVP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kern, WARPS * 32, smem));
-        if (resident < 1)
-            resident = 1;
-        configured_dev = dev;
-        configured_smem = smem;
-    }
-    // persistent grid with a static stride over the tiles: the co-runner headroom works as for the merge kernel
-    static thread_local int env_headroom = -2;
-    if (env_headroom == -2)
-        env_headroom = env_int_early("SMVP_MERGE_HEADROOM", -1, -1, 8);
-    const int headroom = env_headroom >= 0 ? env_headroom : A->merge_headroom;
-    const int res_used = resident - headroom >= 1 ? resident - headroom : 1;
-    int64_t grid = (int64_t)device_props().sms * res_used;
-    const int64_t need = ceil_div64(ceil_div64((int64_t)row_end - row_begin, PatternShape<R>::ROWS), WARPS);
-    if (grid > need)
-        grid = need;
-    if (grid > 0)
-        SMVP_LAUNCH(kern, (unsigned)grid, WARPS * 32, smem, s, A->row_ptr, A->val, A->pat_id, A->pat_off, A->pat_len,
-                    A->pattern_count, maxlen, d_x, d_y, row_begin, row_end, (uint32_t)stage, fanp ? *fanp : YFan());
-    return SMVP_OK;
-}
+    static constexpr int WARPS = 4; // warps per CTA
+    static constexpr int R = 1;     // rounds of 32 rows per tile
+    static constexpr int STAGES = 1; // stages per warp
+    static constexpr int CH = 14;   // gathers in flight per lane
+    static constexpr int MINB = 7;  // min CTAs per SM
+};
 
 // rows [row_begin, row_end) of a handle with the row-pattern plan
 static int csr_mult_pattern(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, cudaStream_t s, int32_t row_begin,
                             int32_t row_end)
 {
-    switch (pick_pattern_cfg())
-    {
-#define X(id, wp, r, st, ch, mb)                                                                        \
-    case id:                                                                                            \
-        return fan ? launch_pattern<wp, r, st, ch, mb, true>(A, d_x, d_y, fan, s, row_begin, row_end) \
-                   : launch_pattern<wp, r, st, ch, mb, false>(A, d_x, d_y, nullptr, s, row_begin, row_end);
-        SMVP_PATTERN_CFGS(X)
-#undef X
-    default:
-        return SMVP_E_ARG;
-    }
+    using C = PatternCfg;
+    const int maxlen = A->pattern_maxlen > 0 ? A->pattern_maxlen : 1;
+    const int stage = PatternShape<C::R>::stage_bytes(maxlen);
+    const int table = (A->pattern_count * (maxlen + 1) * 4 + 127) & ~127;
+    const int smem = table + C::WARPS * C::STAGES * stage;
+    const int64_t need = ceil_div64(ceil_div64((int64_t)row_end - row_begin, PatternShape<C::R>::ROWS), C::WARPS);
+    return with_flag(fan != nullptr, [&](auto F) {
+        auto kern = csr_pattern_kernel<C::WARPS, C::R, C::STAGES, C::CH, C::MINB, decltype(F)::value>;
+        // the shared memory depends on the matrix (longest pattern, pattern count): occupancy is looked up per size
+        static thread_local Residency res;
+        int64_t grid = 0;
+        SMVP_TRY(persistent_grid(kern, C::WARPS * 32, smem, A->merge_headroom, need, res, &grid));
+        if (grid > 0)
+            SMVP_LAUNCH(kern, (unsigned)grid, C::WARPS * 32, smem, s, A->row_ptr, A->val, A->pat_id, A->pat_off, A->pat_len,
+                        A->pattern_count, maxlen, d_x, d_y, row_begin, row_end, (uint32_t)stage, fan ? *fan : YFan());
+        return (int)SMVP_OK;
+    });
 }
 
 // tiles [tile_begin, tile_end) of the plan; (0, -1) = all
@@ -1175,34 +1040,26 @@ static int csr_mult_merge(smvp_csr *A, const double *d_x, double *d_y, const YFa
     // the row-pattern plan serves whole passes (the pipelined host call cuts its ranges on rows: csr_mult_pattern)
     if (A->pattern_state == 1 && tile_begin == 0 && tile_end < 0 && !accum)
         return csr_mult_pattern(A, d_x, d_y, fan, s, 0, A->rows);
-    const int cfg = pick_merge_cfg(A);
-    SMVP_TRY(merge_plan(A, cfg, s));
+    SMVP_TRY(merge_plan(A, s));
     if (tile_end < 0)
         tile_end = A->merge_tiles;
     // a relabelled handle indexes x by popularity rank: the gathers carry cache-retention hints (SMVP_RANKED_HINTS=0: off)
-    const char *rh = getenv("SMVP_RANKED_HINTS");
-    const bool ranked = (A->relabel_state == 1 || A->ranked_cols == 1) && !(rh && rh[0] == '0');
-    switch (cfg)
-    {
-#define X(id, wp, i, st, mb, un)                                                                                       \
-    case id:                                                                                                           \
-        if (ranked)                                                                                                           \
-            return fan ? launch_wmerge<wp, i, st, mb, true, true, un>(A, d_x, d_y, fan, s, tile_begin, tile_end, accum)       \
-                       : launch_wmerge<wp, i, st, mb, false, true, un>(A, d_x, d_y, nullptr, s, tile_begin, tile_end, accum); \
-        return fan ? launch_wmerge<wp, i, st, mb, true, false, un>(A, d_x, d_y, fan, s, tile_begin, tile_end, accum)          \
-                   : launch_wmerge<wp, i, st, mb, false, false, un>(A, d_x, d_y, nullptr, s, tile_begin, tile_end, accum);
-        SMVP_WMERGE_CFGS(X)
-#undef X
-    default:
-        return SMVP_E_ARG;
-    }
+    const bool ranked = (A->relabel_state == 1 || A->ranked_cols == 1) && env_tristate("SMVP_RANKED_HINTS") != -1;
+    const bool skewed = merge_skewed(A);
+    return with_flag(fan != nullptr, [&](auto F) {
+        return with_flag(ranked, [&](auto R) {
+            constexpr bool FANOUT = decltype(F)::value, RANKED = decltype(R)::value;
+            return skewed ? launch_wmerge<MergeSkewed, FANOUT, RANKED>(A, d_x, d_y, fan, s, tile_begin, tile_end, accum)
+                          : launch_wmerge<MergeStencil, FANOUT, RANKED>(A, d_x, d_y, fan, s, tile_begin, tile_end, accum);
+        });
+    });
 }
 
 int csr_resolve_variant(const smvp_csr *A, int variant)
 {
     if (variant == SMVP_CSR_AUTO)
     {
-        const char *env = getenv("SMVP_CSR_VARIANT");
+        const char *env = env_str("SMVP_CSR_VARIANT");
         if (env && (env[0] == '1' || env[0] == '2'))
             return env[0] - '0';
         return A->auto_variant;
@@ -1289,7 +1146,7 @@ static int csr_mult_any(smvp_csr *A, const double *d_x, double *d_y, const YFan 
         if (!x && A->cols > 0)
             return SMVP_E_ARG;
     }
-    const int persist_mb = A->relabel_state == 1 ? env_int_early("SMVP_L2_PERSIST_MB", 0, 0, 4096) : 0;
+    const int persist_mb = A->relabel_state == 1 ? env_int("SMVP_L2_PERSIST_MB", 0, 0, 4096) : 0;
     if (persist_mb > 0)
         SMVP_TRY(l2_persist_window(s, x, (size_t)persist_mb << 20));
     const int rc = csr_mult_launch(A, x, d_y, fan, variant, s);
@@ -1354,14 +1211,6 @@ extern "C" int smvp_csr_mult_device_fanout(smvp_csr *A, const double *d_x, doubl
 constexpr int PIPE_MAX_RANGES = 64;   // == capacity of smvp_csr::pipe_tile / pipe_row / pipe_xneed (common.cuh)
 constexpr int PIPE_MAX_XCHUNKS = 128;
 
-static int env_int(const char *name, int dflt, int lo, int hi)
-{
-    const char *e = getenv(name);
-    if (!e || !e[0])
-        return dflt;
-    const int v = atoi(e);
-    return v < lo ? lo : (v > hi ? hi : v);
-}
 // defaults from the sweep on B200 (tools/sweep_e2e.py, profiles/): tuning hooks SMVP_PIPE_RANGES / SMVP_PIPE_XCHUNKS
 // Piece SIZE, not piece count, is fixed, so the fixed cost of a call shrinks with the block a rank owns (round 1: e2e did
 // not scale with N).  6 MB in both directions: on the 402 MB vectors of the 369^3 stencil that is 64 ranges x 64 upload
@@ -1392,10 +1241,14 @@ static int pipe_xchunks(int64_t x_bytes)
 // middle uses transfers large enough for both PCIe directions to run near their rate.  MEASURED: it loses -- 10.9 ms per call
 // against 9.8 ms for 64 x 64 equal 6 MB pieces in the same run (the upload ends at 9.9 instead of 9.2 ms: with both
 // directions busy, many small equal pieces interleave better than a few large ones).  Default: n equal pieces.
+static bool pipe_ramp()
+{
+    const char *pe = env_str("SMVP_PIPE_PROFILE");
+    return pe && pe[0] == 'r';
+}
 static int pipe_profile(int64_t bytes, int n_uniform, int max_pieces, double *f)
 {
-    const char *pe = getenv("SMVP_PIPE_PROFILE");
-    const bool ramp = pe && pe[0] == 'r';
+    const bool ramp = pipe_ramp();
     const int64_t MB = 1 << 20;
     const int64_t ends[4] = {2 * MB, 4 * MB, 8 * MB, 16 * MB};
     const int64_t big = 24 * MB, ends_sum = 2 * (2 + 4 + 8 + 16) * MB;
@@ -1453,11 +1306,10 @@ static int pipe_plan(smvp_csr *A)
 {
     const bool pat = A->pattern_state == 1;
     if (!pat)
-        SMVP_TRY(merge_plan(A, pick_merge_cfg(A), 0));
+        SMVP_TRY(merge_plan(A, 0));
     double rf[PIPE_MAX_RANGES + 1];
     const int NR = pipe_profile(8 * (int64_t)A->rows, pipe_ranges(8 * (int64_t)A->rows), PIPE_MAX_RANGES, rf);
-    const char *pe = getenv("SMVP_PIPE_PROFILE");
-    const int ramp = pe && pe[0] == 'r' ? 1 : 0;
+    const int ramp = pipe_ramp() ? 1 : 0;
     const int32_t key = pat ? PIPE_CFG_PATTERN : A->merge_cfg;
     if (A->pipe_cfg == key && A->pipe_ranges == NR && A->pipe_ramp == ramp)
         return SMVP_OK;
@@ -1707,7 +1559,7 @@ static int csr_mult_pipelined(smvp_csr *A, const double *x_host, double *y_host,
         total += t;
     }
     *ms = total;
-    if (getenv("SMVP_PIPE_TRACE")) // where the pass spends its time (ms after the start of the pass)
+    if (env_set("SMVP_PIPE_TRACE")) // where the pass spends its time (ms after the start of the pass)
     {
         auto at = [&](cudaEvent_t ev) {
             float t = 0.f;
@@ -1752,8 +1604,8 @@ extern "C" int smvp_csr_mult(smvp_csr *A, const double *x_host, double *y_host, 
         }
         return a.type == cudaMemoryTypeHost || a.type == cudaMemoryTypeManaged;
     };
-    const bool pipelined = merge && ((int64_t)A->rows + A->cols) >= (1 << 21) && getenv("SMVP_NO_OVERLAP") == nullptr &&
-                           (getenv("SMVP_FORCE_OVERLAP") != nullptr || (page_locked(x_host) && page_locked(y_host)));
+    const bool pipelined = merge && ((int64_t)A->rows + A->cols) >= (1 << 21) && !env_set("SMVP_NO_OVERLAP") &&
+                           (env_set("SMVP_FORCE_OVERLAP") || (page_locked(x_host) && page_locked(y_host)));
     int rc = SMVP_OK;
     // plans outside the timed bracket (the reference builds its format before the loop too)
     if (A->rows > 0)
@@ -1761,7 +1613,7 @@ extern "C" int smvp_csr_mult(smvp_csr *A, const double *x_host, double *y_host, 
     if (rc == SMVP_OK && pipelined)
         rc = pipe_plan(A);
     else if (rc == SMVP_OK && merge && A->pattern_state != 1)
-        rc = merge_plan(A, pick_merge_cfg(A), 0);
+        rc = merge_plan(A, 0);
     if (rc != SMVP_OK)
         return rc;
     const bool relabeled = A->relabel_state == 1;
@@ -1782,7 +1634,7 @@ extern "C" int smvp_csr_mult(smvp_csr *A, const double *x_host, double *y_host, 
         const bool small = (int64_t)A->rows + A->cols + A->nnz < SMVP_SMALL_LOOP_ITEMS;
         // (an explicitly requested variant is honoured pass by pass; AUTO may pick the looping kernel)
         const bool tiny = variant == SMVP_CSR_AUTO && A->nnz <= TINY_MAX_NNZ && A->rows <= TINY_MAX_ROWS &&
-                          getenv("SMVP_NO_TINY_LOOP") == nullptr;
+                          !env_set("SMVP_NO_TINY_LOOP");
         std::function<int(cudaStream_t, int)> multi;
         if (tiny)
             multi = [&](cudaStream_t s, int n) {

@@ -154,8 +154,7 @@ int csr_pattern_plan(smvp_csr *A, cudaStream_t s)
     SMVP_TRY(csr_relabel_plan(A, s)); // a relabelled handle reads col_rel: that plan decides first
     if (A->pattern_state != 0)
         return SMVP_OK;
-    const char *env = getenv("SMVP_CSR_PATTERN");
-    if (A->relabel_state == 1 || A->rows == 0 || (env && env[0] == '0'))
+    if (A->relabel_state == 1 || A->rows == 0 || env_tristate("SMVP_CSR_PATTERN") == -1)
     {
         A->pattern_state = -1;
         return SMVP_OK;

@@ -32,14 +32,16 @@ namespace smvp
 // x of 64 MB and more: beyond what L2 keeps next to the matrix streams; 32 MB of x: the part expected to stay L2-resident.
 // SMVP_RELABEL_MIN_COLS / SMVP_RELABEL_HOT_COLS (entries) scale the AUTO test down so that it can be exercised on small
 // matrices (tests); they do not touch the cache hints of the multiply.
-static int64_t env_entries(const char *name, int64_t dflt)
+static int64_t relabel_min_cols()
 {
-    const char *e = getenv(name);
-    const long long v = e && e[0] ? atoll(e) : 0;
-    return v > 0 ? (int64_t)v : dflt;
+    const int v = env_int("SMVP_RELABEL_MIN_COLS", 0, 0, INT32_MAX);
+    return v > 0 ? v : 8 << 20;
 }
-static int64_t relabel_min_cols() { return env_entries("SMVP_RELABEL_MIN_COLS", 8 << 20); }
-static int64_t relabel_hot_cols() { return env_entries("SMVP_RELABEL_HOT_COLS", 4 << 20); }
+static int64_t relabel_hot_cols()
+{
+    const int v = env_int("SMVP_RELABEL_HOT_COLS", 0, 0, INT32_MAX);
+    return v > 0 ? v : 4 << 20;
+}
 
 __global__ void __launch_bounds__(256) relabel_key_kernel(const uint32_t *__restrict__ count, int32_t cols, uint32_t maxc,
                                                           uint32_t *__restrict__ key, uint32_t *__restrict__ idx)
@@ -209,12 +211,6 @@ int relabel_indices(const int32_t *d_idx, int64_t nnz, const int32_t *d_rank, in
     return SMVP_OK;
 }
 
-static int env_forced(const char *name)
-{
-    const char *env = getenv(name);
-    return (env && env[0] == '1') ? 1 : (env && env[0] == '0') ? -1 : 0;
-}
-
 // decides (once per handle) and, if the plan is worth it, builds col_rel / x_order / x_rel.  Synchronous.
 int csr_relabel_plan(smvp_csr *A, cudaStream_t s)
 {
@@ -222,7 +218,7 @@ int csr_relabel_plan(smvp_csr *A, cudaStream_t s)
         return csr_split_plan(A, s); // decided once as well; returns at once afterwards
     int use = 0;
     int32_t *order = nullptr, *rank = nullptr;
-    SMVP_TRY(popularity_plan(A->col_ind, A->nnz, A->cols, env_forced("SMVP_CSR_RELABEL"), 2.0, &order, &rank, &use, s));
+    SMVP_TRY(popularity_plan(A->col_ind, A->nnz, A->cols, env_tristate("SMVP_CSR_RELABEL"), 2.0, &order, &rank, &use, s));
     if (!use)
     {
         A->relabel_state = -1;
@@ -258,7 +254,7 @@ int tjds_relabel_plan(smvp_tjds *A, cudaStream_t s)
         return SMVP_OK;
     int use = 0;
     int32_t *order = nullptr, *rank = nullptr;
-    SMVP_TRY(popularity_plan(A->row_ind, A->nnz, A->rows, env_forced("SMVP_TJDS_RELABEL"), 4.0, &order, &rank, &use, s));
+    SMVP_TRY(popularity_plan(A->row_ind, A->nnz, A->rows, env_tristate("SMVP_TJDS_RELABEL"), 4.0, &order, &rank, &use, s));
     if (!use)
     {
         A->relabel_state = -1;
@@ -343,22 +339,19 @@ __global__ void __launch_bounds__(256) split_scatter_kernel(const int32_t *__res
     }
 }
 
-static int hot_prefix_entries()
-{
-    const char *e = getenv("SMVP_HOT_L2");
-    return e && e[0] ? atoi(e) : (4 << 20);
-}
+// also the L2 retention limit of the ranked gathers (csr_mult.cu hot_limits): one value for both
+int32_t hot_l2_entries() { return env_int("SMVP_HOT_L2", 4 << 20, 0, INT32_MAX); } // 32 MB of x
 
 int csr_split_plan(smvp_csr *A, cudaStream_t s)
 {
     if (A->split_state != 0)
         return SMVP_OK;
     A->split_state = -1;
-    const int forced = env_forced("SMVP_CSR_SPLIT");
+    const int forced = env_tristate("SMVP_CSR_SPLIT");
     // OPT-IN (SMVP_CSR_SPLIT=1), never AUTO: measured on R-MAT scale 26 it LOSES -- see the header comment above
     if (A->relabel_state != 1 || forced <= 0 || A->nnz == 0)
         return SMVP_OK;
-    const int32_t hot = hot_prefix_entries();
+    const int32_t hot = hot_l2_entries();
     if (hot <= 0 || hot >= A->cols)
         return SMVP_OK;
     DevTmp row_of, pos, total, hr, hc, hv, cr, cc, cv;

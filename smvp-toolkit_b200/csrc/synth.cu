@@ -645,8 +645,7 @@ extern "C" int smvp_push_tma_device(void *const *d_dst_list, int n_dst, const vo
             SMVP_CUDA(cudaFuncSetAttribute(push_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
             // same L1 / shared-memory split as the merge-path SpMV (which needs ~200 KB of shared memory per SM): an SM
             // hosts CTAs of two kernels at once only under one split
-            const char *cv = getenv("SMVP_PUSH_CARVEOUT");
-            if (!(cv && cv[0] == '0'))
+            if (env_tristate("SMVP_PUSH_CARVEOUT") != -1)
                 SMVP_CUDA(cudaFuncSetAttribute(push_tma_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
                                                (int)cudaSharedmemCarveoutMaxShared));
             configured_dev = dev;

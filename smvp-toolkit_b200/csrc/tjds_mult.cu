@@ -24,39 +24,8 @@
 namespace smvp
 {
 
-// SMVP_TJDS_STREAM=1 reads the matrix streams with ld.global.nc.L1::no_allocate; measured on B200 it LOSES to
-// plain __ldg (atomic 3.19 vs 3.12 ms, deterministic 4.12 vs 3.83 ms on the 369^3 stencil), so it stays off
-#ifndef SMVP_TJDS_STREAM
-#define SMVP_TJDS_STREAM 0
-#endif
-__device__ __forceinline__ int32_t ld_stream_i32(const int32_t *p)
-{
-#if SMVP_TJDS_STREAM == 2
-    int32_t v; // L2 fetches the whole 256-byte block the load falls into: a sequential stream finds its next lines in L2
-    asm volatile("ld.global.nc.L2::256B.s32 %0, [%1];" : "=r"(v) : "l"(p));
-    return v;
-#elif SMVP_TJDS_STREAM
-    int32_t v;
-    asm volatile("ld.global.nc.L1::no_allocate.s32 %0, [%1];" : "=r"(v) : "l"(p));
-    return v;
-#else
-    return __ldg(p);
-#endif
-}
-__device__ __forceinline__ double ld_stream_f64(const double *p)
-{
-#if SMVP_TJDS_STREAM == 2
-    double v;
-    asm volatile("ld.global.nc.L2::256B.f64 %0, [%1];" : "=d"(v) : "l"(p));
-    return v;
-#elif SMVP_TJDS_STREAM
-    double v;
-    asm volatile("ld.global.nc.L1::no_allocate.f64 %0, [%1];" : "=d"(v) : "l"(p));
-    return v;
-#else
-    return __ldg(p);
-#endif
-}
+// The matrix streams are read with plain __ldg.  Measured on B200 and removed: ld.global.nc.L1::no_allocate streams
+// lose (atomic 3.19 vs 3.12 ms, deterministic 4.12 vs 3.83 ms on the 369^3 stencil); ld.global.nc.L2::256B changed nothing.
 
 constexpr int32_t EXP_LOW_NONE = 0x7fffffff;  // "no row bound seen" for the running minimum
 constexpr int32_t EXP_NONFINITE = 0x40000000; // "an Inf or NaN was seen": above every real exponent
@@ -207,8 +176,8 @@ __global__ void __launch_bounds__(256) tjds_atomic_kernel(const int2 *__restrict
                 if ((uint32_t)q < (uint32_t)(s_sp[i + 1] - sp))
                 {
                     const int32_t j = sp + q;
-                    r[u] = ld_stream_i32(row_ind + j);
-                    v[u] = ld_stream_f64(val + j);
+                    r[u] = __ldg(row_ind + j);
+                    v[u] = __ldg(val + j);
                     if (SKEW)
                         xv[u] = __ldg(x_perm + q);
                 }
@@ -460,8 +429,8 @@ __global__ void __launch_bounds__(256, MINB) tjds_det_kernel(const int2 *__restr
             const int32_t sp = s_sp[i], q = SKEW ? q0 - i : q0;
             const bool live = (uint32_t)q < (uint32_t)(s_sp[i + 1] - sp);
             const int32_t j = live ? sp + q : 0;
-            r[u] = ld_stream_i32(row_ind + j);
-            v[u] = ld_stream_f64(val + j);
+            r[u] = __ldg(row_ind + j);
+            v[u] = __ldg(val + j);
             xv[u] = SKEW ? __ldg(x_perm + (live ? q : 0)) : xq;
             if (!live)
                 r[u] = -1;
@@ -598,8 +567,8 @@ __global__ void __launch_bounds__(256) tjds_transpose_kernel(const int2 *__restr
         {
             const int32_t i = i0 + u, sp = s_sp[i];
             const bool live = q < s_sp[i + 1] - sp;
-            r[u] = live ? ld_stream_i32(row_ind + sp + q) : -1;
-            v[u] = live ? ld_stream_f64(val + sp + q) : 0.0;
+            r[u] = live ? __ldg(row_ind + sp + q) : -1;
+            v[u] = live ? __ldg(val + sp + q) : 0.0;
         }
 #pragma unroll
         for (int u = 0; u < TJDS_TR_UNROLL; u++)
@@ -680,12 +649,6 @@ __global__ void __launch_bounds__(256) tjds_transpose_count_kernel(const int32_t
 
 // the row indices the kernels scatter through: the relabelled copy when that plan is in use (relabel.cu)
 static inline const int32_t *mult_rows(const smvp_tjds *A) { return A->relabel_state == 1 ? A->row_rel : A->row_ind; }
-
-static int env_tristate(const char *name)
-{
-    const char *env = getenv(name);
-    return (env && env[0] == '1') ? 1 : (env && env[0] == '0') ? -1 : 0;
-}
 
 // decides the walk (once per handle) and builds the block table for it.  Synchronous.
 static int tjds_plan(smvp_tjds *A, cudaStream_t s)
@@ -816,7 +779,7 @@ static int tjds_det_route(smvp_tjds *A)
         const int32_t lo_r = A->det_flags[2];
         A->det_fast = (ok && !(A->det_flags[0] & 2) && ex != EXP_NONE && er != EXP_NONE && lo_r != EXP_LOW_NONE &&
                        (int64_t)lo_r + ex >= TJDS_FRAC - 1023 && (int64_t)er + ex <= TJDS_FRAC - TJDS_W + 1022 &&
-                       getenv("SMVP_TJDS_DET_GENERAL") == nullptr)
+                       !env_set("SMVP_TJDS_DET_GENERAL"))
                           ? 1
                           : -1;
     }
@@ -1022,37 +985,24 @@ static int tjds_pass(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit,
             SMVP_CUDA(cudaMemsetAsync(A->acc + (size_t)w * (size_t)A->rows + r_lo, 0, sizeof(long long) * (size_t)(r_hi - r_lo), s));
         if (blocks > 0 && lim > 0)
         {
-#define SMVP_DET_LAUNCH(U, SK, FA, MB, MB1)                                                                                       \
-    do                                                                                                                            \
-    {                                                                                                                             \
-        if (words == 2)                                                                                                           \
-            SMVP_LAUNCH((tjds_det_kernel<U, SK, FA, MB, 2>), blocks, 256, 0, s, SMVP_TJDS_ARGS_COMMON, (const int32_t *)A->row_exp, \
-                        (const int32_t *)A->x_exp, (unsigned long long *)A->acc, A->rows, A->nslots, lim);                         \
-        else                                                                                                                      \
-            SMVP_LAUNCH((tjds_det_kernel<U, SK, FA, MB1, 1>), blocks, 256, 0, s, SMVP_TJDS_ARGS_COMMON, (const int32_t *)A->row_exp, \
-                        (const int32_t *)A->x_exp, (unsigned long long *)A->acc, A->rows, A->nslots, lim);                         \
-    } while (0)
-            const char *ce = getenv("SMVP_TJDS_DET_CFG"); // tuning hook
-            const int cfg = ce && ce[0] ? atoi(ce) : 0;
-            const bool fast = A->det_fast == 1;
-            // CTAs per SM: 6 for the two-word kernel (40 registers).  The one-word kernel runs at 8 (32 registers, at the
-            // price of ONE 4-byte spill outside the loop): 3.0 - 3.1 ms against 3.85 ms at 6 CTAs without the spill
-            // (profiles/r02_logs/r02_tjds_sweep5.log) -- the kernel is latency-bound, residency wins.
-            if (skew && fast)
-            {
-                if (cfg == 1)
-                    SMVP_DET_LAUNCH(3, true, true, 8, 8);
-                else if (cfg == 2)
-                    SMVP_DET_LAUNCH(4, true, true, 6, 6);
-                else
-                    SMVP_DET_LAUNCH(4, true, true, 6, 8);
-            }
-            else if (skew)
-                SMVP_DET_LAUNCH(4, true, false, 6, 6);
-            else if (fast)
-                SMVP_DET_LAUNCH(4, false, true, 6, 6);
-            else
-                SMVP_DET_LAUNCH(4, false, false, 6, 6);
+            // CTAs per SM: 6 for the two-word kernel (40 registers).  The one-word kernel of the skewed fast walk runs at 8
+            // (32 registers, at the price of ONE 4-byte spill outside the loop): 3.0 - 3.1 ms against 3.85 ms at 6 CTAs
+            // without the spill (profiles/r02_logs/r02_tjds_sweep5.log) -- the kernel is latency-bound, residency wins.
+            // The other swept configurations are in DESIGN.md §5.3.
+            with_flag(skew, [&](auto SK) {
+                return with_flag(A->det_fast == 1, [&](auto FA) {
+                    constexpr bool SKEW = decltype(SK)::value, FAST = decltype(FA)::value;
+                    if (words == 2)
+                        SMVP_LAUNCH((tjds_det_kernel<4, SKEW, FAST, 6, 2>), blocks, 256, 0, s, SMVP_TJDS_ARGS_COMMON,
+                                    (const int32_t *)A->row_exp, (const int32_t *)A->x_exp, (unsigned long long *)A->acc, A->rows,
+                                    A->nslots, lim);
+                    else
+                        SMVP_LAUNCH((tjds_det_kernel<4, SKEW, FAST, SKEW && FAST ? 8 : 6, 1>), blocks, 256, 0, s,
+                                    SMVP_TJDS_ARGS_COMMON, (const int32_t *)A->row_exp, (const int32_t *)A->x_exp,
+                                    (unsigned long long *)A->acc, A->rows, A->nslots, lim);
+                    return (int)SMVP_OK;
+                });
+            });
         }
         SMVP_LAUNCH(tjds_det_finalize_kernel, (unsigned)ceil_div64(A->rows, 256), 256, 0, s, (const long long *)A->acc,
                     (const int32_t *)A->row_exp, (const int32_t *)A->x_exp, A->rows, d_y,
@@ -1095,7 +1045,7 @@ extern "C" int smvp_tjds_mult(smvp_tjds *A, const double *x_host, double *y_host
     // reference keeps its vectorInit outside, main-cli.c:1008): conservative.
     const bool small = (int64_t)A->rows + A->cols + A->nnz < SMVP_SMALL_LOOP_ITEMS;
     const bool tiny = variant == SMVP_TJDS_ATOMIC && A->relabel_state != 1 && A->nnz <= 16384 && A->rows <= 4096 && A->cols <= 4096 &&
-                      getenv("SMVP_NO_TINY_LOOP") == nullptr;
+                      !env_set("SMVP_NO_TINY_LOOP");
     std::function<int(cudaStream_t, int)> multi;
     if (tiny)
         multi = [&](cudaStream_t s, int n) {

@@ -1,8 +1,7 @@
 #!/usr/bin/env python3
 """A/B of the popularity relabelling (relabel.cu) on an R-MAT matrix (GPU box):
-    python tools/sweep_rmat.py --scale 26 --cfgs 4,1,6,5 [--steps 10]
-Builds the same CSR twice (SMVP_CSR_RELABEL=0 / 1), times the merge-path configurations and the vector kernel on
-both with x declared once (smvp_csr_set_x_device), times the x permutation itself, and checks that the relabelled
+    python tools/sweep_rmat.py --scale 26 [--steps 10]
+Builds the same CSR twice (SMVP_CSR_RELABEL=0 / 1), times the merge-path and the vector kernel on both with x declared once (smvp_csr_set_x_device), times the x permutation itself, and checks that the relabelled
 y is bit-identical to the plain y."""
 import argparse
 import os
@@ -32,7 +31,6 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--scale", type=int, default=26)
     ap.add_argument("--edge-factor", type=int, default=16)
-    ap.add_argument("--cfgs", default="4,1,6,5")
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--modes", default="0,1")
     ap.add_argument("--hints", default="off,8192x4194304,0x4194304,8192x0,65536x8388608")
@@ -48,7 +46,7 @@ def main():
     x = torch.empty(N, dtype=torch.float64, device="cuda")
     eng.synth_vector(x, N, 999)
     y = torch.empty(M, dtype=torch.float64, device="cuda")
-    y_plain = {}
+    y_plain = None
     for mode in args.modes.split(","):
         os.environ["SMVP_CSR_RELABEL"] = mode
         A = eng.CsrMatrix.build_device(r, c, v, M, N, nnz)
@@ -61,21 +59,18 @@ def main():
             elif hint:
                 os.environ["SMVP_RANKED_HINTS"] = "1"
                 os.environ["SMVP_HOT_L1"], os.environ["SMVP_HOT_L2"] = hint.split("x")
-            for cfg in [int(t) for t in args.cfgs.split(",")]:
-              for pmb in (args.persist.split(",") if mode != "0" else ["0"]):
-                os.environ["SMVP_MERGE_CFG"] = str(cfg)
+            for pmb in (args.persist.split(",") if mode != "0" else ["0"]):
                 os.environ["SMVP_L2_PERSIST_MB"] = pmb
                 y.fill_(float("nan"))
                 ms = timeit(lambda: A.mult_device(None, y, eng.CSR_MERGE), args.steps)
                 tag = ""
                 if mode == "0":
-                    y_plain[cfg] = y.clone()
-                elif cfg in y_plain:
-                    tag = "bit-identical" if torch.equal(y, y_plain[cfg]) else "DIFFERS from plain"
-                print("  hints %-16s persist %3s MB merge cfg %d: %8.3f ms  %8.1f GB/s  %s" % (hint, pmb, cfg, ms, nbytes / ms / 1e6, tag),
-                      flush=True)
+                    y_plain = y.clone()
+                elif y_plain is not None:
+                    tag = "bit-identical" if torch.equal(y, y_plain) else "DIFFERS from plain"
+                print("  hints %-16s persist %3s MB merge: %8.3f ms  %8.1f GB/s  %s" % (hint, pmb, ms, nbytes / ms / 1e6, tag), flush=True)
         os.environ.pop("SMVP_L2_PERSIST_MB", None)
-        for k in ("SMVP_MERGE_CFG", "SMVP_RANKED_HINTS", "SMVP_HOT_L1", "SMVP_HOT_L2"):
+        for k in ("SMVP_RANKED_HINTS", "SMVP_HOT_L1", "SMVP_HOT_L2"):
             os.environ.pop(k, None)
         if not args.no_vector:
             ms = timeit(lambda: A.mult_device(None, y, eng.CSR_VECTOR), args.steps)

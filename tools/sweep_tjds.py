@@ -31,7 +31,6 @@ def main():
     ap.add_argument("--grid", type=int, default=369)
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--modes", default="0,1,auto")
-    ap.add_argument("--det-cfgs", default="", help="comma list of SMVP_TJDS_DET_CFG values timed on each handle")
     args = ap.parse_args()
     g = args.grid
     m = n = g ** 3
@@ -70,13 +69,6 @@ def main():
                     tag += ", vs first walk " + ("bit-identical" if torch.equal(y, det_keep[variant]) else "DIFFERS")
             print("skew=%-4s plan=%s ndiag=%d  %-13s: %8.3f ms  %8.1f GB/s  %s" %
                   (mode, T.plan(), T.ndiag, name, ms, nbytes / ms / 1e6, tag), flush=True)
-        for cfg in [c for c in args.det_cfgs.split(",") if c]:
-            os.environ["SMVP_TJDS_DET_CFG"] = cfg
-            ms = timeit(lambda: T.mult_device(y, eng.TJDS_DETERMINISTIC_FAST), args.steps)
-            ok = eng.TJDS_DETERMINISTIC_FAST in det_keep and torch.equal(y, det_keep[eng.TJDS_DETERMINISTIC_FAST])
-            print("skew=%-4s det cfg %s: %8.3f ms  %8.1f GB/s  %s" % (mode, cfg, ms, nbytes / ms / 1e6,
-                                                                    "bit-identical" if ok else "DIFFERS"), flush=True)
-        os.environ.pop("SMVP_TJDS_DET_CFG", None)
         T.free()
 
 
