@@ -173,6 +173,38 @@ int smvp_tjds_mult_transpose_device(smvp_tjds *A, const double *d_x, double *d_y
  * to the device once and y back once per call; ms_each as there, exact or batched for small matrices)             */
 int smvp_tjds_mult_transpose(smvp_tjds *A, const double *x_host, double *y_host, int iters, double *ms_each);
 
+/* ---- scaled, accumulating multiply y = alpha * A x + beta * y (and alpha * A^T x + beta * y): the update Krylov solvers
+ * repeat -- a residual r = b - A x is alpha = -1, beta = 1 with y = b; LSQR's u <- A v - a u and v <- A^T u - b v.  The
+ * update is fused into the store of the multiply: one read of y instead of a temporary and a second vector pass.
+ *
+ * For every row r let s_r be what the plain call (same handle, variant, plan and diag_limit) stores into y[r], bit for
+ * bit.  These calls store
+ *     beta != 0:  y[r] = fl( fl(alpha * s_r) + fl(beta * y[r]) )   (each product and the sum rounded separately, no FMA)
+ *     beta == 0:  y[r] = fl(alpha * s_r), and y is NEVER READ (uninitialised or NaN-filled y is fine, as in BLAS; -0.0
+ *                 counts as 0)
+ * alpha = 0 does not skip the matrix: the formula holds as written, so an Inf or NaN in A x still propagates.
+ * alpha = 1, beta = 0 is the plain call: the same kernels and launches, the same bits.
+ * Exceptions, both inherited from the plain pass:
+ *   - a CSR handle with the hot / cold split (smvp_csr_info_t.x_split = 1) runs the hot pass with (alpha, beta) and then
+ *     the cold pass with (alpha, 1): within 1e-12 normwise, not bit-identical, like the split's plain pass;
+ *   - SMVP_TJDS_ATOMIC (and the deterministic variants routed to it, det_route = -1): s_r is the atomic pass's value,
+ *     which is not reproducible run to run.  The deterministic variants are bit-exact.
+ * Aliasing: d_y may not be the x the kernels read -- for CSR d_x, or the x of smvp_csr_set_x_device when d_x == NULL;
+ * for the TJDS transposed call d_x.  Those calls return SMVP_E_ARG; a partial overlap is undefined.  TJDS A x reads the
+ * handle's own permuted copy of x, so there d_y may be the caller's x.
+ * Device vectors only, asynchronous on `stream`.  As with the plain calls, the first call on a handle may synchronise
+ * (plans, scratch); later calls only enqueue work and can be captured in a CUDA graph.  Launches per pass: those of the
+ * plain call, except SMVP_TJDS_ATOMIC on a handle with y_relabel = -1, which takes one more (its sums land in a scratch
+ * of `rows` doubles, allocated at the first such call and counted in device_bytes, and a per-row pass applies the
+ * formula).  A TJDS handle without entries: the transposed call stores fl(alpha * 0) + fl(beta * y) with one launch.
+ * Bytes added to a pass: 8 * rows (the read of y) when beta != 0; TJDS atomic in natural order 16 * rows more.       */
+int smvp_csr_mult_device_axpby(smvp_csr *A, double alpha, const double *d_x, double beta, double *d_y, int variant,
+                               void *stream); /* d_x == NULL: the x of smvp_csr_set_x_device */
+int smvp_tjds_mult_device_axpby(smvp_tjds *A, double alpha, double beta, double *d_y, int variant, int32_t diag_limit,
+                                void *stream); /* the x of smvp_tjds_set_x_device, as smvp_tjds_mult_device */
+int smvp_tjds_mult_transpose_device_axpby(smvp_tjds *A, double alpha, const double *d_x, double beta, double *d_y,
+                                          void *stream); /* d_x: rows entries, d_y: cols */
+
 /* ---- introspection ---- */
 typedef struct smvp_csr_info_t
 {

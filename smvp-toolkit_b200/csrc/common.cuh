@@ -54,6 +54,19 @@ static inline int with_flag(bool b, F &&f)
     return b ? f(std::true_type()) : f(std::false_type());
 }
 
+// The store of the scaled, accumulating multiply y = alpha * A x + beta * y (the *_axpby entry points): s is what the plain
+// pass stores for the row, y0 the row's old value.  Products and the sum are rounded separately (no FMA).  beta == 0:
+// fl(alpha * s) and y0 is not used -- callers then never load it.
+struct Axpby
+{
+    double alpha, beta;
+    bool plain() const { return alpha == 1.0 && beta == 0.0; } // fl(1 * s) = s: the plain kernels store exactly this
+};
+__device__ __forceinline__ double axpby(double alpha, double s, double beta, double y0)
+{
+    return beta != 0.0 ? __dadd_rn(__dmul_rn(alpha, s), __dmul_rn(beta, y0)) : __dmul_rn(alpha, s);
+}
+
 // ---------------------------------------------------------------- environment (api.cu)
 // The library's only reader of the environment: every SMVP_* switch goes through these (table in INTEGRATION.md).
 const char *env_str(const char *name);                   // the value; NULL when unset or empty
@@ -259,6 +272,7 @@ struct smvp_tjds
     int32_t *row_rel;        // [nnz]  rank of row_ind[j]; what the kernels scatter through when in use
     int32_t *row_rank;       // [rows] rank of row r
     double *y_rel;           // [rows] y in rank order (atomic variant)
+    double *y_sum;           // [rows] atomic sums of a natural-order handle under the epilogue (*_axpby), built at first use
     // transposed product y = A^T x (tjds_mult.cu), scratch built at its first call.  Columns longer than TJDS_SEG
     // (slots [0, tr_nlong)) are summed per segment into tr_part, then combined; tr_nwide of them are longer than
     // TJDS_SEG^2 entries and are combined by a whole warp.

@@ -142,29 +142,45 @@ struct YFan
     double *p[SMVP_MAX_FANOUT];
     int n;
 };
-// accum != 0 (second pass of a hot / cold split, never with a fan-out): y[row] += v.  Every row has exactly one writer in
-// a pass (the lane that ends it, or the fix-up kernel for rows cut by tile boundaries), so the read-modify-write is safe.
-template <bool FANOUT>
-__device__ __forceinline__ void store_y_acc(double *__restrict__ y, const YFan &fan, int64_t row, double v, int32_t accum)
+// EPI (the *_axpby calls and the second pass of a hot / cold split, never with a fan-out): y[row] = alpha * v + beta *
+// y[row] (axpby, common.cuh).  Every row has exactly one writer in a pass (the lane that ends it, or the fix-up kernel for
+// rows cut by tile boundaries), so the read-modify-write is safe.
+template <bool FANOUT, bool EPI>
+__device__ __forceinline__ void store_y(double *__restrict__ y, const YFan &fan, int64_t row, double v, double alpha, double beta)
 {
+    static_assert(!(FANOUT && EPI), "the epilogue is not instantiated with the fan-out");
     if (FANOUT)
     {
         for (int k = 0; k < fan.n; k++)
             fan.p[k][row] = v;
     }
+    else if (EPI)
+        y[row] = axpby(alpha, v, beta, beta != 0.0 ? y[row] : 0.0);
     else
-        y[row] = accum ? __dadd_rn(y[row], v) : v;
+        y[row] = v;
 }
+// y[r] for the epilogue, loaded ahead of its store: through the coherent path (y is written by the same kernel) and
+// issued where it stands (volatile: not sunk to its use)
+__device__ __forceinline__ double ld_y_early(const double *p)
+{
+    double v;
+    asm volatile("ld.global.f64 %0, [%1];" : "=d"(v) : "l"(p));
+    return v;
+}
+// the instantiations the launchers name: the epilogue exists only without the fan-out
+template <bool FANOUT, bool EPI>
+constexpr bool kernel_exists() { return !(FANOUT && EPI); }
 
 // =====================================================================================  VECTOR
 // LPR >= 16 (WIDE): each lane pulls 4 consecutive entries per step with 128-bit loads (long rows).
 // LPR < 16: lane l takes entries l, l+LPR, ... with 8/4-byte loads (short rows).  With only a few rows per warp
 //           the lanes of one request then sit on consecutive entries of consecutive rows, so the x gather of a
 //           banded matrix touches far fewer sectors per request -- the vector kernel is L1-bound on such rows.
-template <int LPR, bool FANOUT>
+template <int LPR, bool FANOUT, bool EPI>
 __global__ void __launch_bounds__(256) csr_vector_kernel(const int32_t *__restrict__ row_ptr, const int32_t *__restrict__ col_ind,
                                                          const double *__restrict__ val, const double *__restrict__ x,
-                                                         double *__restrict__ y, int32_t rows, const __grid_constant__ YFan fan)
+                                                         double *__restrict__ y, int32_t rows, const __grid_constant__ YFan fan,
+                                                         double alpha, double beta)
 {
     constexpr bool WIDE = LPR >= 16;
     const int64_t gt = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -220,7 +236,7 @@ __global__ void __launch_bounds__(256) csr_vector_kernel(const int32_t *__restri
     for (int o = LPR / 2; o > 0; o >>= 1)
         sum = __dadd_rn(sum, __shfl_xor_sync(0xffffffffu, sum, o));
     if (row < rows && lane == 0)
-        store_y_acc<FANOUT>(y, fan, row, sum, 0);
+        store_y<FANOUT, EPI>(y, fan, row, sum, alpha, beta);
 }
 
 // =====================================================================================  TINY LOOP
@@ -264,35 +280,43 @@ __global__ void __launch_bounds__(TINY_THREADS) csr_tiny_loop_kernel(const int32
 static inline const int32_t *mult_cols(const smvp_csr *A) { return A->relabel_state == 1 ? A->col_rel : A->col_ind; }
 
 template <int LPR>
-static int launch_vector(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, cudaStream_t s)
+static int launch_vector(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, const Axpby &ab, cudaStream_t s)
 {
     const int64_t threads = (int64_t)A->rows * LPR;
     const int64_t blocks = ceil_div64(threads, 256);
     if (blocks > 0x7fffffffLL)
         return SMVP_E_TOOBIG;
     if (blocks > 0)
-        with_flag(fan != nullptr, [&](auto F) {
-            SMVP_LAUNCH((csr_vector_kernel<LPR, decltype(F)::value>), (unsigned)blocks, 256, 0, s, A->row_ptr, mult_cols(A), A->val,
-                        d_x, d_y, A->rows, fan ? *fan : YFan());
-            return SMVP_OK;
+        return with_flag(fan != nullptr, [&](auto F) {
+            return with_flag(!ab.plain(), [&](auto E) {
+                constexpr bool FANOUT = decltype(F)::value, EPI = decltype(E)::value;
+                if constexpr (!kernel_exists<FANOUT, EPI>())
+                    return (int)SMVP_E_ARG;
+                else
+                {
+                    SMVP_LAUNCH((csr_vector_kernel<LPR, FANOUT, EPI>), (unsigned)blocks, 256, 0, s, A->row_ptr, mult_cols(A), A->val,
+                                d_x, d_y, A->rows, fan ? *fan : YFan(), ab.alpha, ab.beta);
+                    return (int)SMVP_OK;
+                }
+            });
         });
     return SMVP_OK;
 }
 
-static int csr_mult_vector(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, cudaStream_t s)
+static int csr_mult_vector(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, const Axpby &ab, cudaStream_t s)
 {
     const double mean = A->rows > 0 ? (double)A->nnz / A->rows : 0.0;
     int rc;
     if (mean <= 8.0)
-        rc = launch_vector<2>(A, d_x, d_y, fan, s);
+        rc = launch_vector<2>(A, d_x, d_y, fan, ab, s);
     else if (mean <= 16.0)
-        rc = launch_vector<4>(A, d_x, d_y, fan, s);
+        rc = launch_vector<4>(A, d_x, d_y, fan, ab, s);
     else if (mean <= 32.0)
-        rc = launch_vector<8>(A, d_x, d_y, fan, s);
+        rc = launch_vector<8>(A, d_x, d_y, fan, ab, s);
     else if (mean <= 64.0)
-        rc = launch_vector<16>(A, d_x, d_y, fan, s);
+        rc = launch_vector<16>(A, d_x, d_y, fan, ab, s);
     else
-        rc = launch_vector<32>(A, d_x, d_y, fan, s);
+        rc = launch_vector<32>(A, d_x, d_y, fan, ab, s);
     return rc;
 }
 
@@ -368,10 +392,10 @@ __device__ __forceinline__ TileView make_tile(int32_t r0, int32_t r1, int32_t t,
 
 // First row of a tile that ends a row there: y[row] = (carries of the tiles the row crossed, in tile order) + (partial
 // of the tile where it ends).  tile_row[u+1] is the row tile u's carry belongs to.
-template <bool FANOUT>
+template <bool FANOUT, bool EPI>
 __device__ __forceinline__ void merge_fixup_tile(int32_t t, const int32_t *__restrict__ tile_row, const double *__restrict__ head_val,
                                                  const double *__restrict__ carry_val, double *__restrict__ y, const YFan &fan,
-                                                 int32_t accum)
+                                                 double alpha, double beta)
 {
     // everything the common case needs is loaded up front (independent loads: one memory round trip)
     const int32_t r = tile_row[t];
@@ -398,7 +422,7 @@ __device__ __forceinline__ void merge_fixup_tile(int32_t t, const int32_t *__res
             acc = __dadd_rn(acc, __ldcg(carry_val + k));
         acc = __dadd_rn(acc, h);
     }
-    store_y_acc<FANOUT>(y, fan, r, acc, accum);
+    store_y<FANOUT, EPI>(y, fan, r, acc, alpha, beta);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -407,13 +431,13 @@ __device__ __forceinline__ void merge_fixup_tile(int32_t t, const int32_t *__res
 // never meets a block-wide barrier: warps of a CTA drift apart freely, so while one waits for HBM
 // or for its x gathers the others walk.  Rows cut by lane boundaries are stitched with a segmented
 // warp scan (__shfl_up_sync), rows cut by tile boundaries by the fix-up kernel -- fixed order, no atomics.
-template <int WARPS, int IPT, int MINB, bool FANOUT, bool RANKED, bool UNI>
+template <int WARPS, int IPT, int MINB, bool FANOUT, bool RANKED, bool UNI, bool EPI>
 __global__ void __launch_bounds__(WARPS * 32, MINB)
     csr_merge_warp_kernel(const int32_t *__restrict__ row_ptr, const int32_t *__restrict__ col_ind, const double *__restrict__ val,
                           const double *__restrict__ x, double *__restrict__ y, const int32_t *__restrict__ tile_row, int32_t rows,
                           int64_t nnz, int32_t tile_begin, int32_t num_tiles, double *__restrict__ head_val,
                           double *__restrict__ carry_val, const __grid_constant__ YFan fan, int32_t hot_l1, int32_t hot_l2,
-                          int32_t early_dependents, int32_t accum)
+                          int32_t early_dependents, double alpha, double beta)
 {
     // Small grids (early_dependents != 0): let the fix-up kernel, launched with programmatic stream serialization, be
     // scheduled NOW; it parks at griddepcontrol.wait until this grid has completed and flushed.  In the batched `-n` loop
@@ -563,6 +587,11 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
         // waits for each load before issuing the next), then the products.  (Pinning the lane's two shared-window bases
         // in registers with an opaque move saves an address instruction per load but makes the 14-item configurations
         // spill; the nested "live slot / row end" walk this one replaced is in profiles/r01_logs/diet_bisect.log.)
+        // EPI: y of my first row end (tile row i0; row 0 of the tile is the fix-up kernel's), loaded before the gathers so
+        // that its latency hides behind them; further row ends of the lane (short rows) load y at their store
+        double y_first = 0.0;
+        if (EPI && beta != 0.0 && i0 < i_next && i0 != 0)
+            y_first = ld_y_early(y + (int64_t)tile_r0 + i0);
         double prod[IPT];
         {
             int32_t cq[IPT];
@@ -607,7 +636,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
                             first_sum = sum;
                         }
                         else
-                            store_y_acc<FANOUT>(y, fan, (int64_t)tile_r0 + row, sum, accum);
+                            store_y<FANOUT, EPI>(y, fan, (int64_t)tile_r0 + row, sum, alpha, beta);
                         sum = 0.0;
                         row++;
                         until = (row < i_next ? row_end(row) : 0x7fffffff) - j0;
@@ -625,7 +654,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
                     first_sum = sum;
                 }
                 else
-                    store_y_acc<FANOUT>(y, fan, (int64_t)tile_r0 + row, sum, accum);
+                    store_y<FANOUT, EPI>(y, fan, (int64_t)tile_r0 + row, sum, alpha, beta);
                 sum = 0.0;
                 row++;
             }
@@ -661,12 +690,15 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
             if (lane > 0 && prev_key == i0)
                 first_sum = __dadd_rn(prev_scan, first_sum);
             // the tile's first row may have started in earlier tiles: its partial goes to the fix-up
-            // kernel, which adds the carries and writes y.  y itself is only ever WRITTEN here (never
-            // read), so it may be a write-only mapping such as an NVSwitch multicast address.
+            // kernel, which adds the carries and writes y -- and, under the epilogue, is the only one to read that
+            // row of y.  Without the epilogue y is only ever WRITTEN here (never read), so it may be a write-only
+            // mapping such as an NVSwitch multicast address.
             if (i0 == 0)
                 head_val[t] = first_sum;
+            else if (EPI)
+                y[(int64_t)tile_r0 + i0] = axpby(alpha, first_sum, beta, y_first);
             else
-                store_y_acc<FANOUT>(y, fan, (int64_t)tile_r0 + i0, first_sum, accum);
+                store_y<FANOUT, false>(y, fan, (int64_t)tile_r0 + i0, first_sum, alpha, beta);
         }
         if (lane == 31)
             carry_val[t] = scan; // partial of the row that continues into the next tile
@@ -676,17 +708,17 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
     }
 }
 
-template <bool FANOUT>
+template <bool FANOUT, bool EPI>
 __global__ void __launch_bounds__(256) merge_fixup_kernel(const int32_t *__restrict__ tile_row, const double *__restrict__ head_val,
                                                           const double *__restrict__ carry_val, int32_t tile_begin,
                                                           int32_t num_tiles, double *__restrict__ y,
-                                                          const __grid_constant__ YFan fan, int32_t accum)
+                                                          const __grid_constant__ YFan fan, double alpha, double beta)
 {
     // no-op unless launched with programmatic stream serialization: then it waits here for the merge kernel's results
     asm volatile("griddepcontrol.wait;" ::: "memory");
     const int32_t t = tile_begin + blockIdx.x * blockDim.x + threadIdx.x;
     if (t < num_tiles)
-        merge_fixup_tile<FANOUT>(t, tile_row, head_val, carry_val, y, fan, accum);
+        merge_fixup_tile<FANOUT, EPI>(t, tile_row, head_val, carry_val, y, fan, alpha, beta);
 }
 
 // ---- the two instantiations AUTO chooses from (merge_skewed).  Measured on B200 (logs under profiles/, the swept
@@ -777,12 +809,12 @@ static int persistent_grid(K kern, int threads, int smem, int handle_headroom, i
     return SMVP_OK;
 }
 
-template <class C, bool FANOUT, bool RANKED>
-static int launch_wmerge(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fanp, cudaStream_t s, int32_t tile_begin,
-                         int32_t tile_end, int32_t accum)
+template <class C, bool FANOUT, bool RANKED, bool EPI>
+static int launch_wmerge(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fanp, const Axpby &ab, cudaStream_t s,
+                         int32_t tile_begin, int32_t tile_end)
 {
     constexpr int SMEM = C::WARPS * MergeShape<32, C::IPT>::SMEM_BYTES;
-    auto kern = csr_merge_warp_kernel<C::WARPS, C::IPT, C::MINB, FANOUT, RANKED, C::UNI>;
+    auto kern = csr_merge_warp_kernel<C::WARPS, C::IPT, C::MINB, FANOUT, RANKED, C::UNI, EPI>;
     int32_t hot_l1 = 0, hot_l2 = 0;
     if (RANKED)
         hot_limits(&hot_l1, &hot_l2);
@@ -799,7 +831,7 @@ static int launch_wmerge(const smvp_csr *A, const double *d_x, double *d_y, cons
         static thread_local const bool pdl_ok = !env_set("SMVP_NO_PDL"); // SMVP_NO_PDL: no early launch of the fix-up
         const bool early = pdl_ok && ntiles <= MERGE_PDL_TILES;
         SMVP_LAUNCH(kern, (unsigned)grid, C::WARPS * 32, SMEM, s, A->row_ptr, mult_cols(A), A->val, d_x, d_y, A->tile_row, A->rows,
-                    A->nnz, tile_begin, tile_end, A->head_val, A->carry_val, fan, hot_l1, hot_l2, early ? 1 : 0, accum);
+                    A->nnz, tile_begin, tile_end, A->head_val, A->carry_val, fan, hot_l1, hot_l2, early ? 1 : 0, ab.alpha, ab.beta);
         if (early)
         {
             cudaLaunchConfig_t cfg = {};
@@ -812,13 +844,13 @@ static int launch_wmerge(const smvp_csr *A, const double *d_x, double *d_y, cons
             attr[0].val.programmaticStreamSerializationAllowed = 1;
             cfg.attrs = attr;
             cfg.numAttrs = 1;
-            SMVP_CUDA(cudaLaunchKernelEx(&cfg, merge_fixup_kernel<FANOUT>, (const int32_t *)A->tile_row, (const double *)A->head_val,
-                                         (const double *)A->carry_val, tile_begin, tile_end, d_y, fan, accum));
+            SMVP_CUDA(cudaLaunchKernelEx(&cfg, merge_fixup_kernel<FANOUT, EPI>, (const int32_t *)A->tile_row, (const double *)A->head_val,
+                                         (const double *)A->carry_val, tile_begin, tile_end, d_y, fan, ab.alpha, ab.beta));
             ::smvp::g_launches.fetch_add(1, std::memory_order_relaxed);
         }
         else
-            SMVP_LAUNCH(merge_fixup_kernel<FANOUT>, (unsigned)ceil_div64(ntiles, 256), 256, 0, s, (const int32_t *)A->tile_row,
-                        (const double *)A->head_val, (const double *)A->carry_val, tile_begin, tile_end, d_y, fan, accum);
+            SMVP_LAUNCH((merge_fixup_kernel<FANOUT, EPI>), (unsigned)ceil_div64(ntiles, 256), 256, 0, s, (const int32_t *)A->tile_row,
+                        (const double *)A->head_val, (const double *)A->carry_val, tile_begin, tile_end, d_y, fan, ab.alpha, ab.beta);
     }
     return SMVP_OK;
 }
@@ -840,13 +872,14 @@ struct PatternShape
     static int stage_bytes(int maxlen) { return (((ROWS * maxlen + 2) * 8 + 15) / 16 * 16 + ROWS + 32 + 127) & ~127; }
 };
 
-template <int WARPS, int R, int STAGES, int CH, int MINB, bool FANOUT>
+template <int WARPS, int R, int STAGES, int CH, int MINB, bool FANOUT, bool EPI>
 __global__ void __launch_bounds__(WARPS * 32, MINB)
     csr_pattern_kernel(const int32_t *__restrict__ row_ptr, const double *__restrict__ val, const uint8_t *__restrict__ pat_id,
                        const int32_t *__restrict__ pat_off, const int32_t *__restrict__ pat_len, int32_t npat, int32_t maxlen,
                        const double *__restrict__ x, double *__restrict__ y, int32_t row_begin, int32_t row_end,
-                       uint32_t stage_bytes, const __grid_constant__ YFan fan)
+                       uint32_t stage_bytes, const __grid_constant__ YFan fan, double alpha, double beta)
 {
+    static_assert(!EPI || (R == 1 && !FANOUT), "the epilogue keeps one y value per lane: one round per tile");
     constexpr int ROWS = PatternShape<R>::ROWS;
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ __align__(8) uint64_t full_bar[WARPS * STAGES];
@@ -917,6 +950,10 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
         int32_t nn0 = 0, nn1 = 0;
         if (tn < ntiles && tn > t)
             bounds(tn, &nn0, &nn1);
+        // the epilogue's y[r]: issued before the wait for the stage, its latency hides behind the staging and the gathers
+        double y0 = 0.0;
+        if (EPI && beta != 0.0 && row_begin + t * ROWS + lane < row_end)
+            y0 = ld_y_early(y + row_begin + t * ROWS + lane);
 
         mbar_wait(&bars[s], (phase >> s) & 1u);
         phase ^= 1u << s;
@@ -975,7 +1012,12 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
                         sum = __dadd_rn(sum, __dmul_rn(lds_f64(vrow + 8u * (uint32_t)(k0 + q)), xv[q]));
             }
             if (live)
-                store_y_acc<FANOUT>(y, fan, r, sum, 0);
+            {
+                if (EPI)
+                    y[r] = axpby(alpha, sum, beta, y0);
+                else
+                    store_y<FANOUT, false>(y, fan, r, sum, alpha, beta);
+            }
         }
         // the stage is consumed: refill it with tile tn
         __syncwarp();
@@ -1003,8 +1045,8 @@ struct PatternCfg
 };
 
 // rows [row_begin, row_end) of a handle with the row-pattern plan
-static int csr_mult_pattern(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, cudaStream_t s, int32_t row_begin,
-                            int32_t row_end)
+static int csr_mult_pattern(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, const Axpby &ab, cudaStream_t s,
+                            int32_t row_begin, int32_t row_end)
 {
     using C = PatternCfg;
     const int maxlen = A->pattern_maxlen > 0 ? A->pattern_maxlen : 1;
@@ -1013,33 +1055,43 @@ static int csr_mult_pattern(const smvp_csr *A, const double *d_x, double *d_y, c
     const int smem = table + C::WARPS * C::STAGES * stage;
     const int64_t need = ceil_div64(ceil_div64((int64_t)row_end - row_begin, PatternShape<C::R>::ROWS), C::WARPS);
     return with_flag(fan != nullptr, [&](auto F) {
-        auto kern = csr_pattern_kernel<C::WARPS, C::R, C::STAGES, C::CH, C::MINB, decltype(F)::value>;
-        // the shared memory depends on the matrix (longest pattern, pattern count): occupancy is looked up per size
-        static thread_local Residency res;
-        int64_t grid = 0;
-        SMVP_TRY(persistent_grid(kern, C::WARPS * 32, smem, A->merge_headroom, need, res, &grid));
-        if (grid > 0)
-            SMVP_LAUNCH(kern, (unsigned)grid, C::WARPS * 32, smem, s, A->row_ptr, A->val, A->pat_id, A->pat_off, A->pat_len,
-                        A->pattern_count, maxlen, d_x, d_y, row_begin, row_end, (uint32_t)stage, fan ? *fan : YFan());
-        return (int)SMVP_OK;
+        return with_flag(!ab.plain(), [&](auto E) {
+            constexpr bool FANOUT = decltype(F)::value, EPI = decltype(E)::value;
+            if constexpr (!kernel_exists<FANOUT, EPI>())
+                return (int)SMVP_E_ARG;
+            else
+            {
+                auto kern = csr_pattern_kernel<C::WARPS, C::R, C::STAGES, C::CH, C::MINB, FANOUT, EPI>;
+                // the shared memory depends on the matrix (longest pattern, pattern count): occupancy is looked up per size
+                static thread_local Residency res;
+                int64_t grid = 0;
+                SMVP_TRY(persistent_grid(kern, C::WARPS * 32, smem, A->merge_headroom, need, res, &grid));
+                if (grid > 0)
+                    SMVP_LAUNCH(kern, (unsigned)grid, C::WARPS * 32, smem, s, A->row_ptr, A->val, A->pat_id, A->pat_off, A->pat_len,
+                                A->pattern_count, maxlen, d_x, d_y, row_begin, row_end, (uint32_t)stage, fan ? *fan : YFan(),
+                                ab.alpha, ab.beta);
+                return (int)SMVP_OK;
+            }
+        });
     });
 }
 
+constexpr Axpby AXPBY_PLAIN = {1.0, 0.0};
+
 // tiles [tile_begin, tile_end) of the plan; (0, -1) = all
-static int csr_mult_merge(smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, cudaStream_t s, int32_t tile_begin = 0,
-                          int32_t tile_end = -1, int32_t accum = 0)
+static int csr_mult_merge(smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, const Axpby &ab, cudaStream_t s,
+                          int32_t tile_begin = 0, int32_t tile_end = -1)
 {
-    // hot / cold split (relabel.cu): whole passes without a fan-out run as y = hot * x_rel, then y += cold * x_rel
-    if (A->split_state == 1 && !fan && tile_begin == 0 && tile_end < 0 && !accum)
+    // hot / cold split (relabel.cu): whole passes without a fan-out run as y = alpha * hot * x_rel + beta * y, then
+    // y = alpha * cold * x_rel + y (the parts are never split themselves)
+    if (A->split_state == 1 && !fan && tile_begin == 0 && tile_end < 0)
     {
-        SMVP_TRY(csr_mult_merge(A->hot, d_x, d_y, nullptr, s, 0, -1, 0));
-        return csr_mult_merge(A->cold, d_x, d_y, nullptr, s, 0, -1, 1);
+        SMVP_TRY(csr_mult_merge(A->hot, d_x, d_y, nullptr, ab, s));
+        return csr_mult_merge(A->cold, d_x, d_y, nullptr, Axpby{ab.alpha, 1.0}, s);
     }
-    if (accum && fan)
-        return SMVP_E_ARG;
     // the row-pattern plan serves whole passes (the pipelined host call cuts its ranges on rows: csr_mult_pattern)
-    if (A->pattern_state == 1 && tile_begin == 0 && tile_end < 0 && !accum)
-        return csr_mult_pattern(A, d_x, d_y, fan, s, 0, A->rows);
+    if (A->pattern_state == 1 && tile_begin == 0 && tile_end < 0)
+        return csr_mult_pattern(A, d_x, d_y, fan, ab, s, 0, A->rows);
     SMVP_TRY(merge_plan(A, s));
     if (tile_end < 0)
         tile_end = A->merge_tiles;
@@ -1048,9 +1100,14 @@ static int csr_mult_merge(smvp_csr *A, const double *d_x, double *d_y, const YFa
     const bool skewed = merge_skewed(A);
     return with_flag(fan != nullptr, [&](auto F) {
         return with_flag(ranked, [&](auto R) {
-            constexpr bool FANOUT = decltype(F)::value, RANKED = decltype(R)::value;
-            return skewed ? launch_wmerge<MergeSkewed, FANOUT, RANKED>(A, d_x, d_y, fan, s, tile_begin, tile_end, accum)
-                          : launch_wmerge<MergeStencil, FANOUT, RANKED>(A, d_x, d_y, fan, s, tile_begin, tile_end, accum);
+            return with_flag(!ab.plain(), [&](auto E) {
+                constexpr bool FANOUT = decltype(F)::value, RANKED = decltype(R)::value, EPI = decltype(E)::value;
+                if constexpr (!kernel_exists<FANOUT, EPI>())
+                    return (int)SMVP_E_ARG;
+                else
+                    return skewed ? launch_wmerge<MergeSkewed, FANOUT, RANKED, EPI>(A, d_x, d_y, fan, ab, s, tile_begin, tile_end)
+                                  : launch_wmerge<MergeStencil, FANOUT, RANKED, EPI>(A, d_x, d_y, fan, ab, s, tile_begin, tile_end);
+            });
         });
     });
 }
@@ -1072,12 +1129,12 @@ int csr_resolve_variant(const smvp_csr *A, int variant)
 using namespace smvp;
 
 // x is already in the space the kernels index (x itself, or x_rel when the relabelling plan is in use)
-static int csr_mult_launch(smvp_csr *A, const double *x, double *d_y, const YFan *fan, int variant, cudaStream_t s)
+static int csr_mult_launch(smvp_csr *A, const double *x, double *d_y, const YFan *fan, const Axpby &ab, int variant, cudaStream_t s)
 {
     if (A->rows == 0)
         return SMVP_OK;
     const int v = csr_resolve_variant(A, variant);
-    int rc = (v == SMVP_CSR_VECTOR) ? csr_mult_vector(A, x, d_y, fan, s) : csr_mult_merge(A, x, d_y, fan, s);
+    int rc = (v == SMVP_CSR_VECTOR) ? csr_mult_vector(A, x, d_y, fan, ab, s) : csr_mult_merge(A, x, d_y, fan, ab, s);
     if (rc != SMVP_OK)
         return rc;
     SMVP_CUDA(cudaGetLastError());
@@ -1123,7 +1180,7 @@ static int l2_persist_window(cudaStream_t s, const void *base, size_t bytes)
     return SMVP_OK;
 }
 
-static int csr_mult_any(smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, int variant, void *stream)
+static int csr_mult_any(smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, const Axpby &ab, int variant, void *stream)
 {
     if (variant != SMVP_CSR_AUTO && variant != SMVP_CSR_VECTOR && variant != SMVP_CSR_MERGE)
         return SMVP_E_ARG;
@@ -1149,7 +1206,7 @@ static int csr_mult_any(smvp_csr *A, const double *d_x, double *d_y, const YFan 
     const int persist_mb = A->relabel_state == 1 ? env_int("SMVP_L2_PERSIST_MB", 0, 0, 4096) : 0;
     if (persist_mb > 0)
         SMVP_TRY(l2_persist_window(s, x, (size_t)persist_mb << 20));
-    const int rc = csr_mult_launch(A, x, d_y, fan, variant, s);
+    const int rc = csr_mult_launch(A, x, d_y, fan, ab, variant, s);
     if (persist_mb > 0)
         SMVP_TRY(l2_persist_window(s, nullptr, 0));
     return rc;
@@ -1178,7 +1235,17 @@ extern "C" int smvp_csr_mult_device(smvp_csr *A, const double *d_x, double *d_y,
 {
     if (!A || (A->rows > 0 && !d_y))
         return SMVP_E_ARG;
-    return csr_mult_any(A, d_x, d_y, nullptr, variant, stream);
+    return csr_mult_any(A, d_x, d_y, nullptr, AXPBY_PLAIN, variant, stream);
+}
+
+extern "C" int smvp_csr_mult_device_axpby(smvp_csr *A, double alpha, const double *d_x, double beta, double *d_y, int variant,
+                                          void *stream)
+{
+    if (!A || (A->rows > 0 && !d_y))
+        return SMVP_E_ARG;
+    if (d_y && d_y == (d_x ? d_x : A->x_set))
+        return SMVP_E_ARG; // y would be read and written while the kernels gather it as x
+    return csr_mult_any(A, d_x, d_y, nullptr, Axpby{alpha, beta}, variant, stream);
 }
 
 extern "C" int smvp_csr_mult_device_fanout(smvp_csr *A, const double *d_x, double *const *d_y_list, int n_out, int variant,
@@ -1193,7 +1260,7 @@ extern "C" int smvp_csr_mult_device_fanout(smvp_csr *A, const double *d_x, doubl
     for (int k = 0; k < n_out; k++)
         if (A->rows > 0 && !fan.p[k])
             return SMVP_E_ARG;
-    return csr_mult_any(A, d_x, fan.p[0], &fan, variant, stream);
+    return csr_mult_any(A, d_x, fan.p[0], &fan, AXPBY_PLAIN, variant, stream);
 }
 
 // ------------------------------------------------------------------ host-vector entry point
@@ -1522,8 +1589,9 @@ static int csr_mult_pipelined(smvp_csr *A, const double *x_host, double *y_host,
         }
         PIPE_CK(cudaEventRecord(R.t0[c], cs));
         if (A->pipe_tile[c + 1] > A->pipe_tile[c] && e == cudaSuccess)
-            rc = A->pattern_state == 1 ? csr_mult_pattern(A, xm, A->d_y, nullptr, cs, A->pipe_row[c], A->pipe_row[c + 1])
-                                       : csr_mult_merge(A, xm, A->d_y, nullptr, cs, A->pipe_tile[c], A->pipe_tile[c + 1]);
+            rc = A->pattern_state == 1
+                     ? csr_mult_pattern(A, xm, A->d_y, nullptr, AXPBY_PLAIN, cs, A->pipe_row[c], A->pipe_row[c + 1])
+                     : csr_mult_merge(A, xm, A->d_y, nullptr, AXPBY_PLAIN, cs, A->pipe_tile[c], A->pipe_tile[c + 1]);
         PIPE_CK(cudaEventRecord(R.t1[c], cs));
         if (y_host)
         {
@@ -1655,7 +1723,7 @@ extern "C" int smvp_csr_mult(smvp_csr *A, const double *x_host, double *y_host, 
                 return (int)SMVP_OK;
             };
         if (A->rows > 0)
-            rc = timed_loop(iters, ms_each, small, [&](cudaStream_t s) { return csr_mult_launch(A, xm, A->d_y, nullptr, variant, s); },
+            rc = timed_loop(iters, ms_each, small, [&](cudaStream_t s) { return csr_mult_launch(A, xm, A->d_y, nullptr, AXPBY_PLAIN, variant, s); },
                             multi);
         else if (ms_each)
             for (int it = 0; it < iters; it++)
@@ -1683,7 +1751,7 @@ extern "C" int smvp_csr_mult(smvp_csr *A, const double *x_host, double *y_host, 
             else
             {
                 cudaEventRecord(e0, 0);
-                rc = csr_mult_launch(A, xm, A->d_y, nullptr, variant, 0);
+                rc = csr_mult_launch(A, xm, A->d_y, nullptr, AXPBY_PLAIN, variant, 0);
                 cudaEventRecord(e1, 0);
                 if (rc != SMVP_OK)
                     break;

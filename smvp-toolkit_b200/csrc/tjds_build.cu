@@ -106,6 +106,7 @@ void tjds_release(smvp_tjds *A)
     cudaFree(A->tr_part);
     cudaFree(A->d_xt);
     cudaFree(A->d_yt);
+    cudaFree(A->y_sum);
     tjds_relabel_release(A);
     delete A;
 }

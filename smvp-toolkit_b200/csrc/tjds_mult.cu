@@ -487,10 +487,13 @@ __global__ void __launch_bounds__(256, MINB) tjds_det_kernel(const int2 *__restr
         flush();
 }
 
-// row_rank != NULL: the accumulators and row_exp are in popularity-rank order (relabelled handle), y is not
+// row_rank != NULL: the accumulators and row_exp are in popularity-rank order (relabelled handle), y is not.
+// EPI: y[row] = alpha * (row sum) + beta * y[row] (axpby, common.cuh) instead of the row sum.
+template <bool EPI>
 __global__ void __launch_bounds__(256) tjds_det_finalize_kernel(const long long *__restrict__ acc, const int32_t *__restrict__ row_exp,
                                                                 const int32_t *__restrict__ x_exp, int32_t rows, double *__restrict__ y,
-                                                                const int32_t *__restrict__ row_rank, int words, int32_t r_lo, int32_t r_hi)
+                                                                const int32_t *__restrict__ row_rank, int words, int32_t r_lo, int32_t r_hi,
+                                                                double alpha, double beta)
 {
     // accumulators exist (are cleared and filled) only for rows [r_lo, r_hi) of the index space the kernels use
     const int32_t row = blockIdx.x * blockDim.x + threadIdx.x;
@@ -499,7 +502,7 @@ __global__ void __launch_bounds__(256) tjds_det_finalize_kernel(const long long 
     const int32_t r = row_rank ? row_rank[row] : row;
     if (r < r_lo || r >= r_hi)
     {
-        y[row] = 0.0;
+        y[row] = EPI ? axpby(alpha, 0.0, beta, beta != 0.0 ? y[row] : 0.0) : 0.0;
         return;
     }
     longlong2 a;
@@ -513,15 +516,26 @@ __global__ void __launch_bounds__(256) tjds_det_finalize_kernel(const long long 
         const int32_t T = row_exp[r] + *x_exp;
         out = scalbn(s, T - TJDS_FRAC);
     }
-    y[row] = out;
+    y[row] = EPI ? axpby(alpha, out, beta, beta != 0.0 ? y[row] : 0.0) : out;
 }
 
-// y[r] = y_rel[rank[r]]: the atomic variant of a relabelled handle sums in rank order
+// y[r] = y_rel[rank[r]]: the atomic variant of a relabelled handle sums in rank order.  EPI: y[r] = alpha * y_rel[rank[r]]
+// + beta * y[r] (axpby, common.cuh), and row_rank == NULL stands for the identity (the atomic sums of a natural-order
+// handle, which land in a scratch vector under the epilogue).
+template <bool EPI>
 __global__ void __launch_bounds__(256) tjds_unrank_y_kernel(const double *__restrict__ y_rel, const int32_t *__restrict__ row_rank,
-                                                            int32_t rows, double *__restrict__ y)
+                                                            int32_t rows, double *__restrict__ y, double alpha, double beta)
 {
     for (int32_t r = blockIdx.x * blockDim.x + threadIdx.x; r < rows; r += gridDim.x * blockDim.x)
-        y[r] = __ldg(y_rel + __ldg(row_rank + r));
+    {
+        if (EPI)
+        {
+            const double s = __ldg(y_rel + (row_rank ? __ldg(row_rank + r) : r));
+            y[r] = axpby(alpha, s, beta, beta != 0.0 ? y[r] : 0.0);
+        }
+        else
+            y[r] = __ldg(y_rel + __ldg(row_rank + r));
+    }
 }
 
 // ---- transposed product y = A^T x --------------------------------------------------------------------------------
@@ -534,19 +548,25 @@ __global__ void __launch_bounds__(256) tjds_unrank_y_kernel(const double *__rest
 // go to tr_part[tr_seg_off[g] + q] (one coalesced store per warp) and tjds_transpose_combine_kernel adds them in
 // segment order.  The table is walked straight whatever walk A x uses: a skewed table only has extra slots past the
 // end of each segment's first diagonal, and those threads find nothing to do.  row_ind is read, never row_rel.
+// EPI: every store of a column's value s becomes y = alpha * s + beta * y (axpby, common.cuh), empty columns too (s = +0.0).
 constexpr int TJDS_TR_UNROLL = 8; // entries whose loads are issued before the first of them is used
+__device__ __forceinline__ void tr_store(bool epi, double *__restrict__ y, int32_t c, double s, double alpha, double beta)
+{
+    y[c] = epi ? axpby(alpha, s, beta, beta != 0.0 ? y[c] : 0.0) : s;
+}
+template <bool EPI>
 __global__ void __launch_bounds__(256) tjds_transpose_kernel(const int2 *__restrict__ blocks, const int32_t *__restrict__ start_pos,
                                                              const int32_t *__restrict__ row_ind, const double *__restrict__ val,
                                                              const int32_t *__restrict__ perm, const double *__restrict__ x,
                                                              double *__restrict__ y, double *__restrict__ part,
                                                              const uint32_t *__restrict__ seg_off, int32_t ndiag, int32_t nslots,
-                                                             int32_t cols, int32_t nlong)
+                                                             int32_t cols, int32_t nlong, double alpha, double beta)
 {
     static_assert(TJDS_SEG % TJDS_TR_UNROLL == 0, "s_sp holds TJDS_SEG + 1 entries");
     __shared__ int32_t s_sp[TJDS_SEG + 1];
     // empty columns (slots nslots .. cols-1) get +0.0, spread over the whole grid
     for (int64_t p = (int64_t)nslots + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < cols; p += (int64_t)gridDim.x * blockDim.x)
-        y[__ldg(perm + p)] = 0.0;
+        tr_store(EPI, y, __ldg(perm + p), 0.0, alpha, beta);
     const int2 blk = __ldg(blocks + blockIdx.x);
     const int32_t d_begin = blk.x * TJDS_SEG;
     const int32_t nd = min(TJDS_SEG, ndiag - d_begin);
@@ -579,7 +599,7 @@ __global__ void __launch_bounds__(256) tjds_transpose_kernel(const int2 *__restr
                 s = __dadd_rn(s, __dmul_rn(v[u], xv[u]));
     }
     if (q >= nlong)
-        y[__ldg(perm + q)] = s; // a column of at most TJDS_SEG entries lives in segment 0 alone
+        tr_store(EPI, y, __ldg(perm + q), s, alpha, beta); // a column of at most TJDS_SEG entries lives in segment 0 alone
     else
         part[(int64_t)__ldg(seg_off + blk.x) + q] = s;
 }
@@ -589,9 +609,11 @@ __global__ void __launch_bounds__(256) tjds_transpose_kernel(const int2 *__restr
 // round, TJDS_TR_ROUNDS rounds ahead, and every lane adds them in order from shuffles (the additions are the serial
 // part, the loads are not).  Slots [nwide, nlong) take one thread each.
 constexpr int TJDS_TR_ROUNDS = 4;
+template <bool EPI>
 __global__ void __launch_bounds__(256) tjds_transpose_combine_kernel(const double *__restrict__ part, const uint32_t *__restrict__ seg_off,
                                                                      const int32_t *__restrict__ slot_len, const int32_t *__restrict__ perm,
-                                                                     int32_t nlong, int32_t nwide, double *__restrict__ y)
+                                                                     int32_t nlong, int32_t nwide, double *__restrict__ y, double alpha,
+                                                                     double beta)
 {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, wide_threads = (int64_t)nwide * 32;
     if (t < wide_threads)
@@ -620,7 +642,7 @@ __global__ void __launch_bounds__(256) tjds_transpose_combine_kernel(const doubl
                 }
         }
         if (lane == 0)
-            y[__ldg(perm + q)] = s;
+            tr_store(EPI, y, __ldg(perm + q), s, alpha, beta);
         return;
     }
     const int64_t qq = (int64_t)nwide + (t - wide_threads);
@@ -632,7 +654,14 @@ __global__ void __launch_bounds__(256) tjds_transpose_combine_kernel(const doubl
 #pragma unroll 4
     for (int32_t g = 0; g < nch; g++)
         s = __dadd_rn(s, __ldg(part + __ldg(seg_off + g) + q));
-    y[__ldg(perm + q)] = s;
+    tr_store(EPI, y, __ldg(perm + q), s, alpha, beta);
+}
+
+// y = alpha * (+0.0) + beta * y: the scaled, accumulating transposed product of a handle without entries
+__global__ void __launch_bounds__(256) tjds_axpby_empty_kernel(double *__restrict__ y, int32_t n, double alpha, double beta)
+{
+    for (int32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+        y[i] = axpby(alpha, 0.0, beta, beta != 0.0 ? y[i] : 0.0);
 }
 
 // partials segment g holds: the long columns (slots [0, nlong), nlong = length of diagonal TJDS_SEG) in segment 0, the
@@ -833,23 +862,39 @@ static int tjds_transpose_prepare(smvp_tjds *A, cudaStream_t s)
     return SMVP_OK;
 }
 
+constexpr Axpby AXPBY_PLAIN = {1.0, 0.0};
+
 // one transposed pass, asynchronous on s; tjds_transpose_prepare has run and A->cols > 0
-static int tjds_transpose_pass(smvp_tjds *A, const double *d_x, double *d_y, cudaStream_t s)
+static int tjds_transpose_pass(smvp_tjds *A, const double *d_x, double *d_y, const Axpby &ab, cudaStream_t s)
 {
-    if (A->ndiag == 0)
+    const bool epi = !ab.plain();
+    if (A->ndiag == 0) // no entries: every column is empty
     {
-        SMVP_CUDA(cudaMemsetAsync(d_y, 0, sizeof(double) * (size_t)A->cols, s)); // no entries: every column is empty
+        if (!epi)
+            SMVP_CUDA(cudaMemsetAsync(d_y, 0, sizeof(double) * (size_t)A->cols, s));
+        else
+        {
+            int64_t blocks = ceil_div64(A->cols, 256 * 4);
+            const int64_t cap = (int64_t)device_props().sms * 8;
+            SMVP_LAUNCH(tjds_axpby_empty_kernel, (unsigned)(blocks < cap ? blocks : cap), 256, 0, s, d_y, A->cols, ab.alpha, ab.beta);
+            SMVP_CUDA(cudaGetLastError());
+        }
         return SMVP_OK;
     }
-    SMVP_LAUNCH(tjds_transpose_kernel, (unsigned)A->num_seg_blocks, 256, 0, s, (const int2 *)A->seg_blocks, (const int32_t *)A->start_pos,
-                (const int32_t *)A->row_ind, (const double *)A->val, (const int32_t *)A->perm, d_x, d_y, A->tr_part,
-                (const uint32_t *)A->tr_seg_off, A->ndiag, A->nslots, A->cols, A->tr_nlong);
-    if (A->ndiag > TJDS_SEG)
-    {
-        const int64_t threads = 32 * (int64_t)A->tr_nwide + (A->tr_nlong - A->tr_nwide);
-        SMVP_LAUNCH(tjds_transpose_combine_kernel, (unsigned)ceil_div64(threads, 256), 256, 0, s, (const double *)A->tr_part,
-                    (const uint32_t *)A->tr_seg_off, (const int32_t *)A->slot_len, (const int32_t *)A->perm, A->tr_nlong, A->tr_nwide, d_y);
-    }
+    with_flag(epi, [&](auto E) {
+        constexpr bool EPI = decltype(E)::value;
+        SMVP_LAUNCH(tjds_transpose_kernel<EPI>, (unsigned)A->num_seg_blocks, 256, 0, s, (const int2 *)A->seg_blocks,
+                    (const int32_t *)A->start_pos, (const int32_t *)A->row_ind, (const double *)A->val, (const int32_t *)A->perm, d_x, d_y,
+                    A->tr_part, (const uint32_t *)A->tr_seg_off, A->ndiag, A->nslots, A->cols, A->tr_nlong, ab.alpha, ab.beta);
+        if (A->ndiag > TJDS_SEG)
+        {
+            const int64_t threads = 32 * (int64_t)A->tr_nwide + (A->tr_nlong - A->tr_nwide);
+            SMVP_LAUNCH(tjds_transpose_combine_kernel<EPI>, (unsigned)ceil_div64(threads, 256), 256, 0, s, (const double *)A->tr_part,
+                        (const uint32_t *)A->tr_seg_off, (const int32_t *)A->slot_len, (const int32_t *)A->perm, A->tr_nlong, A->tr_nwide,
+                        d_y, ab.alpha, ab.beta);
+        }
+        return (int)SMVP_OK;
+    });
     SMVP_CUDA(cudaGetLastError());
     return SMVP_OK;
 }
@@ -866,7 +911,21 @@ extern "C" int smvp_tjds_mult_transpose_device(smvp_tjds *A, const double *d_x, 
         return SMVP_OK;
     cudaStream_t s = (cudaStream_t)stream;
     SMVP_TRY(tjds_transpose_prepare(A, s));
-    return tjds_transpose_pass(A, d_x, d_y, s);
+    return tjds_transpose_pass(A, d_x, d_y, AXPBY_PLAIN, s);
+}
+
+extern "C" int smvp_tjds_mult_transpose_device_axpby(smvp_tjds *A, double alpha, const double *d_x, double beta, double *d_y,
+                                                     void *stream)
+{
+    if (!A || (A->rows > 0 && !d_x) || (A->cols > 0 && !d_y))
+        return SMVP_E_ARG;
+    if (d_y && d_y == d_x)
+        return SMVP_E_ARG; // y would be read and written while the kernels gather it as x
+    if (A->cols == 0)
+        return SMVP_OK;
+    cudaStream_t s = (cudaStream_t)stream;
+    SMVP_TRY(tjds_transpose_prepare(A, s));
+    return tjds_transpose_pass(A, d_x, d_y, Axpby{alpha, beta}, s);
 }
 
 extern "C" int smvp_tjds_mult_transpose(smvp_tjds *A, const double *x_host, double *y_host, int iters, double *ms_each)
@@ -882,7 +941,7 @@ extern "C" int smvp_tjds_mult_transpose(smvp_tjds *A, const double *x_host, doub
     SMVP_TRY(tjds_transpose_prepare(A, 0));
     const bool small = (int64_t)A->rows + A->cols + A->nnz < SMVP_SMALL_LOOP_ITEMS;
     if (A->cols > 0)
-        SMVP_TRY(timed_loop(iters, ms_each, small, [&](cudaStream_t s) { return tjds_transpose_pass(A, A->d_xt, A->d_yt, s); }));
+        SMVP_TRY(timed_loop(iters, ms_each, small, [&](cudaStream_t s) { return tjds_transpose_pass(A, A->d_xt, A->d_yt, AXPBY_PLAIN, s); }));
     else if (ms_each)
         for (int it = 0; it < iters; it++)
             ms_each[it] = 0.0;
@@ -931,7 +990,7 @@ static int32_t tjds_effective_limit(const smvp_tjds *A, int32_t diag_limit)
 
 // plans, auxiliary arrays and the host-side routing decision: everything that may synchronise, so that the pass
 // itself only enqueues work (and can be captured in a CUDA graph)
-static int tjds_prepare(smvp_tjds *A, int variant, cudaStream_t s)
+static int tjds_prepare(smvp_tjds *A, int variant, const Axpby &ab, cudaStream_t s)
 {
     if (A->rows == 0)
         return SMVP_OK;
@@ -944,22 +1003,30 @@ static int tjds_prepare(smvp_tjds *A, int variant, cudaStream_t s)
         SMVP_TRY(tjds_prepare_det(A, s));
         SMVP_TRY(tjds_det_route(A));
     }
+    // the atomic sums of a natural-order handle land in a scratch vector under the epilogue (relabelled handles use y_rel)
+    if (!ab.plain() && A->relabel_state != 1 && (variant == SMVP_TJDS_ATOMIC || A->det_route != 1) && !A->y_sum)
+    {
+        SMVP_CUDA(dev_alloc(&A->y_sum, A->rows));
+        A->device_bytes += 8 * (int64_t)A->rows;
+    }
     return SMVP_OK;
 }
 
 #define SMVP_TJDS_ARGS_COMMON (const int2 *)A->seg_blocks, (const int32_t *)A->start_pos, mult_rows(A), (const double *)A->val, (const double *)A->x_perm
 
-// one pass, asynchronous on s; tjds_prepare has run
-static int tjds_pass(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit, cudaStream_t s)
+// one pass, asynchronous on s; tjds_prepare has run (with the same ab)
+static int tjds_pass(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit, const Axpby &ab, cudaStream_t s)
 {
     const int32_t lim = tjds_effective_limit(A, diag_limit);
-    const bool ranked = A->relabel_state == 1, skew = A->skew == 1;
+    const bool ranked = A->relabel_state == 1, skew = A->skew == 1, epi = !ab.plain();
     const unsigned blocks = (unsigned)A->num_seg_blocks;
     if (variant == SMVP_TJDS_ATOMIC || A->det_route != 1)
     {
         double *y_caller = d_y;
         if (ranked)
             d_y = A->y_rel; // sums land in rank order; tjds_unrank_y_kernel puts them back
+        else if (epi)
+            d_y = A->y_sum; // sums land beside y; tjds_unrank_y_kernel (identity rank) applies the epilogue
         SMVP_CUDA(cudaMemsetAsync(d_y, 0, sizeof(double) * (size_t)A->rows, s));
         if (blocks > 0 && lim > 0)
         {
@@ -968,12 +1035,16 @@ static int tjds_pass(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit,
             else
                 SMVP_LAUNCH((tjds_atomic_kernel<4, false>), blocks, 256, 0, s, SMVP_TJDS_ARGS_COMMON, d_y, A->nslots, lim);
         }
-        if (ranked)
+        if (ranked || epi)
         {
             int64_t ub = ceil_div64(A->rows, 256 * 4);
             const int64_t cap = (int64_t)device_props().sms * 8;
-            SMVP_LAUNCH(tjds_unrank_y_kernel, (unsigned)(ub < cap ? ub : cap), 256, 0, s, (const double *)A->y_rel,
-                        (const int32_t *)A->row_rank, A->rows, y_caller);
+            const int32_t *rank = ranked ? (const int32_t *)A->row_rank : nullptr;
+            with_flag(epi, [&](auto E) {
+                SMVP_LAUNCH(tjds_unrank_y_kernel<decltype(E)::value>, (unsigned)(ub < cap ? ub : cap), 256, 0, s, (const double *)d_y, rank,
+                            A->rows, y_caller, ab.alpha, ab.beta);
+                return (int)SMVP_OK;
+            });
         }
     }
     else
@@ -1004,15 +1075,18 @@ static int tjds_pass(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit,
                 });
             });
         }
-        SMVP_LAUNCH(tjds_det_finalize_kernel, (unsigned)ceil_div64(A->rows, 256), 256, 0, s, (const long long *)A->acc,
-                    (const int32_t *)A->row_exp, (const int32_t *)A->x_exp, A->rows, d_y,
-                    ranked ? (const int32_t *)A->row_rank : nullptr, words, r_lo, r_hi);
+        with_flag(epi, [&](auto E) {
+            SMVP_LAUNCH(tjds_det_finalize_kernel<decltype(E)::value>, (unsigned)ceil_div64(A->rows, 256), 256, 0, s,
+                        (const long long *)A->acc, (const int32_t *)A->row_exp, (const int32_t *)A->x_exp, A->rows, d_y,
+                        ranked ? (const int32_t *)A->row_rank : nullptr, words, r_lo, r_hi, ab.alpha, ab.beta);
+            return (int)SMVP_OK;
+        });
     }
     SMVP_CUDA(cudaGetLastError());
     return SMVP_OK;
 }
 
-extern "C" int smvp_tjds_mult_device(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit, void *stream)
+static int tjds_mult_any(smvp_tjds *A, const Axpby &ab, double *d_y, int variant, int32_t diag_limit, void *stream)
 {
     if (!A || (A->rows > 0 && !d_y))
         return SMVP_E_ARG;
@@ -1021,8 +1095,19 @@ extern "C" int smvp_tjds_mult_device(smvp_tjds *A, double *d_y, int variant, int
     if (A->rows == 0)
         return SMVP_OK;
     cudaStream_t s = (cudaStream_t)stream;
-    SMVP_TRY(tjds_prepare(A, variant, s));
-    return tjds_pass(A, d_y, variant, diag_limit, s);
+    SMVP_TRY(tjds_prepare(A, variant, ab, s));
+    return tjds_pass(A, d_y, variant, diag_limit, ab, s);
+}
+
+extern "C" int smvp_tjds_mult_device(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit, void *stream)
+{
+    return tjds_mult_any(A, AXPBY_PLAIN, d_y, variant, diag_limit, stream);
+}
+
+extern "C" int smvp_tjds_mult_device_axpby(smvp_tjds *A, double alpha, double beta, double *d_y, int variant, int32_t diag_limit,
+                                           void *stream)
+{
+    return tjds_mult_any(A, Axpby{alpha, beta}, d_y, variant, diag_limit, stream);
 }
 
 extern "C" int smvp_tjds_mult(smvp_tjds *A, const double *x_host, double *y_host, int iters, double *ms_each, int variant,
@@ -1040,7 +1125,7 @@ extern "C" int smvp_tjds_mult(smvp_tjds *A, const double *x_host, double *y_host
         SMVP_CUDA(cudaMemcpy(A->d_x, x_host, sizeof(double) * (size_t)A->cols, cudaMemcpyHostToDevice));
     // x is permuted once, before the loop, as the reference does at build time (main-cli.c:907-923)
     SMVP_TRY(smvp_tjds_set_x_device(A, A->d_x, nullptr));
-    SMVP_TRY(tjds_prepare(A, variant, 0));
+    SMVP_TRY(tjds_prepare(A, variant, AXPBY_PLAIN, 0));
     // the zero-fill of y / of the accumulators is part of the pass and therefore INSIDE the timed bracket (the
     // reference keeps its vectorInit outside, main-cli.c:1008): conservative.
     const bool small = (int64_t)A->rows + A->cols + A->nnz < SMVP_SMALL_LOOP_ITEMS;
@@ -1056,7 +1141,7 @@ extern "C" int smvp_tjds_mult(smvp_tjds *A, const double *x_host, double *y_host
             return (int)SMVP_OK;
         };
     if (A->rows > 0)
-        SMVP_TRY(timed_loop(iters, ms_each, small, [&](cudaStream_t s) { return tjds_pass(A, A->d_y, variant, diag_limit, s); }, multi));
+        SMVP_TRY(timed_loop(iters, ms_each, small, [&](cudaStream_t s) { return tjds_pass(A, A->d_y, variant, diag_limit, AXPBY_PLAIN, s); }, multi));
     else if (ms_each)
         for (int it = 0; it < iters; it++)
             ms_each[it] = 0.0;

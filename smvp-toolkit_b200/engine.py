@@ -82,6 +82,9 @@ SIGNATURES = {
     "smvp_csr_transpose": (_int, [_vp, _pp]),
     "smvp_tjds_mult_transpose_device": (_int, [_vp, _vp, _vp, _vp]),
     "smvp_tjds_mult_transpose": (_int, [_vp, _vp, _vp, _int, _vp]),
+    "smvp_csr_mult_device_axpby": (_int, [_vp, _dbl, _vp, _dbl, _vp, _int, _vp]),
+    "smvp_tjds_mult_device_axpby": (_int, [_vp, _dbl, _dbl, _vp, _int, _i32, _vp]),
+    "smvp_tjds_mult_transpose_device_axpby": (_int, [_vp, _dbl, _vp, _dbl, _vp, _vp]),
     "smvp_csr_info": (_int, [_vp, ctypes.POINTER(_CsrInfo)]),
     "smvp_tjds_info": (_int, [_vp, ctypes.POINTER(_TjdsInfo)]),
     "smvp_csr_export": (_int, [_vp, _vp, _vp, _vp]),
@@ -266,6 +269,12 @@ class CsrMatrix:
         """One pass y = A x; d_x=None uses the x last given to set_x_device."""
         _check(lib().smvp_csr_mult_device(self._h, _ptr(d_x), _ptr(d_y), variant, _stream(stream)), "smvp_csr_mult_device")
 
+    def mult_device_axpby(self, alpha, d_x, beta, d_y, variant=CSR_AUTO, stream=None):
+        """One pass y = alpha * A x + beta * y fused into the multiply (beta == 0: y is not read); d_x=None uses the x
+        last given to set_x_device.  See smvp_csr_mult_device_axpby in include/smvp_cuda.h."""
+        _check(lib().smvp_csr_mult_device_axpby(self._h, alpha, _ptr(d_x), beta, _ptr(d_y), variant, _stream(stream)),
+               "smvp_csr_mult_device_axpby")
+
     @property
     def x_relabel(self):
         """1: the multiply reads popularity-relabelled columns, -1: natural order, 0: not decided yet."""
@@ -388,12 +397,22 @@ class TjdsMatrix:
         _check(lib().smvp_tjds_mult_transpose_device(self._h, _ptr(d_x), _ptr(d_y), _stream(stream)),
                "smvp_tjds_mult_transpose_device")
 
+    def mult_transpose_device_axpby(self, alpha, d_x, beta, d_y, stream=None):
+        """One pass y = alpha * A^T x + beta * y (d_x: `rows` entries, d_y: `cols`; beta == 0: y is not read)."""
+        _check(lib().smvp_tjds_mult_transpose_device_axpby(self._h, alpha, _ptr(d_x), beta, _ptr(d_y), _stream(stream)),
+               "smvp_tjds_mult_transpose_device_axpby")
+
     def set_x_device(self, d_x, stream=None):
         _check(lib().smvp_tjds_set_x_device(self._h, _ptr(d_x), _stream(stream)), "smvp_tjds_set_x_device")
 
     def mult_device(self, d_y, variant=TJDS_ATOMIC, diag_limit=0, stream=None):
         _check(lib().smvp_tjds_mult_device(self._h, _ptr(d_y), variant, diag_limit, _stream(stream)),
                "smvp_tjds_mult_device")
+
+    def mult_device_axpby(self, alpha, beta, d_y, variant=TJDS_ATOMIC, diag_limit=0, stream=None):
+        """One pass y = alpha * A x + beta * y with the x last given to set_x_device (beta == 0: y is not read)."""
+        _check(lib().smvp_tjds_mult_device_axpby(self._h, alpha, beta, _ptr(d_y), variant, diag_limit, _stream(stream)),
+               "smvp_tjds_mult_device_axpby")
 
     def export(self):
         perm = np.zeros(self.cols, np.int32)
