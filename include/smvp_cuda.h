@@ -205,6 +205,49 @@ int smvp_tjds_mult_device_axpby(smvp_tjds *A, double alpha, double beta, double 
 int smvp_tjds_mult_transpose_device_axpby(smvp_tjds *A, double alpha, const double *d_x, double beta, double *d_y,
                                           void *stream); /* d_x: rows entries, d_y: cols */
 
+/* ---- the same update with an inner product of the new y fused into it: CG's p^T (A p), a residual's ||b - A x||^2,
+ * BiCG's and LSQR's products with A^T -- without a second kernel that reads y (and w) again.
+ *
+ * y: bit for bit what the matching *_axpby call (same handle, variant, plan, diag_limit and arguments, (1, 0) included)
+ *    stores, with its two exceptions unchanged (the hot / cold split, TJDS atomic).
+ * *d_dot = sum over every row r of y of fl(w[r] * y_new[r]) -- for the transposed call the `cols` entries of y.
+ *    d_w == NULL means w = y_new (||y_new||^2); d_w may be the x the kernels read (CG's p^T A p).  d_dot is ONE device
+ *    double, overwritten (never accumulated), written on `stream`.  When every term is zero (no rows; a handle without
+ *    entries and beta = 0) it is +0.0.  Inf and NaN propagate as IEEE arithmetic says.
+ * Order of the sum: each product is rounded once (no FMA).  The kernel that stores y adds the products of a WORK UNIT, a
+ *    fixed set of rows of the handle's plan, into one partial:
+ *        CSR row-pattern plan         a tile of 32 rows                       products added in a pairwise tree    d = 5
+ *        CSR merge-path plan          a warp tile (its row ends, lane by lane, then a pairwise tree over the lanes) plus
+ *                                     the fix-up's first row of the tile                                            d = 20
+ *        CSR hot / cold split         the cold pass's merge-path tiles (the hot pass forms no dot)                 d = 20
+ *        CSR vector variant           the rows of one 256-thread CTA, pairwise tree over the threads               d = 8
+ *        TJDS A x (every variant)     a block of 256 rows of y, pairwise tree                                       d = 8
+ *        TJDS A^T x                   one CTA of the gather (its empty columns, then its short column) or of the
+ *                                     combine kernel, pairwise tree over the threads      d = 9 + ceil((cols - nslots) /
+ *                                     (256 * gather CTAs)), nslots the columns that hold entries; no entries: 256-entry
+ *                                     blocks, d = 8
+ *    The P partials are then summed in a tree that depends on P alone (at most 48 + ceil(P / 2^21) additions deep).
+ *    With k = 1 + d + 48 + ceil(P / 2^21) and u = 2^-53:  |dot - sum_r w_r y_r| <= k u / (1 - k u) * sum_r |w_r y_r|.
+ *    The bits are a function of the handle, its plan, the variant and the vectors -- never of the grid, the SM count,
+ *    smvp_csr_set_corunner_headroom or timing: wherever y is reproducible the dot is bit-identical run to run (TJDS atomic
+ *    and inputs routed to it, det_route = -1, are not).
+ * Arguments: SMVP_E_ARG when d_dot is NULL, d_w == d_y (pass NULL for the new y), d_dot equals d_x, d_y or d_w, or a rule
+ *    of the *_axpby call is broken.
+ * Launches: those of the *_axpby call with (alpha, beta) != (1, 0) on the handle, plus one reduction -- a dot pass always
+ *    runs the epilogue, so TJDS atomic on a handle with y_relabel = -1 uses the scratch y and the per-row pass even for
+ *    (1, 0).  Bytes added to the *_axpby pass: 8 * rows for w when d_w != NULL, plus 16 bytes per work unit.  The
+ *    per-handle scratch of the partials -- 8 * (U + ceil(U / 8192) + 1) bytes, U the most units the handle can use (CSR:
+ *    any variant or plan; TJDS: A x, and A^T x once its plan exists) -- is allocated at the first dot call, which may
+ *    synchronise, and counted in device_bytes; later calls only enqueue work.  The one exception: a TJDS handle whose
+ *    first transposed dot call comes after an A x one grows it then, synchronising once.  Only one dot pass may be in
+ *    flight per handle.                                                                                              */
+int smvp_csr_mult_device_axpby_dot(smvp_csr *A, double alpha, const double *d_x, double beta, double *d_y,
+                                   const double *d_w, double *d_dot, int variant, void *stream);
+int smvp_tjds_mult_device_axpby_dot(smvp_tjds *A, double alpha, double beta, double *d_y, const double *d_w,
+                                    double *d_dot, int variant, int32_t diag_limit, void *stream);
+int smvp_tjds_mult_transpose_device_axpby_dot(smvp_tjds *A, double alpha, const double *d_x, double beta, double *d_y,
+                                              const double *d_w, double *d_dot, void *stream);
+
 /* ---- introspection ---- */
 typedef struct smvp_csr_info_t
 {

@@ -67,6 +67,61 @@ __device__ __forceinline__ double axpby(double alpha, double s, double beta, dou
     return beta != 0.0 ? __dadd_rn(__dmul_rn(alpha, s), __dmul_rn(beta, y0)) : __dmul_rn(alpha, s);
 }
 
+// The inner product fused into the store (the *_axpby_dot entry points, DESIGN.md §5.7).  The kernel that stores row r of
+// y also forms dot_term = fl(w[r] * y_new[r]) (w == NULL: y_new[r] itself) and sums the terms of its WORK UNIT -- a fixed
+// set of rows the plan defines -- into part[unit].  dot_reduce then sums the partials in a fixed tree that depends on
+// their number only, so the bits never depend on the grid, the SM count or timing.
+struct DotOut
+{
+    const double *w; // NULL: w = y_new
+    double *part;    // one partial per work unit
+};
+__device__ __forceinline__ double dot_term(const double *w, int64_t r, double v) { return __dmul_rn(w ? __ldg(w + r) : v, v); }
+// the epilogue's store of a dot pass: y[r] = fl(alpha * s) + fl(beta * y[r]) and the running sum acc += dot_term
+__device__ __forceinline__ void store_axpby_dot(double *__restrict__ y, int64_t r, double s, double alpha, double beta,
+                                                const double *__restrict__ w, double &acc)
+{
+    const double v = axpby(alpha, s, beta, beta != 0.0 ? y[r] : 0.0);
+    y[r] = v;
+    acc = __dadd_rn(acc, dot_term(w, r, v));
+}
+// pairwise tree over the 32 lanes in lane order (a butterfly: every lane ends with the same bits)
+__device__ __forceinline__ double warp_tree_sum(double v)
+{
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1)
+        v = __dadd_rn(v, __shfl_xor_sync(0xffffffffu, v, o));
+    return v;
+}
+// pairwise tree over the THREADS threads of a CTA in thread order; the sum is valid in thread 0.  Every thread calls it.
+template <int THREADS>
+__device__ __forceinline__ double cta_tree_sum(double v)
+{
+    constexpr int W = THREADS / 32;
+    static_assert(W >= 1 && W <= 32 && (W & (W - 1)) == 0, "a power of two of warps");
+    __shared__ double s_w[W];
+    v = warp_tree_sum(v);
+    if (W == 1)
+        return v;
+    const int lane = threadIdx.x & 31, wi = threadIdx.x >> 5;
+    if (lane == 0)
+        s_w[wi] = v;
+    __syncthreads();
+    if (wi == 0)
+    {
+        v = lane < W ? s_w[lane] : 0.0;
+#pragma unroll
+        for (int o = 1; o < W; o <<= 1)
+            v = __dadd_rn(v, __shfl_xor_sync(0xffffffffu, v, o));
+    }
+    return v;
+}
+// Per-handle scratch of a dot pass (dot.cu): the partials of `units` work units, the reduction's CTA sums and its counter.
+// Grows *buf (counted in *device_bytes) when the plan needs more room; may synchronise then.
+int dot_scratch(double **buf, int64_t *cap, int64_t *device_bytes, int64_t units, cudaStream_t s);
+// one launch: *out = the partials buf[0, units) summed in the fixed tree (DESIGN.md §5.7)
+int dot_reduce(double *buf, int64_t cap, int64_t units, double *out, cudaStream_t s);
+
 // ---------------------------------------------------------------- environment (api.cu)
 // The library's only reader of the environment: every SMVP_* switch goes through these (table in INTEGRATION.md).
 const char *env_str(const char *name);                   // the value; NULL when unset or empty
@@ -217,6 +272,9 @@ struct smvp_csr
     uint8_t *pat_id;                       // [rows]
     int32_t *pat_off;                      // [pattern_count * PAT_LMAX]
     int32_t *pat_len;                      // [pattern_count]
+    // scratch of the fused inner product (*_axpby_dot, dot.cu): unit partials, reduction sums and counter; built at first use
+    double *dot_buf;
+    int64_t dot_cap;
 };
 namespace smvp
 {
@@ -281,6 +339,8 @@ struct smvp_tjds
     uint32_t *tr_seg_off;    // [nseg] first partial of segment g; slot q of segment g writes tr_part[tr_seg_off[g] + q]
     double *tr_part;         // one partial per (segment, slot) pair of the long columns
     double *d_xt, *d_yt;     // [rows] / [cols]: scratch of the host-vector entry point
+    double *dot_buf;         // scratch of the fused inner product (*_axpby_dot, dot.cu), built at first use
+    int64_t dot_cap;
 };
 namespace smvp
 {

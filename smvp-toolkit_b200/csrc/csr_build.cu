@@ -75,6 +75,7 @@ void csr_release(smvp_csr *A)
     cudaFree(A->carry_val);
     cudaFree(A->d_x);
     cudaFree(A->d_y);
+    cudaFree(A->dot_buf);
     csr_pipe_release(A);
     csr_relabel_release(A);
     csr_pattern_release(A);

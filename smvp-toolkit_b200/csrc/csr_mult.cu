@@ -167,6 +167,13 @@ __device__ __forceinline__ double ld_y_early(const double *p)
     asm volatile("ld.global.f64 %0, [%1];" : "=d"(v) : "l"(p));
     return v;
 }
+// w[r] for the dot, loaded ahead of its use like ld_y_early (read-only: w is never y)
+__device__ __forceinline__ double ld_w_early(const double *p)
+{
+    double v;
+    asm volatile("ld.global.nc.f64 %0, [%1];" : "=d"(v) : "l"(p));
+    return v;
+}
 // the instantiations the launchers name: the epilogue exists only without the fan-out
 template <bool FANOUT, bool EPI>
 constexpr bool kernel_exists() { return !(FANOUT && EPI); }
@@ -176,12 +183,14 @@ constexpr bool kernel_exists() { return !(FANOUT && EPI); }
 // LPR < 16: lane l takes entries l, l+LPR, ... with 8/4-byte loads (short rows).  With only a few rows per warp
 //           the lanes of one request then sit on consecutive entries of consecutive rows, so the x gather of a
 //           banded matrix touches far fewer sectors per request -- the vector kernel is L1-bound on such rows.
-template <int LPR, bool FANOUT, bool EPI>
-__global__ void __launch_bounds__(256) csr_vector_kernel(const int32_t *__restrict__ row_ptr, const int32_t *__restrict__ col_ind,
-                                                         const double *__restrict__ val, const double *__restrict__ x,
-                                                         double *__restrict__ y, int32_t rows, const __grid_constant__ YFan fan,
-                                                         double alpha, double beta)
+// DOT (csr_vector_dot_kernel): the work unit is the CTA -- the rows its sub-warps end, in thread order
+template <int LPR, bool FANOUT, bool EPI, bool DOT>
+__device__ __forceinline__ void csr_vector_body(const int32_t *__restrict__ row_ptr, const int32_t *__restrict__ col_ind,
+                                                const double *__restrict__ val, const double *__restrict__ x, double *__restrict__ y,
+                                                int32_t rows, const YFan &fan, double alpha, double beta, const double *__restrict__ w,
+                                                double *__restrict__ part)
 {
+    static_assert(!DOT || (EPI && !FANOUT), "the dot is formed by the epilogue");
     constexpr bool WIDE = LPR >= 16;
     const int64_t gt = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const int64_t row = gt / LPR;
@@ -235,8 +244,41 @@ __global__ void __launch_bounds__(256) csr_vector_kernel(const int32_t *__restri
 #pragma unroll
     for (int o = LPR / 2; o > 0; o >>= 1)
         sum = __dadd_rn(sum, __shfl_xor_sync(0xffffffffu, sum, o));
-    if (row < rows && lane == 0)
-        store_y<FANOUT, EPI>(y, fan, row, sum, alpha, beta);
+    if (!DOT)
+    {
+        if (row < rows && lane == 0)
+            store_y<FANOUT, EPI>(y, fan, row, sum, alpha, beta);
+    }
+    else
+    {
+        double d = 0.0;
+        if (row < rows && lane == 0)
+        {
+            const double v = axpby(alpha, sum, beta, beta != 0.0 ? y[row] : 0.0);
+            y[row] = v;
+            d = dot_term(w, row, v);
+        }
+        d = cta_tree_sum<256>(d);
+        if (threadIdx.x == 0)
+            part[blockIdx.x] = d;
+    }
+}
+template <int LPR, bool FANOUT, bool EPI>
+__global__ void __launch_bounds__(256) csr_vector_kernel(const int32_t *__restrict__ row_ptr, const int32_t *__restrict__ col_ind,
+                                                         const double *__restrict__ val, const double *__restrict__ x,
+                                                         double *__restrict__ y, int32_t rows, const __grid_constant__ YFan fan,
+                                                         double alpha, double beta)
+{
+    csr_vector_body<LPR, FANOUT, EPI, false>(row_ptr, col_ind, val, x, y, rows, fan, alpha, beta, nullptr, nullptr);
+}
+// (6 CTAs per SM: at the default bound ptxas keeps 32 registers and spills in the 128-bit configurations)
+template <int LPR>
+__global__ void __launch_bounds__(256, 6) csr_vector_dot_kernel(const int32_t *__restrict__ row_ptr, const int32_t *__restrict__ col_ind,
+                                                             const double *__restrict__ val, const double *__restrict__ x,
+                                                             double *__restrict__ y, int32_t rows, double alpha, double beta,
+                                                             const double *__restrict__ w, double *__restrict__ part)
+{
+    csr_vector_body<LPR, false, true, true>(row_ptr, col_ind, val, x, y, rows, YFan(), alpha, beta, w, part);
 }
 
 // =====================================================================================  TINY LOOP
@@ -279,14 +321,25 @@ __global__ void __launch_bounds__(TINY_THREADS) csr_tiny_loop_kernel(const int32
 // the column indices the multiply kernels read: the relabelled copy when that plan is in use (relabel.cu)
 static inline const int32_t *mult_cols(const smvp_csr *A) { return A->relabel_state == 1 ? A->col_rel : A->col_ind; }
 
+// lanes per row of the vector kernel, from the mean row length
+static int vector_lpr(const smvp_csr *A)
+{
+    const double mean = A->rows > 0 ? (double)A->nnz / A->rows : 0.0;
+    return mean <= 8.0 ? 2 : mean <= 16.0 ? 4 : mean <= 32.0 ? 8 : mean <= 64.0 ? 16 : 32;
+}
+
 template <int LPR>
-static int launch_vector(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, const Axpby &ab, cudaStream_t s)
+static int launch_vector(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, const Axpby &ab, const DotOut *dot,
+                         cudaStream_t s)
 {
     const int64_t threads = (int64_t)A->rows * LPR;
     const int64_t blocks = ceil_div64(threads, 256);
     if (blocks > 0x7fffffffLL)
         return SMVP_E_TOOBIG;
-    if (blocks > 0)
+    if (blocks > 0 && dot)
+        SMVP_LAUNCH(csr_vector_dot_kernel<LPR>, (unsigned)blocks, 256, 0, s, A->row_ptr, mult_cols(A), A->val, d_x, d_y, A->rows,
+                    ab.alpha, ab.beta, dot->w, dot->part);
+    else if (blocks > 0)
         return with_flag(fan != nullptr, [&](auto F) {
             return with_flag(!ab.plain(), [&](auto E) {
                 constexpr bool FANOUT = decltype(F)::value, EPI = decltype(E)::value;
@@ -303,21 +356,22 @@ static int launch_vector(const smvp_csr *A, const double *d_x, double *d_y, cons
     return SMVP_OK;
 }
 
-static int csr_mult_vector(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, const Axpby &ab, cudaStream_t s)
+static int csr_mult_vector(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, const Axpby &ab, const DotOut *dot,
+                           cudaStream_t s)
 {
-    const double mean = A->rows > 0 ? (double)A->nnz / A->rows : 0.0;
-    int rc;
-    if (mean <= 8.0)
-        rc = launch_vector<2>(A, d_x, d_y, fan, ab, s);
-    else if (mean <= 16.0)
-        rc = launch_vector<4>(A, d_x, d_y, fan, ab, s);
-    else if (mean <= 32.0)
-        rc = launch_vector<8>(A, d_x, d_y, fan, ab, s);
-    else if (mean <= 64.0)
-        rc = launch_vector<16>(A, d_x, d_y, fan, ab, s);
-    else
-        rc = launch_vector<32>(A, d_x, d_y, fan, ab, s);
-    return rc;
+    switch (vector_lpr(A))
+    {
+    case 2:
+        return launch_vector<2>(A, d_x, d_y, fan, ab, dot, s);
+    case 4:
+        return launch_vector<4>(A, d_x, d_y, fan, ab, dot, s);
+    case 8:
+        return launch_vector<8>(A, d_x, d_y, fan, ab, dot, s);
+    case 16:
+        return launch_vector<16>(A, d_x, d_y, fan, ab, dot, s);
+    default:
+        return launch_vector<32>(A, d_x, d_y, fan, ab, dot, s);
+    }
 }
 
 // =====================================================================================  MERGE
@@ -392,10 +446,12 @@ __device__ __forceinline__ TileView make_tile(int32_t r0, int32_t r1, int32_t t,
 
 // First row of a tile that ends a row there: y[row] = (carries of the tiles the row crossed, in tile order) + (partial
 // of the tile where it ends).  tile_row[u+1] is the row tile u's carry belongs to.
-template <bool FANOUT, bool EPI>
+// DOT: the row's dot term is added to tile t's partial, which the merge kernel left (its unit: the tile plus this row).
+template <bool FANOUT, bool EPI, bool DOT = false>
 __device__ __forceinline__ void merge_fixup_tile(int32_t t, const int32_t *__restrict__ tile_row, const double *__restrict__ head_val,
                                                  const double *__restrict__ carry_val, double *__restrict__ y, const YFan &fan,
-                                                 double alpha, double beta)
+                                                 double alpha, double beta, const double *__restrict__ w = nullptr,
+                                                 double *__restrict__ part = nullptr)
 {
     // everything the common case needs is loaded up front (independent loads: one memory round trip)
     const int32_t r = tile_row[t];
@@ -422,7 +478,14 @@ __device__ __forceinline__ void merge_fixup_tile(int32_t t, const int32_t *__res
             acc = __dadd_rn(acc, __ldcg(carry_val + k));
         acc = __dadd_rn(acc, h);
     }
-    store_y<FANOUT, EPI>(y, fan, r, acc, alpha, beta);
+    if (!DOT)
+        store_y<FANOUT, EPI>(y, fan, r, acc, alpha, beta);
+    else
+    {
+        const double v = axpby(alpha, acc, beta, beta != 0.0 ? y[r] : 0.0);
+        y[r] = v;
+        part[t] = __dadd_rn(__ldcg(part + t), dot_term(w, r, v));
+    }
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -439,273 +502,26 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
                           double *__restrict__ carry_val, const __grid_constant__ YFan fan, int32_t hot_l1, int32_t hot_l2,
                           int32_t early_dependents, double alpha, double beta)
 {
-    // Small grids (early_dependents != 0): let the fix-up kernel, launched with programmatic stream serialization, be
-    // scheduled NOW; it parks at griddepcontrol.wait until this grid has completed and flushed.  In the batched `-n` loop
-    // of a matrix like memplus that hides the second launch's latency (a pass lasts as long as a launch).
-    if (early_dependents)
-        asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    // processes tiles [tile_begin, num_tiles): a sub-range lets the host overlap the copy-out of finished rows.
-    // One stage per warp: deeper rings lost to more resident warps in every sweep.
-    using Shape = MergeShape<32, IPT>;
-    extern __shared__ __align__(128) unsigned char stage_mem[];
-    __shared__ __align__(8) uint64_t full_bar[WARPS];
-
-    // UNI: the warp index and the tile coordinates below are broadcast from lane 0.  The values are the same in every lane
-    // anyway, but the broadcast lets the compiler PROVE it and keep the whole tile bookkeeping (and the operands of the
-    // bulk copies) in uniform registers instead of electing a lane and converting per copy.  Measured on B200
-    // (profiles/r01_logs/diet_bisect.log): stencil configuration 2.78 -> 2.69 ms, but the R-MAT configuration 5.67 ->
-    // 6.39 ms, so it is a per-configuration choice (MergeStencil::UNI, MergeSkewed::UNI).
-#define SMVP_BCAST(v) (UNI ? __shfl_sync(0xffffffffu, (v), 0) : (v))
-    const int lane = threadIdx.x & 31, w = SMVP_BCAST((int)(threadIdx.x >> 5));
-    const int64_t total = (int64_t)rows + nnz;
-    unsigned char *base = stage_mem + (size_t)w * Shape::SMEM_BYTES;
-    uint64_t *my_bar = &full_bar[w];
-    uint64_t policy = 0;
-    if (lane == 0)
-    {
-        mbar_init(my_bar, 1);
-        fence_mbar_init();
-        policy = l2_evict_first_policy();
-    }
-    __syncwarp();
-
-    const uint64_t pol_last = RANKED ? l2_evict_last_policy() : 0, pol_first = RANKED ? l2_evict_first_policy() : 0;
-    const int32_t warp_stride = (int32_t)gridDim.x * WARPS;
-    auto issue = [&](const TileView &v) { // lane 0 only
-        mbar_expect_tx(my_bar, v.vb + v.cb + v.rb);
-        if (v.vb)
-            bulk_g2s(base, val + v.va, v.vb, my_bar, policy);
-        if (v.cb)
-            bulk_g2s(base + v.vb, col_ind + v.ca, v.cb, my_bar, policy);
-        if (v.rb)
-            bulk_g2s(base + v.vb + v.cb, row_ptr + v.ra, v.rb, my_bar, policy);
-    };
-
-    int32_t t = tile_begin + (int32_t)blockIdx.x * WARPS + w;
-    int32_t cur_r0 = 0, cur_r1 = 0; // merge coordinates of the tile in flight: the only tile state kept across the loop
-    if (t < num_tiles)
-    {
-        cur_r0 = SMVP_BCAST(__ldg(tile_row + t));
-        cur_r1 = SMVP_BCAST(__ldg(tile_row + t + 1));
-        if (lane == 0)
-            issue(make_tile(cur_r0, cur_r1, t, Shape::TILE, total));
-    }
-    uint32_t parity = 0;
-
-    while (t < num_tiles)
-    {
-        // per-tile scalars: only what the walk needs stays live (the rest of the TileView dies here)
-        int32_t n0, tile_r0, rows_t, nnz_t, items_t;
-        uint32_t sval, scol, srow; // shared-window byte addresses of TILE-LOCAL nonzero 0 / row 0
-        {
-            const TileView v = make_tile(cur_r0, cur_r1, t, Shape::TILE, total);
-            n0 = (int32_t)v.n0;
-            tile_r0 = v.r0;
-            rows_t = v.rows_t;
-            nnz_t = v.nnz_t;
-            items_t = v.items_t;
-            const uint32_t b = smem_u32(base);
-            sval = b + 8u * (uint32_t)(n0 - v.va);
-            scol = b + v.vb + 4u * (uint32_t)(n0 - v.ca);
-            srow = b + v.vb + v.cb + 4u * (uint32_t)(v.r0 + 1 - v.ra);
-        }
-        auto row_end = [&](int32_t i) -> int32_t { return lds_s32(srow + 4u * (uint32_t)i) - n0; };
-
-        mbar_wait(my_bar, parity);
-        parity ^= 1u;
-
-        // ---- my first merge item: interpolate, gallop, bisect (2 probes on regular matrices)
-        int32_t d = lane * IPT;
-        if (d > items_t)
-            d = items_t;
-        int32_t lo = d > nnz_t ? d - nnz_t : 0, hi = d < rows_t ? d : rows_t;
-        if (lo < hi)
-        {
-            // first guess by interpolation.  The divisor is the FULL tile size (a compile-time constant: multiply-shift
-            // instead of a 25-instruction integer division); only the matrix's last tile is shorter, and there the guess
-            // is merely a little low before the gallop corrects it.
-            int32_t g = (int32_t)(((uint32_t)d * (uint32_t)rows_t) / (uint32_t)Shape::TILE); // < 2^20: 32-bit is exact
-            g = g < lo ? lo : (g > hi - 1 ? hi - 1 : g);
-            int32_t step = 1;
-            if (row_end(g) <= d - g - 1)
-            {
-                lo = g + 1;
-                while (lo < hi)
-                {
-                    const int32_t m = (lo + step - 1 < hi - 1) ? lo + step - 1 : hi - 1;
-                    if (row_end(m) <= d - m - 1)
-                    {
-                        lo = m + 1;
-                        step <<= 1;
-                    }
-                    else
-                    {
-                        hi = m;
-                        break;
-                    }
-                }
-            }
-            else
-            {
-                hi = g;
-                while (lo < hi)
-                {
-                    const int32_t m = (hi - step > lo) ? hi - step : lo;
-                    if (!(row_end(m) <= d - m - 1))
-                    {
-                        hi = m;
-                        step <<= 1;
-                    }
-                    else
-                    {
-                        lo = m + 1;
-                        break;
-                    }
-                }
-            }
-            while (lo < hi)
-            {
-                const int32_t mid = (lo + hi) >> 1;
-                if (row_end(mid) <= d - mid - 1)
-                    lo = mid + 1;
-                else
-                    hi = mid;
-            }
-        }
-        const int32_t i0 = lo, j0 = d - lo;
-        int32_t d_next = (lane + 1) * IPT;
-        if (d_next > items_t)
-            d_next = items_t;
-        int32_t j_next = __shfl_down_sync(0xffffffffu, j0, 1);
-        if (lane == 31)
-            j_next = nnz_t;
-        const int32_t i_next = d_next - j_next;
-        const int32_t cnt = j_next - j0;
-
-        // ---- all my gathers first, in three phases pinned by volatile asm: the column indices, then every x gather of
-        // the lane (IPT independent loads in flight together -- left alone, the compiler reuses one register pair and
-        // waits for each load before issuing the next), then the products.  (Pinning the lane's two shared-window bases
-        // in registers with an opaque move saves an address instruction per load but makes the 14-item configurations
-        // spill; the nested "live slot / row end" walk this one replaced is in profiles/r01_logs/diet_bisect.log.)
-        // EPI: y of my first row end (tile row i0; row 0 of the tile is the fix-up kernel's), loaded before the gathers so
-        // that its latency hides behind them; further row ends of the lane (short rows) load y at their store
-        double y_first = 0.0;
-        if (EPI && beta != 0.0 && i0 < i_next && i0 != 0)
-            y_first = ld_y_early(y + (int64_t)tile_r0 + i0);
-        double prod[IPT];
-        {
-            int32_t cq[IPT];
-            uint32_t cbase = scol + 4u * (uint32_t)j0, vbase = sval + 8u * (uint32_t)j0;
-            // (every slot gets a defined value: leaving the dead ones undefined makes the compiler carry the previous
-            // tile's registers through the loop and spill them)
-#pragma unroll
-            for (int q = 0; q < IPT; q++)
-                cq[q] = q < cnt ? lds_s32(cbase + 4u * q) : 0;
-#pragma unroll
-            for (int q = 0; q < IPT; q++)
-            {
-                prod[q] = 0.0;
-                if (q < cnt)
-                    prod[q] = RANKED ? ldg_x_ranked(x, cq[q], hot_l1, hot_l2, pol_last, pol_first) : ldg_x_pinned(x, cq[q]);
-            }
-#pragma unroll
-            for (int q = 0; q < IPT; q++)
-                if (q < cnt)
-                    prod[q] = __dmul_rn(lds_f64(vbase + 8u * q), prod[q]);
-        }
-
-        double sum = 0.0, first_sum = 0.0;
-        bool has_first = false;
-        {
-            // Walk.  `until` = nonzeros of mine before my next row end (relative to j0, so each test is against a constant;
-            // "no further row end of mine" = never).  Dead slots (q >= cnt) hold +0.0, and a partial sum that starts at
-            // +0.0 can never become -0.0, so adding them is exact: the loop needs no "is this slot live" test, and the row
-            // ends that follow my last nonzero are flushed by the same test at the first dead slot.
-            int32_t row = i0;
-            int32_t until = (row < i_next ? row_end(row) : 0x7fffffff) - j0;
-#pragma unroll
-            for (int q = 0; q < IPT; q++)
-            {
-                if (until <= q) // rare: a row end (or a run of empty rows) sits before item q
-                {
-                    do
-                    {
-                        if (!has_first)
-                        {
-                            has_first = true;
-                            first_sum = sum;
-                        }
-                        else
-                            store_y<FANOUT, EPI>(y, fan, (int64_t)tile_r0 + row, sum, alpha, beta);
-                        sum = 0.0;
-                        row++;
-                        until = (row < i_next ? row_end(row) : 0x7fffffff) - j0;
-                    } while (until <= q);
-                }
-                sum = __dadd_rn(sum, prod[q]);
-            }
-            // every row end of mine has at most IPT - 1 of my nonzeros before it, so the loop above has seen them all;
-            // this is only a safety net
-            while (row < i_next)
-            {
-                if (!has_first)
-                {
-                    has_first = true;
-                    first_sum = sum;
-                }
-                else
-                    store_y<FANOUT, EPI>(y, fan, (int64_t)tile_r0 + row, sum, alpha, beta);
-                sum = 0.0;
-                row++;
-            }
-        }
-
-        // ---- the stage is consumed: refill it for my next tile while the warp stitches
-        __syncwarp();
-        const int32_t tn = t + warp_stride;
-        if (tn < num_tiles && tn > t)
-        {
-            cur_r0 = SMVP_BCAST(__ldg(tile_row + tn));
-            cur_r1 = SMVP_BCAST(__ldg(tile_row + tn + 1));
-            if (lane == 0)
-                issue(make_tile(cur_r0, cur_r1, tn, Shape::TILE, total));
-        }
-
-        // ---- stitch rows cut by lane boundaries: segmented inclusive scan of (carry row, carry sum)
-        const int32_t key = i_next; // the row my trailing partial belongs to
-        double scan = sum;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1)
-        {
-            const int32_t pk = __shfl_up_sync(0xffffffffu, key, o);
-            const bool take = lane >= o && pk == key;
-            const double pv = __shfl_up_sync(0xffffffffu, scan, o);
-            if (take)
-                scan = __dadd_rn(pv, scan);
-        }
-        const double prev_scan = __shfl_up_sync(0xffffffffu, scan, 1);
-        const int32_t prev_key = __shfl_up_sync(0xffffffffu, key, 1);
-        if (has_first)
-        {
-            if (lane > 0 && prev_key == i0)
-                first_sum = __dadd_rn(prev_scan, first_sum);
-            // the tile's first row may have started in earlier tiles: its partial goes to the fix-up
-            // kernel, which adds the carries and writes y -- and, under the epilogue, is the only one to read that
-            // row of y.  Without the epilogue y is only ever WRITTEN here (never read), so it may be a write-only
-            // mapping such as an NVSwitch multicast address.
-            if (i0 == 0)
-                head_val[t] = first_sum;
-            else if (EPI)
-                y[(int64_t)tile_r0 + i0] = axpby(alpha, first_sum, beta, y_first);
-            else
-                store_y<FANOUT, false>(y, fan, (int64_t)tile_r0 + i0, first_sum, alpha, beta);
-        }
-        if (lane == 31)
-            carry_val[t] = scan; // partial of the row that continues into the next tile
-        if (tn <= t)
-            break; // 32-bit overflow guard
-        t = tn;
-    }
+#define SMVP_MERGE_DOT 0
+#include "merge_warp_body.cuh"
+#undef SMVP_MERGE_DOT
+}
+// The dot pass (DESIGN.md §5.7): the work unit is the warp tile -- each lane adds the dot terms of the rows it stores in
+// the order it stores them, the lanes are added in a pairwise tree into part[t], and the fix-up kernel adds the term of
+// the tile's first row (merge_fixup_tile).  Whole passes only, with the epilogue, never with the fan-out.
+template <int WARPS, int IPT, int MINB, bool RANKED, bool UNI>
+__global__ void __launch_bounds__(WARPS * 32, MINB)
+    csr_merge_warp_dot_kernel(const int32_t *__restrict__ row_ptr, const int32_t *__restrict__ col_ind, const double *__restrict__ val,
+                              const double *__restrict__ x, double *__restrict__ y, const int32_t *__restrict__ tile_row, int32_t rows,
+                              int64_t nnz, int32_t num_tiles, double *__restrict__ head_val, double *__restrict__ carry_val,
+                              int32_t hot_l1, int32_t hot_l2, int32_t early_dependents, double alpha, double beta,
+                              const double *__restrict__ dot_w, double *__restrict__ part)
+{
+    constexpr bool EPI = true;
+    constexpr int32_t tile_begin = 0;
+#define SMVP_MERGE_DOT 1
+#include "merge_warp_body.cuh"
+#undef SMVP_MERGE_DOT
 }
 
 template <bool FANOUT, bool EPI>
@@ -719,6 +535,20 @@ __global__ void __launch_bounds__(256) merge_fixup_kernel(const int32_t *__restr
     const int32_t t = tile_begin + blockIdx.x * blockDim.x + threadIdx.x;
     if (t < num_tiles)
         merge_fixup_tile<FANOUT, EPI>(t, tile_row, head_val, carry_val, y, fan, alpha, beta);
+}
+// The dot pass's fix-up.  griddepcontrol.wait returns only once the merge kernel has completed and its writes are
+// visible, and every thread of this grid executes it before it exits: so when this grid has completed -- which the
+// reduction launched after it in stream order waits for -- the merge kernel's partials are final, also when this grid
+// was launched early.  The reduction itself is an ordinary launch.
+__global__ void __launch_bounds__(256) merge_fixup_dot_kernel(const int32_t *__restrict__ tile_row, const double *__restrict__ head_val,
+                                                              const double *__restrict__ carry_val, int32_t num_tiles,
+                                                              double *__restrict__ y, double alpha, double beta,
+                                                              const double *__restrict__ w, double *__restrict__ part)
+{
+    asm volatile("griddepcontrol.wait;" ::: "memory");
+    const int32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t < num_tiles)
+        merge_fixup_tile<false, true, true>(t, tile_row, head_val, carry_val, y, YFan(), alpha, beta, w, part);
 }
 
 // ---- the two instantiations AUTO chooses from (merge_skewed).  Measured on B200 (logs under profiles/, the swept
@@ -809,6 +639,40 @@ static int persistent_grid(K kern, int threads, int smem, int handle_headroom, i
     return SMVP_OK;
 }
 
+// The fix-up after the merge kernel: launched early with programmatic stream serialization (it parks at
+// griddepcontrol.wait) when `early`, an ordinary launch otherwise
+template <typename K, typename... Args>
+static int launch_fixup(bool early, int32_t ntiles, cudaStream_t s, K kern, Args... args)
+{
+    if (early)
+    {
+        cudaLaunchConfig_t cfg = {};
+        cfg.gridDim = dim3((unsigned)ceil_div64(ntiles, 256));
+        cfg.blockDim = dim3(256);
+        cfg.dynamicSmemBytes = 0;
+        cfg.stream = s;
+        cudaLaunchAttribute attr[1];
+        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+        attr[0].val.programmaticStreamSerializationAllowed = 1;
+        cfg.attrs = attr;
+        cfg.numAttrs = 1;
+        SMVP_CUDA(cudaLaunchKernelEx(&cfg, kern, args...));
+        ::smvp::g_launches.fetch_add(1, std::memory_order_relaxed);
+    }
+    else
+        SMVP_LAUNCH(kern, (unsigned)ceil_div64(ntiles, 256), 256, 0, s, args...);
+    return SMVP_OK;
+}
+
+// (a fix-up fused into the kernel -- the last warp of the grid to finish walks the tiles -- was tried for the batched `-n`
+// loop of small matrices: one warp serialises the few hundred tiles of a matrix like memplus, 12.1 us per pass against
+// 5.7 us with the second launch.  Two launches it stays.)
+static bool merge_fixup_early(int32_t ntiles)
+{
+    static thread_local const bool pdl_ok = !env_set("SMVP_NO_PDL"); // SMVP_NO_PDL: no early launch of the fix-up
+    return pdl_ok && ntiles <= MERGE_PDL_TILES;
+}
+
 template <class C, bool FANOUT, bool RANKED, bool EPI>
 static int launch_wmerge(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fanp, const Axpby &ab, cudaStream_t s,
                          int32_t tile_begin, int32_t tile_end)
@@ -825,32 +689,35 @@ static int launch_wmerge(const smvp_csr *A, const double *d_x, double *d_y, cons
     SMVP_TRY(persistent_grid(kern, C::WARPS * 32, SMEM, A->merge_headroom, ceil_div64(ntiles, C::WARPS), res, &grid));
     if (grid > 0)
     {
-        // (a fix-up fused into the kernel -- the last warp of the grid to finish walks the tiles -- was tried for the
-        // batched `-n` loop of small matrices: one warp serialises the few hundred tiles of a matrix like memplus,
-        // 12.1 us per pass against 5.7 us with the second launch.  Two launches it stays.)
-        static thread_local const bool pdl_ok = !env_set("SMVP_NO_PDL"); // SMVP_NO_PDL: no early launch of the fix-up
-        const bool early = pdl_ok && ntiles <= MERGE_PDL_TILES;
+        const bool early = merge_fixup_early(ntiles);
         SMVP_LAUNCH(kern, (unsigned)grid, C::WARPS * 32, SMEM, s, A->row_ptr, mult_cols(A), A->val, d_x, d_y, A->tile_row, A->rows,
                     A->nnz, tile_begin, tile_end, A->head_val, A->carry_val, fan, hot_l1, hot_l2, early ? 1 : 0, ab.alpha, ab.beta);
-        if (early)
-        {
-            cudaLaunchConfig_t cfg = {};
-            cfg.gridDim = dim3((unsigned)ceil_div64(ntiles, 256));
-            cfg.blockDim = dim3(256);
-            cfg.dynamicSmemBytes = 0;
-            cfg.stream = s;
-            cudaLaunchAttribute attr[1];
-            attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-            attr[0].val.programmaticStreamSerializationAllowed = 1;
-            cfg.attrs = attr;
-            cfg.numAttrs = 1;
-            SMVP_CUDA(cudaLaunchKernelEx(&cfg, merge_fixup_kernel<FANOUT, EPI>, (const int32_t *)A->tile_row, (const double *)A->head_val,
-                                         (const double *)A->carry_val, tile_begin, tile_end, d_y, fan, ab.alpha, ab.beta));
-            ::smvp::g_launches.fetch_add(1, std::memory_order_relaxed);
-        }
-        else
-            SMVP_LAUNCH((merge_fixup_kernel<FANOUT, EPI>), (unsigned)ceil_div64(ntiles, 256), 256, 0, s, (const int32_t *)A->tile_row,
-                        (const double *)A->head_val, (const double *)A->carry_val, tile_begin, tile_end, d_y, fan, ab.alpha, ab.beta);
+        SMVP_TRY(launch_fixup(early, ntiles, s, merge_fixup_kernel<FANOUT, EPI>, (const int32_t *)A->tile_row, (const double *)A->head_val,
+                              (const double *)A->carry_val, tile_begin, tile_end, d_y, fan, ab.alpha, ab.beta));
+    }
+    return SMVP_OK;
+}
+
+// the whole-pass merge-path multiply with the dot partials of its tiles in dot->part[0, merge_tiles)
+template <class C, bool RANKED>
+static int launch_wmerge_dot(const smvp_csr *A, const double *d_x, double *d_y, const Axpby &ab, const DotOut &dot, cudaStream_t s)
+{
+    constexpr int SMEM = C::WARPS * MergeShape<32, C::IPT>::SMEM_BYTES;
+    auto kern = csr_merge_warp_dot_kernel<C::WARPS, C::IPT, C::MINB, RANKED, C::UNI>;
+    int32_t hot_l1 = 0, hot_l2 = 0;
+    if (RANKED)
+        hot_limits(&hot_l1, &hot_l2);
+    static thread_local Residency res;
+    const int32_t ntiles = A->merge_tiles;
+    int64_t grid = 0;
+    SMVP_TRY(persistent_grid(kern, C::WARPS * 32, SMEM, A->merge_headroom, ceil_div64(ntiles, C::WARPS), res, &grid));
+    if (grid > 0)
+    {
+        const bool early = merge_fixup_early(ntiles);
+        SMVP_LAUNCH(kern, (unsigned)grid, C::WARPS * 32, SMEM, s, A->row_ptr, mult_cols(A), A->val, d_x, d_y, A->tile_row, A->rows,
+                    A->nnz, ntiles, A->head_val, A->carry_val, hot_l1, hot_l2, early ? 1 : 0, ab.alpha, ab.beta, dot.w, dot.part);
+        SMVP_TRY(launch_fixup(early, ntiles, s, merge_fixup_dot_kernel, (const int32_t *)A->tile_row, (const double *)A->head_val,
+                              (const double *)A->carry_val, ntiles, d_y, ab.alpha, ab.beta, dot.w, dot.part));
     }
     return SMVP_OK;
 }
@@ -872,14 +739,17 @@ struct PatternShape
     static int stage_bytes(int maxlen) { return (((ROWS * maxlen + 2) * 8 + 15) / 16 * 16 + ROWS + 32 + 127) & ~127; }
 };
 
-template <int WARPS, int R, int STAGES, int CH, int MINB, bool FANOUT, bool EPI>
-__global__ void __launch_bounds__(WARPS * 32, MINB)
-    csr_pattern_kernel(const int32_t *__restrict__ row_ptr, const double *__restrict__ val, const uint8_t *__restrict__ pat_id,
-                       const int32_t *__restrict__ pat_off, const int32_t *__restrict__ pat_len, int32_t npat, int32_t maxlen,
-                       const double *__restrict__ x, double *__restrict__ y, int32_t row_begin, int32_t row_end,
-                       uint32_t stage_bytes, const __grid_constant__ YFan fan, double alpha, double beta)
+// DOT (csr_pattern_dot_kernel): the work unit is the tile of 32 rows; the lanes' dot terms are added in a pairwise tree
+// into part[t].  w[r] is loaded beside the early load of y[r].
+template <int WARPS, int R, int STAGES, int CH, int MINB, bool FANOUT, bool EPI, bool DOT>
+__device__ __forceinline__ void
+csr_pattern_body(const int32_t *__restrict__ row_ptr, const double *__restrict__ val, const uint8_t *__restrict__ pat_id,
+                 const int32_t *__restrict__ pat_off, const int32_t *__restrict__ pat_len, int32_t npat, int32_t maxlen,
+                 const double *__restrict__ x, double *__restrict__ y, int32_t row_begin, int32_t row_end, uint32_t stage_bytes,
+                 const YFan &fan, double alpha, double beta, const double *__restrict__ dot_w, double *__restrict__ part)
 {
     static_assert(!EPI || (R == 1 && !FANOUT), "the epilogue keeps one y value per lane: one round per tile");
+    static_assert(!DOT || EPI, "the dot is formed by the epilogue");
     constexpr int ROWS = PatternShape<R>::ROWS;
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ __align__(8) uint64_t full_bar[WARPS * STAGES];
@@ -951,9 +821,12 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
         if (tn < ntiles && tn > t)
             bounds(tn, &nn0, &nn1);
         // the epilogue's y[r]: issued before the wait for the stage, its latency hides behind the staging and the gathers
-        double y0 = 0.0;
+        double y0 = 0.0, w0 = 0.0;
         if (EPI && beta != 0.0 && row_begin + t * ROWS + lane < row_end)
             y0 = ld_y_early(y + row_begin + t * ROWS + lane);
+        if (DOT && dot_w && row_begin + t * ROWS + lane < row_end)
+            w0 = ld_w_early(dot_w + row_begin + t * ROWS + lane);
+        double d = 0.0; // DOT: the lane's dot term
 
         mbar_wait(&bars[s], (phase >> s) & 1u);
         phase ^= 1u << s;
@@ -1013,11 +886,23 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
             }
             if (live)
             {
-                if (EPI)
+                if (DOT)
+                {
+                    const double v = axpby(alpha, sum, beta, y0);
+                    y[r] = v;
+                    d = __dmul_rn(dot_w ? w0 : v, v);
+                }
+                else if (EPI)
                     y[r] = axpby(alpha, sum, beta, y0);
                 else
                     store_y<FANOUT, false>(y, fan, r, sum, alpha, beta);
             }
+        }
+        if (DOT)
+        {
+            d = warp_tree_sum(d);
+            if (lane == 0)
+                part[t] = d;
         }
         // the stage is consumed: refill it with tile tn
         __syncwarp();
@@ -1029,6 +914,26 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
         t += warp_stride;
         s = s + 1 == STAGES ? 0 : s + 1;
     }
+}
+template <int WARPS, int R, int STAGES, int CH, int MINB, bool FANOUT, bool EPI>
+__global__ void __launch_bounds__(WARPS * 32, MINB)
+    csr_pattern_kernel(const int32_t *__restrict__ row_ptr, const double *__restrict__ val, const uint8_t *__restrict__ pat_id,
+                       const int32_t *__restrict__ pat_off, const int32_t *__restrict__ pat_len, int32_t npat, int32_t maxlen,
+                       const double *__restrict__ x, double *__restrict__ y, int32_t row_begin, int32_t row_end,
+                       uint32_t stage_bytes, const __grid_constant__ YFan fan, double alpha, double beta)
+{
+    csr_pattern_body<WARPS, R, STAGES, CH, MINB, FANOUT, EPI, false>(row_ptr, val, pat_id, pat_off, pat_len, npat, maxlen, x, y, row_begin,
+                                                                    row_end, stage_bytes, fan, alpha, beta, nullptr, nullptr);
+}
+template <int WARPS, int R, int STAGES, int CH, int MINB>
+__global__ void __launch_bounds__(WARPS * 32, MINB)
+    csr_pattern_dot_kernel(const int32_t *__restrict__ row_ptr, const double *__restrict__ val, const uint8_t *__restrict__ pat_id,
+                           const int32_t *__restrict__ pat_off, const int32_t *__restrict__ pat_len, int32_t npat, int32_t maxlen,
+                           const double *__restrict__ x, double *__restrict__ y, int32_t rows, uint32_t stage_bytes, double alpha,
+                           double beta, const double *__restrict__ w, double *__restrict__ part)
+{
+    csr_pattern_body<WARPS, R, STAGES, CH, MINB, false, true, true>(row_ptr, val, pat_id, pat_off, pat_len, npat, maxlen, x, y, 0, rows,
+                                                                   stage_bytes, YFan(), alpha, beta, w, part);
 }
 
 // ---- the pattern kernel's configuration.  Measured on B200 (profiles/r03_logs/sweep_pattern.log, stencil 369^3, the
@@ -1046,7 +951,7 @@ struct PatternCfg
 
 // rows [row_begin, row_end) of a handle with the row-pattern plan
 static int csr_mult_pattern(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, const Axpby &ab, cudaStream_t s,
-                            int32_t row_begin, int32_t row_end)
+                            int32_t row_begin, int32_t row_end, const DotOut *dot = nullptr)
 {
     using C = PatternCfg;
     const int maxlen = A->pattern_maxlen > 0 ? A->pattern_maxlen : 1;
@@ -1054,6 +959,17 @@ static int csr_mult_pattern(const smvp_csr *A, const double *d_x, double *d_y, c
     const int table = (A->pattern_count * (maxlen + 1) * 4 + 127) & ~127;
     const int smem = table + C::WARPS * C::STAGES * stage;
     const int64_t need = ceil_div64(ceil_div64((int64_t)row_end - row_begin, PatternShape<C::R>::ROWS), C::WARPS);
+    if (dot) // whole passes only: the partial of tile t goes to dot->part[t]
+    {
+        auto kern = csr_pattern_dot_kernel<C::WARPS, C::R, C::STAGES, C::CH, C::MINB>;
+        static thread_local Residency res;
+        int64_t grid = 0;
+        SMVP_TRY(persistent_grid(kern, C::WARPS * 32, smem, A->merge_headroom, need, res, &grid));
+        if (grid > 0)
+            SMVP_LAUNCH(kern, (unsigned)grid, C::WARPS * 32, smem, s, A->row_ptr, A->val, A->pat_id, A->pat_off, A->pat_len,
+                        A->pattern_count, maxlen, d_x, d_y, A->rows, (uint32_t)stage, ab.alpha, ab.beta, dot->w, dot->part);
+        return (int)SMVP_OK;
+    }
     return with_flag(fan != nullptr, [&](auto F) {
         return with_flag(!ab.plain(), [&](auto E) {
             constexpr bool FANOUT = decltype(F)::value, EPI = decltype(E)::value;
@@ -1079,25 +995,33 @@ static int csr_mult_pattern(const smvp_csr *A, const double *d_x, double *d_y, c
 constexpr Axpby AXPBY_PLAIN = {1.0, 0.0};
 
 // tiles [tile_begin, tile_end) of the plan; (0, -1) = all
+// dot != NULL: a whole pass with the epilogue whose dot partials go to dot->part (csr_dot_units counts them)
 static int csr_mult_merge(smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, const Axpby &ab, cudaStream_t s,
-                          int32_t tile_begin = 0, int32_t tile_end = -1)
+                          int32_t tile_begin = 0, int32_t tile_end = -1, const DotOut *dot = nullptr)
 {
     // hot / cold split (relabel.cu): whole passes without a fan-out run as y = alpha * hot * x_rel + beta * y, then
-    // y = alpha * cold * x_rel + y (the parts are never split themselves)
+    // y = alpha * cold * x_rel + y (the parts are never split themselves).  The dot is formed by the cold pass, which
+    // stores every row last.
     if (A->split_state == 1 && !fan && tile_begin == 0 && tile_end < 0)
     {
         SMVP_TRY(csr_mult_merge(A->hot, d_x, d_y, nullptr, ab, s));
-        return csr_mult_merge(A->cold, d_x, d_y, nullptr, Axpby{ab.alpha, 1.0}, s);
+        return csr_mult_merge(A->cold, d_x, d_y, nullptr, Axpby{ab.alpha, 1.0}, s, 0, -1, dot);
     }
     // the row-pattern plan serves whole passes (the pipelined host call cuts its ranges on rows: csr_mult_pattern)
     if (A->pattern_state == 1 && tile_begin == 0 && tile_end < 0)
-        return csr_mult_pattern(A, d_x, d_y, fan, ab, s, 0, A->rows);
+        return csr_mult_pattern(A, d_x, d_y, fan, ab, s, 0, A->rows, dot);
     SMVP_TRY(merge_plan(A, s));
     if (tile_end < 0)
         tile_end = A->merge_tiles;
     // a relabelled handle indexes x by popularity rank: the gathers carry cache-retention hints (SMVP_RANKED_HINTS=0: off)
     const bool ranked = (A->relabel_state == 1 || A->ranked_cols == 1) && env_tristate("SMVP_RANKED_HINTS") != -1;
     const bool skewed = merge_skewed(A);
+    if (dot)
+        return with_flag(ranked, [&](auto R) {
+            constexpr bool RANKED = decltype(R)::value;
+            return skewed ? launch_wmerge_dot<MergeSkewed, RANKED>(A, d_x, d_y, ab, *dot, s)
+                          : launch_wmerge_dot<MergeStencil, RANKED>(A, d_x, d_y, ab, *dot, s);
+        });
     return with_flag(fan != nullptr, [&](auto F) {
         return with_flag(ranked, [&](auto R) {
             return with_flag(!ab.plain(), [&](auto E) {
@@ -1110,6 +1034,38 @@ static int csr_mult_merge(smvp_csr *A, const double *d_x, double *d_y, const YFa
             });
         });
     });
+}
+
+// work units of a dot pass with resolved variant v (DESIGN.md §5.7); builds the plan they depend on
+static int csr_dot_units(smvp_csr *A, int v, cudaStream_t s, int64_t *units)
+{
+    if (v == SMVP_CSR_VECTOR)
+        *units = ceil_div64((int64_t)A->rows * vector_lpr(A), 256); // the vector kernel's CTAs
+    else if (A->split_state == 1)
+    {
+        SMVP_TRY(merge_plan(A->cold, s)); // the cold pass's tiles
+        *units = A->cold->merge_tiles;
+    }
+    else if (A->pattern_state == 1)
+        *units = ceil_div64(A->rows, PatternShape<PatternCfg::R>::ROWS);
+    else
+    {
+        SMVP_TRY(merge_plan(A, s));
+        *units = A->merge_tiles;
+    }
+    return SMVP_OK;
+}
+
+// the most work units any plan of the handle can give a dot pass: the scratch is sized for it at the first dot call, so
+// that a later call with another variant or plan never allocates (nor synchronises)
+static int64_t csr_dot_units_max(const smvp_csr *A)
+{
+    constexpr int32_t min_tile = 32 * (MergeSkewed::IPT < MergeStencil::IPT ? MergeSkewed::IPT : MergeStencil::IPT);
+    const int64_t vec = ceil_div64((int64_t)A->rows * vector_lpr(A), 256);
+    const int64_t pat = ceil_div64(A->rows, PatternShape<PatternCfg::R>::ROWS);
+    const int64_t merge = ceil_div64((int64_t)A->rows + A->nnz, min_tile); // also bounds the cold part of a split
+    const int64_t m = vec > pat ? vec : pat;
+    return m > merge ? m : merge;
 }
 
 int csr_resolve_variant(const smvp_csr *A, int variant)
@@ -1129,12 +1085,13 @@ int csr_resolve_variant(const smvp_csr *A, int variant)
 using namespace smvp;
 
 // x is already in the space the kernels index (x itself, or x_rel when the relabelling plan is in use)
-static int csr_mult_launch(smvp_csr *A, const double *x, double *d_y, const YFan *fan, const Axpby &ab, int variant, cudaStream_t s)
+static int csr_mult_launch(smvp_csr *A, const double *x, double *d_y, const YFan *fan, const Axpby &ab, int variant, cudaStream_t s,
+                           const DotOut *dot = nullptr)
 {
     if (A->rows == 0)
         return SMVP_OK;
     const int v = csr_resolve_variant(A, variant);
-    int rc = (v == SMVP_CSR_VECTOR) ? csr_mult_vector(A, x, d_y, fan, ab, s) : csr_mult_merge(A, x, d_y, fan, ab, s);
+    int rc = (v == SMVP_CSR_VECTOR) ? csr_mult_vector(A, x, d_y, fan, ab, dot, s) : csr_mult_merge(A, x, d_y, fan, ab, s, 0, -1, dot);
     if (rc != SMVP_OK)
         return rc;
     SMVP_CUDA(cudaGetLastError());
@@ -1180,13 +1137,20 @@ static int l2_persist_window(cudaStream_t s, const void *base, size_t bytes)
     return SMVP_OK;
 }
 
-static int csr_mult_any(smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, const Axpby &ab, int variant, void *stream)
+// d_dot != NULL: a dot pass (smvp_csr_mult_device_axpby_dot), *d_dot = sum of w[r] * y_new[r] (w = d_w, or y_new)
+static int csr_mult_any(smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, const Axpby &ab, int variant, void *stream,
+                        const double *d_w = nullptr, double *d_dot = nullptr)
 {
     if (variant != SMVP_CSR_AUTO && variant != SMVP_CSR_VECTOR && variant != SMVP_CSR_MERGE)
         return SMVP_E_ARG;
-    if (A->rows == 0)
-        return SMVP_OK;
     cudaStream_t s = (cudaStream_t)stream;
+    if (A->rows == 0)
+    {
+        if (!d_dot)
+            return SMVP_OK;
+        SMVP_TRY(dot_scratch(&A->dot_buf, &A->dot_cap, &A->device_bytes, csr_dot_units_max(A), s));
+        return dot_reduce(A->dot_buf, A->dot_cap, 0, d_dot, s); // no rows: +0.0
+    }
     SMVP_TRY(csr_pattern_plan(A, s)); // decides the relabelling first
     const double *x = d_x; // NULL: the x last given to smvp_csr_set_x_device
     if (A->relabel_state == 1)
@@ -1206,7 +1170,21 @@ static int csr_mult_any(smvp_csr *A, const double *d_x, double *d_y, const YFan 
     const int persist_mb = A->relabel_state == 1 ? env_int("SMVP_L2_PERSIST_MB", 0, 0, 4096) : 0;
     if (persist_mb > 0)
         SMVP_TRY(l2_persist_window(s, x, (size_t)persist_mb << 20));
-    const int rc = csr_mult_launch(A, x, d_y, fan, ab, variant, s);
+    int rc = SMVP_OK;
+    if (!d_dot)
+        rc = csr_mult_launch(A, x, d_y, fan, ab, variant, s);
+    else
+    {
+        int64_t units = 0;
+        rc = csr_dot_units(A, csr_resolve_variant(A, variant), s, &units);
+        if (rc == SMVP_OK)
+            rc = dot_scratch(&A->dot_buf, &A->dot_cap, &A->device_bytes, csr_dot_units_max(A), s);
+        const DotOut dot = {d_w, A->dot_buf};
+        if (rc == SMVP_OK)
+            rc = csr_mult_launch(A, x, d_y, nullptr, ab, variant, s, &dot);
+        if (rc == SMVP_OK)
+            rc = dot_reduce(A->dot_buf, A->dot_cap, units, d_dot, s);
+    }
     if (persist_mb > 0)
         SMVP_TRY(l2_persist_window(s, nullptr, 0));
     return rc;
@@ -1246,6 +1224,19 @@ extern "C" int smvp_csr_mult_device_axpby(smvp_csr *A, double alpha, const doubl
     if (d_y && d_y == (d_x ? d_x : A->x_set))
         return SMVP_E_ARG; // y would be read and written while the kernels gather it as x
     return csr_mult_any(A, d_x, d_y, nullptr, Axpby{alpha, beta}, variant, stream);
+}
+
+extern "C" int smvp_csr_mult_device_axpby_dot(smvp_csr *A, double alpha, const double *d_x, double beta, double *d_y,
+                                              const double *d_w, double *d_dot, int variant, void *stream)
+{
+    if (!A || (A->rows > 0 && !d_y) || !d_dot)
+        return SMVP_E_ARG;
+    const double *x = d_x ? d_x : A->x_set;
+    if (d_y && d_y == x)
+        return SMVP_E_ARG; // y would be read and written while the kernels gather it as x
+    if ((d_w && d_w == d_y) || d_dot == x || d_dot == d_y || d_dot == d_w)
+        return SMVP_E_ARG;
+    return csr_mult_any(A, d_x, d_y, nullptr, Axpby{alpha, beta}, variant, stream, d_w, d_dot);
 }
 
 extern "C" int smvp_csr_mult_device_fanout(smvp_csr *A, const double *d_x, double *const *d_y_list, int n_out, int variant,

@@ -107,6 +107,7 @@ void tjds_release(smvp_tjds *A)
     cudaFree(A->d_xt);
     cudaFree(A->d_yt);
     cudaFree(A->y_sum);
+    cudaFree(A->dot_buf);
     tjds_relabel_release(A);
     delete A;
 }

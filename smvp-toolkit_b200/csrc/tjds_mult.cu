@@ -489,21 +489,20 @@ __global__ void __launch_bounds__(256, MINB) tjds_det_kernel(const int2 *__restr
 
 // row_rank != NULL: the accumulators and row_exp are in popularity-rank order (relabelled handle), y is not.
 // EPI: y[row] = alpha * (row sum) + beta * y[row] (axpby, common.cuh) instead of the row sum.
+// DOT (tjds_det_finalize_dot_kernel): the work unit is the CTA's 256 rows of y; their dot terms are added in a pairwise tree.
 template <bool EPI>
-__global__ void __launch_bounds__(256) tjds_det_finalize_kernel(const long long *__restrict__ acc, const int32_t *__restrict__ row_exp,
-                                                                const int32_t *__restrict__ x_exp, int32_t rows, double *__restrict__ y,
-                                                                const int32_t *__restrict__ row_rank, int words, int32_t r_lo, int32_t r_hi,
-                                                                double alpha, double beta)
+__device__ __forceinline__ double tjds_det_finalize_row(int32_t row, const long long *__restrict__ acc, const int32_t *__restrict__ row_exp,
+                                                        const int32_t *__restrict__ x_exp, int32_t rows, double *__restrict__ y,
+                                                        const int32_t *__restrict__ row_rank, int words, int32_t r_lo, int32_t r_hi,
+                                                        double alpha, double beta)
 {
     // accumulators exist (are cleared and filled) only for rows [r_lo, r_hi) of the index space the kernels use
-    const int32_t row = blockIdx.x * blockDim.x + threadIdx.x;
-    if (row >= rows)
-        return;
     const int32_t r = row_rank ? row_rank[row] : row;
     if (r < r_lo || r >= r_hi)
     {
-        y[row] = EPI ? axpby(alpha, 0.0, beta, beta != 0.0 ? y[row] : 0.0) : 0.0;
-        return;
+        const double v = EPI ? axpby(alpha, 0.0, beta, beta != 0.0 ? y[row] : 0.0) : 0.0;
+        y[row] = v;
+        return v;
     }
     longlong2 a;
     a.x = acc[r];
@@ -516,7 +515,34 @@ __global__ void __launch_bounds__(256) tjds_det_finalize_kernel(const long long 
         const int32_t T = row_exp[r] + *x_exp;
         out = scalbn(s, T - TJDS_FRAC);
     }
-    y[row] = EPI ? axpby(alpha, out, beta, beta != 0.0 ? y[row] : 0.0) : out;
+    const double v = EPI ? axpby(alpha, out, beta, beta != 0.0 ? y[row] : 0.0) : out;
+    y[row] = v;
+    return v;
+}
+template <bool EPI>
+__global__ void __launch_bounds__(256) tjds_det_finalize_kernel(const long long *__restrict__ acc, const int32_t *__restrict__ row_exp,
+                                                                const int32_t *__restrict__ x_exp, int32_t rows, double *__restrict__ y,
+                                                                const int32_t *__restrict__ row_rank, int words, int32_t r_lo, int32_t r_hi,
+                                                                double alpha, double beta)
+{
+    const int32_t row = blockIdx.x * blockDim.x + threadIdx.x;
+    if (row >= rows)
+        return;
+    tjds_det_finalize_row<EPI>(row, acc, row_exp, x_exp, rows, y, row_rank, words, r_lo, r_hi, alpha, beta);
+}
+__global__ void __launch_bounds__(256) tjds_det_finalize_dot_kernel(const long long *__restrict__ acc, const int32_t *__restrict__ row_exp,
+                                                                    const int32_t *__restrict__ x_exp, int32_t rows, double *__restrict__ y,
+                                                                    const int32_t *__restrict__ row_rank, int words, int32_t r_lo,
+                                                                    int32_t r_hi, double alpha, double beta, const double *__restrict__ w,
+                                                                    double *__restrict__ part)
+{
+    const int32_t row = blockIdx.x * blockDim.x + threadIdx.x;
+    double d = 0.0;
+    if (row < rows)
+        d = dot_term(w, row, tjds_det_finalize_row<true>(row, acc, row_exp, x_exp, rows, y, row_rank, words, r_lo, r_hi, alpha, beta));
+    d = cta_tree_sum<256>(d);
+    if (threadIdx.x == 0)
+        part[blockIdx.x] = d;
 }
 
 // y[r] = y_rel[rank[r]]: the atomic variant of a relabelled handle sums in rank order.  EPI: y[r] = alpha * y_rel[rank[r]]
@@ -537,6 +563,19 @@ __global__ void __launch_bounds__(256) tjds_unrank_y_kernel(const double *__rest
             y[r] = __ldg(y_rel + __ldg(row_rank + r));
     }
 }
+// the dot pass's unrank: one row per thread, so that the work unit is a 256-row block of y whatever the grid
+__global__ void __launch_bounds__(256) tjds_unrank_y_dot_kernel(const double *__restrict__ y_rel, const int32_t *__restrict__ row_rank,
+                                                                int32_t rows, double *__restrict__ y, double alpha, double beta,
+                                                                const double *__restrict__ w, double *__restrict__ part)
+{
+    const int32_t r = blockIdx.x * blockDim.x + threadIdx.x;
+    double d = 0.0;
+    if (r < rows)
+        store_axpby_dot(y, r, __ldg(y_rel + (row_rank ? __ldg(row_rank + r) : r)), alpha, beta, w, d);
+    d = cta_tree_sum<256>(d);
+    if (threadIdx.x == 0)
+        part[blockIdx.x] = d;
+}
 
 // ---- transposed product y = A^T x --------------------------------------------------------------------------------
 // Slot q of every diagonal belongs to column perm[q], and the d-th entry of a column is its d-th by row, so
@@ -554,19 +593,28 @@ __device__ __forceinline__ void tr_store(bool epi, double *__restrict__ y, int32
 {
     y[c] = epi ? axpby(alpha, s, beta, beta != 0.0 ? y[c] : 0.0) : s;
 }
-template <bool EPI>
-__global__ void __launch_bounds__(256) tjds_transpose_kernel(const int2 *__restrict__ blocks, const int32_t *__restrict__ start_pos,
-                                                             const int32_t *__restrict__ row_ind, const double *__restrict__ val,
-                                                             const int32_t *__restrict__ perm, const double *__restrict__ x,
-                                                             double *__restrict__ y, double *__restrict__ part,
-                                                             const uint32_t *__restrict__ seg_off, int32_t ndiag, int32_t nslots,
-                                                             int32_t cols, int32_t nlong, double alpha, double beta)
+// DOT (the *_dot_kernel wrappers): a CTA of either kernel is a work unit.  A thread adds the dot terms of the columns it
+// stores in the order it stores them, and the CTA's threads are added in a pairwise tree into dot_part[unit].
+template <bool EPI, bool DOT>
+__device__ __forceinline__ void tjds_transpose_body(const int2 *__restrict__ blocks, const int32_t *__restrict__ start_pos,
+                                                    const int32_t *__restrict__ row_ind, const double *__restrict__ val,
+                                                    const int32_t *__restrict__ perm, const double *__restrict__ x, double *__restrict__ y,
+                                                    double *__restrict__ part, const uint32_t *__restrict__ seg_off, int32_t ndiag,
+                                                    int32_t nslots, int32_t cols, int32_t nlong, double alpha, double beta,
+                                                    const double *__restrict__ dot_w, double *__restrict__ dot_part)
 {
     static_assert(TJDS_SEG % TJDS_TR_UNROLL == 0, "s_sp holds TJDS_SEG + 1 entries");
+    static_assert(!DOT || EPI, "the dot is formed by the epilogue");
     __shared__ int32_t s_sp[TJDS_SEG + 1];
+    double d = 0.0; // DOT: this thread's dot terms
     // empty columns (slots nslots .. cols-1) get +0.0, spread over the whole grid
     for (int64_t p = (int64_t)nslots + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < cols; p += (int64_t)gridDim.x * blockDim.x)
-        tr_store(EPI, y, __ldg(perm + p), 0.0, alpha, beta);
+    {
+        if (DOT)
+            store_axpby_dot(y, __ldg(perm + p), 0.0, alpha, beta, dot_w, d);
+        else
+            tr_store(EPI, y, __ldg(perm + p), 0.0, alpha, beta);
+    }
     const int2 blk = __ldg(blocks + blockIdx.x);
     const int32_t d_begin = blk.x * TJDS_SEG;
     const int32_t nd = min(TJDS_SEG, ndiag - d_begin);
@@ -575,10 +623,11 @@ __global__ void __launch_bounds__(256) tjds_transpose_kernel(const int2 *__restr
         s_sp[threadIdx.x] = __ldg(start_pos + d_begin + min((int32_t)threadIdx.x, nd));
     __syncthreads();
     const int32_t q = blk.y + (int32_t)threadIdx.x;
-    if (q >= s_sp[1] - s_sp[0])
+    const bool has = q < s_sp[1] - s_sp[0];
+    if (!DOT && !has)
         return; // the column at this slot ends before the segment (or the slot is past the table's diagonals)
     double s = 0.0;
-    for (int32_t i0 = 0; i0 < nd; i0 += TJDS_TR_UNROLL)
+    for (int32_t i0 = 0; has && i0 < nd; i0 += TJDS_TR_UNROLL)
     {
         int32_t r[TJDS_TR_UNROLL];
         double v[TJDS_TR_UNROLL], xv[TJDS_TR_UNROLL];
@@ -598,10 +647,43 @@ __global__ void __launch_bounds__(256) tjds_transpose_kernel(const int2 *__restr
             if (r[u] >= 0)
                 s = __dadd_rn(s, __dmul_rn(v[u], xv[u]));
     }
-    if (q >= nlong)
-        tr_store(EPI, y, __ldg(perm + q), s, alpha, beta); // a column of at most TJDS_SEG entries lives in segment 0 alone
-    else
+    if (has && q >= nlong) // a column of at most TJDS_SEG entries lives in segment 0 alone
+    {
+        if (DOT)
+            store_axpby_dot(y, __ldg(perm + q), s, alpha, beta, dot_w, d);
+        else
+            tr_store(EPI, y, __ldg(perm + q), s, alpha, beta);
+    }
+    else if (has)
         part[(int64_t)__ldg(seg_off + blk.x) + q] = s;
+    if (DOT)
+    {
+        d = cta_tree_sum<256>(d);
+        if (threadIdx.x == 0)
+            dot_part[blockIdx.x] = d;
+    }
+}
+template <bool EPI>
+__global__ void __launch_bounds__(256) tjds_transpose_kernel(const int2 *__restrict__ blocks, const int32_t *__restrict__ start_pos,
+                                                             const int32_t *__restrict__ row_ind, const double *__restrict__ val,
+                                                             const int32_t *__restrict__ perm, const double *__restrict__ x,
+                                                             double *__restrict__ y, double *__restrict__ part,
+                                                             const uint32_t *__restrict__ seg_off, int32_t ndiag, int32_t nslots,
+                                                             int32_t cols, int32_t nlong, double alpha, double beta)
+{
+    tjds_transpose_body<EPI, false>(blocks, start_pos, row_ind, val, perm, x, y, part, seg_off, ndiag, nslots, cols, nlong, alpha, beta,
+                                    nullptr, nullptr);
+}
+__global__ void __launch_bounds__(256) tjds_transpose_dot_kernel(const int2 *__restrict__ blocks, const int32_t *__restrict__ start_pos,
+                                                                 const int32_t *__restrict__ row_ind, const double *__restrict__ val,
+                                                                 const int32_t *__restrict__ perm, const double *__restrict__ x,
+                                                                 double *__restrict__ y, double *__restrict__ part,
+                                                                 const uint32_t *__restrict__ seg_off, int32_t ndiag, int32_t nslots,
+                                                                 int32_t cols, int32_t nlong, double alpha, double beta,
+                                                                 const double *__restrict__ w, double *__restrict__ dot_part)
+{
+    tjds_transpose_body<true, true>(blocks, start_pos, row_ind, val, perm, x, y, part, seg_off, ndiag, nslots, cols, nlong, alpha, beta,
+                                    w, dot_part);
 }
 
 // y[perm[q]] = tr_part partials of long column q added left to right from +0.0, chunk 0 first.  Slots [0, nwide) hold
@@ -609,12 +691,14 @@ __global__ void __launch_bounds__(256) tjds_transpose_kernel(const int2 *__restr
 // round, TJDS_TR_ROUNDS rounds ahead, and every lane adds them in order from shuffles (the additions are the serial
 // part, the loads are not).  Slots [nwide, nlong) take one thread each.
 constexpr int TJDS_TR_ROUNDS = 4;
-template <bool EPI>
-__global__ void __launch_bounds__(256) tjds_transpose_combine_kernel(const double *__restrict__ part, const uint32_t *__restrict__ seg_off,
-                                                                     const int32_t *__restrict__ slot_len, const int32_t *__restrict__ perm,
-                                                                     int32_t nlong, int32_t nwide, double *__restrict__ y, double alpha,
-                                                                     double beta)
+template <bool EPI, bool DOT>
+__device__ __forceinline__ void tjds_transpose_combine_body(const double *__restrict__ part, const uint32_t *__restrict__ seg_off,
+                                                            const int32_t *__restrict__ slot_len, const int32_t *__restrict__ perm,
+                                                            int32_t nlong, int32_t nwide, double *__restrict__ y, double alpha, double beta,
+                                                            const double *__restrict__ dot_w, double *__restrict__ dot_part)
 {
+    static_assert(!DOT || EPI, "the dot is formed by the epilogue");
+    double d = 0.0; // DOT: this thread's dot term
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, wide_threads = (int64_t)nwide * 32;
     if (t < wide_threads)
     {
@@ -642,19 +726,56 @@ __global__ void __launch_bounds__(256) tjds_transpose_combine_kernel(const doubl
                 }
         }
         if (lane == 0)
-            tr_store(EPI, y, __ldg(perm + q), s, alpha, beta);
-        return;
+        {
+            if (DOT)
+                store_axpby_dot(y, __ldg(perm + q), s, alpha, beta, dot_w, d);
+            else
+                tr_store(EPI, y, __ldg(perm + q), s, alpha, beta);
+        }
+        if (!DOT)
+            return;
     }
-    const int64_t qq = (int64_t)nwide + (t - wide_threads);
-    if (qq >= nlong)
-        return;
-    const int32_t q = (int32_t)qq;
-    const int32_t nch = (__ldg(slot_len + q) + TJDS_SEG - 1) / TJDS_SEG;
-    double s = 0.0;
+    else
+    {
+        const int64_t qq = (int64_t)nwide + (t - wide_threads);
+        if (!DOT && qq >= nlong)
+            return;
+        if (qq < nlong)
+        {
+            const int32_t q = (int32_t)qq;
+            const int32_t nch = (__ldg(slot_len + q) + TJDS_SEG - 1) / TJDS_SEG;
+            double s = 0.0;
 #pragma unroll 4
-    for (int32_t g = 0; g < nch; g++)
-        s = __dadd_rn(s, __ldg(part + __ldg(seg_off + g) + q));
-    tr_store(EPI, y, __ldg(perm + q), s, alpha, beta);
+            for (int32_t g = 0; g < nch; g++)
+                s = __dadd_rn(s, __ldg(part + __ldg(seg_off + g) + q));
+            if (DOT)
+                store_axpby_dot(y, __ldg(perm + q), s, alpha, beta, dot_w, d);
+            else
+                tr_store(EPI, y, __ldg(perm + q), s, alpha, beta);
+        }
+    }
+    if (DOT)
+    {
+        d = cta_tree_sum<256>(d);
+        if (threadIdx.x == 0)
+            dot_part[blockIdx.x] = d;
+    }
+}
+template <bool EPI>
+__global__ void __launch_bounds__(256) tjds_transpose_combine_kernel(const double *__restrict__ part, const uint32_t *__restrict__ seg_off,
+                                                                     const int32_t *__restrict__ slot_len, const int32_t *__restrict__ perm,
+                                                                     int32_t nlong, int32_t nwide, double *__restrict__ y, double alpha,
+                                                                     double beta)
+{
+    tjds_transpose_combine_body<EPI, false>(part, seg_off, slot_len, perm, nlong, nwide, y, alpha, beta, nullptr, nullptr);
+}
+__global__ void __launch_bounds__(256) tjds_transpose_combine_dot_kernel(const double *__restrict__ part, const uint32_t *__restrict__ seg_off,
+                                                                         const int32_t *__restrict__ slot_len,
+                                                                         const int32_t *__restrict__ perm, int32_t nlong, int32_t nwide,
+                                                                         double *__restrict__ y, double alpha, double beta,
+                                                                         const double *__restrict__ w, double *__restrict__ dot_part)
+{
+    tjds_transpose_combine_body<true, true>(part, seg_off, slot_len, perm, nlong, nwide, y, alpha, beta, w, dot_part);
 }
 
 // y = alpha * (+0.0) + beta * y: the scaled, accumulating transposed product of a handle without entries
@@ -662,6 +783,18 @@ __global__ void __launch_bounds__(256) tjds_axpby_empty_kernel(double *__restric
 {
     for (int32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
         y[i] = axpby(alpha, 0.0, beta, beta != 0.0 ? y[i] : 0.0);
+}
+// its dot pass: one entry per thread, the work unit is a 256-entry block of y
+__global__ void __launch_bounds__(256) tjds_axpby_empty_dot_kernel(double *__restrict__ y, int32_t n, double alpha, double beta,
+                                                                   const double *__restrict__ w, double *__restrict__ part)
+{
+    const int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    double d = 0.0;
+    if (i < n)
+        store_axpby_dot(y, i, 0.0, alpha, beta, w, d);
+    d = cta_tree_sum<256>(d);
+    if (threadIdx.x == 0)
+        part[blockIdx.x] = d;
 }
 
 // partials segment g holds: the long columns (slots [0, nlong), nlong = length of diagonal TJDS_SEG) in segment 0, the
@@ -864,6 +997,48 @@ static int tjds_transpose_prepare(smvp_tjds *A, cudaStream_t s)
 
 constexpr Axpby AXPBY_PLAIN = {1.0, 0.0};
 
+// work units of a transposed dot pass: the CTAs of the gather and of the combine kernel, or of the empty-handle kernel
+static int64_t tjds_transpose_units(const smvp_tjds *A)
+{
+    if (A->ndiag == 0)
+        return ceil_div64(A->cols, 256);
+    const int64_t combine = A->ndiag > TJDS_SEG ? ceil_div64(32 * (int64_t)A->tr_nwide + (A->tr_nlong - A->tr_nwide), 256) : 0;
+    return A->num_seg_blocks + combine;
+}
+
+// the most work units a dot pass of the handle can have: A x (256-row blocks) and, once its plan exists, A^T x -- the
+// scratch is sized for both, so it grows at most once, at the first transposed dot call after an A x one
+static int64_t tjds_dot_units_max(const smvp_tjds *A)
+{
+    const int64_t ax = ceil_div64(A->rows, 256);
+    const int64_t atx = A->cols > 0 && (A->tr_ready || A->ndiag == 0) ? tjds_transpose_units(A) : 0;
+    return ax > atx ? ax : atx;
+}
+
+// the transposed dot pass: the kernels of the epilogue with their dot partials in dot.part (tjds_transpose_units of them)
+static int tjds_transpose_pass_dot(smvp_tjds *A, const double *d_x, double *d_y, const Axpby &ab, const DotOut &dot, cudaStream_t s)
+{
+    if (A->ndiag == 0)
+        SMVP_LAUNCH(tjds_axpby_empty_dot_kernel, (unsigned)ceil_div64(A->cols, 256), 256, 0, s, d_y, A->cols, ab.alpha, ab.beta, dot.w,
+                    dot.part);
+    else
+    {
+        SMVP_LAUNCH(tjds_transpose_dot_kernel, (unsigned)A->num_seg_blocks, 256, 0, s, (const int2 *)A->seg_blocks,
+                    (const int32_t *)A->start_pos, (const int32_t *)A->row_ind, (const double *)A->val, (const int32_t *)A->perm, d_x, d_y,
+                    A->tr_part, (const uint32_t *)A->tr_seg_off, A->ndiag, A->nslots, A->cols, A->tr_nlong, ab.alpha, ab.beta, dot.w,
+                    dot.part);
+        if (A->ndiag > TJDS_SEG)
+        {
+            const int64_t threads = 32 * (int64_t)A->tr_nwide + (A->tr_nlong - A->tr_nwide);
+            SMVP_LAUNCH(tjds_transpose_combine_dot_kernel, (unsigned)ceil_div64(threads, 256), 256, 0, s, (const double *)A->tr_part,
+                        (const uint32_t *)A->tr_seg_off, (const int32_t *)A->slot_len, (const int32_t *)A->perm, A->tr_nlong, A->tr_nwide,
+                        d_y, ab.alpha, ab.beta, dot.w, dot.part + A->num_seg_blocks);
+        }
+    }
+    SMVP_CUDA(cudaGetLastError());
+    return SMVP_OK;
+}
+
 // one transposed pass, asynchronous on s; tjds_transpose_prepare has run and A->cols > 0
 static int tjds_transpose_pass(smvp_tjds *A, const double *d_x, double *d_y, const Axpby &ab, cudaStream_t s)
 {
@@ -928,6 +1103,25 @@ extern "C" int smvp_tjds_mult_transpose_device_axpby(smvp_tjds *A, double alpha,
     return tjds_transpose_pass(A, d_x, d_y, Axpby{alpha, beta}, s);
 }
 
+extern "C" int smvp_tjds_mult_transpose_device_axpby_dot(smvp_tjds *A, double alpha, const double *d_x, double beta, double *d_y,
+                                                         const double *d_w, double *d_dot, void *stream)
+{
+    if (!A || (A->rows > 0 && !d_x) || (A->cols > 0 && !d_y) || !d_dot)
+        return SMVP_E_ARG;
+    if (d_y && d_y == d_x)
+        return SMVP_E_ARG; // y would be read and written while the kernels gather it as x
+    if ((d_w && d_w == d_y) || d_dot == d_x || d_dot == d_y || d_dot == d_w)
+        return SMVP_E_ARG;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (A->cols > 0)
+        SMVP_TRY(tjds_transpose_prepare(A, s));
+    const int64_t units = A->cols > 0 ? tjds_transpose_units(A) : 0;
+    SMVP_TRY(dot_scratch(&A->dot_buf, &A->dot_cap, &A->device_bytes, tjds_dot_units_max(A), s));
+    if (A->cols > 0)
+        SMVP_TRY(tjds_transpose_pass_dot(A, d_x, d_y, Axpby{alpha, beta}, DotOut{d_w, A->dot_buf}, s));
+    return dot_reduce(A->dot_buf, A->dot_cap, units, d_dot, s);
+}
+
 extern "C" int smvp_tjds_mult_transpose(smvp_tjds *A, const double *x_host, double *y_host, int iters, double *ms_each)
 {
     if (!A || iters < 1 || (A->rows > 0 && !x_host) || (A->cols > 0 && !y_host))
@@ -990,7 +1184,7 @@ static int32_t tjds_effective_limit(const smvp_tjds *A, int32_t diag_limit)
 
 // plans, auxiliary arrays and the host-side routing decision: everything that may synchronise, so that the pass
 // itself only enqueues work (and can be captured in a CUDA graph)
-static int tjds_prepare(smvp_tjds *A, int variant, const Axpby &ab, cudaStream_t s)
+static int tjds_prepare(smvp_tjds *A, int variant, const Axpby &ab, cudaStream_t s, bool dot = false)
 {
     if (A->rows == 0)
         return SMVP_OK;
@@ -1003,8 +1197,9 @@ static int tjds_prepare(smvp_tjds *A, int variant, const Axpby &ab, cudaStream_t
         SMVP_TRY(tjds_prepare_det(A, s));
         SMVP_TRY(tjds_det_route(A));
     }
-    // the atomic sums of a natural-order handle land in a scratch vector under the epilogue (relabelled handles use y_rel)
-    if (!ab.plain() && A->relabel_state != 1 && (variant == SMVP_TJDS_ATOMIC || A->det_route != 1) && !A->y_sum)
+    // the atomic sums of a natural-order handle land in a scratch vector under the epilogue (relabelled handles use y_rel);
+    // a dot pass always runs the epilogue
+    if ((!ab.plain() || dot) && A->relabel_state != 1 && (variant == SMVP_TJDS_ATOMIC || A->det_route != 1) && !A->y_sum)
     {
         SMVP_CUDA(dev_alloc(&A->y_sum, A->rows));
         A->device_bytes += 8 * (int64_t)A->rows;
@@ -1014,11 +1209,13 @@ static int tjds_prepare(smvp_tjds *A, int variant, const Axpby &ab, cudaStream_t
 
 #define SMVP_TJDS_ARGS_COMMON (const int2 *)A->seg_blocks, (const int32_t *)A->start_pos, mult_rows(A), (const double *)A->val, (const double *)A->x_perm
 
-// one pass, asynchronous on s; tjds_prepare has run (with the same ab)
-static int tjds_pass(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit, const Axpby &ab, cudaStream_t s)
+// one pass, asynchronous on s; tjds_prepare has run (with the same ab and dot).  dot != NULL: the per-row kernel that
+// stores y (unrank or det-finalize) also leaves the dot partials of its 256-row blocks in dot->part.
+static int tjds_pass(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit, const Axpby &ab, cudaStream_t s,
+                     const DotOut *dot = nullptr)
 {
     const int32_t lim = tjds_effective_limit(A, diag_limit);
-    const bool ranked = A->relabel_state == 1, skew = A->skew == 1, epi = !ab.plain();
+    const bool ranked = A->relabel_state == 1, skew = A->skew == 1, epi = !ab.plain() || dot;
     const unsigned blocks = (unsigned)A->num_seg_blocks;
     if (variant == SMVP_TJDS_ATOMIC || A->det_route != 1)
     {
@@ -1035,7 +1232,10 @@ static int tjds_pass(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit,
             else
                 SMVP_LAUNCH((tjds_atomic_kernel<4, false>), blocks, 256, 0, s, SMVP_TJDS_ARGS_COMMON, d_y, A->nslots, lim);
         }
-        if (ranked || epi)
+        if (dot)
+            SMVP_LAUNCH(tjds_unrank_y_dot_kernel, (unsigned)ceil_div64(A->rows, 256), 256, 0, s, (const double *)d_y,
+                        ranked ? (const int32_t *)A->row_rank : nullptr, A->rows, y_caller, ab.alpha, ab.beta, dot->w, dot->part);
+        else if (ranked || epi)
         {
             int64_t ub = ceil_div64(A->rows, 256 * 4);
             const int64_t cap = (int64_t)device_props().sms * 8;
@@ -1075,28 +1275,47 @@ static int tjds_pass(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit,
                 });
             });
         }
-        with_flag(epi, [&](auto E) {
-            SMVP_LAUNCH(tjds_det_finalize_kernel<decltype(E)::value>, (unsigned)ceil_div64(A->rows, 256), 256, 0, s,
-                        (const long long *)A->acc, (const int32_t *)A->row_exp, (const int32_t *)A->x_exp, A->rows, d_y,
-                        ranked ? (const int32_t *)A->row_rank : nullptr, words, r_lo, r_hi, ab.alpha, ab.beta);
-            return (int)SMVP_OK;
-        });
+        if (dot)
+            SMVP_LAUNCH(tjds_det_finalize_dot_kernel, (unsigned)ceil_div64(A->rows, 256), 256, 0, s, (const long long *)A->acc,
+                        (const int32_t *)A->row_exp, (const int32_t *)A->x_exp, A->rows, d_y,
+                        ranked ? (const int32_t *)A->row_rank : nullptr, words, r_lo, r_hi, ab.alpha, ab.beta, dot->w, dot->part);
+        else
+            with_flag(epi, [&](auto E) {
+                SMVP_LAUNCH(tjds_det_finalize_kernel<decltype(E)::value>, (unsigned)ceil_div64(A->rows, 256), 256, 0, s,
+                            (const long long *)A->acc, (const int32_t *)A->row_exp, (const int32_t *)A->x_exp, A->rows, d_y,
+                            ranked ? (const int32_t *)A->row_rank : nullptr, words, r_lo, r_hi, ab.alpha, ab.beta);
+                return (int)SMVP_OK;
+            });
     }
     SMVP_CUDA(cudaGetLastError());
     return SMVP_OK;
 }
 
-static int tjds_mult_any(smvp_tjds *A, const Axpby &ab, double *d_y, int variant, int32_t diag_limit, void *stream)
+// d_dot != NULL: a dot pass (smvp_tjds_mult_device_axpby_dot), *d_dot = sum of w[r] * y_new[r] (w = d_w, or y_new)
+static int tjds_mult_any(smvp_tjds *A, const Axpby &ab, double *d_y, int variant, int32_t diag_limit, void *stream,
+                         const double *d_w = nullptr, double *d_dot = nullptr)
 {
     if (!A || (A->rows > 0 && !d_y))
         return SMVP_E_ARG;
     if (variant != SMVP_TJDS_ATOMIC && variant != SMVP_TJDS_DETERMINISTIC && variant != SMVP_TJDS_DETERMINISTIC_FAST)
         return SMVP_E_ARG;
-    if (A->rows == 0)
-        return SMVP_OK;
     cudaStream_t s = (cudaStream_t)stream;
-    SMVP_TRY(tjds_prepare(A, variant, ab, s));
-    return tjds_pass(A, d_y, variant, diag_limit, ab, s);
+    if (!d_dot)
+    {
+        if (A->rows == 0)
+            return SMVP_OK;
+        SMVP_TRY(tjds_prepare(A, variant, ab, s));
+        return tjds_pass(A, d_y, variant, diag_limit, ab, s);
+    }
+    const int64_t units = ceil_div64(A->rows, 256); // 256-row blocks of the kernel that stores y
+    SMVP_TRY(tjds_prepare(A, variant, ab, s, true));
+    SMVP_TRY(dot_scratch(&A->dot_buf, &A->dot_cap, &A->device_bytes, tjds_dot_units_max(A), s));
+    if (A->rows > 0)
+    {
+        const DotOut dot = {d_w, A->dot_buf};
+        SMVP_TRY(tjds_pass(A, d_y, variant, diag_limit, ab, s, &dot));
+    }
+    return dot_reduce(A->dot_buf, A->dot_cap, units, d_dot, s);
 }
 
 extern "C" int smvp_tjds_mult_device(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit, void *stream)
@@ -1108,6 +1327,14 @@ extern "C" int smvp_tjds_mult_device_axpby(smvp_tjds *A, double alpha, double be
                                            void *stream)
 {
     return tjds_mult_any(A, Axpby{alpha, beta}, d_y, variant, diag_limit, stream);
+}
+
+extern "C" int smvp_tjds_mult_device_axpby_dot(smvp_tjds *A, double alpha, double beta, double *d_y, const double *d_w, double *d_dot,
+                                               int variant, int32_t diag_limit, void *stream)
+{
+    if (!A || !d_dot || (d_w && d_w == d_y) || d_dot == d_y || d_dot == d_w)
+        return SMVP_E_ARG;
+    return tjds_mult_any(A, Axpby{alpha, beta}, d_y, variant, diag_limit, stream, d_w, d_dot);
 }
 
 extern "C" int smvp_tjds_mult(smvp_tjds *A, const double *x_host, double *y_host, int iters, double *ms_each, int variant,

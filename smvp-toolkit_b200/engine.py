@@ -85,6 +85,9 @@ SIGNATURES = {
     "smvp_csr_mult_device_axpby": (_int, [_vp, _dbl, _vp, _dbl, _vp, _int, _vp]),
     "smvp_tjds_mult_device_axpby": (_int, [_vp, _dbl, _dbl, _vp, _int, _i32, _vp]),
     "smvp_tjds_mult_transpose_device_axpby": (_int, [_vp, _dbl, _vp, _dbl, _vp, _vp]),
+    "smvp_csr_mult_device_axpby_dot": (_int, [_vp, _dbl, _vp, _dbl, _vp, _vp, _vp, _int, _vp]),
+    "smvp_tjds_mult_device_axpby_dot": (_int, [_vp, _dbl, _dbl, _vp, _vp, _vp, _int, _i32, _vp]),
+    "smvp_tjds_mult_transpose_device_axpby_dot": (_int, [_vp, _dbl, _vp, _dbl, _vp, _vp, _vp, _vp]),
     "smvp_csr_info": (_int, [_vp, ctypes.POINTER(_CsrInfo)]),
     "smvp_tjds_info": (_int, [_vp, ctypes.POINTER(_TjdsInfo)]),
     "smvp_csr_export": (_int, [_vp, _vp, _vp, _vp]),
@@ -275,6 +278,13 @@ class CsrMatrix:
         _check(lib().smvp_csr_mult_device_axpby(self._h, alpha, _ptr(d_x), beta, _ptr(d_y), variant, _stream(stream)),
                "smvp_csr_mult_device_axpby")
 
+    def mult_device_axpby_dot(self, alpha, d_x, beta, d_y, d_w, d_dot, variant=CSR_AUTO, stream=None):
+        """mult_device_axpby with d_dot[0] = sum of w[r] * y_new[r] formed in the same pass (d_w=None: w = y_new, the
+        squared norm).  d_dot is a one-element device tensor, overwritten.  See smvp_csr_mult_device_axpby_dot in
+        include/smvp_cuda.h for the order of the sum and its error bound."""
+        _check(lib().smvp_csr_mult_device_axpby_dot(self._h, alpha, _ptr(d_x), beta, _ptr(d_y), _ptr(d_w), _ptr(d_dot), variant,
+                                                    _stream(stream)), "smvp_csr_mult_device_axpby_dot")
+
     @property
     def x_relabel(self):
         """1: the multiply reads popularity-relabelled columns, -1: natural order, 0: not decided yet."""
@@ -402,6 +412,11 @@ class TjdsMatrix:
         _check(lib().smvp_tjds_mult_transpose_device_axpby(self._h, alpha, _ptr(d_x), beta, _ptr(d_y), _stream(stream)),
                "smvp_tjds_mult_transpose_device_axpby")
 
+    def mult_transpose_device_axpby_dot(self, alpha, d_x, beta, d_y, d_w, d_dot, stream=None):
+        """mult_transpose_device_axpby with d_dot[0] = sum over the `cols` entries of w[c] * y_new[c] (d_w=None: w = y_new)."""
+        _check(lib().smvp_tjds_mult_transpose_device_axpby_dot(self._h, alpha, _ptr(d_x), beta, _ptr(d_y), _ptr(d_w), _ptr(d_dot),
+                                                               _stream(stream)), "smvp_tjds_mult_transpose_device_axpby_dot")
+
     def set_x_device(self, d_x, stream=None):
         _check(lib().smvp_tjds_set_x_device(self._h, _ptr(d_x), _stream(stream)), "smvp_tjds_set_x_device")
 
@@ -413,6 +428,11 @@ class TjdsMatrix:
         """One pass y = alpha * A x + beta * y with the x last given to set_x_device (beta == 0: y is not read)."""
         _check(lib().smvp_tjds_mult_device_axpby(self._h, alpha, beta, _ptr(d_y), variant, diag_limit, _stream(stream)),
                "smvp_tjds_mult_device_axpby")
+
+    def mult_device_axpby_dot(self, alpha, beta, d_y, d_w, d_dot, variant=TJDS_ATOMIC, diag_limit=0, stream=None):
+        """mult_device_axpby with d_dot[0] = sum of w[r] * y_new[r] formed in the same pass (d_w=None: w = y_new)."""
+        _check(lib().smvp_tjds_mult_device_axpby_dot(self._h, alpha, beta, _ptr(d_y), _ptr(d_w), _ptr(d_dot), variant, diag_limit,
+                                                     _stream(stream)), "smvp_tjds_mult_device_axpby_dot")
 
     def export(self):
         perm = np.zeros(self.cols, np.int32)
