@@ -184,11 +184,9 @@ int smvp_tjds_mult_transpose(smvp_tjds *A, const double *x_host, double *y_host,
  *                 counts as 0)
  * alpha = 0 does not skip the matrix: the formula holds as written, so an Inf or NaN in A x still propagates.
  * alpha = 1, beta = 0 is the plain call: the same kernels and launches, the same bits.
- * Exceptions, both inherited from the plain pass:
- *   - a CSR handle with the hot / cold split (smvp_csr_info_t.x_split = 1) runs the hot pass with (alpha, beta) and then
- *     the cold pass with (alpha, 1): within 1e-12 normwise, not bit-identical, like the split's plain pass;
- *   - SMVP_TJDS_ATOMIC (and the deterministic variants routed to it, det_route = -1): s_r is the atomic pass's value,
- *     which is not reproducible run to run.  The deterministic variants are bit-exact.
+ * Exception, inherited from the plain pass: SMVP_TJDS_ATOMIC (and the deterministic variants routed to it,
+ * det_route = -1): s_r is the atomic pass's value, which is not reproducible run to run.  The deterministic variants are
+ * bit-exact.
  * Aliasing: d_y may not be the x the kernels read -- for CSR d_x, or the x of smvp_csr_set_x_device when d_x == NULL;
  * for the TJDS transposed call d_x.  Those calls return SMVP_E_ARG; a partial overlap is undefined.  TJDS A x reads the
  * handle's own permuted copy of x, so there d_y may be the caller's x.
@@ -209,7 +207,7 @@ int smvp_tjds_mult_transpose_device_axpby(smvp_tjds *A, double alpha, const doub
  * BiCG's and LSQR's products with A^T -- without a second kernel that reads y (and w) again.
  *
  * y: bit for bit what the matching *_axpby call (same handle, variant, plan, diag_limit and arguments, (1, 0) included)
- *    stores, with its two exceptions unchanged (the hot / cold split, TJDS atomic).
+ *    stores, with its exception unchanged (TJDS atomic).
  * *d_dot = sum over every row r of y of fl(w[r] * y_new[r]) -- for the transposed call the `cols` entries of y.
  *    d_w == NULL means w = y_new (||y_new||^2); d_w may be the x the kernels read (CG's p^T A p).  d_dot is ONE device
  *    double, overwritten (never accumulated), written on `stream`.  When every term is zero (no rows; a handle without
@@ -219,7 +217,6 @@ int smvp_tjds_mult_transpose_device_axpby(smvp_tjds *A, double alpha, const doub
  *        CSR row-pattern plan         a tile of 32 rows                       products added in a pairwise tree    d = 5
  *        CSR merge-path plan          a warp tile (its row ends, lane by lane, then a pairwise tree over the lanes) plus
  *                                     the fix-up's first row of the tile                                            d = 20
- *        CSR hot / cold split         the cold pass's merge-path tiles (the hot pass forms no dot)                 d = 20
  *        CSR vector variant           the rows of one 256-thread CTA, pairwise tree over the threads               d = 8
  *        TJDS A x (every variant)     a block of 256 rows of y, pairwise tree                                       d = 8
  *        TJDS A^T x                   one CTA of the gather (its empty columns, then its short column) or of the
@@ -262,11 +259,6 @@ typedef struct smvp_csr_info_t
     int32_t x_relabel;        /* multiply plan: 1 = the kernels read popularity-relabelled column indices
                                  and a permuted copy of x (row sums keep their order: y is bit-identical),
                                  -1 = natural order kept, 0 = not decided yet (decided at the first pass) */
-    int32_t x_split;          /* multiply plan of a relabelled handle: 1 = the merge-path multiply runs in two passes, the
-                                 entries whose column is among the 4 Mi most popular (their part of x stays in L2) and
-                                 the others (y += ...): a row sum is then taken in two parts -- within 1e-12, not
-                                 bit-identical to the one-pass order; -1 = one pass (the default: the split is an
-                                 opt-in experiment, SMVP_CSR_SPLIT=1, that loses on R-MAT); 0 = not decided yet   */
     int32_t row_patterns;     /* multiply plan: P > 0 = every row's column offsets (col - row) are one of P lists of at most
                                  32 entries (stencils, banded matrices); the merge variant then streams a one-byte pattern id
                                  per row instead of col_ind and sums each row in the reference's order (y bit-identical to

@@ -249,7 +249,6 @@ struct smvp_csr
     double *d_x, *d_y;
     // plan of the pipelined host-vector pass (csr_mult.cu): tile ranges, the rows each completes and how much of x
     // (a leading part, x arrives front to back) each reads.  Host-side copies; pipe_cfg = tile size they were cut for.
-    int32_t pipe_ramp;                       // 1: the ranges were cut with the ramped piece profile (SMVP_PIPE_PROFILE)
     int32_t pipe_cfg, pipe_ranges, pipe_xlo; // pipe_xlo: first entry of x any nonzero reads (rounded down to 64)
     int32_t pipe_tile[65], pipe_row[65], pipe_xneed[64];
     void *pipe_res; // streams and events of that pass, created on first use (csr_mult.cu)
@@ -259,12 +258,6 @@ struct smvp_csr
     int32_t *x_order;    // [cols] column with rank p
     double *x_rel;       // [cols] x in rank order
     const double *x_set; // the x last given to smvp_csr_set_x_device (caller-owned)
-    // hot / cold split of a relabelled handle (relabel.cu): two CSR matrices over the SAME rank-ordered column space,
-    // `hot` holding the entries whose column rank is below the L2-resident prefix of x_rel, `cold` the others.  The
-    // merge-path multiply runs hot (every gather an L2 hit) then cold (+=).  0 undecided, 1 in use, -1 not used.
-    int32_t split_state;
-    int32_t ranked_cols; // 1: col_ind already holds popularity ranks (a hot / cold part): the ranked gather hints apply
-    smvp_csr *hot, *cold;
     // row-pattern plan (pattern.cu): 0 undecided, 1 in use, -1 not used.  Row r's k-th nonzero sits in column
     // r + pat_off[pat_id[r] * PAT_LMAX + k]; the multiply reads pat_id instead of col_ind.
     int32_t pattern_state;
@@ -282,15 +275,8 @@ void csr_pipe_release(smvp_csr *A);                                // csr_mult.c
 int csr_relabel_plan(smvp_csr *A, cudaStream_t s);                 // relabel.cu
 int csr_relabel_x(smvp_csr *A, const double *d_x, cudaStream_t s); // relabel.cu
 void csr_relabel_release(smvp_csr *A);                             // relabel.cu
-int csr_split_plan(smvp_csr *A, cudaStream_t s);                   // relabel.cu: after csr_relabel_plan
-int32_t hot_l2_entries(); // relabel.cu: rank-ordered x entries expected to stay L2-resident (SMVP_HOT_L2)
 int csr_pattern_plan(smvp_csr *A, cudaStream_t s);                // pattern.cu: decides the relabelling first
 void csr_pattern_release(smvp_csr *A);                             // pattern.cu
-void csr_release(smvp_csr *A);                                     // csr_build.cu
-int csr_build_impl(const int32_t *d_row, const int32_t *d_col, const double *d_val, int32_t rows, int32_t cols, int64_t nnz,
-                   smvp_csr *A, cudaStream_t s);                   // csr_build.cu
-// row_of[j] = row of nonzero j, from row_ptr[rows+1] (asynchronous on s)
-int csr_expand_rows(const int32_t *row_ptr, int32_t rows, int64_t nnz, int32_t *row_of, cudaStream_t s); // csr_build.cu
 } // namespace smvp
 
 struct smvp_tjds

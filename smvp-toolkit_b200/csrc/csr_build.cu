@@ -51,7 +51,8 @@ __global__ void __launch_bounds__(256) expand_rows_kernel(const int32_t *__restr
     }
 }
 
-int csr_expand_rows(const int32_t *row_ptr, int32_t rows, int64_t nnz, int32_t *row_of, cudaStream_t s)
+// row_of[j] = row of nonzero j, from row_ptr[rows+1] (asynchronous on s)
+static int csr_expand_rows(const int32_t *row_ptr, int32_t rows, int64_t nnz, int32_t *row_of, cudaStream_t s)
 {
     if (nnz == 0)
         return SMVP_OK;
@@ -61,12 +62,10 @@ int csr_expand_rows(const int32_t *row_ptr, int32_t rows, int64_t nnz, int32_t *
     return SMVP_OK;
 }
 
-void csr_release(smvp_csr *A)
+static void csr_release(smvp_csr *A)
 {
     if (!A)
         return;
-    csr_release(A->hot);
-    csr_release(A->cold);
     cudaFree(A->row_ptr);
     cudaFree(A->col_ind);
     cudaFree(A->val);
@@ -82,7 +81,7 @@ void csr_release(smvp_csr *A)
     delete A;
 }
 
-int csr_build_impl(const int32_t *d_row, const int32_t *d_col, const double *d_val, int32_t rows, int32_t cols,
+static int csr_build_impl(const int32_t *d_row, const int32_t *d_col, const double *d_val, int32_t rows, int32_t cols,
                           int64_t nnz, smvp_csr *A, cudaStream_t s)
 {
     int order = ORDER_ROW_COL;
@@ -213,7 +212,7 @@ extern "C" int smvp_csr_build(const smvp_coo *coo, int32_t rows, int32_t cols, i
 
 // A^T from A's arrays: the entries of A, read in its (row, col) order, are the entries of A^T in (col, row) order, so
 // coo_inspect reports ORDER_COL_ROW and the build's stable sort on the row key alone keeps each row of A^T in ascending
-// column order.  A's natural col_ind is read whatever plan A uses (relabelled and split handles keep it).
+// column order.  A's natural col_ind is read whatever plan A uses (a relabelled handle keeps it).
 extern "C" int smvp_csr_transpose(const smvp_csr *A, smvp_csr **out)
 {
     if (!out)

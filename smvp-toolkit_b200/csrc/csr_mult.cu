@@ -75,6 +75,9 @@ __device__ __forceinline__ uint64_t l2_evict_last_policy()
 // x gather of a popularity-relabelled matrix (relabel.cu): the column index IS the popularity rank, so the
 // load can say how long the line deserves to live.  rank < hot_l1: keep in L1; rank < hot_l2: keep in L2
 // (evict-last) while the matrix streams and the cold gathers pass through evict-first and do not allocate in L1.
+// Every other L1 / L2 size measured on R-MAT scale 26 lost (DESIGN.md §5.4).
+constexpr int32_t HOT_L1_ENTRIES = 8192;    // 64 KB of x
+constexpr int32_t HOT_L2_ENTRIES = 4 << 20; // 32 MB of x
 __device__ __forceinline__ double ldg_x_ranked(const double *x, int32_t c, int32_t hot_l1, int32_t hot_l2, uint64_t pol_last,
                                                uint64_t pol_first)
 {
@@ -142,9 +145,9 @@ struct YFan
     double *p[SMVP_MAX_FANOUT];
     int n;
 };
-// EPI (the *_axpby calls and the second pass of a hot / cold split, never with a fan-out): y[row] = alpha * v + beta *
-// y[row] (axpby, common.cuh).  Every row has exactly one writer in a pass (the lane that ends it, or the fix-up kernel for
-// rows cut by tile boundaries), so the read-modify-write is safe.
+// EPI (the *_axpby calls, never with a fan-out): y[row] = alpha * v + beta * y[row] (axpby, common.cuh).  Every row has
+// exactly one writer in a pass (the lane that ends it, or the fix-up kernel for rows cut by tile boundaries), so the
+// read-modify-write is safe.
 template <bool FANOUT, bool EPI>
 __device__ __forceinline__ void store_y(double *__restrict__ y, const YFan &fan, int64_t row, double v, double alpha, double beta)
 {
@@ -601,13 +604,6 @@ static int merge_plan(smvp_csr *A, cudaStream_t s)
     return SMVP_OK;
 }
 
-// how much of the rank-ordered x a relabelled multiply asks L1 / L2 to retain (entries; SMVP_HOT_L1 / SMVP_HOT_L2)
-static void hot_limits(int32_t *l1, int32_t *l2)
-{
-    *l1 = env_int("SMVP_HOT_L1", 8192, 0, INT32_MAX); // 64 KB
-    *l2 = hot_l2_entries();                           // 32 MB
-}
-
 // Persistent grid with a static stride over the tiles: the CTAs that fit on the device at once, at most `need`.
 // smvp_csr_set_corunner_headroom / SMVP_MERGE_HEADROOM=k: leave room for k more CTAs per SM.  Every CTA must be resident
 // from the start: a CTA that has to wait for a co-running kernel's CTA to retire (the exchange kernel of the multi-GPU
@@ -679,9 +675,7 @@ static int launch_wmerge(const smvp_csr *A, const double *d_x, double *d_y, cons
 {
     constexpr int SMEM = C::WARPS * MergeShape<32, C::IPT>::SMEM_BYTES;
     auto kern = csr_merge_warp_kernel<C::WARPS, C::IPT, C::MINB, FANOUT, RANKED, C::UNI, EPI>;
-    int32_t hot_l1 = 0, hot_l2 = 0;
-    if (RANKED)
-        hot_limits(&hot_l1, &hot_l2);
+    const int32_t hot_l1 = RANKED ? HOT_L1_ENTRIES : 0, hot_l2 = RANKED ? HOT_L2_ENTRIES : 0;
     const YFan fan = fanp ? *fanp : YFan();
     static thread_local Residency res;
     const int32_t ntiles = tile_end - tile_begin;
@@ -704,9 +698,7 @@ static int launch_wmerge_dot(const smvp_csr *A, const double *d_x, double *d_y, 
 {
     constexpr int SMEM = C::WARPS * MergeShape<32, C::IPT>::SMEM_BYTES;
     auto kern = csr_merge_warp_dot_kernel<C::WARPS, C::IPT, C::MINB, RANKED, C::UNI>;
-    int32_t hot_l1 = 0, hot_l2 = 0;
-    if (RANKED)
-        hot_limits(&hot_l1, &hot_l2);
+    const int32_t hot_l1 = RANKED ? HOT_L1_ENTRIES : 0, hot_l2 = RANKED ? HOT_L2_ENTRIES : 0;
     static thread_local Residency res;
     const int32_t ntiles = A->merge_tiles;
     int64_t grid = 0;
@@ -999,22 +991,15 @@ constexpr Axpby AXPBY_PLAIN = {1.0, 0.0};
 static int csr_mult_merge(smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, const Axpby &ab, cudaStream_t s,
                           int32_t tile_begin = 0, int32_t tile_end = -1, const DotOut *dot = nullptr)
 {
-    // hot / cold split (relabel.cu): whole passes without a fan-out run as y = alpha * hot * x_rel + beta * y, then
-    // y = alpha * cold * x_rel + y (the parts are never split themselves).  The dot is formed by the cold pass, which
-    // stores every row last.
-    if (A->split_state == 1 && !fan && tile_begin == 0 && tile_end < 0)
-    {
-        SMVP_TRY(csr_mult_merge(A->hot, d_x, d_y, nullptr, ab, s));
-        return csr_mult_merge(A->cold, d_x, d_y, nullptr, Axpby{ab.alpha, 1.0}, s, 0, -1, dot);
-    }
     // the row-pattern plan serves whole passes (the pipelined host call cuts its ranges on rows: csr_mult_pattern)
     if (A->pattern_state == 1 && tile_begin == 0 && tile_end < 0)
         return csr_mult_pattern(A, d_x, d_y, fan, ab, s, 0, A->rows, dot);
     SMVP_TRY(merge_plan(A, s));
     if (tile_end < 0)
         tile_end = A->merge_tiles;
-    // a relabelled handle indexes x by popularity rank: the gathers carry cache-retention hints (SMVP_RANKED_HINTS=0: off)
-    const bool ranked = (A->relabel_state == 1 || A->ranked_cols == 1) && env_tristate("SMVP_RANKED_HINTS") != -1;
+    // a relabelled handle indexes x by popularity rank: the gathers carry cache-retention hints (without them: 7.62 against
+    // 6.69 ms on R-MAT scale 26, DESIGN.md §5.4)
+    const bool ranked = A->relabel_state == 1;
     const bool skewed = merge_skewed(A);
     if (dot)
         return with_flag(ranked, [&](auto R) {
@@ -1041,11 +1026,6 @@ static int csr_dot_units(smvp_csr *A, int v, cudaStream_t s, int64_t *units)
 {
     if (v == SMVP_CSR_VECTOR)
         *units = ceil_div64((int64_t)A->rows * vector_lpr(A), 256); // the vector kernel's CTAs
-    else if (A->split_state == 1)
-    {
-        SMVP_TRY(merge_plan(A->cold, s)); // the cold pass's tiles
-        *units = A->cold->merge_tiles;
-    }
     else if (A->pattern_state == 1)
         *units = ceil_div64(A->rows, PatternShape<PatternCfg::R>::ROWS);
     else
@@ -1063,7 +1043,7 @@ static int64_t csr_dot_units_max(const smvp_csr *A)
     constexpr int32_t min_tile = 32 * (MergeSkewed::IPT < MergeStencil::IPT ? MergeSkewed::IPT : MergeStencil::IPT);
     const int64_t vec = ceil_div64((int64_t)A->rows * vector_lpr(A), 256);
     const int64_t pat = ceil_div64(A->rows, PatternShape<PatternCfg::R>::ROWS);
-    const int64_t merge = ceil_div64((int64_t)A->rows + A->nnz, min_tile); // also bounds the cold part of a split
+    const int64_t merge = ceil_div64((int64_t)A->rows + A->nnz, min_tile);
     const int64_t m = vec > pat ? vec : pat;
     return m > merge ? m : merge;
 }
@@ -1098,45 +1078,6 @@ static int csr_mult_launch(smvp_csr *A, const double *x, double *d_y, const YFan
     return SMVP_OK;
 }
 
-// L2 persisting carve-out for the hot prefix of a relabelled x (tuning hook SMVP_L2_PERSIST_MB, off by default): the
-// top-ranked entries of x_rel are declared "persisting" for the stream of the pass, everything else streams.
-static int l2_persist_window(cudaStream_t s, const void *base, size_t bytes)
-{
-    static thread_local int dev_done = -1;
-    static thread_local size_t max_win = 0, max_persist = 0;
-    int dev = 0;
-    SMVP_CUDA(cudaGetDevice(&dev));
-    if (dev_done != dev)
-    {
-        int v = 0;
-        SMVP_CUDA(cudaDeviceGetAttribute(&v, cudaDevAttrMaxAccessPolicyWindowSize, dev));
-        max_win = (size_t)v;
-        SMVP_CUDA(cudaDeviceGetAttribute(&v, cudaDevAttrMaxPersistingL2CacheSize, dev));
-        max_persist = (size_t)v;
-        dev_done = dev;
-    }
-    cudaStreamAttrValue attr = {};
-    if (bytes > 0)
-    {
-        if (bytes > max_win)
-            bytes = max_win;
-        SMVP_CUDA(cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, bytes < max_persist ? bytes : max_persist));
-        attr.accessPolicyWindow.base_ptr = const_cast<void *>(base);
-        attr.accessPolicyWindow.num_bytes = bytes;
-        attr.accessPolicyWindow.hitRatio = bytes <= max_persist ? 1.0f : (float)max_persist / (float)bytes;
-        attr.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-        attr.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-    }
-    else
-    {
-        attr.accessPolicyWindow.num_bytes = 0;
-        attr.accessPolicyWindow.hitProp = cudaAccessPropertyNormal;
-        attr.accessPolicyWindow.missProp = cudaAccessPropertyNormal;
-    }
-    SMVP_CUDA(cudaStreamSetAttribute(s, cudaStreamAttributeAccessPolicyWindow, &attr));
-    return SMVP_OK;
-}
-
 // d_dot != NULL: a dot pass (smvp_csr_mult_device_axpby_dot), *d_dot = sum of w[r] * y_new[r] (w = d_w, or y_new)
 static int csr_mult_any(smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, const Axpby &ab, int variant, void *stream,
                         const double *d_w = nullptr, double *d_dot = nullptr)
@@ -1167,27 +1108,14 @@ static int csr_mult_any(smvp_csr *A, const double *d_x, double *d_y, const YFan 
         if (!x && A->cols > 0)
             return SMVP_E_ARG;
     }
-    const int persist_mb = A->relabel_state == 1 ? env_int("SMVP_L2_PERSIST_MB", 0, 0, 4096) : 0;
-    if (persist_mb > 0)
-        SMVP_TRY(l2_persist_window(s, x, (size_t)persist_mb << 20));
-    int rc = SMVP_OK;
     if (!d_dot)
-        rc = csr_mult_launch(A, x, d_y, fan, ab, variant, s);
-    else
-    {
-        int64_t units = 0;
-        rc = csr_dot_units(A, csr_resolve_variant(A, variant), s, &units);
-        if (rc == SMVP_OK)
-            rc = dot_scratch(&A->dot_buf, &A->dot_cap, &A->device_bytes, csr_dot_units_max(A), s);
-        const DotOut dot = {d_w, A->dot_buf};
-        if (rc == SMVP_OK)
-            rc = csr_mult_launch(A, x, d_y, nullptr, ab, variant, s, &dot);
-        if (rc == SMVP_OK)
-            rc = dot_reduce(A->dot_buf, A->dot_cap, units, d_dot, s);
-    }
-    if (persist_mb > 0)
-        SMVP_TRY(l2_persist_window(s, nullptr, 0));
-    return rc;
+        return csr_mult_launch(A, x, d_y, fan, ab, variant, s);
+    int64_t units = 0;
+    SMVP_TRY(csr_dot_units(A, csr_resolve_variant(A, variant), s, &units));
+    SMVP_TRY(dot_scratch(&A->dot_buf, &A->dot_cap, &A->device_bytes, csr_dot_units_max(A), s));
+    const DotOut dot = {d_w, A->dot_buf};
+    SMVP_TRY(csr_mult_launch(A, x, d_y, nullptr, ab, variant, s, &dot));
+    return dot_reduce(A->dot_buf, A->dot_cap, units, d_dot, s);
 }
 
 extern "C" int smvp_csr_set_x_device(smvp_csr *A, const double *d_x, void *stream)
@@ -1266,17 +1194,17 @@ extern "C" int smvp_csr_mult_device_fanout(smvp_csr *A, const double *d_x, doubl
 // With iters == 1 both happen in the same pass and the call costs about ONE vector transfer (PCIe is full
 // duplex) instead of upload + multiply + download back to back.  ms_each still reports the multiply alone: the
 // sum of the ranges' own event brackets, each opened after the range's wait for x.
-constexpr int PIPE_MAX_RANGES = 64;   // == capacity of smvp_csr::pipe_tile / pipe_row / pipe_xneed (common.cuh)
-constexpr int PIPE_MAX_XCHUNKS = 128;
+constexpr int PIPE_MAX_RANGES = 64;  // == capacity of smvp_csr::pipe_tile / pipe_row / pipe_xneed (common.cuh)
+constexpr int PIPE_MAX_XCHUNKS = 64;
 
-// defaults from the sweep on B200 (tools/sweep_e2e.py, profiles/): tuning hooks SMVP_PIPE_RANGES / SMVP_PIPE_XCHUNKS
-// Piece SIZE, not piece count, is fixed, so the fixed cost of a call shrinks with the block a rank owns (round 1: e2e did
-// not scale with N).  6 MB in both directions: on the 402 MB vectors of the 369^3 stencil that is 64 ranges x 64 upload
-// pieces, the best of every sweep (tools/sweep_e2e.py with SMVP_PIPE_TRACE=1, round 2: 9.8 ms per call against 12.2 ms
-// for 32 x 64 and 11.2 ms for 16 x 16 in the same run; the PCIe floor with both directions busy is 8.05 ms).  The trace
-// shows why the numbers scatter: with both directions busy the UPLOAD of the 402 MB ends anywhere between 8.3 and 11.5 ms
-// depending on how the pieces of the two directions interleave, equal-sized pieces interleave best.  Price: a pass cut
-// into 64 ranges spends 5.7 ms of GPU time instead of 2.7 (short launches), which is what ms_each reports for it.
+// Piece sizes from the sweep on B200 (DESIGN.md §6, profiles/).  Piece SIZE, not piece count, is fixed, so the fixed cost
+// of a call shrinks with the block a rank owns (round 1: e2e did not scale with N).  6 MB in both directions: on the
+// 402 MB vectors of the 369^3 stencil that is 64 ranges x 64 upload pieces, the best of every sweep (round 2: 9.8 ms per
+// call against 12.2 ms for 32 x 64 and 11.2 ms for 16 x 16 in the same run; the PCIe floor with both directions busy is
+// 8.05 ms).  SMVP_PIPE_TRACE=1 shows why the numbers scatter: with both directions busy the UPLOAD of the 402 MB ends
+// anywhere between 8.3 and 11.5 ms depending on how the pieces of the two directions interleave, equal-sized pieces
+// interleave best.  Price: a pass cut into 64 ranges spends 5.7 ms of GPU time instead of 2.7 (short launches), which is
+// what ms_each reports for it.
 // Shorter vectors (the row block of one GPU out of N) download in 12 MB pieces: 17 ranges x 33 upload pieces measured
 // 6.8 ms per call on the 201 MB blocks of 2 GPUs, 32 x 33 measured 7.95 ms.
 constexpr int64_t PIPE_DOWN_PIECE_BYTES = 12 << 20;
@@ -1285,52 +1213,21 @@ constexpr int64_t PIPE_UP_PIECE_BYTES = 6 << 20;
 static int pipe_ranges(int64_t y_bytes)
 {
     const int64_t want = ceil_div64(y_bytes, y_bytes >= (300ll << 20) ? PIPE_DOWN_PIECE_BYTES_LONG : PIPE_DOWN_PIECE_BYTES);
-    return env_int("SMVP_PIPE_RANGES", (int)(want < 2 ? 2 : (want > 64 ? 64 : want)), 1, PIPE_MAX_RANGES);
+    return (int)(want < 2 ? 2 : (want > PIPE_MAX_RANGES ? PIPE_MAX_RANGES : want));
 }
 static int pipe_xchunks(int64_t x_bytes)
 {
     const int64_t want = ceil_div64(x_bytes, PIPE_UP_PIECE_BYTES);
-    return env_int("SMVP_PIPE_XCHUNKS", (int)(want < 2 ? 2 : (want > 64 ? 64 : want)), 1, PIPE_MAX_XCHUNKS);
+    return (int)(want < 2 ? 2 : (want > PIPE_MAX_XCHUNKS ? PIPE_MAX_XCHUNKS : want));
 }
 
-// Piece boundaries as fractions of the whole (f[0] = 0 ... f[n] = 1).  SMVP_PIPE_PROFILE=ramp (tuning hook): small pieces at
-// both ends, large ones in the middle -- 2, 4, 8, 16 MB, then 24 MB pieces, then 16, 8, 4, 2 MB.  The first range can start
-// (and the first rows go down) after 2 MB instead of 6, the tail after the last upload is one 2 MB piece, and the long
-// middle uses transfers large enough for both PCIe directions to run near their rate.  MEASURED: it loses -- 10.9 ms per call
-// against 9.8 ms for 64 x 64 equal 6 MB pieces in the same run (the upload ends at 9.9 instead of 9.2 ms: with both
-// directions busy, many small equal pieces interleave better than a few large ones).  Default: n equal pieces.
-static bool pipe_ramp()
+// n equal pieces: boundaries f[0] = 0 ... f[n] = 1 as fractions of the whole.  (Ramped pieces -- 2, 4, 8, 16 MB at both
+// ends, 24 MB in the middle -- lost: 10.9 ms per call against 9.8 ms; with both directions busy, many small equal pieces
+// interleave better than a few large ones.)
+static void pipe_profile(int n, double *f)
 {
-    const char *pe = env_str("SMVP_PIPE_PROFILE");
-    return pe && pe[0] == 'r';
-}
-static int pipe_profile(int64_t bytes, int n_uniform, int max_pieces, double *f)
-{
-    const bool ramp = pipe_ramp();
-    const int64_t MB = 1 << 20;
-    const int64_t ends[4] = {2 * MB, 4 * MB, 8 * MB, 16 * MB};
-    const int64_t big = 24 * MB, ends_sum = 2 * (2 + 4 + 8 + 16) * MB;
-    int n = 0;
-    if (ramp && bytes >= ends_sum + 2 * big)
-    {
-        const int64_t mid = bytes - ends_sum;
-        int nmid = (int)ceil_div64(mid, big);
-        if (8 + nmid > max_pieces)
-            nmid = max_pieces - 8;
-        double at = 0.0;
-        f[n++] = 0.0;
-        for (int i = 0; i < 4; i++)
-            f[n++] = (at += (double)ends[i] / (double)bytes);
-        for (int i = 0; i < nmid; i++)
-            f[n++] = (at += (double)mid / nmid / (double)bytes);
-        for (int i = 3; i >= 0; i--)
-            f[n++] = (at += (double)ends[i] / (double)bytes);
-        f[n - 1] = 1.0;
-        return n - 1;
-    }
-    for (int i = 0; i <= n_uniform; i++)
-        f[i] = (double)i / n_uniform;
-    return n_uniform;
+    for (int i = 0; i <= n; i++)
+        f[i] = (double)i / n;
 }
 
 // largest and smallest column index among nonzeros [n0, n1): out[0] = max (start -1), out[1] = min (start INT32_MAX)
@@ -1365,13 +1262,12 @@ static int pipe_plan(smvp_csr *A)
     const bool pat = A->pattern_state == 1;
     if (!pat)
         SMVP_TRY(merge_plan(A, 0));
-    double rf[PIPE_MAX_RANGES + 1];
-    const int NR = pipe_profile(8 * (int64_t)A->rows, pipe_ranges(8 * (int64_t)A->rows), PIPE_MAX_RANGES, rf);
-    const int ramp = pipe_ramp() ? 1 : 0;
+    const int NR = pipe_ranges(8 * (int64_t)A->rows);
     const int32_t key = pat ? PIPE_CFG_PATTERN : A->merge_cfg;
-    if (A->pipe_cfg == key && A->pipe_ranges == NR && A->pipe_ramp == ramp)
+    if (A->pipe_cfg == key && A->pipe_ranges == NR)
         return SMVP_OK;
-    A->pipe_ramp = ramp;
+    double rf[PIPE_MAX_RANGES + 1];
+    pipe_profile(NR, rf);
     const int32_t T = pat ? 0 : A->merge_tiles;
     const int64_t tile_items = pat ? 0 : A->merge_cfg;
     int32_t *d_max = nullptr; // per range: {largest, smallest} column index
@@ -1431,15 +1327,11 @@ static int pipe_plan(smvp_csr *A)
     return SMVP_OK;
 }
 
-constexpr int PIPE_MAX_STREAMS = 4;
-// pieces may alternate over several streams per direction (SMVP_PIPE_STREAMS).  Measured on B200 (profiles/r01_logs/
-// e2e_sweep.log): one stream 10.15 ms per call, two 11.9 ms, three 13.2 ms -- concurrent pieces only share the link
-// and finish later, so one stream per direction is the default
-static int pipe_streams() { return env_int("SMVP_PIPE_STREAMS", 1, 1, PIPE_MAX_STREAMS); }
-
+// One stream per direction: pieces on two or three streams per direction only share the link and finish later (10.15 ms
+// per call with one, 11.9 with two, 13.2 with three; profiles/r01_logs/e2e_sweep.log).
 struct PipeResources
 {
-    cudaStream_t up[PIPE_MAX_STREAMS] = {}, down[PIPE_MAX_STREAMS] = {}, compute = nullptr;
+    cudaStream_t up = nullptr, down = nullptr, compute = nullptr;
     cudaEvent_t x_ready[PIPE_MAX_XCHUNKS] = {}, done[PIPE_MAX_RANGES] = {}, t0[PIPE_MAX_RANGES] = {}, t1[PIPE_MAX_RANGES] = {};
     cudaEvent_t begin = nullptr, down_done[PIPE_MAX_RANGES] = {};
     cudaError_t create()
@@ -1449,12 +1341,10 @@ struct PipeResources
         cudaError_t e = cudaStreamCreateWithFlags(&compute, cudaStreamNonBlocking);
         if (e == cudaSuccess)
             e = cudaEventCreate(&begin);
-        for (int k = 0; k < PIPE_MAX_STREAMS && e == cudaSuccess; k++)
-        {
-            e = cudaStreamCreateWithFlags(&up[k], cudaStreamNonBlocking);
-            if (e == cudaSuccess)
-                e = cudaStreamCreateWithFlags(&down[k], cudaStreamNonBlocking);
-        }
+        if (e == cudaSuccess)
+            e = cudaStreamCreateWithFlags(&up, cudaStreamNonBlocking);
+        if (e == cudaSuccess)
+            e = cudaStreamCreateWithFlags(&down, cudaStreamNonBlocking);
         for (int c = 0; c < PIPE_MAX_XCHUNKS && e == cudaSuccess; c++)
             e = cudaEventCreate(&x_ready[c]);
         for (int c = 0; c < PIPE_MAX_RANGES && e == cudaSuccess; c++)
@@ -1489,13 +1379,10 @@ struct PipeResources
             if (t1[c])
                 cudaEventDestroy(t1[c]);
         }
-        for (int k = 0; k < PIPE_MAX_STREAMS; k++)
-        {
-            if (up[k])
-                cudaStreamDestroy(up[k]);
-            if (down[k])
-                cudaStreamDestroy(down[k]);
-        }
+        if (up)
+            cudaStreamDestroy(up);
+        if (down)
+            cudaStreamDestroy(down);
     }
 };
 
@@ -1528,11 +1415,12 @@ static int csr_mult_pipelined(smvp_csr *A, const double *x_host, double *y_host,
     }
     PipeResources &R = *static_cast<PipeResources *>(A->pipe_res);
     // the part of x this matrix reads: [xlo, xhi).  Entries outside it are never gathered, so they are not uploaded
-    const int NR = A->pipe_ranges, NS = pipe_streams();
+    const int NR = A->pipe_ranges;
     const int64_t xlo = A->pipe_xlo, xhi = NR > 0 ? A->pipe_xneed[NR - 1] : 0;
     const int64_t xlen = xhi > xlo ? xhi - xlo : 0;
+    const int NX = pipe_xchunks(8 * xlen);
     double xf[PIPE_MAX_XCHUNKS + 1];
-    const int NX = pipe_profile(8 * xlen, pipe_xchunks(8 * xlen), PIPE_MAX_XCHUNKS, xf);
+    pipe_profile(NX, xf);
     int64_t xb[PIPE_MAX_XCHUNKS + 1]; // piece k uploads x[xb[k], xb[k+1]) (boundaries on 512-byte multiples)
     for (int k = 0; k <= NX; k++)
     {
@@ -1550,19 +1438,16 @@ static int csr_mult_pipelined(smvp_csr *A, const double *x_host, double *y_host,
     // everything queued on the legacy stream before the call (the zero-fill of y, an earlier pass) comes first
     PIPE_CK(cudaEventRecord(R.begin, 0));
     PIPE_CK(cudaStreamWaitEvent(cs, R.begin, 0));
-    for (int k = 0; k < NS; k++)
-    {
-        PIPE_CK(cudaStreamWaitEvent(R.up[k], R.begin, 0));
-        PIPE_CK(cudaStreamWaitEvent(R.down[k], R.begin, 0));
-    }
+    PIPE_CK(cudaStreamWaitEvent(R.up, R.begin, 0));
+    PIPE_CK(cudaStreamWaitEvent(R.down, R.begin, 0));
     if (x_host)
     {
         for (int k = 0; k < NX; k++)
         {
             const int64_t a = xb[k], b = xb[k + 1];
             if (b > a)
-                PIPE_CK(cudaMemcpyAsync(A->d_x + a, x_host + a, sizeof(double) * (size_t)(b - a), cudaMemcpyHostToDevice, R.up[k % NS]));
-            PIPE_CK(cudaEventRecord(R.x_ready[k], R.up[k % NS]));
+                PIPE_CK(cudaMemcpyAsync(A->d_x + a, x_host + a, sizeof(double) * (size_t)(b - a), cudaMemcpyHostToDevice, R.up));
+            PIPE_CK(cudaEventRecord(R.x_ready[k], R.up));
         }
     }
     int rc = SMVP_OK;
@@ -1575,8 +1460,11 @@ static int csr_mult_pipelined(smvp_csr *A, const double *x_host, double *y_host,
             int k = waited < 0 ? 0 : waited; // first piece whose end covers what the range reads
             while (k < NX - 1 && xb[k + 1] < (int64_t)A->pipe_xneed[c])
                 k++;
-            for (; waited < k; waited++) // pieces alternate over NS streams: wait for each one up to k
-                PIPE_CK(cudaStreamWaitEvent(cs, R.x_ready[waited + 1], 0));
+            if (k > waited) // the pieces complete in order on one stream: piece k's event covers every earlier one
+            {
+                PIPE_CK(cudaStreamWaitEvent(cs, R.x_ready[k], 0));
+                waited = k;
+            }
         }
         PIPE_CK(cudaEventRecord(R.t0[c], cs));
         if (A->pipe_tile[c + 1] > A->pipe_tile[c] && e == cudaSuccess)
@@ -1587,22 +1475,19 @@ static int csr_mult_pipelined(smvp_csr *A, const double *x_host, double *y_host,
         if (y_host)
         {
             PIPE_CK(cudaEventRecord(R.done[c], cs));
-            PIPE_CK(cudaStreamWaitEvent(R.down[c % NS], R.done[c], 0));
+            PIPE_CK(cudaStreamWaitEvent(R.down, R.done[c], 0));
             const int32_t r0 = A->pipe_row[c], r1 = A->pipe_row[c + 1];
             if (r1 > r0)
-                PIPE_CK(cudaMemcpyAsync(y_host + r0, A->d_y + r0, sizeof(double) * (size_t)(r1 - r0), cudaMemcpyDeviceToHost,
-                                        R.down[c % NS]));
-            PIPE_CK(cudaEventRecord(R.down_done[c], R.down[c % NS]));
+                PIPE_CK(cudaMemcpyAsync(y_host + r0, A->d_y + r0, sizeof(double) * (size_t)(r1 - r0), cudaMemcpyDeviceToHost, R.down));
+            PIPE_CK(cudaEventRecord(R.down_done[c], R.down));
         }
     }
     // drain every stream of the pass, also after a failure (nothing may still touch the caller's buffers on return)
     cudaError_t es = cudaStreamSynchronize(cs);
-    for (int k = 0; k < NS; k++) // the upload streams too: a matrix may read less than all of x
-    {
-        const cudaError_t eu = cudaStreamSynchronize(R.up[k]), ed = cudaStreamSynchronize(R.down[k]);
-        if (es == cudaSuccess)
-            es = eu != cudaSuccess ? eu : ed;
-    }
+    // the upload stream too: a matrix may read less than all of x
+    const cudaError_t eu = cudaStreamSynchronize(R.up), ed = cudaStreamSynchronize(R.down);
+    if (es == cudaSuccess)
+        es = eu != cudaSuccess ? eu : ed;
 #undef PIPE_CK
     if (rc != SMVP_OK)
         return rc;
@@ -1780,12 +1665,9 @@ extern "C" int smvp_csr_info(const smvp_csr *A, smvp_csr_info_t *out)
     out->bytes_per_mult = 12 * A->nnz + 4 * ((int64_t)A->rows + 1) + 8 * (int64_t)A->cols + 8 * (int64_t)A->rows;
     out->device_bytes = A->device_bytes;
     out->launches_per_mult[SMVP_CSR_VECTOR] = 1;
-    out->launches_per_mult[SMVP_CSR_MERGE] = 2;
+    out->launches_per_mult[SMVP_CSR_MERGE] = A->pattern_state == 1 ? 1 : 2;
     out->launches_per_mult[SMVP_CSR_AUTO] = out->launches_per_mult[out->auto_variant];
     out->x_relabel = A->relabel_state;
-    out->x_split = A->split_state;
-    out->launches_per_mult[SMVP_CSR_MERGE] = A->pattern_state == 1 ? 1 : A->split_state == 1 ? 4 : 2;
-    out->launches_per_mult[SMVP_CSR_AUTO] = out->launches_per_mult[out->auto_variant];
     out->row_patterns = A->pattern_state == 1 ? A->pattern_count : A->pattern_state;
     return SMVP_OK;
 }

@@ -215,14 +215,13 @@ int relabel_indices(const int32_t *d_idx, int64_t nnz, const int32_t *d_rank, in
 int csr_relabel_plan(smvp_csr *A, cudaStream_t s)
 {
     if (A->relabel_state != 0)
-        return csr_split_plan(A, s); // decided once as well; returns at once afterwards
+        return SMVP_OK;
     int use = 0;
     int32_t *order = nullptr, *rank = nullptr;
     SMVP_TRY(popularity_plan(A->col_ind, A->nnz, A->cols, env_tristate("SMVP_CSR_RELABEL"), 2.0, &order, &rank, &use, s));
     if (!use)
     {
         A->relabel_state = -1;
-        A->split_state = -1;
         return SMVP_OK;
     }
     A->x_order = order;
@@ -242,7 +241,7 @@ int csr_relabel_plan(smvp_csr *A, cudaStream_t s)
     }
     A->device_bytes += 4 * A->nnz + 12 * (int64_t)A->cols;
     A->relabel_state = 1;
-    return csr_split_plan(A, s);
+    return SMVP_OK;
 }
 
 // the same for the ROWS of a TJDS handle: the multiply scatters into y[row_ind[j]], and on a power-law matrix whose
@@ -287,139 +286,6 @@ void tjds_relabel_release(smvp_tjds *A)
     cudaFree(A->y_rel);
     A->row_rank = A->row_rel = nullptr;
     A->y_rel = nullptr;
-}
-
-// ---------------------------------------------------------------------------------------------- hot / cold split
-// Round-2 ncu of the relabelled + hinted kernel on R-MAT scale 26 (profiles/r02_csr_merge_warp_rmat26_relabel_hints.txt):
-// 24.35 GB of DRAM traffic for 14.07 GB algorithmic, L2 hit rate 47 %, DRAM 56 % busy -- the hot prefix of x_rel does not
-// stay resident while the cold gathers (11 % of the entries, one 32-byte sector each) and the streams pass through, and
-// the kernel waits on the misses.  The split separates the two populations: `hot` = the entries whose column rank is
-// below the prefix, a matrix whose whole x (32 MB) sits in L2, so it streams at the roofline; `cold` = the rest, few
-// entries, every gather a miss, nothing else to disturb.  y = hot * x_rel, then y += cold * x_rel (the row sum is
-// taken in two parts: within the 1e-12 bar, no longer bit-identical to the natural order).  Costs 12 more bytes per
-// nonzero of HBM and one more pass over y.
-// MEASURED (profiles/r02_logs/r02_split_launches.csv, ncu per launch): the hot pass moves 12.3 GB of DRAM traffic --
-// exactly its algorithmic bytes, L2 hit rate 61 % -- and still takes 4.59 ms: with the misses gone the kernel is bound by
-// the gather RATE (945 M 8-byte gathers, each its own 32-byte sector through L1 and the crossbar: ~206 G gathers/s),
-// not by DRAM.  The cold pass takes 2.10 ms for 11.0 GB (a missed 8-byte gather costs a 64-byte DRAM burst).  Together
-// 6.9 ms against 5.33 ms for the one-pass relabelled kernel, which overlaps the cold misses with the hot hits.  So the
-// split stays an opt-in experiment (SMVP_CSR_SPLIT=1), and the R-MAT multiply is gather-rate-bound: the next lever is
-// fewer sector accesses per gather (the hottest few thousand x entries held in shared memory), not less DRAM traffic.
-__global__ void __launch_bounds__(256) split_flag_kernel(const int32_t *__restrict__ col_rel, int64_t nnz, int32_t hot,
-                                                         uint32_t *__restrict__ flag)
-{
-    for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < nnz; j += (int64_t)gridDim.x * blockDim.x)
-        flag[j] = __ldg(col_rel + j) < hot ? 1u : 0u;
-}
-
-// pos = exclusive scan of the hot flags: hot entry j lands at pos[j], cold entry j at j - pos[j] (both keep their order)
-__global__ void __launch_bounds__(256) split_scatter_kernel(const int32_t *__restrict__ row_of, const int32_t *__restrict__ col_rel,
-                                                            const double *__restrict__ val, int64_t nnz, int32_t hot,
-                                                            const uint32_t *__restrict__ pos, int32_t *__restrict__ hr,
-                                                            int32_t *__restrict__ hc, double *__restrict__ hv, int32_t *__restrict__ cr,
-                                                            int32_t *__restrict__ cc, double *__restrict__ cv)
-{
-    for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < nnz; j += (int64_t)gridDim.x * blockDim.x)
-    {
-        const int32_t c = __ldg(col_rel + j);
-        const uint32_t p = pos[j];
-        if (c < hot)
-        {
-            hr[p] = row_of[j];
-            hc[p] = c;
-            hv[p] = val[j];
-        }
-        else
-        {
-            const int64_t q = j - (int64_t)p;
-            cr[q] = row_of[j];
-            cc[q] = c;
-            cv[q] = val[j];
-        }
-    }
-}
-
-// also the L2 retention limit of the ranked gathers (csr_mult.cu hot_limits): one value for both
-int32_t hot_l2_entries() { return env_int("SMVP_HOT_L2", 4 << 20, 0, INT32_MAX); } // 32 MB of x
-
-int csr_split_plan(smvp_csr *A, cudaStream_t s)
-{
-    if (A->split_state != 0)
-        return SMVP_OK;
-    A->split_state = -1;
-    const int forced = env_tristate("SMVP_CSR_SPLIT");
-    // OPT-IN (SMVP_CSR_SPLIT=1), never AUTO: measured on R-MAT scale 26 it LOSES -- see the header comment above
-    if (A->relabel_state != 1 || forced <= 0 || A->nnz == 0)
-        return SMVP_OK;
-    const int32_t hot = hot_l2_entries();
-    if (hot <= 0 || hot >= A->cols)
-        return SMVP_OK;
-    DevTmp row_of, pos, total, hr, hc, hv, cr, cc, cv;
-    smvp_csr *H = nullptr, *C = nullptr;
-    auto body = [&]() -> int {
-        const int64_t nnz = A->nnz;
-        int64_t blocks = ceil_div64(nnz, 256 * 8);
-        const int64_t cap = (int64_t)device_props().sms * 16;
-        const unsigned grid = (unsigned)(blocks < cap ? blocks : cap);
-        SMVP_CUDA(row_of.alloc<int32_t>(nnz));
-        SMVP_CUDA(pos.alloc<uint32_t>(nnz));
-        SMVP_CUDA(total.alloc<uint32_t>(1));
-        SMVP_TRY(csr_expand_rows(A->row_ptr, A->rows, nnz, row_of.as<int32_t>(), s));
-        SMVP_LAUNCH(split_flag_kernel, grid, 256, 0, s, (const int32_t *)A->col_rel, nnz, hot, pos.as<uint32_t>());
-        SMVP_TRY(exclusive_scan_u32(pos.as<uint32_t>(), pos.as<uint32_t>(), nnz, total.as<uint32_t>(), s));
-        uint32_t nh = 0;
-        SMVP_CUDA(cudaMemcpyAsync(&nh, total.p, sizeof(nh), cudaMemcpyDeviceToHost, s));
-        SMVP_CUDA(cudaStreamSynchronize(s));
-        const int64_t nc = nnz - (int64_t)nh;
-        if (nh == 0 || nc == 0)
-            return SMVP_OK; // nothing to separate
-        SMVP_CUDA(hr.alloc<int32_t>(nh));
-        SMVP_CUDA(hc.alloc<int32_t>(nh));
-        SMVP_CUDA(hv.alloc<double>(nh));
-        SMVP_CUDA(cr.alloc<int32_t>(nc));
-        SMVP_CUDA(cc.alloc<int32_t>(nc));
-        SMVP_CUDA(cv.alloc<double>(nc));
-        SMVP_LAUNCH(split_scatter_kernel, grid, 256, 0, s, (const int32_t *)row_of.as<int32_t>(), (const int32_t *)A->col_rel,
-                    (const double *)A->val, nnz, hot, (const uint32_t *)pos.as<uint32_t>(), hr.as<int32_t>(), hc.as<int32_t>(),
-                    hv.as<double>(), cr.as<int32_t>(), cc.as<int32_t>(), cv.as<double>());
-        SMVP_CUDA(cudaStreamSynchronize(s));
-        SMVP_CUDA(cudaGetLastError());
-        cudaFree(row_of.p); // make room before the two builds
-        row_of.p = nullptr;
-        cudaFree(pos.p);
-        pos.p = nullptr;
-        for (int part = 0; part < 2; part++)
-        {
-            smvp_csr *P = new (std::nothrow) smvp_csr();
-            if (!P)
-                return SMVP_E_ALLOC;
-            (part == 0 ? H : C) = P;
-            P->rows = A->rows;
-            P->cols = A->cols;
-            P->nnz = part == 0 ? (int64_t)nh : nc;
-            P->relabel_state = -1; // its column indices ARE ranks already
-            P->split_state = -1;
-            P->ranked_cols = 1;
-            P->merge_cfg = -1;
-            P->pipe_cfg = -1;
-            SMVP_TRY(csr_build_impl(part == 0 ? hr.as<int32_t>() : cr.as<int32_t>(), part == 0 ? hc.as<int32_t>() : cc.as<int32_t>(),
-                                    part == 0 ? hv.as<double>() : cv.as<double>(), A->rows, A->cols, P->nnz, P, s));
-            P->auto_variant = SMVP_CSR_MERGE;
-        }
-        return SMVP_OK;
-    };
-    const int rc = body();
-    if (rc != SMVP_OK || !H || !C)
-    {
-        csr_release(H);
-        csr_release(C);
-        return rc;
-    }
-    A->hot = H;
-    A->cold = C;
-    A->device_bytes += H->device_bytes + C->device_bytes;
-    A->split_state = 1;
-    return SMVP_OK;
 }
 
 // x_rel = x in rank order (asynchronous on s)

@@ -44,7 +44,7 @@ class _CsrInfo(ctypes.Structure):
     _fields_ = [("rows", ctypes.c_int32), ("cols", ctypes.c_int32), ("nnz", ctypes.c_int64),
                 ("max_row_nnz", ctypes.c_int32), ("auto_variant", ctypes.c_int32), ("input_order", ctypes.c_int32),
                 ("bytes_per_mult", ctypes.c_int64), ("device_bytes", ctypes.c_int64),
-                ("launches_per_mult", ctypes.c_int32 * 3), ("x_relabel", ctypes.c_int32), ("x_split", ctypes.c_int32),
+                ("launches_per_mult", ctypes.c_int32 * 3), ("x_relabel", ctypes.c_int32),
                 ("row_patterns", ctypes.c_int32)]
 
 
@@ -291,13 +291,6 @@ class CsrMatrix:
         info = _CsrInfo()
         _check(lib().smvp_csr_info(self._h, ctypes.byref(info)), "smvp_csr_info")
         return info.x_relabel
-
-    @property
-    def x_split(self):
-        """1: a relabelled handle multiplies in a hot and a cold pass, -1: one pass, 0: not decided yet."""
-        info = _CsrInfo()
-        _check(lib().smvp_csr_info(self._h, ctypes.byref(info)), "smvp_csr_info")
-        return info.x_split
 
     @property
     def row_patterns(self):

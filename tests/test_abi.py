@@ -88,6 +88,43 @@ def test_no_gpu_means_loud_failure_not_fallback(eng):
         eng.smvp_tjds_compute(coo, m, n, len(coo), 1)
 
 
+def _header_fields(struct):
+    """field names of a struct typedef in include/smvp_cuda.h, in declaration order"""
+    text = open(os.path.join(REPO, "include", "smvp_cuda.h")).read()
+    body = re.search(r"typedef struct %s\s*\{(.*?)\}\s*%s;" % (struct, struct), text, re.S).group(1)
+    body = re.sub(r"/\*.*?\*/", "", body, flags=re.S)
+    names = []
+    for decl in filter(None, (d.strip() for d in body.split(";"))):
+        _, declarators = decl.split(None, 1)  # every field type is one token (int32_t, int64_t)
+        names += [re.match(r"\s*(\w+)", d).group(1) for d in declarators.split(",")]
+    return names
+
+
+def test_info_structs_match_the_header(tmp_path):
+    """engine.py's ctypes mirrors of smvp_csr_info_t and smvp_tjds_info_t have the header's fields, offsets and size, as
+    gcc lays the header out (no library build, no GPU)."""
+    from smvp_toolkit_b200 import engine
+
+    mirrors = {"smvp_csr_info_t": engine._CsrInfo, "smvp_tjds_info_t": engine._TjdsInfo}
+    fields = {s: _header_fields(s) for s in mirrors}
+    for s, py in mirrors.items():
+        assert fields[s] == [f[0] for f in py._fields_], s
+    src = ["#include <stddef.h>", "#include <stdio.h>", '#include "smvp_cuda.h"', "int main(void)", "{"]
+    for s in mirrors:
+        src.append('    printf("%s sizeof %%zu\\n", sizeof(%s));' % (s, s))
+        src += ['    printf("%s %s %%zu\\n", offsetof(%s, %s));' % (s, f, s, f) for f in fields[s]]
+    src += ["    return 0;", "}"]
+    (tmp_path / "layout.c").write_text("\n".join(src) + "\n")
+    exe = str(tmp_path / "layout")
+    subprocess.run(["gcc", "-std=c11", "-I" + os.path.join(REPO, "include"), "-o", exe, str(tmp_path / "layout.c")], check=True)
+    c = {tuple(ln.split()[:2]): int(ln.split()[2]) for ln in subprocess.run([exe], capture_output=True, text=True,
+                                                                            check=True).stdout.splitlines()}
+    for s, py in mirrors.items():
+        assert c[(s, "sizeof")] == ctypes.sizeof(py), s
+        for f in fields[s]:
+            assert c[(s, f)] == getattr(py, f).offset, (s, f)
+
+
 def test_time_stats_is_host_side(eng):
     td = eng.TimeData(np.array([1.0, 2.0, 3.0, 2.0]))
     assert td.time_total == 8.0 and td.time_avg == 2.0 and td.time_min == 1.0 and td.time_max == 3.0

@@ -366,18 +366,15 @@ def _dot_bits(A, alpha, dx, beta, y0, w, variant=0):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("plan", ["pattern", "merge", "relabel", "split"])
+@pytest.mark.parametrize("plan", ["pattern", "merge", "relabel"])
 def test_dot_does_not_depend_on_the_grid(eng, monkeypatch, plan):
     """The same handle at co-runner headroom 0 and 1 gives the same dot bits.  The matrices are large enough that the
     persistent grid is capped by residency, so the headroom changes the grid and which CTA walks which tile."""
     import torch
 
     rng = np.random.default_rng(12)
-    if plan in ("relabel", "split"):
+    if plan == "relabel":
         monkeypatch.setenv("SMVP_CSR_RELABEL", "1")
-        if plan == "split":
-            monkeypatch.setenv("SMVP_CSR_SPLIT", "1")
-            monkeypatch.setenv("SMVP_HOT_L2", "1024")
         n = 1 << 18
         r, c, v = eng.synth_rmat(18, 16 << 18, seed=42)
         A = eng.CsrMatrix.build_device(r, c, v, n, n, r.n)
@@ -402,11 +399,7 @@ def test_dot_does_not_depend_on_the_grid(eng, monkeypatch, plan):
         assert [_dot_bits(A, -1.0, dx, 1.0, y0, wv, eng.CSR_MERGE) for wv in (None, w, dx)] == want
     A.set_corunner_headroom(1)
     assert [_dot_bits(A, -1.0, dx, 1.0, y0, wv, eng.CSR_MERGE) for wv in (None, w, dx)] == want
-    assert {"pattern": A.row_patterns > 0, "merge": A.row_patterns < 0, "relabel": A.x_relabel == 1,
-            "split": A.x_split == 1}[plan]
-    if plan == "split":  # y within the split's 1e-12 of the one-pass order; the dot within the bound of its own y
-        y, dot = _csr_run(A, -1.0, dx, 1.0, y0, None, eng.CSR_MERGE)
-        _check_dot(dot, None, y, DEPTH["merge"], "split")
+    assert {"pattern": A.row_patterns > 0, "merge": A.row_patterns < 0, "relabel": A.x_relabel == 1}[plan]
     A.free()
 
 
@@ -508,17 +501,14 @@ def _launches(eng, fn):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("plan", ["pattern", "merge", "vector", "relabel", "split"])
+@pytest.mark.parametrize("plan", ["pattern", "merge", "vector", "relabel"])
 def test_csr_launches(eng, monkeypatch, plan):
     """A CSR dot pass launches what the *_axpby call with (alpha, beta) != (1, 0) launches, plus the reduction."""
     import torch
 
     rng = np.random.default_rng(14)
-    if plan in ("relabel", "split"):
+    if plan == "relabel":
         monkeypatch.setenv("SMVP_CSR_RELABEL", "1")
-        if plan == "split":
-            monkeypatch.setenv("SMVP_CSR_SPLIT", "1")
-            monkeypatch.setenv("SMVP_HOT_L2", "1024")
         coo, n = synth_ref.rmat(14, 16 << 14), 1 << 14
     elif plan == "pattern":
         coo, n = _stencil(12, rng), 12 ** 3

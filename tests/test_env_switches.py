@@ -9,11 +9,14 @@ CSRC = os.path.join(REPO, "smvp-toolkit_b200", "csrc")
 HELPERS = ("env_str", "env_set", "env_int", "env_tristate")
 HELPER_CALL = re.compile(r"\b(%s)\(\s*([^)\s,]*)" % "|".join(HELPERS))
 
-# compile-time switches, tuning hooks and configuration tables that selected swept kernel variants; the measurements that
-# retired them are in DESIGN.md §5.2 / §5.3
+# compile-time switches, tuning hooks and configuration tables that selected swept kernel variants, and the plan-level
+# and host-side switches that selected a losing or neutral arm; the measurements that retired them are in DESIGN.md
+# §5.2 / §5.3 / §5.4 / §6
 REMOVED = ("SMVP_ASM_LDS", "SMVP_SCAN_EXIT", "SMVP_UNIFORM_TILES", "SMVP_X_EVICT_LAST", "SMVP_TJDS_STREAM", "SMVP_MERGE_CFG",
            "SMVP_WMERGE_CFGS", "SMVP_PATTERN_CFG", "SMVP_PATTERN_CFGS", "SMVP_VECTOR_WIDE", "SMVP_TJDS_DET_CFG",
-           "SMVP_TJDS_UNROLL", "SMVP_MERGE_CHUNK", "SMVP_MERGE_ALIGNED", "SMVP_PHASED_PLAIN", "SMVP_CUDA_LIB")
+           "SMVP_TJDS_UNROLL", "SMVP_MERGE_CHUNK", "SMVP_MERGE_ALIGNED", "SMVP_PHASED_PLAIN", "SMVP_CUDA_LIB",
+           "SMVP_CSR_SPLIT", "SMVP_L2_PERSIST_MB", "SMVP_RANKED_HINTS", "SMVP_HOT_L1", "SMVP_HOT_L2", "SMVP_PIPE_PROFILE",
+           "SMVP_PIPE_STREAMS", "SMVP_PIPE_RANGES", "SMVP_PIPE_XCHUNKS")
 
 
 def _sources():

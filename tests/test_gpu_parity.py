@@ -652,7 +652,7 @@ def test_full_size_rmat_scale26(eng, monkeypatch):
     eng.synth_vector(d_x, n, 4242)
     x = d_x.cpu().numpy()
 
-    # ---- (b) full matrix, CSR: AUTO (relabelled at this size), the opt-in hot / cold split, and the natural order
+    # ---- (b) full matrix, CSR: AUTO (relabelled at this size) and the natural order
     A = eng.CsrMatrix.build_device(r, c, v, m, n, nnz)
     y_auto = torch.empty(m, dtype=torch.float64, device="cuda")
     A.set_x_device(d_x)
@@ -660,31 +660,21 @@ def test_full_size_rmat_scale26(eng, monkeypatch):
     torch.cuda.synchronize()
     if scale >= 26:
         assert A.x_relabel == 1, "AUTO is expected to relabel the column space of R-MAT scale 26"
-        assert A.x_split == -1, "the hot / cold split is opt-in (it loses on this matrix)"
     y_vec = torch.empty_like(y_auto)
     A.mult_device(None, y_vec, eng.CSR_VECTOR)
     torch.cuda.synchronize()
     assert float(torch.linalg.norm(y_vec - y_auto) / torch.linalg.norm(y_auto)) <= TOL
     A.free()
-    monkeypatch.setenv("SMVP_CSR_SPLIT", "1")
-    R = eng.CsrMatrix.build_device(r, c, v, m, n, nnz)
-    y_split = torch.empty_like(y_auto)
-    R.mult_device(d_x, y_split, eng.CSR_MERGE)
-    torch.cuda.synchronize()
-    assert scale < 26 or (R.x_relabel == 1 and R.x_split == 1)
-    R.free()
-    monkeypatch.delenv("SMVP_CSR_SPLIT")
     monkeypatch.setenv("SMVP_CSR_RELABEL", "0")
     P = eng.CsrMatrix.build_device(r, c, v, m, n, nnz)
     y_plain = torch.empty_like(y_auto)
     P.mult_device(d_x, y_plain, eng.CSR_MERGE)
     torch.cuda.synchronize()
-    assert P.x_relabel == -1 and P.x_split == -1
+    assert P.x_relabel == -1
     assert torch.equal(y_plain, y_auto), "relabelled and natural-order CSR must agree bit for bit"
-    assert float(torch.linalg.norm(y_split - y_plain) / torch.linalg.norm(y_plain)) <= TOL  # two-pass row sums
     P.free()
     monkeypatch.delenv("SMVP_CSR_RELABEL")
-    del y_vec, y_plain, y_split
+    del y_vec, y_plain
 
     # ---- (c) full matrix, TJDS
     T = eng.TjdsMatrix.build_device(r, c, v, m, n, nnz)
@@ -841,15 +831,12 @@ def test_nonfinite_inputs_follow_ieee_propagation(eng):
     T.free()
 
 
-def test_csr_hot_cold_split_forced(eng, monkeypatch):
-    """The hot / cold split of a relabelled handle (relabel.cu: csr_split_plan) on a small matrix with the prefix scaled
-    down: y within 1e-12 of the oracle through every entry point, the exported CSR arrays untouched, the vector kernel
-    and fan-out passes (which do not split) still right, empty rows / rows with only hot or only cold entries handled."""
+def test_csr_relabel_forced_empty_rows_and_batched_loop(eng, monkeypatch):
+    """A relabelled handle on a small power-law matrix with empty rows: y within 1e-12 of the oracle and bit-identical to
+    a natural-order handle through the host entry point (iters 1 / 3 / 40; 40 takes the batched graph loop), the vector
+    kernel, the device and the fan-out passes; the exported CSR arrays untouched."""
     import torch
 
-    monkeypatch.setenv("SMVP_CSR_RELABEL", "1")
-    monkeypatch.setenv("SMVP_CSR_SPLIT", "1")
-    monkeypatch.setenv("SMVP_HOT_L2", "3000")  # entries of x_rel that count as hot
     rng = np.random.default_rng(91)
     m, n = 50021, 40009
     coo = _powerlaw_coo(rng, m, n, 700000, 4.0)
@@ -857,13 +844,26 @@ def test_csr_hot_cold_split_forced(eng, monkeypatch):
     x = rng.uniform(-1, 1, n)
     rp, ci, va = oracle.csr_build(coo, m, n)
     y_ref = oracle.csr_mult(rp, ci, va, x)
+
+    def same(a, b):
+        return np.array_equal(a.view(np.int64), b.view(np.int64))
+
+    monkeypatch.setenv("SMVP_CSR_RELABEL", "0")
+    B = eng.CsrMatrix.build(coo, m, n)
+    y_nat, _ = B.mult(x, iters=1, variant=eng.CSR_MERGE)
+    yv_nat, _ = B.mult(x, iters=1, variant=eng.CSR_VECTOR)
+    assert B.x_relabel == -1
+    B.free()
+    monkeypatch.setenv("SMVP_CSR_RELABEL", "1")
     A = eng.CsrMatrix.build(coo, m, n)
     for iters in (1, 3, 40):
         y, _ = A.mult(x, iters=iters, variant=eng.CSR_MERGE)
         assert util.rel_l2(y, y_ref) <= TOL, iters
-    assert A.x_relabel == 1 and A.x_split == 1
+        assert same(y, y_nat), iters
+    assert A.x_relabel == 1
     yv, _ = A.mult(x, iters=1, variant=eng.CSR_VECTOR)
     assert util.rel_l2(yv, y_ref) <= TOL
+    assert same(yv, yv_nat)
     g = A.export()
     assert np.array_equal(g[0], rp) and np.array_equal(g[1], ci) and np.array_equal(g[2].view(np.int64), va.view(np.int64))
     d_x = torch.as_tensor(x, device="cuda")
@@ -872,8 +872,10 @@ def test_csr_hot_cold_split_forced(eng, monkeypatch):
     A.mult_device(None, d_y, eng.CSR_MERGE)
     torch.cuda.synchronize()
     assert util.rel_l2(d_y.cpu().numpy(), y_ref) <= TOL
+    assert same(d_y.cpu().numpy(), y_nat)
     outs = [torch.full((m,), float("nan"), dtype=torch.float64, device="cuda") for _ in range(2)]
     A.mult_device_fanout(None, [o.data_ptr() for o in outs], eng.CSR_MERGE)
     torch.cuda.synchronize()
     assert util.rel_l2(outs[0].cpu().numpy(), y_ref) <= TOL and torch.equal(outs[0], outs[1])
+    assert same(outs[0].cpu().numpy(), y_nat)
     A.free()

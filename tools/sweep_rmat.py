@@ -33,9 +33,7 @@ def main():
     ap.add_argument("--edge-factor", type=int, default=16)
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--modes", default="0,1")
-    ap.add_argument("--hints", default="off,8192x4194304,0x4194304,8192x0,65536x8388608")
     ap.add_argument("--no-vector", action="store_true")
-    ap.add_argument("--persist", default="0", help="comma list of SMVP_L2_PERSIST_MB values tried with every hint setting")
     args = ap.parse_args()
     src = sdist.RmatSource(eng, args.scale, args.edge_factor << args.scale)
     M = N = src.rows
@@ -52,26 +50,14 @@ def main():
         A = eng.CsrMatrix.build_device(r, c, v, M, N, nnz)
         t_plan = timeit(lambda: A.set_x_device(x), 1)  # first call decides and builds the plan; then 3 warm + 1
         print("relabel=%s state=%d   set_x %.3f ms" % (mode, A.x_relabel, t_plan), flush=True)
-        hints = [""] if mode == "0" else args.hints.split(",")
-        for hint in hints:  # "off" | "L1xL2" in entries (ranked cache-retention hints of the relabelled kernel)
-            if hint == "off":
-                os.environ["SMVP_RANKED_HINTS"] = "0"
-            elif hint:
-                os.environ["SMVP_RANKED_HINTS"] = "1"
-                os.environ["SMVP_HOT_L1"], os.environ["SMVP_HOT_L2"] = hint.split("x")
-            for pmb in (args.persist.split(",") if mode != "0" else ["0"]):
-                os.environ["SMVP_L2_PERSIST_MB"] = pmb
-                y.fill_(float("nan"))
-                ms = timeit(lambda: A.mult_device(None, y, eng.CSR_MERGE), args.steps)
-                tag = ""
-                if mode == "0":
-                    y_plain = y.clone()
-                elif y_plain is not None:
-                    tag = "bit-identical" if torch.equal(y, y_plain) else "DIFFERS from plain"
-                print("  hints %-16s persist %3s MB merge: %8.3f ms  %8.1f GB/s  %s" % (hint, pmb, ms, nbytes / ms / 1e6, tag), flush=True)
-        os.environ.pop("SMVP_L2_PERSIST_MB", None)
-        for k in ("SMVP_RANKED_HINTS", "SMVP_HOT_L1", "SMVP_HOT_L2"):
-            os.environ.pop(k, None)
+        y.fill_(float("nan"))
+        ms = timeit(lambda: A.mult_device(None, y, eng.CSR_MERGE), args.steps)
+        tag = ""
+        if mode == "0":
+            y_plain = y.clone()
+        elif y_plain is not None:
+            tag = "bit-identical" if torch.equal(y, y_plain) else "DIFFERS from plain"
+        print("  merge      : %8.3f ms  %8.1f GB/s  %s" % (ms, nbytes / ms / 1e6, tag), flush=True)
         if not args.no_vector:
             ms = timeit(lambda: A.mult_device(None, y, eng.CSR_VECTOR), args.steps)
             print("  vector     : %8.3f ms  %8.1f GB/s" % (ms, nbytes / ms / 1e6), flush=True)
