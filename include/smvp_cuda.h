@@ -264,6 +264,11 @@ typedef struct smvp_csr_info_t
                                  per row instead of col_ind and sums each row in the reference's order (y bit-identical to
                                  main-cli.c:410-416); -1 = not used (more than 256 lists, a longer row, a relabelled handle,
                                  or SMVP_CSR_PATTERN=0); 0 = not decided yet (decided at the first pass)              */
+    int32_t value_bytes;      /* with row_patterns > 0: the width the pattern kernel streams the values at -- 2 (fp16) or
+                                 4 (fp32) when EVERY value converts to that type and back with the same 64 bits (pattern
+                                 and integer matrices, constant-coefficient stencils; a copy at that width is held and
+                                 counted in device_bytes, y stays bit-identical), else 8; 0 = not decided yet.
+                                 Meaningless when row_patterns <= 0.                                                  */
 } smvp_csr_info_t;
 
 typedef struct smvp_tjds_info_t

@@ -223,6 +223,33 @@ constexpr int32_t EXP_NONE = (int32_t)0x80808080; // memset(0x80) pattern: "no e
 // row-pattern plan (pattern.cu): at most PAT_MAX distinct column-offset lists (ids are one byte), none longer than PAT_LMAX
 constexpr int PAT_MAX = 256;
 constexpr int PAT_LMAX = 32;
+// Value widths of that plan: fp64 (double), fp32 (float) or fp16 held as its 16 bits (uint16_t).  pattern.cu keeps a
+// narrow width only where narrow_value then widen_value gives back the same 64 bits for EVERY value, and the pattern
+// kernel widens with the same instruction, so its products see exactly the fp64 operands.
+__device__ __forceinline__ double widen_value(double v) { return v; }
+__device__ __forceinline__ double widen_value(float v)
+{
+    double d;
+    asm("cvt.f64.f32 %0, %1;" : "=d"(d) : "f"(v));
+    return d;
+}
+__device__ __forceinline__ double widen_value(uint16_t v)
+{
+    double d;
+    asm("cvt.f64.f16 %0, %1;" : "=d"(d) : "h"(v));
+    return d;
+}
+template <typename V>
+__device__ __forceinline__ V narrow_value(double v)
+{
+    static_assert(std::is_same<V, float>::value || std::is_same<V, uint16_t>::value, "fp32 or fp16");
+    V n;
+    if constexpr (std::is_same<V, float>::value)
+        asm("cvt.rn.f32.f64 %0, %1;" : "=f"(n) : "d"(v));
+    else
+        asm("cvt.rn.f16.f64 %0, %1;" : "=h"(n) : "d"(v));
+    return n;
+}
 
 } // namespace smvp
 
@@ -265,6 +292,10 @@ struct smvp_csr
     uint8_t *pat_id;                       // [rows]
     int32_t *pat_off;                      // [pattern_count * PAT_LMAX]
     int32_t *pat_len;                      // [pattern_count]
+    // the values the pattern kernel streams: val itself (pat_vbytes 8) or, when every value converts to fp32 / fp16 and
+    // back with the same 64 bits, a copy at that width (pat_vbytes 4 / 2).  0 = not decided.  val stays for every other path.
+    int32_t pat_vbytes;
+    void *pat_val; // [nnz] narrow copy (NULL at width 8)
     // scratch of the fused inner product (*_axpby_dot, dot.cu): unit partials, reduction sums and counter; built at first use
     double *dot_buf;
     int64_t dot_cap;

@@ -727,15 +727,41 @@ template <int R>
 struct PatternShape
 {
     static constexpr int ROWS = 32 * R;
-    // val slice (16-byte aligned start: up to one extra double at each end) + pat_id slice (16-byte aligned)
-    static int stage_bytes(int maxlen) { return (((ROWS * maxlen + 2) * 8 + 15) / 16 * 16 + ROWS + 32 + 127) & ~127; }
+    // value slice of vsize-byte values (16-byte aligned start and length: up to 16 / vsize - 1 extra values at each end)
+    // + pat_id slice (16-byte aligned)
+    static int stage_bytes(int maxlen, int vsize)
+    {
+        return (((ROWS * maxlen + 2 * (16 / vsize - 1)) * vsize + 15) / 16 * 16 + ROWS + 32 + 127) & ~127;
+    }
 };
+
+// a value of the stage at shared address a, widened to fp64 (V: double, float or fp16 as uint16_t)
+template <typename V>
+__device__ __forceinline__ double lds_value(uint32_t a)
+{
+    if constexpr (std::is_same<V, double>::value)
+        return lds_f64(a);
+    else if constexpr (std::is_same<V, float>::value)
+    {
+        float v;
+        asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(a));
+        return widen_value(v);
+    }
+    else
+    {
+        uint16_t v;
+        asm volatile("ld.shared.b16 %0, [%1];" : "=h"(v) : "r"(a));
+        return widen_value(v);
+    }
+}
 
 // DOT (csr_pattern_dot_kernel): the work unit is the tile of 32 rows; the lanes' dot terms are added in a pairwise tree
 // into part[t].  w[r] is loaded beside the early load of y[r].
-template <int WARPS, int R, int STAGES, int CH, int MINB, bool FANOUT, bool EPI, bool DOT>
+// V: the width the values are streamed at (A->pat_vbytes).  Narrow values are widened exactly (pattern.cu checked every
+// one), so the products and sums are those of the fp64 kernel.
+template <typename V, int WARPS, int R, int STAGES, int CH, int MINB, bool FANOUT, bool EPI, bool DOT>
 __device__ __forceinline__ void
-csr_pattern_body(const int32_t *__restrict__ row_ptr, const double *__restrict__ val, const uint8_t *__restrict__ pat_id,
+csr_pattern_body(const int32_t *__restrict__ row_ptr, const V *__restrict__ val, const uint8_t *__restrict__ pat_id,
                  const int32_t *__restrict__ pat_off, const int32_t *__restrict__ pat_len, int32_t npat, int32_t maxlen,
                  const double *__restrict__ x, double *__restrict__ y, int32_t row_begin, int32_t row_end, uint32_t stage_bytes,
                  const YFan &fan, double alpha, double beta, const double *__restrict__ dot_w, double *__restrict__ part)
@@ -743,6 +769,7 @@ csr_pattern_body(const int32_t *__restrict__ row_ptr, const double *__restrict__
     static_assert(!EPI || (R == 1 && !FANOUT), "the epilogue keeps one y value per lane: one round per tile");
     static_assert(!DOT || EPI, "the dot is formed by the epilogue");
     constexpr int ROWS = PatternShape<R>::ROWS;
+    constexpr int VA = 16 / (int)sizeof(V); // values per 16 bytes: the alignment of a bulk copy
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ __align__(8) uint64_t full_bar[WARPS * STAGES];
     __shared__ int32_t stage_n0[WARPS * STAGES]; // first nonzero of the tile in each stage
@@ -773,8 +800,8 @@ csr_pattern_body(const int32_t *__restrict__ row_ptr, const double *__restrict__
     // rows [r0, r1) of tile t; lane 0 stages it (n0 = row_ptr[r0], n1 = row_ptr[r1] loaded by the caller)
     auto issue = [&](int32_t t, int s, int32_t n0, int32_t n1) {
         const int32_t r0 = row_begin + t * ROWS, r1 = min(r0 + ROWS, row_end);
-        const int32_t va = n0 & ~1, pa = r0 & ~15;
-        const uint32_t vb = n1 > n0 ? (uint32_t)(((n1 + 1) & ~1) - va) * 8u : 0u;
+        const int32_t va = n0 & ~(VA - 1), pa = r0 & ~15;
+        const uint32_t vb = n1 > n0 ? (uint32_t)(((n1 + VA - 1) & ~(VA - 1)) - va) * (uint32_t)sizeof(V) : 0u;
         const uint32_t pb = (uint32_t)(((r1 + 15) & ~15) - pa);
         unsigned char *dst = smem + (base - smem_u32(smem)) + (uint32_t)s * stage_bytes;
         stage_n0[w * STAGES + s] = n0;
@@ -825,7 +852,7 @@ csr_pattern_body(const int32_t *__restrict__ row_ptr, const double *__restrict__
         const int32_t r0 = row_begin + t * ROWS, r1 = min(r0 + ROWS, row_end);
         const int32_t n0 = stage_n0[w * STAGES + s];
         const uint32_t sb = base + (uint32_t)s * stage_bytes;
-        const uint32_t sval = sb + 8u * (uint32_t)(n0 - (n0 & ~1)); // nonzero n0
+        const uint32_t sval = sb + (uint32_t)sizeof(V) * (uint32_t)(n0 - (n0 & ~(VA - 1))); // nonzero n0
         const uint32_t spid = sb + val_bytes + (uint32_t)(r0 - (r0 & ~15)); // row r0
         int32_t done = 0; // nonzeros of the tile before the current round
 #pragma unroll 1
@@ -850,7 +877,7 @@ csr_pattern_body(const int32_t *__restrict__ row_ptr, const double *__restrict__
                 if (lane >= o)
                     incl += v;
             }
-            const uint32_t vrow = sval + 8u * (uint32_t)(done + incl - len);
+            const uint32_t vrow = sval + (uint32_t)sizeof(V) * (uint32_t)(done + incl - len);
             const uint32_t orow = smem_u32(s_off) + 4u * (uint32_t)(p * maxlen);
             done += __shfl_sync(0xffffffffu, incl, 31);
             const int32_t kmax = __reduce_max_sync(0xffffffffu, len);
@@ -874,7 +901,7 @@ csr_pattern_body(const int32_t *__restrict__ row_ptr, const double *__restrict__
 #pragma unroll
                 for (int q = 0; q < CH; q++)
                     if (k0 + q < len)
-                        sum = __dadd_rn(sum, __dmul_rn(lds_f64(vrow + 8u * (uint32_t)(k0 + q)), xv[q]));
+                        sum = __dadd_rn(sum, __dmul_rn(lds_value<V>(vrow + (uint32_t)sizeof(V) * (uint32_t)(k0 + q)), xv[q]));
             }
             if (live)
             {
@@ -907,6 +934,7 @@ csr_pattern_body(const int32_t *__restrict__ row_ptr, const double *__restrict__
         s = s + 1 == STAGES ? 0 : s + 1;
     }
 }
+// fp64 values: the kernels read val itself
 template <int WARPS, int R, int STAGES, int CH, int MINB, bool FANOUT, bool EPI>
 __global__ void __launch_bounds__(WARPS * 32, MINB)
     csr_pattern_kernel(const int32_t *__restrict__ row_ptr, const double *__restrict__ val, const uint8_t *__restrict__ pat_id,
@@ -914,8 +942,9 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
                        const double *__restrict__ x, double *__restrict__ y, int32_t row_begin, int32_t row_end,
                        uint32_t stage_bytes, const __grid_constant__ YFan fan, double alpha, double beta)
 {
-    csr_pattern_body<WARPS, R, STAGES, CH, MINB, FANOUT, EPI, false>(row_ptr, val, pat_id, pat_off, pat_len, npat, maxlen, x, y, row_begin,
-                                                                    row_end, stage_bytes, fan, alpha, beta, nullptr, nullptr);
+    csr_pattern_body<double, WARPS, R, STAGES, CH, MINB, FANOUT, EPI, false>(row_ptr, val, pat_id, pat_off, pat_len, npat, maxlen, x,
+                                                                            y, row_begin, row_end, stage_bytes, fan, alpha, beta,
+                                                                            nullptr, nullptr);
 }
 template <int WARPS, int R, int STAGES, int CH, int MINB>
 __global__ void __launch_bounds__(WARPS * 32, MINB)
@@ -924,8 +953,48 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
                            const double *__restrict__ x, double *__restrict__ y, int32_t rows, uint32_t stage_bytes, double alpha,
                            double beta, const double *__restrict__ w, double *__restrict__ part)
 {
-    csr_pattern_body<WARPS, R, STAGES, CH, MINB, false, true, true>(row_ptr, val, pat_id, pat_off, pat_len, npat, maxlen, x, y, 0, rows,
-                                                                   stage_bytes, YFan(), alpha, beta, w, part);
+    csr_pattern_body<double, WARPS, R, STAGES, CH, MINB, false, true, true>(row_ptr, val, pat_id, pat_off, pat_len, npat, maxlen, x, y,
+                                                                           0, rows, stage_bytes, YFan(), alpha, beta, w, part);
+}
+// narrow values (V = float or fp16 as uint16_t): the kernels read the plan's copy A->pat_val
+template <typename V, int WARPS, int R, int STAGES, int CH, int MINB, bool FANOUT, bool EPI>
+__global__ void __launch_bounds__(WARPS * 32, MINB)
+    csr_pattern_kernel_narrow(const int32_t *__restrict__ row_ptr, const V *__restrict__ val, const uint8_t *__restrict__ pat_id,
+                              const int32_t *__restrict__ pat_off, const int32_t *__restrict__ pat_len, int32_t npat, int32_t maxlen,
+                              const double *__restrict__ x, double *__restrict__ y, int32_t row_begin, int32_t row_end,
+                              uint32_t stage_bytes, const __grid_constant__ YFan fan, double alpha, double beta)
+{
+    csr_pattern_body<V, WARPS, R, STAGES, CH, MINB, FANOUT, EPI, false>(row_ptr, val, pat_id, pat_off, pat_len, npat, maxlen, x, y,
+                                                                       row_begin, row_end, stage_bytes, fan, alpha, beta, nullptr,
+                                                                       nullptr);
+}
+template <typename V, int WARPS, int R, int STAGES, int CH, int MINB>
+__global__ void __launch_bounds__(WARPS * 32, MINB)
+    csr_pattern_dot_kernel_narrow(const int32_t *__restrict__ row_ptr, const V *__restrict__ val, const uint8_t *__restrict__ pat_id,
+                                  const int32_t *__restrict__ pat_off, const int32_t *__restrict__ pat_len, int32_t npat,
+                                  int32_t maxlen, const double *__restrict__ x, double *__restrict__ y, int32_t rows,
+                                  uint32_t stage_bytes, double alpha, double beta, const double *__restrict__ w,
+                                  double *__restrict__ part)
+{
+    csr_pattern_body<V, WARPS, R, STAGES, CH, MINB, false, true, true>(row_ptr, val, pat_id, pat_off, pat_len, npat, maxlen, x, y, 0,
+                                                                      rows, stage_bytes, YFan(), alpha, beta, w, part);
+}
+// the instantiation of each kernel for value type V
+template <typename V, class C, bool FANOUT, bool EPI>
+constexpr auto pattern_kernel()
+{
+    if constexpr (std::is_same<V, double>::value)
+        return csr_pattern_kernel<C::WARPS, C::R, C::STAGES, C::CH, C::MINB, FANOUT, EPI>;
+    else
+        return csr_pattern_kernel_narrow<V, C::WARPS, C::R, C::STAGES, C::CH, C::MINB, FANOUT, EPI>;
+}
+template <typename V, class C>
+constexpr auto pattern_dot_kernel()
+{
+    if constexpr (std::is_same<V, double>::value)
+        return csr_pattern_dot_kernel<C::WARPS, C::R, C::STAGES, C::CH, C::MINB>;
+    else
+        return csr_pattern_dot_kernel_narrow<V, C::WARPS, C::R, C::STAGES, C::CH, C::MINB>;
 }
 
 // ---- the pattern kernel's configuration.  Measured on B200 (profiles/r03_logs/sweep_pattern.log, stencil 369^3, the
@@ -940,25 +1009,38 @@ struct PatternCfg
     static constexpr int CH = 14;   // gathers in flight per lane
     static constexpr int MINB = 7;  // min CTAs per SM
 };
-
-// rows [row_begin, row_end) of a handle with the row-pattern plan
-static int csr_mult_pattern(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, const Axpby &ab, cudaStream_t s,
-                            int32_t row_begin, int32_t row_end, const DotOut *dot = nullptr)
+// narrow values: a smaller stage per warp, so more CTAs fit.  Swept per width on the same stencil over {CH, CTAs/SM} =
+// {14, 7}, {14, 8}, {14, 9}, {10, 10}, {8, 12}, {6, 16 (fp32: 13)} (profiles/r05_logs/sweep_width.log, DESIGN.md §5.2):
+// fp16 keeps fp64's configuration, fp32 takes 8 CTAs/SM.  WARPS and R stay those of fp64 at every width: the dot's work
+// units are tiles of 32 rows.
+template <typename V>
+struct PatternCfgOf : PatternCfg
 {
-    using C = PatternCfg;
+};
+template <>
+struct PatternCfgOf<float> : PatternCfg
+{
+    static constexpr int MINB = 8;
+};
+
+template <typename V>
+static int launch_pattern(const smvp_csr *A, const V *val, const double *d_x, double *d_y, const YFan *fan, const Axpby &ab,
+                          cudaStream_t s, int32_t row_begin, int32_t row_end, const DotOut *dot)
+{
+    using C = PatternCfgOf<V>;
     const int maxlen = A->pattern_maxlen > 0 ? A->pattern_maxlen : 1;
-    const int stage = PatternShape<C::R>::stage_bytes(maxlen);
+    const int stage = PatternShape<C::R>::stage_bytes(maxlen, (int)sizeof(V));
     const int table = (A->pattern_count * (maxlen + 1) * 4 + 127) & ~127;
     const int smem = table + C::WARPS * C::STAGES * stage;
     const int64_t need = ceil_div64(ceil_div64((int64_t)row_end - row_begin, PatternShape<C::R>::ROWS), C::WARPS);
     if (dot) // whole passes only: the partial of tile t goes to dot->part[t]
     {
-        auto kern = csr_pattern_dot_kernel<C::WARPS, C::R, C::STAGES, C::CH, C::MINB>;
+        auto kern = pattern_dot_kernel<V, C>();
         static thread_local Residency res;
         int64_t grid = 0;
         SMVP_TRY(persistent_grid(kern, C::WARPS * 32, smem, A->merge_headroom, need, res, &grid));
         if (grid > 0)
-            SMVP_LAUNCH(kern, (unsigned)grid, C::WARPS * 32, smem, s, A->row_ptr, A->val, A->pat_id, A->pat_off, A->pat_len,
+            SMVP_LAUNCH(kern, (unsigned)grid, C::WARPS * 32, smem, s, A->row_ptr, val, A->pat_id, A->pat_off, A->pat_len,
                         A->pattern_count, maxlen, d_x, d_y, A->rows, (uint32_t)stage, ab.alpha, ab.beta, dot->w, dot->part);
         return (int)SMVP_OK;
     }
@@ -969,19 +1051,30 @@ static int csr_mult_pattern(const smvp_csr *A, const double *d_x, double *d_y, c
                 return (int)SMVP_E_ARG;
             else
             {
-                auto kern = csr_pattern_kernel<C::WARPS, C::R, C::STAGES, C::CH, C::MINB, FANOUT, EPI>;
+                auto kern = pattern_kernel<V, C, FANOUT, EPI>();
                 // the shared memory depends on the matrix (longest pattern, pattern count): occupancy is looked up per size
                 static thread_local Residency res;
                 int64_t grid = 0;
                 SMVP_TRY(persistent_grid(kern, C::WARPS * 32, smem, A->merge_headroom, need, res, &grid));
                 if (grid > 0)
-                    SMVP_LAUNCH(kern, (unsigned)grid, C::WARPS * 32, smem, s, A->row_ptr, A->val, A->pat_id, A->pat_off, A->pat_len,
+                    SMVP_LAUNCH(kern, (unsigned)grid, C::WARPS * 32, smem, s, A->row_ptr, val, A->pat_id, A->pat_off, A->pat_len,
                                 A->pattern_count, maxlen, d_x, d_y, row_begin, row_end, (uint32_t)stage, fan ? *fan : YFan(),
                                 ab.alpha, ab.beta);
                 return (int)SMVP_OK;
             }
         });
     });
+}
+
+// rows [row_begin, row_end) of a handle with the row-pattern plan, its values streamed at the plan's width
+static int csr_mult_pattern(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, const Axpby &ab, cudaStream_t s,
+                            int32_t row_begin, int32_t row_end, const DotOut *dot = nullptr)
+{
+    if (A->pat_vbytes == 2)
+        return launch_pattern(A, (const uint16_t *)A->pat_val, d_x, d_y, fan, ab, s, row_begin, row_end, dot);
+    if (A->pat_vbytes == 4)
+        return launch_pattern(A, (const float *)A->pat_val, d_x, d_y, fan, ab, s, row_begin, row_end, dot);
+    return launch_pattern(A, (const double *)A->val, d_x, d_y, fan, ab, s, row_begin, row_end, dot);
 }
 
 constexpr Axpby AXPBY_PLAIN = {1.0, 0.0};
@@ -1669,5 +1762,6 @@ extern "C" int smvp_csr_info(const smvp_csr *A, smvp_csr_info_t *out)
     out->launches_per_mult[SMVP_CSR_AUTO] = out->launches_per_mult[out->auto_variant];
     out->x_relabel = A->relabel_state;
     out->row_patterns = A->pattern_state == 1 ? A->pattern_count : A->pattern_state;
+    out->value_bytes = A->pat_vbytes;
     return SMVP_OK;
 }

@@ -18,6 +18,12 @@
 //      collision) rejects the plan.  A hash match alone never decides a column.
 // The plan is given up when a row is longer than PAT_LMAX, when more than PAT_MAX patterns occur, or when the handle is
 // relabelled (that plan decides first).  SMVP_CSR_PATTERN=0 keeps it off.
+//
+// Value width: with col_ind gone, val is 93 % of what the pattern kernel streams.  Once the plan is accepted, one pass
+// over val checks which of fp16 and fp32 hold every value with the same 64 bits (pattern and integer matrices,
+// constant-coefficient stencils such as the benchmark's {26, -1}); the kernel then streams a copy at the narrowest such
+// width and widens each value exactly, so y is unchanged.  It depends on the precision the values need, not on how many
+// distinct values there are.  val itself stays for every other path.
 #include "common.cuh"
 
 #include <algorithm>
@@ -139,13 +145,73 @@ __global__ void __launch_bounds__(256) pattern_assign_kernel(const int32_t *__re
     }
 }
 
+// flags |= 1 when some value does not survive fp16 and back with its 64 bits, |= 2 when some value does not survive fp32.
+// Bits, not ==: -0.0 keeps its sign, subnormals and out-of-range values fail, a NaN passes only with its payload intact.
+__global__ void __launch_bounds__(256) pattern_width_kernel(const double *__restrict__ val, int64_t nnz, int32_t *flags)
+{
+    unsigned f = 0;
+    for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < nnz; j += (int64_t)gridDim.x * blockDim.x)
+    {
+        const double v = val[j];
+        const long long b = __double_as_longlong(v);
+        if (__double_as_longlong(widen_value(narrow_value<uint16_t>(v))) != b)
+            f |= 1u;
+        if (__double_as_longlong(widen_value(narrow_value<float>(v))) != b)
+            f |= 2u;
+    }
+    f = __reduce_or_sync(0xffffffffu, f);
+    if ((threadIdx.x & 31) == 0 && f)
+        atomicOr(flags, (int32_t)f);
+}
+
+template <typename V>
+__global__ void __launch_bounds__(256) pattern_narrow_kernel(const double *__restrict__ val, int64_t nnz, V *__restrict__ out)
+{
+    for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < nnz; j += (int64_t)gridDim.x * blockDim.x)
+        out[j] = narrow_value<V>(val[j]);
+}
+
+// the narrowest width (2, 4 or 8 bytes) that holds every value exactly, and the copy of val at that width
+static int pattern_values(smvp_csr *A, unsigned grid, cudaStream_t s)
+{
+    DevTmp g_flags;
+    SMVP_CUDA(g_flags.alloc<int32_t>(1));
+    int32_t *flags = g_flags.as<int32_t>(), h_flags = 0;
+    SMVP_CUDA(cudaMemsetAsync(flags, 0, sizeof(int32_t), s));
+    if (A->nnz > 0)
+        SMVP_LAUNCH(pattern_width_kernel, grid, 256, 0, s, (const double *)A->val, A->nnz, flags);
+    SMVP_CUDA(cudaGetLastError());
+    SMVP_CUDA(cudaMemcpyAsync(&h_flags, flags, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    SMVP_CUDA(cudaStreamSynchronize(s));
+    const int32_t vbytes = !(h_flags & 1) ? 2 : !(h_flags & 2) ? 4 : 8;
+    if (vbytes == 2)
+    {
+        SMVP_CUDA(dev_alloc((uint16_t **)&A->pat_val, A->nnz));
+        if (A->nnz > 0)
+            SMVP_LAUNCH(pattern_narrow_kernel<uint16_t>, grid, 256, 0, s, (const double *)A->val, A->nnz, (uint16_t *)A->pat_val);
+    }
+    else if (vbytes == 4)
+    {
+        SMVP_CUDA(dev_alloc((float **)&A->pat_val, A->nnz));
+        if (A->nnz > 0)
+            SMVP_LAUNCH(pattern_narrow_kernel<float>, grid, 256, 0, s, (const double *)A->val, A->nnz, (float *)A->pat_val);
+    }
+    SMVP_CUDA(cudaGetLastError());
+    SMVP_CUDA(cudaStreamSynchronize(s));
+    A->pat_vbytes = vbytes;
+    return SMVP_OK;
+}
+
 void csr_pattern_release(smvp_csr *A)
 {
     cudaFree(A->pat_id);
     cudaFree(A->pat_off);
     cudaFree(A->pat_len);
+    cudaFree(A->pat_val);
     A->pat_id = nullptr;
     A->pat_off = A->pat_len = nullptr;
+    A->pat_val = nullptr;
+    A->pat_vbytes = 0;
 }
 
 // decides (once per handle) and, when every row matches one of at most PAT_MAX patterns, builds the plan.  Synchronous.
@@ -224,8 +290,14 @@ int csr_pattern_plan(smvp_csr *A, cudaStream_t s)
         A->pattern_state = rc == SMVP_OK ? -1 : 0;
         return rc;
     }
+    const int rv = pattern_values(A, grid, s);
+    if (rv != SMVP_OK)
+    {
+        csr_pattern_release(A);
+        return rv; // undecided: the next pass tries again
+    }
     A->pattern_count = npat;
-    A->device_bytes += (int64_t)A->rows + 4 * (int64_t)npat * (PAT_LMAX + 1);
+    A->device_bytes += (int64_t)A->rows + 4 * (int64_t)npat * (PAT_LMAX + 1) + (A->pat_vbytes < 8 ? A->pat_vbytes * A->nnz : 0);
     A->pattern_state = 1;
     return SMVP_OK;
 }

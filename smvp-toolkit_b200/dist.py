@@ -714,7 +714,9 @@ class RowBlockCsr:
         """What the multiply does beyond the plain kernel (decided by the library from the matrix, reported as is)."""
         if self.variant_name == "merge" and self.A.row_patterns > 0:
             return ("rows share %d column-offset patterns (smvp_csr_info_t.row_patterns): the kernel streams pattern ids "
-                    "instead of col_ind" % self.A.row_patterns)
+                    "instead of col_ind, and the values as %s (smvp_csr_info_t.value_bytes = %d: %s)"
+                    % (self.A.row_patterns, {2: "fp16", 4: "fp32", 8: "fp64"}.get(self.A.value_bytes, "?"), self.A.value_bytes,
+                       "fp64" if self.A.value_bytes == 8 else "every value converts to it and back exactly"))
         if self.A.x_relabel == 1:
             return ("column space relabelled by popularity (smvp_csr_info_t.x_relabel = 1): the kernels read rank-ordered "
                     "column indices and a permuted copy of x formed ONCE per x by smvp_csr_set_x_device, outside the "

@@ -45,7 +45,7 @@ class _CsrInfo(ctypes.Structure):
                 ("max_row_nnz", ctypes.c_int32), ("auto_variant", ctypes.c_int32), ("input_order", ctypes.c_int32),
                 ("bytes_per_mult", ctypes.c_int64), ("device_bytes", ctypes.c_int64),
                 ("launches_per_mult", ctypes.c_int32 * 3), ("x_relabel", ctypes.c_int32),
-                ("row_patterns", ctypes.c_int32)]
+                ("row_patterns", ctypes.c_int32), ("value_bytes", ctypes.c_int32)]
 
 
 class _TjdsInfo(ctypes.Structure):
@@ -298,6 +298,14 @@ class CsrMatrix:
         info = _CsrInfo()
         _check(lib().smvp_csr_info(self._h, ctypes.byref(info)), "smvp_csr_info")
         return info.row_patterns
+
+    @property
+    def value_bytes(self):
+        """With row_patterns > 0: 2 / 4 / 8 = the pattern kernel streams the values as fp16 / fp32 / fp64 (a narrow width
+        only when every value converts to it and back exactly), 0: not decided yet."""
+        info = _CsrInfo()
+        _check(lib().smvp_csr_info(self._h, ctypes.byref(info)), "smvp_csr_info")
+        return info.value_bytes
 
     def mult_device_fanout(self, d_x, y_ptrs, variant=CSR_AUTO, stream=None):
         """y = A x stored into every destination of y_ptrs (device addresses, possibly peer-mapped)."""
