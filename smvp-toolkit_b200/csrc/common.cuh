@@ -77,13 +77,67 @@ struct DotOut
     double *part;    // one partial per work unit
 };
 __device__ __forceinline__ double dot_term(const double *w, int64_t r, double v) { return __dmul_rn(w ? __ldg(w + r) : v, v); }
-// the epilogue's store of a dot pass: y[r] = fl(alpha * s) + fl(beta * y[r]) and the running sum acc += dot_term
-__device__ __forceinline__ void store_axpby_dot(double *__restrict__ y, int64_t r, double s, double alpha, double beta,
-                                                const double *__restrict__ w, double &acc)
+
+// Multi GPU (row blocks, SURVEY.md 8e): every rank must end with the whole y, so the CSR multiply kernels store each
+// finished row straight into every peer's copy of y over NVLink (peer-mapped symmetric memory): the "allgather" is fused
+// into the SpMV epilogue and overlaps the streaming of the matrix instead of following it.
+constexpr int SMVP_MAX_FANOUT = 8;
+struct YFan
 {
-    const double v = axpby(alpha, s, beta, beta != 0.0 ? y[r] : 0.0);
-    y[r] = v;
-    acc = __dadd_rn(acc, dot_term(w, r, v));
+    double *p[SMVP_MAX_FANOUT];
+    int n;
+};
+
+// How a kernel stores a finished row s of y.  Every kernel that stores y takes the mode as a template parameter, so each
+// instantiation stores one way:
+//   Plain   y[r] = s
+//   Fanout  s into every copy of y in a YFan; y is only ever written, never read, so it may be a write-only mapping
+//   Axpby   y[r] = fl(alpha * s) + fl(beta * y[r])   (the *_axpby entry points)
+//   Dot     Axpby, and the row's dot term goes to the kernel's work-unit partial   (the *_axpby_dot entry points)
+enum class YStore
+{
+    Plain,
+    Fanout,
+    Axpby,
+    Dot
+};
+__host__ __device__ constexpr bool reads_y(YStore m) { return m == YStore::Axpby || m == YStore::Dot; } // only when beta != 0
+// the mode of a pass: a dot pass runs the epilogue and never fans out; the fan-out only serves y = A x
+static inline YStore store_mode(bool dot, bool fan, const Axpby &ab)
+{
+    return dot ? YStore::Dot : fan ? YStore::Fanout : ab.plain() ? YStore::Plain : YStore::Axpby;
+}
+// Lifts a run-time store mode into a template argument, like with_flag: f(std::integral_constant<YStore, m>()) for the
+// modes Ms a kernel family is instantiated with (the launcher lists them), so that each launcher names every
+// instantiation once.  Store modes are picked by store_mode, so m is always one of Ms.
+template <YStore... Ms, typename F>
+static inline int with_store(YStore m, F &&f)
+{
+    int rc = SMVP_E_ARG;
+    (void)((m == Ms && ((rc = f(std::integral_constant<YStore, Ms>())), true)) || ...);
+    return rc;
+}
+// The store of row r in mode M (fan: the copies of a Fanout store).  Returns the row's dot term in Dot mode, +0.0 otherwise.
+// Every row has exactly one writer in a pass, so the read-modify-write of Axpby and Dot is safe; beta == 0 never loads y.
+template <YStore M>
+__device__ __forceinline__ double store_row(double *__restrict__ y, int64_t r, double s, double alpha, double beta,
+                                            const double *__restrict__ w, const YFan *fan = nullptr)
+{
+    if constexpr (M == YStore::Plain)
+        y[r] = s;
+    else if constexpr (M == YStore::Fanout)
+    {
+        for (int k = 0; k < fan->n; k++)
+            fan->p[k][r] = s;
+    }
+    else
+    {
+        const double v = axpby(alpha, s, beta, beta != 0.0 ? y[r] : 0.0);
+        y[r] = v;
+        if constexpr (M == YStore::Dot)
+            return dot_term(w, r, v);
+    }
+    return 0.0;
 }
 // pairwise tree over the 32 lanes in lane order (a butterfly: every lane ends with the same bits)
 __device__ __forceinline__ double warp_tree_sum(double v)

@@ -135,33 +135,9 @@ __device__ __forceinline__ int32_t lds_s32(uint32_t a)
 }
 
 // ------------------------------------------------------------------ where y goes
-// Single GPU: one pointer.  Multi GPU (row blocks, SURVEY.md 8e): every rank must end with the whole y, so
-// the multiply kernels store each finished row straight into every peer's copy of y over NVLink
-// (peer-mapped symmetric memory): the "allgather" is fused into the SpMV epilogue and overlaps the
-// streaming of the matrix instead of following it.  y is only ever written, never read.
-constexpr int SMVP_MAX_FANOUT = 8;
-struct YFan
-{
-    double *p[SMVP_MAX_FANOUT];
-    int n;
-};
-// EPI (the *_axpby calls, never with a fan-out): y[row] = alpha * v + beta * y[row] (axpby, common.cuh).  Every row has
-// exactly one writer in a pass (the lane that ends it, or the fix-up kernel for rows cut by tile boundaries), so the
-// read-modify-write is safe.
-template <bool FANOUT, bool EPI>
-__device__ __forceinline__ void store_y(double *__restrict__ y, const YFan &fan, int64_t row, double v, double alpha, double beta)
-{
-    static_assert(!(FANOUT && EPI), "the epilogue is not instantiated with the fan-out");
-    if (FANOUT)
-    {
-        for (int k = 0; k < fan.n; k++)
-            fan.p[k][row] = v;
-    }
-    else if (EPI)
-        y[row] = axpby(alpha, v, beta, beta != 0.0 ? y[row] : 0.0);
-    else
-        y[row] = v;
-}
+// The kernels below store y in one of the modes of common.cuh (YStore, store_row).  Under Axpby and Dot the lane that ends
+// a row, or the fix-up kernel for rows cut by tile boundaries, is the row's one writer.
+
 // y[r] for the epilogue, loaded ahead of its store: through the coherent path (y is written by the same kernel) and
 // issued where it stands (volatile: not sunk to its use)
 __device__ __forceinline__ double ld_y_early(const double *p)
@@ -177,23 +153,22 @@ __device__ __forceinline__ double ld_w_early(const double *p)
     asm volatile("ld.global.nc.f64 %0, [%1];" : "=d"(v) : "l"(p));
     return v;
 }
-// the instantiations the launchers name: the epilogue exists only without the fan-out
-template <bool FANOUT, bool EPI>
-constexpr bool kernel_exists() { return !(FANOUT && EPI); }
 
 // =====================================================================================  VECTOR
 // LPR >= 16 (WIDE): each lane pulls 4 consecutive entries per step with 128-bit loads (long rows).
 // LPR < 16: lane l takes entries l, l+LPR, ... with 8/4-byte loads (short rows).  With only a few rows per warp
 //           the lanes of one request then sit on consecutive entries of consecutive rows, so the x gather of a
 //           banded matrix touches far fewer sectors per request -- the vector kernel is L1-bound on such rows.
-// DOT (csr_vector_dot_kernel): the work unit is the CTA -- the rows its sub-warps end, in thread order
-template <int LPR, bool FANOUT, bool EPI, bool DOT>
-__device__ __forceinline__ void csr_vector_body(const int32_t *__restrict__ row_ptr, const int32_t *__restrict__ col_ind,
-                                                const double *__restrict__ val, const double *__restrict__ x, double *__restrict__ y,
-                                                int32_t rows, const YFan &fan, double alpha, double beta, const double *__restrict__ w,
-                                                double *__restrict__ part)
+// Dot: the work unit is the CTA -- the rows its sub-warps end, in thread order.  It runs at 6 CTAs per SM: at the default
+// bound ptxas keeps 32 registers and spills in the 128-bit configurations.
+template <YStore M>
+__host__ __device__ constexpr int vector_min_ctas() { return M == YStore::Dot ? 6 : 0; }
+template <int LPR, YStore M>
+__global__ void __launch_bounds__(256, vector_min_ctas<M>())
+    csr_vector_kernel(const int32_t *__restrict__ row_ptr, const int32_t *__restrict__ col_ind, const double *__restrict__ val,
+                      const double *__restrict__ x, double *__restrict__ y, int32_t rows, const __grid_constant__ YFan fan, double alpha,
+                      double beta, const double *__restrict__ w, double *__restrict__ part)
 {
-    static_assert(!DOT || (EPI && !FANOUT), "the dot is formed by the epilogue");
     constexpr bool WIDE = LPR >= 16;
     const int64_t gt = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const int64_t row = gt / LPR;
@@ -247,41 +222,15 @@ __device__ __forceinline__ void csr_vector_body(const int32_t *__restrict__ row_
 #pragma unroll
     for (int o = LPR / 2; o > 0; o >>= 1)
         sum = __dadd_rn(sum, __shfl_xor_sync(0xffffffffu, sum, o));
-    if (!DOT)
+    double d = 0.0;
+    if (row < rows && lane == 0)
+        d = store_row<M>(y, row, sum, alpha, beta, w, &fan);
+    if constexpr (M == YStore::Dot)
     {
-        if (row < rows && lane == 0)
-            store_y<FANOUT, EPI>(y, fan, row, sum, alpha, beta);
-    }
-    else
-    {
-        double d = 0.0;
-        if (row < rows && lane == 0)
-        {
-            const double v = axpby(alpha, sum, beta, beta != 0.0 ? y[row] : 0.0);
-            y[row] = v;
-            d = dot_term(w, row, v);
-        }
         d = cta_tree_sum<256>(d);
         if (threadIdx.x == 0)
             part[blockIdx.x] = d;
     }
-}
-template <int LPR, bool FANOUT, bool EPI>
-__global__ void __launch_bounds__(256) csr_vector_kernel(const int32_t *__restrict__ row_ptr, const int32_t *__restrict__ col_ind,
-                                                         const double *__restrict__ val, const double *__restrict__ x,
-                                                         double *__restrict__ y, int32_t rows, const __grid_constant__ YFan fan,
-                                                         double alpha, double beta)
-{
-    csr_vector_body<LPR, FANOUT, EPI, false>(row_ptr, col_ind, val, x, y, rows, fan, alpha, beta, nullptr, nullptr);
-}
-// (6 CTAs per SM: at the default bound ptxas keeps 32 registers and spills in the 128-bit configurations)
-template <int LPR>
-__global__ void __launch_bounds__(256, 6) csr_vector_dot_kernel(const int32_t *__restrict__ row_ptr, const int32_t *__restrict__ col_ind,
-                                                             const double *__restrict__ val, const double *__restrict__ x,
-                                                             double *__restrict__ y, int32_t rows, double alpha, double beta,
-                                                             const double *__restrict__ w, double *__restrict__ part)
-{
-    csr_vector_body<LPR, false, true, true>(row_ptr, col_ind, val, x, y, rows, YFan(), alpha, beta, w, part);
 }
 
 // =====================================================================================  TINY LOOP
@@ -339,24 +288,13 @@ static int launch_vector(const smvp_csr *A, const double *d_x, double *d_y, cons
     const int64_t blocks = ceil_div64(threads, 256);
     if (blocks > 0x7fffffffLL)
         return SMVP_E_TOOBIG;
-    if (blocks > 0 && dot)
-        SMVP_LAUNCH(csr_vector_dot_kernel<LPR>, (unsigned)blocks, 256, 0, s, A->row_ptr, mult_cols(A), A->val, d_x, d_y, A->rows,
-                    ab.alpha, ab.beta, dot->w, dot->part);
-    else if (blocks > 0)
-        return with_flag(fan != nullptr, [&](auto F) {
-            return with_flag(!ab.plain(), [&](auto E) {
-                constexpr bool FANOUT = decltype(F)::value, EPI = decltype(E)::value;
-                if constexpr (!kernel_exists<FANOUT, EPI>())
-                    return (int)SMVP_E_ARG;
-                else
-                {
-                    SMVP_LAUNCH((csr_vector_kernel<LPR, FANOUT, EPI>), (unsigned)blocks, 256, 0, s, A->row_ptr, mult_cols(A), A->val,
-                                d_x, d_y, A->rows, fan ? *fan : YFan(), ab.alpha, ab.beta);
-                    return (int)SMVP_OK;
-                }
-            });
-        });
-    return SMVP_OK;
+    if (blocks == 0)
+        return SMVP_OK;
+    return with_store<YStore::Plain, YStore::Fanout, YStore::Axpby, YStore::Dot>(store_mode(dot, fan, ab), [&](auto S) {
+        SMVP_LAUNCH((csr_vector_kernel<LPR, decltype(S)::value>), (unsigned)blocks, 256, 0, s, A->row_ptr, mult_cols(A), A->val, d_x,
+                    d_y, A->rows, fan ? *fan : YFan(), ab.alpha, ab.beta, dot ? dot->w : nullptr, dot ? dot->part : nullptr);
+        return (int)SMVP_OK;
+    });
 }
 
 static int csr_mult_vector(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fan, const Axpby &ab, const DotOut *dot,
@@ -449,12 +387,11 @@ __device__ __forceinline__ TileView make_tile(int32_t r0, int32_t r1, int32_t t,
 
 // First row of a tile that ends a row there: y[row] = (carries of the tiles the row crossed, in tile order) + (partial
 // of the tile where it ends).  tile_row[u+1] is the row tile u's carry belongs to.
-// DOT: the row's dot term is added to tile t's partial, which the merge kernel left (its unit: the tile plus this row).
-template <bool FANOUT, bool EPI, bool DOT = false>
+// Dot: the row's dot term is added to tile t's partial, which the merge kernel left (its unit: the tile plus this row).
+template <YStore M>
 __device__ __forceinline__ void merge_fixup_tile(int32_t t, const int32_t *__restrict__ tile_row, const double *__restrict__ head_val,
                                                  const double *__restrict__ carry_val, double *__restrict__ y, const YFan &fan,
-                                                 double alpha, double beta, const double *__restrict__ w = nullptr,
-                                                 double *__restrict__ part = nullptr)
+                                                 double alpha, double beta, const double *__restrict__ w, double *__restrict__ part)
 {
     // everything the common case needs is loaded up front (independent loads: one memory round trip)
     const int32_t r = tile_row[t];
@@ -481,14 +418,9 @@ __device__ __forceinline__ void merge_fixup_tile(int32_t t, const int32_t *__res
             acc = __dadd_rn(acc, __ldcg(carry_val + k));
         acc = __dadd_rn(acc, h);
     }
-    if (!DOT)
-        store_y<FANOUT, EPI>(y, fan, r, acc, alpha, beta);
-    else
-    {
-        const double v = axpby(alpha, acc, beta, beta != 0.0 ? y[r] : 0.0);
-        y[r] = v;
-        part[t] = __dadd_rn(__ldcg(part + t), dot_term(w, r, v));
-    }
+    const double d = store_row<M>(y, r, acc, alpha, beta, w, &fan);
+    if constexpr (M == YStore::Dot)
+        part[t] = __dadd_rn(__ldcg(part + t), d);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -497,61 +429,326 @@ __device__ __forceinline__ void merge_fixup_tile(int32_t t, const int32_t *__res
 // never meets a block-wide barrier: warps of a CTA drift apart freely, so while one waits for HBM
 // or for its x gathers the others walk.  Rows cut by lane boundaries are stitched with a segmented
 // warp scan (__shfl_up_sync), rows cut by tile boundaries by the fix-up kernel -- fixed order, no atomics.
-template <int WARPS, int IPT, int MINB, bool FANOUT, bool RANKED, bool UNI, bool EPI>
+// Dot (DESIGN.md §5.7): whole passes only.  The work unit is the warp tile -- each lane adds the dot terms of the rows it
+// stores in the order it stores them, the lanes are added in a pairwise tree into part[t], and the fix-up kernel adds the
+// term of the tile's first row (merge_fixup_tile).
+template <int WARPS, int IPT, int MINB, bool RANKED, bool UNI, YStore M>
 __global__ void __launch_bounds__(WARPS * 32, MINB)
     csr_merge_warp_kernel(const int32_t *__restrict__ row_ptr, const int32_t *__restrict__ col_ind, const double *__restrict__ val,
                           const double *__restrict__ x, double *__restrict__ y, const int32_t *__restrict__ tile_row, int32_t rows,
                           int64_t nnz, int32_t tile_begin, int32_t num_tiles, double *__restrict__ head_val,
                           double *__restrict__ carry_val, const __grid_constant__ YFan fan, int32_t hot_l1, int32_t hot_l2,
-                          int32_t early_dependents, double alpha, double beta)
+                          int32_t early_dependents, double alpha, double beta, const double *__restrict__ dot_w,
+                          double *__restrict__ part)
 {
-#define SMVP_MERGE_DOT 0
-#include "merge_warp_body.cuh"
-#undef SMVP_MERGE_DOT
-}
-// The dot pass (DESIGN.md §5.7): the work unit is the warp tile -- each lane adds the dot terms of the rows it stores in
-// the order it stores them, the lanes are added in a pairwise tree into part[t], and the fix-up kernel adds the term of
-// the tile's first row (merge_fixup_tile).  Whole passes only, with the epilogue, never with the fan-out.
-template <int WARPS, int IPT, int MINB, bool RANKED, bool UNI>
-__global__ void __launch_bounds__(WARPS * 32, MINB)
-    csr_merge_warp_dot_kernel(const int32_t *__restrict__ row_ptr, const int32_t *__restrict__ col_ind, const double *__restrict__ val,
-                              const double *__restrict__ x, double *__restrict__ y, const int32_t *__restrict__ tile_row, int32_t rows,
-                              int64_t nnz, int32_t num_tiles, double *__restrict__ head_val, double *__restrict__ carry_val,
-                              int32_t hot_l1, int32_t hot_l2, int32_t early_dependents, double alpha, double beta,
-                              const double *__restrict__ dot_w, double *__restrict__ part)
-{
-    constexpr bool EPI = true;
-    constexpr int32_t tile_begin = 0;
-#define SMVP_MERGE_DOT 1
-#include "merge_warp_body.cuh"
-#undef SMVP_MERGE_DOT
+    // Small grids (early_dependents != 0): let the fix-up kernel, launched with programmatic stream serialization, be
+    // scheduled NOW; it parks at griddepcontrol.wait until this grid has completed and flushed.  In the batched `-n` loop
+    // of a matrix like memplus that hides the second launch's latency (a pass lasts as long as a launch).
+    if (early_dependents)
+        asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+    // processes tiles [tile_begin, num_tiles): a sub-range lets the host overlap the copy-out of finished rows.
+    // One stage per warp: deeper rings lost to more resident warps in every sweep.
+    using Shape = MergeShape<32, IPT>;
+    extern __shared__ __align__(128) unsigned char stage_mem[];
+    __shared__ __align__(8) uint64_t full_bar[WARPS];
+
+    // UNI: the warp index and the tile coordinates below are broadcast from lane 0.  The values are the same in every lane
+    // anyway, but the broadcast lets the compiler PROVE it and keep the whole tile bookkeeping (and the operands of the
+    // bulk copies) in uniform registers instead of electing a lane and converting per copy.  Measured on B200
+    // (profiles/r01_logs/diet_bisect.log): stencil configuration 2.78 -> 2.69 ms, but the R-MAT configuration 5.67 ->
+    // 6.39 ms, so it is a per-configuration choice (MergeStencil::UNI, MergeSkewed::UNI).
+#define SMVP_BCAST(v) (UNI ? __shfl_sync(0xffffffffu, (v), 0) : (v))
+    const int lane = threadIdx.x & 31, w = SMVP_BCAST((int)(threadIdx.x >> 5));
+    const int64_t total = (int64_t)rows + nnz;
+    unsigned char *base = stage_mem + (size_t)w * Shape::SMEM_BYTES;
+    uint64_t *my_bar = &full_bar[w];
+    uint64_t policy = 0;
+    if (lane == 0)
+    {
+        mbar_init(my_bar, 1);
+        fence_mbar_init();
+        policy = l2_evict_first_policy();
+    }
+    __syncwarp();
+
+    const uint64_t pol_last = RANKED ? l2_evict_last_policy() : 0, pol_first = RANKED ? l2_evict_first_policy() : 0;
+    const int32_t warp_stride = (int32_t)gridDim.x * WARPS;
+    auto issue = [&](const TileView &v) { // lane 0 only
+        mbar_expect_tx(my_bar, v.vb + v.cb + v.rb);
+        if (v.vb)
+            bulk_g2s(base, val + v.va, v.vb, my_bar, policy);
+        if (v.cb)
+            bulk_g2s(base + v.vb, col_ind + v.ca, v.cb, my_bar, policy);
+        if (v.rb)
+            bulk_g2s(base + v.vb + v.cb, row_ptr + v.ra, v.rb, my_bar, policy);
+    };
+
+    int32_t t = (M == YStore::Dot ? 0 : tile_begin) + (int32_t)blockIdx.x * WARPS + w; // a dot pass is a whole pass
+    int32_t cur_r0 = 0, cur_r1 = 0; // merge coordinates of the tile in flight: the only tile state kept across the loop
+    if (t < num_tiles)
+    {
+        cur_r0 = SMVP_BCAST(__ldg(tile_row + t));
+        cur_r1 = SMVP_BCAST(__ldg(tile_row + t + 1));
+        if (lane == 0)
+            issue(make_tile(cur_r0, cur_r1, t, Shape::TILE, total));
+    }
+    uint32_t parity = 0;
+
+    while (t < num_tiles)
+    {
+        // per-tile scalars: only what the walk needs stays live (the rest of the TileView dies here)
+        int32_t n0, tile_r0, rows_t, nnz_t, items_t;
+        uint32_t sval, scol, srow; // shared-window byte addresses of TILE-LOCAL nonzero 0 / row 0
+        {
+            const TileView v = make_tile(cur_r0, cur_r1, t, Shape::TILE, total);
+            n0 = (int32_t)v.n0;
+            tile_r0 = v.r0;
+            rows_t = v.rows_t;
+            nnz_t = v.nnz_t;
+            items_t = v.items_t;
+            const uint32_t b = smem_u32(base);
+            sval = b + 8u * (uint32_t)(n0 - v.va);
+            scol = b + v.vb + 4u * (uint32_t)(n0 - v.ca);
+            srow = b + v.vb + v.cb + 4u * (uint32_t)(v.r0 + 1 - v.ra);
+        }
+        auto row_end = [&](int32_t i) -> int32_t { return lds_s32(srow + 4u * (uint32_t)i) - n0; };
+
+        mbar_wait(my_bar, parity);
+        parity ^= 1u;
+
+        // ---- my first merge item: interpolate, gallop, bisect (2 probes on regular matrices)
+        int32_t d = lane * IPT;
+        if (d > items_t)
+            d = items_t;
+        int32_t lo = d > nnz_t ? d - nnz_t : 0, hi = d < rows_t ? d : rows_t;
+        if (lo < hi)
+        {
+            // first guess by interpolation.  The divisor is the FULL tile size (a compile-time constant: multiply-shift
+            // instead of a 25-instruction integer division); only the matrix's last tile is shorter, and there the guess
+            // is merely a little low before the gallop corrects it.
+            int32_t g = (int32_t)(((uint32_t)d * (uint32_t)rows_t) / (uint32_t)Shape::TILE); // < 2^20: 32-bit is exact
+            g = g < lo ? lo : (g > hi - 1 ? hi - 1 : g);
+            int32_t step = 1;
+            if (row_end(g) <= d - g - 1)
+            {
+                lo = g + 1;
+                while (lo < hi)
+                {
+                    const int32_t m = (lo + step - 1 < hi - 1) ? lo + step - 1 : hi - 1;
+                    if (row_end(m) <= d - m - 1)
+                    {
+                        lo = m + 1;
+                        step <<= 1;
+                    }
+                    else
+                    {
+                        hi = m;
+                        break;
+                    }
+                }
+            }
+            else
+            {
+                hi = g;
+                while (lo < hi)
+                {
+                    const int32_t m = (hi - step > lo) ? hi - step : lo;
+                    if (!(row_end(m) <= d - m - 1))
+                    {
+                        hi = m;
+                        step <<= 1;
+                    }
+                    else
+                    {
+                        lo = m + 1;
+                        break;
+                    }
+                }
+            }
+            while (lo < hi)
+            {
+                const int32_t mid = (lo + hi) >> 1;
+                if (row_end(mid) <= d - mid - 1)
+                    lo = mid + 1;
+                else
+                    hi = mid;
+            }
+        }
+        const int32_t i0 = lo, j0 = d - lo;
+        int32_t d_next = (lane + 1) * IPT;
+        if (d_next > items_t)
+            d_next = items_t;
+        int32_t j_next = __shfl_down_sync(0xffffffffu, j0, 1);
+        if (lane == 31)
+            j_next = nnz_t;
+        const int32_t i_next = d_next - j_next;
+        const int32_t cnt = j_next - j0;
+
+        // ---- all my gathers first, in three phases pinned by volatile asm: the column indices, then every x gather of
+        // the lane (IPT independent loads in flight together -- left alone, the compiler reuses one register pair and
+        // waits for each load before issuing the next), then the products.  (Pinning the lane's two shared-window bases
+        // in registers with an opaque move saves an address instruction per load but makes the 14-item configurations
+        // spill; the nested "live slot / row end" walk this one replaced is in profiles/r01_logs/diet_bisect.log.)
+        // Axpby / Dot: y of my first row end (tile row i0; row 0 of the tile is the fix-up kernel's), loaded before the gathers so
+        // that its latency hides behind them; further row ends of the lane (short rows) load y at their store
+        double y_first = 0.0;
+        if (reads_y(M) && beta != 0.0 && i0 < i_next && i0 != 0)
+            y_first = ld_y_early(y + (int64_t)tile_r0 + i0);
+        double w_first = 0.0; // Dot: w of that row, loaded beside it
+        if (M == YStore::Dot && dot_w && i0 < i_next && i0 != 0)
+            w_first = __ldg(dot_w + (int64_t)tile_r0 + i0);
+        double prod[IPT];
+        {
+            int32_t cq[IPT];
+            uint32_t cbase = scol + 4u * (uint32_t)j0, vbase = sval + 8u * (uint32_t)j0;
+            // (every slot gets a defined value: leaving the dead ones undefined makes the compiler carry the previous
+            // tile's registers through the loop and spill them)
+#pragma unroll
+            for (int q = 0; q < IPT; q++)
+                cq[q] = q < cnt ? lds_s32(cbase + 4u * q) : 0;
+#pragma unroll
+            for (int q = 0; q < IPT; q++)
+            {
+                prod[q] = 0.0;
+                if (q < cnt)
+                    prod[q] = RANKED ? ldg_x_ranked(x, cq[q], hot_l1, hot_l2, pol_last, pol_first) : ldg_x_pinned(x, cq[q]);
+            }
+#pragma unroll
+            for (int q = 0; q < IPT; q++)
+                if (q < cnt)
+                    prod[q] = __dmul_rn(lds_f64(vbase + 8u * q), prod[q]);
+        }
+
+        double sum = 0.0, first_sum = 0.0;
+        double dl = 0.0; // Dot: this lane's dot terms, in the order it stores its rows
+        // a row end of mine that is not my first (Dot: the add exists only there -- a dead add of +0.0 moves the schedule of
+        // the Fanout store loop)
+        auto store_end = [&](int32_t row, double s) {
+            const double d = store_row<M>(y, (int64_t)tile_r0 + row, s, alpha, beta, dot_w, &fan);
+            if constexpr (M == YStore::Dot)
+                dl = __dadd_rn(dl, d);
+        };
+        bool has_first = false;
+        {
+            // Walk.  `until` = nonzeros of mine before my next row end (relative to j0, so each test is against a constant;
+            // "no further row end of mine" = never).  Dead slots (q >= cnt) hold +0.0, and a partial sum that starts at
+            // +0.0 can never become -0.0, so adding them is exact: the loop needs no "is this slot live" test, and the row
+            // ends that follow my last nonzero are flushed by the same test at the first dead slot.
+            int32_t row = i0;
+            int32_t until = (row < i_next ? row_end(row) : 0x7fffffff) - j0;
+#pragma unroll
+            for (int q = 0; q < IPT; q++)
+            {
+                if (until <= q) // rare: a row end (or a run of empty rows) sits before item q
+                {
+                    do
+                    {
+                        if (!has_first)
+                        {
+                            has_first = true;
+                            first_sum = sum;
+                        }
+                        else
+                            store_end(row, sum);
+                        sum = 0.0;
+                        row++;
+                        until = (row < i_next ? row_end(row) : 0x7fffffff) - j0;
+                    } while (until <= q);
+                }
+                sum = __dadd_rn(sum, prod[q]);
+            }
+            // every row end of mine has at most IPT - 1 of my nonzeros before it, so the loop above has seen them all;
+            // this is only a safety net
+            while (row < i_next)
+            {
+                if (!has_first)
+                {
+                    has_first = true;
+                    first_sum = sum;
+                }
+                else
+                    store_end(row, sum);
+                sum = 0.0;
+                row++;
+            }
+        }
+
+        // ---- the stage is consumed: refill it for my next tile while the warp stitches
+        __syncwarp();
+        const int32_t tn = t + warp_stride;
+        if (tn < num_tiles && tn > t)
+        {
+            cur_r0 = SMVP_BCAST(__ldg(tile_row + tn));
+            cur_r1 = SMVP_BCAST(__ldg(tile_row + tn + 1));
+            if (lane == 0)
+                issue(make_tile(cur_r0, cur_r1, tn, Shape::TILE, total));
+        }
+
+        // ---- stitch rows cut by lane boundaries: segmented inclusive scan of (carry row, carry sum)
+        const int32_t key = i_next; // the row my trailing partial belongs to
+        double scan = sum;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1)
+        {
+            const int32_t pk = __shfl_up_sync(0xffffffffu, key, o);
+            const bool take = lane >= o && pk == key;
+            const double pv = __shfl_up_sync(0xffffffffu, scan, o);
+            if (take)
+                scan = __dadd_rn(pv, scan);
+        }
+        const double prev_scan = __shfl_up_sync(0xffffffffu, scan, 1);
+        const int32_t prev_key = __shfl_up_sync(0xffffffffu, key, 1);
+        if (has_first)
+        {
+            if (lane > 0 && prev_key == i0)
+                first_sum = __dadd_rn(prev_scan, first_sum);
+            // the tile's first row may have started in earlier tiles: its partial goes to the fix-up
+            // kernel, which adds the carries and writes y -- and, under the epilogue, is the only one to read that
+            // row of y.  Without the epilogue y is only ever WRITTEN here (never read), so it may be a write-only
+            // mapping such as an NVSwitch multicast address.
+            if (i0 == 0)
+                head_val[t] = first_sum;
+            else if constexpr (reads_y(M))
+            {
+                const double v = axpby(alpha, first_sum, beta, y_first);
+                y[(int64_t)tile_r0 + i0] = v;
+                if constexpr (M == YStore::Dot)
+                    dl = __dadd_rn(dl, __dmul_rn(dot_w ? w_first : v, v));
+            }
+            else
+                store_row<M>(y, (int64_t)tile_r0 + i0, first_sum, alpha, beta, dot_w, &fan);
+        }
+        if (lane == 31)
+            carry_val[t] = scan; // partial of the row that continues into the next tile
+        if constexpr (M == YStore::Dot)
+        {
+            dl = warp_tree_sum(dl); // the lanes in a pairwise tree: the tile's partial (the fix-up adds its first row)
+            if (lane == 0)
+                part[t] = dl;
+        }
+        if (tn <= t)
+            break; // 32-bit overflow guard
+        t = tn;
+    }
+#undef SMVP_BCAST
 }
 
-template <bool FANOUT, bool EPI>
-__global__ void __launch_bounds__(256) merge_fixup_kernel(const int32_t *__restrict__ tile_row, const double *__restrict__ head_val,
-                                                          const double *__restrict__ carry_val, int32_t tile_begin,
-                                                          int32_t num_tiles, double *__restrict__ y,
-                                                          const __grid_constant__ YFan fan, double alpha, double beta)
-{
-    // no-op unless launched with programmatic stream serialization: then it waits here for the merge kernel's results
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-    const int32_t t = tile_begin + blockIdx.x * blockDim.x + threadIdx.x;
-    if (t < num_tiles)
-        merge_fixup_tile<FANOUT, EPI>(t, tile_row, head_val, carry_val, y, fan, alpha, beta);
-}
-// The dot pass's fix-up.  griddepcontrol.wait returns only once the merge kernel has completed and its writes are
+// The fix-up.  Under Dot: griddepcontrol.wait returns only once the merge kernel has completed and its writes are
 // visible, and every thread of this grid executes it before it exits: so when this grid has completed -- which the
 // reduction launched after it in stream order waits for -- the merge kernel's partials are final, also when this grid
 // was launched early.  The reduction itself is an ordinary launch.
-__global__ void __launch_bounds__(256) merge_fixup_dot_kernel(const int32_t *__restrict__ tile_row, const double *__restrict__ head_val,
-                                                              const double *__restrict__ carry_val, int32_t num_tiles,
-                                                              double *__restrict__ y, double alpha, double beta,
-                                                              const double *__restrict__ w, double *__restrict__ part)
+template <YStore M>
+__global__ void __launch_bounds__(256) merge_fixup_kernel(const int32_t *__restrict__ tile_row, const double *__restrict__ head_val,
+                                                          const double *__restrict__ carry_val, int32_t tile_begin,
+                                                          int32_t num_tiles, double *__restrict__ y,
+                                                          const __grid_constant__ YFan fan, double alpha, double beta,
+                                                          const double *__restrict__ w, double *__restrict__ part)
 {
+    // no-op unless launched with programmatic stream serialization: then it waits here for the merge kernel's results
     asm volatile("griddepcontrol.wait;" ::: "memory");
-    const int32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+    const int32_t t = (M == YStore::Dot ? 0 : tile_begin) + blockIdx.x * blockDim.x + threadIdx.x;
     if (t < num_tiles)
-        merge_fixup_tile<false, true, true>(t, tile_row, head_val, carry_val, y, YFan(), alpha, beta, w, part);
+        merge_fixup_tile<M>(t, tile_row, head_val, carry_val, y, fan, alpha, beta, w, part);
 }
 
 // ---- the two instantiations AUTO chooses from (merge_skewed).  Measured on B200 (logs under profiles/, the swept
@@ -669,14 +866,18 @@ static bool merge_fixup_early(int32_t ntiles)
     return pdl_ok && ntiles <= MERGE_PDL_TILES;
 }
 
-template <class C, bool FANOUT, bool RANKED, bool EPI>
-static int launch_wmerge(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fanp, const Axpby &ab, cudaStream_t s,
-                         int32_t tile_begin, int32_t tile_end)
+// tiles [tile_begin, tile_end) of the plan; a dot pass (whole passes only) leaves the partials of its tiles in
+// dot->part[0, merge_tiles)
+template <class C, bool RANKED, YStore M>
+static int launch_wmerge(const smvp_csr *A, const double *d_x, double *d_y, const YFan *fanp, const Axpby &ab, const DotOut *dot,
+                         cudaStream_t s, int32_t tile_begin, int32_t tile_end)
 {
     constexpr int SMEM = C::WARPS * MergeShape<32, C::IPT>::SMEM_BYTES;
-    auto kern = csr_merge_warp_kernel<C::WARPS, C::IPT, C::MINB, FANOUT, RANKED, C::UNI, EPI>;
+    auto kern = csr_merge_warp_kernel<C::WARPS, C::IPT, C::MINB, RANKED, C::UNI, M>;
     const int32_t hot_l1 = RANKED ? HOT_L1_ENTRIES : 0, hot_l2 = RANKED ? HOT_L2_ENTRIES : 0;
     const YFan fan = fanp ? *fanp : YFan();
+    const double *w = dot ? dot->w : nullptr;
+    double *part = dot ? dot->part : nullptr;
     static thread_local Residency res;
     const int32_t ntiles = tile_end - tile_begin;
     int64_t grid = 0;
@@ -685,31 +886,10 @@ static int launch_wmerge(const smvp_csr *A, const double *d_x, double *d_y, cons
     {
         const bool early = merge_fixup_early(ntiles);
         SMVP_LAUNCH(kern, (unsigned)grid, C::WARPS * 32, SMEM, s, A->row_ptr, mult_cols(A), A->val, d_x, d_y, A->tile_row, A->rows,
-                    A->nnz, tile_begin, tile_end, A->head_val, A->carry_val, fan, hot_l1, hot_l2, early ? 1 : 0, ab.alpha, ab.beta);
-        SMVP_TRY(launch_fixup(early, ntiles, s, merge_fixup_kernel<FANOUT, EPI>, (const int32_t *)A->tile_row, (const double *)A->head_val,
-                              (const double *)A->carry_val, tile_begin, tile_end, d_y, fan, ab.alpha, ab.beta));
-    }
-    return SMVP_OK;
-}
-
-// the whole-pass merge-path multiply with the dot partials of its tiles in dot->part[0, merge_tiles)
-template <class C, bool RANKED>
-static int launch_wmerge_dot(const smvp_csr *A, const double *d_x, double *d_y, const Axpby &ab, const DotOut &dot, cudaStream_t s)
-{
-    constexpr int SMEM = C::WARPS * MergeShape<32, C::IPT>::SMEM_BYTES;
-    auto kern = csr_merge_warp_dot_kernel<C::WARPS, C::IPT, C::MINB, RANKED, C::UNI>;
-    const int32_t hot_l1 = RANKED ? HOT_L1_ENTRIES : 0, hot_l2 = RANKED ? HOT_L2_ENTRIES : 0;
-    static thread_local Residency res;
-    const int32_t ntiles = A->merge_tiles;
-    int64_t grid = 0;
-    SMVP_TRY(persistent_grid(kern, C::WARPS * 32, SMEM, A->merge_headroom, ceil_div64(ntiles, C::WARPS), res, &grid));
-    if (grid > 0)
-    {
-        const bool early = merge_fixup_early(ntiles);
-        SMVP_LAUNCH(kern, (unsigned)grid, C::WARPS * 32, SMEM, s, A->row_ptr, mult_cols(A), A->val, d_x, d_y, A->tile_row, A->rows,
-                    A->nnz, ntiles, A->head_val, A->carry_val, hot_l1, hot_l2, early ? 1 : 0, ab.alpha, ab.beta, dot.w, dot.part);
-        SMVP_TRY(launch_fixup(early, ntiles, s, merge_fixup_dot_kernel, (const int32_t *)A->tile_row, (const double *)A->head_val,
-                              (const double *)A->carry_val, ntiles, d_y, ab.alpha, ab.beta, dot.w, dot.part));
+                    A->nnz, tile_begin, tile_end, A->head_val, A->carry_val, fan, hot_l1, hot_l2, early ? 1 : 0, ab.alpha, ab.beta, w,
+                    part);
+        SMVP_TRY(launch_fixup(early, ntiles, s, merge_fixup_kernel<M>, (const int32_t *)A->tile_row, (const double *)A->head_val,
+                              (const double *)A->carry_val, tile_begin, tile_end, d_y, fan, ab.alpha, ab.beta, w, part));
     }
     return SMVP_OK;
 }
@@ -755,19 +935,21 @@ __device__ __forceinline__ double lds_value(uint32_t a)
     }
 }
 
-// DOT (csr_pattern_dot_kernel): the work unit is the tile of 32 rows; the lanes' dot terms are added in a pairwise tree
-// into part[t].  w[r] is loaded beside the early load of y[r].
-// V: the width the values are streamed at (A->pat_vbytes).  Narrow values are widened exactly (pattern.cu checked every
-// one), so the products and sums are those of the fp64 kernel.
-template <typename V, int WARPS, int R, int STAGES, int CH, int MINB, bool FANOUT, bool EPI, bool DOT>
-__device__ __forceinline__ void
-csr_pattern_body(const int32_t *__restrict__ row_ptr, const V *__restrict__ val, const uint8_t *__restrict__ pat_id,
-                 const int32_t *__restrict__ pat_off, const int32_t *__restrict__ pat_len, int32_t npat, int32_t maxlen,
-                 const double *__restrict__ x, double *__restrict__ y, int32_t row_begin, int32_t row_end, uint32_t stage_bytes,
-                 const YFan &fan, double alpha, double beta, const double *__restrict__ dot_w, double *__restrict__ part)
+// Dot: whole passes only.  The work unit is the tile of 32 rows; the lanes' dot terms are added in a pairwise tree into
+// part[t].  w[r] is loaded beside the early load of y[r].
+// V: the width the values are streamed at (A->pat_vbytes): val itself (double), or the plan's copy A->pat_val (float or
+// fp16 as uint16_t).  Narrow values are widened exactly (pattern.cu checked every one), so the products and sums are
+// those of the fp64 kernel.
+template <typename V, int WARPS, int R, int STAGES, int CH, int MINB, YStore M>
+__global__ void __launch_bounds__(WARPS * 32, MINB)
+    csr_pattern_kernel(const int32_t *__restrict__ row_ptr, const V *__restrict__ val, const uint8_t *__restrict__ pat_id,
+                       const int32_t *__restrict__ pat_off, const int32_t *__restrict__ pat_len, int32_t npat, int32_t maxlen,
+                       const double *__restrict__ x, double *__restrict__ y, int32_t row_first, int32_t row_end, uint32_t stage_bytes,
+                       const __grid_constant__ YFan fan, double alpha, double beta, const double *__restrict__ dot_w,
+                       double *__restrict__ part)
 {
-    static_assert(!EPI || (R == 1 && !FANOUT), "the epilogue keeps one y value per lane: one round per tile");
-    static_assert(!DOT || EPI, "the dot is formed by the epilogue");
+    static_assert(!reads_y(M) || R == 1, "the epilogue keeps one y value per lane: one round per tile");
+    const int32_t row_begin = M == YStore::Dot ? 0 : row_first;
     constexpr int ROWS = PatternShape<R>::ROWS;
     constexpr int VA = 16 / (int)sizeof(V); // values per 16 bytes: the alignment of a bulk copy
     extern __shared__ __align__(128) unsigned char smem[];
@@ -841,11 +1023,11 @@ csr_pattern_body(const int32_t *__restrict__ row_ptr, const V *__restrict__ val,
             bounds(tn, &nn0, &nn1);
         // the epilogue's y[r]: issued before the wait for the stage, its latency hides behind the staging and the gathers
         double y0 = 0.0, w0 = 0.0;
-        if (EPI && beta != 0.0 && row_begin + t * ROWS + lane < row_end)
+        if (reads_y(M) && beta != 0.0 && row_begin + t * ROWS + lane < row_end)
             y0 = ld_y_early(y + row_begin + t * ROWS + lane);
-        if (DOT && dot_w && row_begin + t * ROWS + lane < row_end)
+        if (M == YStore::Dot && dot_w && row_begin + t * ROWS + lane < row_end)
             w0 = ld_w_early(dot_w + row_begin + t * ROWS + lane);
-        double d = 0.0; // DOT: the lane's dot term
+        double d = 0.0; // Dot: the lane's dot term
 
         mbar_wait(&bars[s], (phase >> s) & 1u);
         phase ^= 1u << s;
@@ -905,19 +1087,18 @@ csr_pattern_body(const int32_t *__restrict__ row_ptr, const V *__restrict__ val,
             }
             if (live)
             {
-                if (DOT)
+                if constexpr (reads_y(M))
                 {
                     const double v = axpby(alpha, sum, beta, y0);
                     y[r] = v;
-                    d = __dmul_rn(dot_w ? w0 : v, v);
+                    if constexpr (M == YStore::Dot)
+                        d = __dmul_rn(dot_w ? w0 : v, v);
                 }
-                else if (EPI)
-                    y[r] = axpby(alpha, sum, beta, y0);
                 else
-                    store_y<FANOUT, false>(y, fan, r, sum, alpha, beta);
+                    store_row<M>(y, r, sum, alpha, beta, dot_w, &fan);
             }
         }
-        if (DOT)
+        if constexpr (M == YStore::Dot)
         {
             d = warp_tree_sum(d);
             if (lane == 0)
@@ -934,69 +1115,6 @@ csr_pattern_body(const int32_t *__restrict__ row_ptr, const V *__restrict__ val,
         s = s + 1 == STAGES ? 0 : s + 1;
     }
 }
-// fp64 values: the kernels read val itself
-template <int WARPS, int R, int STAGES, int CH, int MINB, bool FANOUT, bool EPI>
-__global__ void __launch_bounds__(WARPS * 32, MINB)
-    csr_pattern_kernel(const int32_t *__restrict__ row_ptr, const double *__restrict__ val, const uint8_t *__restrict__ pat_id,
-                       const int32_t *__restrict__ pat_off, const int32_t *__restrict__ pat_len, int32_t npat, int32_t maxlen,
-                       const double *__restrict__ x, double *__restrict__ y, int32_t row_begin, int32_t row_end,
-                       uint32_t stage_bytes, const __grid_constant__ YFan fan, double alpha, double beta)
-{
-    csr_pattern_body<double, WARPS, R, STAGES, CH, MINB, FANOUT, EPI, false>(row_ptr, val, pat_id, pat_off, pat_len, npat, maxlen, x,
-                                                                            y, row_begin, row_end, stage_bytes, fan, alpha, beta,
-                                                                            nullptr, nullptr);
-}
-template <int WARPS, int R, int STAGES, int CH, int MINB>
-__global__ void __launch_bounds__(WARPS * 32, MINB)
-    csr_pattern_dot_kernel(const int32_t *__restrict__ row_ptr, const double *__restrict__ val, const uint8_t *__restrict__ pat_id,
-                           const int32_t *__restrict__ pat_off, const int32_t *__restrict__ pat_len, int32_t npat, int32_t maxlen,
-                           const double *__restrict__ x, double *__restrict__ y, int32_t rows, uint32_t stage_bytes, double alpha,
-                           double beta, const double *__restrict__ w, double *__restrict__ part)
-{
-    csr_pattern_body<double, WARPS, R, STAGES, CH, MINB, false, true, true>(row_ptr, val, pat_id, pat_off, pat_len, npat, maxlen, x, y,
-                                                                           0, rows, stage_bytes, YFan(), alpha, beta, w, part);
-}
-// narrow values (V = float or fp16 as uint16_t): the kernels read the plan's copy A->pat_val
-template <typename V, int WARPS, int R, int STAGES, int CH, int MINB, bool FANOUT, bool EPI>
-__global__ void __launch_bounds__(WARPS * 32, MINB)
-    csr_pattern_kernel_narrow(const int32_t *__restrict__ row_ptr, const V *__restrict__ val, const uint8_t *__restrict__ pat_id,
-                              const int32_t *__restrict__ pat_off, const int32_t *__restrict__ pat_len, int32_t npat, int32_t maxlen,
-                              const double *__restrict__ x, double *__restrict__ y, int32_t row_begin, int32_t row_end,
-                              uint32_t stage_bytes, const __grid_constant__ YFan fan, double alpha, double beta)
-{
-    csr_pattern_body<V, WARPS, R, STAGES, CH, MINB, FANOUT, EPI, false>(row_ptr, val, pat_id, pat_off, pat_len, npat, maxlen, x, y,
-                                                                       row_begin, row_end, stage_bytes, fan, alpha, beta, nullptr,
-                                                                       nullptr);
-}
-template <typename V, int WARPS, int R, int STAGES, int CH, int MINB>
-__global__ void __launch_bounds__(WARPS * 32, MINB)
-    csr_pattern_dot_kernel_narrow(const int32_t *__restrict__ row_ptr, const V *__restrict__ val, const uint8_t *__restrict__ pat_id,
-                                  const int32_t *__restrict__ pat_off, const int32_t *__restrict__ pat_len, int32_t npat,
-                                  int32_t maxlen, const double *__restrict__ x, double *__restrict__ y, int32_t rows,
-                                  uint32_t stage_bytes, double alpha, double beta, const double *__restrict__ w,
-                                  double *__restrict__ part)
-{
-    csr_pattern_body<V, WARPS, R, STAGES, CH, MINB, false, true, true>(row_ptr, val, pat_id, pat_off, pat_len, npat, maxlen, x, y, 0,
-                                                                      rows, stage_bytes, YFan(), alpha, beta, w, part);
-}
-// the instantiation of each kernel for value type V
-template <typename V, class C, bool FANOUT, bool EPI>
-constexpr auto pattern_kernel()
-{
-    if constexpr (std::is_same<V, double>::value)
-        return csr_pattern_kernel<C::WARPS, C::R, C::STAGES, C::CH, C::MINB, FANOUT, EPI>;
-    else
-        return csr_pattern_kernel_narrow<V, C::WARPS, C::R, C::STAGES, C::CH, C::MINB, FANOUT, EPI>;
-}
-template <typename V, class C>
-constexpr auto pattern_dot_kernel()
-{
-    if constexpr (std::is_same<V, double>::value)
-        return csr_pattern_dot_kernel<C::WARPS, C::R, C::STAGES, C::CH, C::MINB>;
-    else
-        return csr_pattern_dot_kernel_narrow<V, C::WARPS, C::R, C::STAGES, C::CH, C::MINB>;
-}
-
 // ---- the pattern kernel's configuration.  Measured on B200 (profiles/r03_logs/sweep_pattern.log, stencil 369^3, the
 // swept configurations in DESIGN.md §5.2): one stage per warp and 28 warps per SM (1.75 ms) against 2.1-3.2 ms for every
 // configuration with two stages or two rounds per tile -- a 7 KB stage per warp, so resident warps, not staging depth,
@@ -1023,6 +1141,7 @@ struct PatternCfgOf<float> : PatternCfg
     static constexpr int MINB = 8;
 };
 
+// rows [row_begin, row_end); a dot pass (whole passes only) leaves the partial of tile t in dot->part[t]
 template <typename V>
 static int launch_pattern(const smvp_csr *A, const V *val, const double *d_x, double *d_y, const YFan *fan, const Axpby &ab,
                           cudaStream_t s, int32_t row_begin, int32_t row_end, const DotOut *dot)
@@ -1033,36 +1152,17 @@ static int launch_pattern(const smvp_csr *A, const V *val, const double *d_x, do
     const int table = (A->pattern_count * (maxlen + 1) * 4 + 127) & ~127;
     const int smem = table + C::WARPS * C::STAGES * stage;
     const int64_t need = ceil_div64(ceil_div64((int64_t)row_end - row_begin, PatternShape<C::R>::ROWS), C::WARPS);
-    if (dot) // whole passes only: the partial of tile t goes to dot->part[t]
-    {
-        auto kern = pattern_dot_kernel<V, C>();
+    return with_store<YStore::Plain, YStore::Fanout, YStore::Axpby, YStore::Dot>(store_mode(dot, fan, ab), [&](auto S) {
+        auto kern = csr_pattern_kernel<V, C::WARPS, C::R, C::STAGES, C::CH, C::MINB, decltype(S)::value>;
+        // the shared memory depends on the matrix (longest pattern, pattern count): occupancy is looked up per size
         static thread_local Residency res;
         int64_t grid = 0;
         SMVP_TRY(persistent_grid(kern, C::WARPS * 32, smem, A->merge_headroom, need, res, &grid));
         if (grid > 0)
             SMVP_LAUNCH(kern, (unsigned)grid, C::WARPS * 32, smem, s, A->row_ptr, val, A->pat_id, A->pat_off, A->pat_len,
-                        A->pattern_count, maxlen, d_x, d_y, A->rows, (uint32_t)stage, ab.alpha, ab.beta, dot->w, dot->part);
+                        A->pattern_count, maxlen, d_x, d_y, row_begin, row_end, (uint32_t)stage, fan ? *fan : YFan(), ab.alpha,
+                        ab.beta, dot ? dot->w : nullptr, dot ? dot->part : nullptr);
         return (int)SMVP_OK;
-    }
-    return with_flag(fan != nullptr, [&](auto F) {
-        return with_flag(!ab.plain(), [&](auto E) {
-            constexpr bool FANOUT = decltype(F)::value, EPI = decltype(E)::value;
-            if constexpr (!kernel_exists<FANOUT, EPI>())
-                return (int)SMVP_E_ARG;
-            else
-            {
-                auto kern = pattern_kernel<V, C, FANOUT, EPI>();
-                // the shared memory depends on the matrix (longest pattern, pattern count): occupancy is looked up per size
-                static thread_local Residency res;
-                int64_t grid = 0;
-                SMVP_TRY(persistent_grid(kern, C::WARPS * 32, smem, A->merge_headroom, need, res, &grid));
-                if (grid > 0)
-                    SMVP_LAUNCH(kern, (unsigned)grid, C::WARPS * 32, smem, s, A->row_ptr, val, A->pat_id, A->pat_off, A->pat_len,
-                                A->pattern_count, maxlen, d_x, d_y, row_begin, row_end, (uint32_t)stage, fan ? *fan : YFan(),
-                                ab.alpha, ab.beta);
-                return (int)SMVP_OK;
-            }
-        });
     });
 }
 
@@ -1094,22 +1194,12 @@ static int csr_mult_merge(smvp_csr *A, const double *d_x, double *d_y, const YFa
     // 6.69 ms on R-MAT scale 26, DESIGN.md §5.4)
     const bool ranked = A->relabel_state == 1;
     const bool skewed = merge_skewed(A);
-    if (dot)
-        return with_flag(ranked, [&](auto R) {
+    return with_flag(ranked, [&](auto R) {
+        return with_store<YStore::Plain, YStore::Fanout, YStore::Axpby, YStore::Dot>(store_mode(dot, fan, ab), [&](auto S) {
             constexpr bool RANKED = decltype(R)::value;
-            return skewed ? launch_wmerge_dot<MergeSkewed, RANKED>(A, d_x, d_y, ab, *dot, s)
-                          : launch_wmerge_dot<MergeStencil, RANKED>(A, d_x, d_y, ab, *dot, s);
-        });
-    return with_flag(fan != nullptr, [&](auto F) {
-        return with_flag(ranked, [&](auto R) {
-            return with_flag(!ab.plain(), [&](auto E) {
-                constexpr bool FANOUT = decltype(F)::value, RANKED = decltype(R)::value, EPI = decltype(E)::value;
-                if constexpr (!kernel_exists<FANOUT, EPI>())
-                    return (int)SMVP_E_ARG;
-                else
-                    return skewed ? launch_wmerge<MergeSkewed, FANOUT, RANKED, EPI>(A, d_x, d_y, fan, ab, s, tile_begin, tile_end)
-                                  : launch_wmerge<MergeStencil, FANOUT, RANKED, EPI>(A, d_x, d_y, fan, ab, s, tile_begin, tile_end);
-            });
+            constexpr YStore M = decltype(S)::value;
+            return skewed ? launch_wmerge<MergeSkewed, RANKED, M>(A, d_x, d_y, fan, ab, dot, s, tile_begin, tile_end)
+                          : launch_wmerge<MergeStencil, RANKED, M>(A, d_x, d_y, fan, ab, dot, s, tile_begin, tile_end);
         });
     });
 }

@@ -487,23 +487,40 @@ __global__ void __launch_bounds__(256, MINB) tjds_det_kernel(const int2 *__restr
         flush();
 }
 
+// Calls store(i) for the rows i in [0, n) of y, store returning the row's dot term.  Dot: one row per thread, so that
+// the work unit is the CTA's 256 rows whatever the grid; their terms are added in a pairwise tree into part[blockIdx.x].
+// The other modes: a grid-stride loop.
+template <YStore M, typename F>
+__device__ __forceinline__ void for_rows_of_y(int32_t n, double *__restrict__ part, F &&store)
+{
+    if constexpr (M == YStore::Dot)
+    {
+        const int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+        double d = 0.0;
+        if (i < n)
+            d = __dadd_rn(d, store(i));
+        d = cta_tree_sum<256>(d);
+        if (threadIdx.x == 0)
+            part[blockIdx.x] = d;
+    }
+    else
+        for (int32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+            store(i);
+}
+
 // row_rank != NULL: the accumulators and row_exp are in popularity-rank order (relabelled handle), y is not.
-// EPI: y[row] = alpha * (row sum) + beta * y[row] (axpby, common.cuh) instead of the row sum.
-// DOT (tjds_det_finalize_dot_kernel): the work unit is the CTA's 256 rows of y; their dot terms are added in a pairwise tree.
-template <bool EPI>
+// Returns the row's dot term (store_row).  Dot: the work unit is the CTA's 256 rows of y; their dot terms are added in a
+// pairwise tree.
+template <YStore M>
 __device__ __forceinline__ double tjds_det_finalize_row(int32_t row, const long long *__restrict__ acc, const int32_t *__restrict__ row_exp,
                                                         const int32_t *__restrict__ x_exp, int32_t rows, double *__restrict__ y,
                                                         const int32_t *__restrict__ row_rank, int words, int32_t r_lo, int32_t r_hi,
-                                                        double alpha, double beta)
+                                                        double alpha, double beta, const double *__restrict__ w)
 {
     // accumulators exist (are cleared and filled) only for rows [r_lo, r_hi) of the index space the kernels use
     const int32_t r = row_rank ? row_rank[row] : row;
     if (r < r_lo || r >= r_hi)
-    {
-        const double v = EPI ? axpby(alpha, 0.0, beta, beta != 0.0 ? y[row] : 0.0) : 0.0;
-        y[row] = v;
-        return v;
-    }
+        return store_row<M>(y, row, 0.0, alpha, beta, w);
     longlong2 a;
     a.x = acc[r];
     a.y = words == 2 ? acc[(int64_t)rows + r] : 0; // one word: the value is hi * 2^(T - 62), i.e. lo = 0 below
@@ -515,66 +532,39 @@ __device__ __forceinline__ double tjds_det_finalize_row(int32_t row, const long 
         const int32_t T = row_exp[r] + *x_exp;
         out = scalbn(s, T - TJDS_FRAC);
     }
-    const double v = EPI ? axpby(alpha, out, beta, beta != 0.0 ? y[row] : 0.0) : out;
-    y[row] = v;
-    return v;
+    return store_row<M>(y, row, out, alpha, beta, w);
 }
-template <bool EPI>
+template <YStore M>
 __global__ void __launch_bounds__(256) tjds_det_finalize_kernel(const long long *__restrict__ acc, const int32_t *__restrict__ row_exp,
                                                                 const int32_t *__restrict__ x_exp, int32_t rows, double *__restrict__ y,
                                                                 const int32_t *__restrict__ row_rank, int words, int32_t r_lo, int32_t r_hi,
-                                                                double alpha, double beta)
-{
-    const int32_t row = blockIdx.x * blockDim.x + threadIdx.x;
-    if (row >= rows)
-        return;
-    tjds_det_finalize_row<EPI>(row, acc, row_exp, x_exp, rows, y, row_rank, words, r_lo, r_hi, alpha, beta);
-}
-__global__ void __launch_bounds__(256) tjds_det_finalize_dot_kernel(const long long *__restrict__ acc, const int32_t *__restrict__ row_exp,
-                                                                    const int32_t *__restrict__ x_exp, int32_t rows, double *__restrict__ y,
-                                                                    const int32_t *__restrict__ row_rank, int words, int32_t r_lo,
-                                                                    int32_t r_hi, double alpha, double beta, const double *__restrict__ w,
-                                                                    double *__restrict__ part)
+                                                                double alpha, double beta, const double *__restrict__ w,
+                                                                double *__restrict__ part)
 {
     const int32_t row = blockIdx.x * blockDim.x + threadIdx.x;
     double d = 0.0;
     if (row < rows)
-        d = dot_term(w, row, tjds_det_finalize_row<true>(row, acc, row_exp, x_exp, rows, y, row_rank, words, r_lo, r_hi, alpha, beta));
-    d = cta_tree_sum<256>(d);
-    if (threadIdx.x == 0)
-        part[blockIdx.x] = d;
-}
-
-// y[r] = y_rel[rank[r]]: the atomic variant of a relabelled handle sums in rank order.  EPI: y[r] = alpha * y_rel[rank[r]]
-// + beta * y[r] (axpby, common.cuh), and row_rank == NULL stands for the identity (the atomic sums of a natural-order
-// handle, which land in a scratch vector under the epilogue).
-template <bool EPI>
-__global__ void __launch_bounds__(256) tjds_unrank_y_kernel(const double *__restrict__ y_rel, const int32_t *__restrict__ row_rank,
-                                                            int32_t rows, double *__restrict__ y, double alpha, double beta)
-{
-    for (int32_t r = blockIdx.x * blockDim.x + threadIdx.x; r < rows; r += gridDim.x * blockDim.x)
+        d = tjds_det_finalize_row<M>(row, acc, row_exp, x_exp, rows, y, row_rank, words, r_lo, r_hi, alpha, beta, w);
+    if constexpr (M == YStore::Dot)
     {
-        if (EPI)
-        {
-            const double s = __ldg(y_rel + (row_rank ? __ldg(row_rank + r) : r));
-            y[r] = axpby(alpha, s, beta, beta != 0.0 ? y[r] : 0.0);
-        }
-        else
-            y[r] = __ldg(y_rel + __ldg(row_rank + r));
+        d = cta_tree_sum<256>(d);
+        if (threadIdx.x == 0)
+            part[blockIdx.x] = d;
     }
 }
-// the dot pass's unrank: one row per thread, so that the work unit is a 256-row block of y whatever the grid
-__global__ void __launch_bounds__(256) tjds_unrank_y_dot_kernel(const double *__restrict__ y_rel, const int32_t *__restrict__ row_rank,
-                                                                int32_t rows, double *__restrict__ y, double alpha, double beta,
-                                                                const double *__restrict__ w, double *__restrict__ part)
+
+// y[r] = y_rel[rank[r]]: the atomic variant of a relabelled handle sums in rank order.  Axpby / Dot: y[r] = alpha *
+// y_rel[rank[r]] + beta * y[r] (axpby, common.cuh), and row_rank == NULL stands for the identity (the atomic sums of a
+// natural-order handle, which land in a scratch vector under the epilogue).
+template <YStore M>
+__global__ void __launch_bounds__(256) tjds_unrank_y_kernel(const double *__restrict__ y_rel, const int32_t *__restrict__ row_rank,
+                                                            int32_t rows, double *__restrict__ y, double alpha, double beta,
+                                                            const double *__restrict__ w, double *__restrict__ part)
 {
-    const int32_t r = blockIdx.x * blockDim.x + threadIdx.x;
-    double d = 0.0;
-    if (r < rows)
-        store_axpby_dot(y, r, __ldg(y_rel + (row_rank ? __ldg(row_rank + r) : r)), alpha, beta, w, d);
-    d = cta_tree_sum<256>(d);
-    if (threadIdx.x == 0)
-        part[blockIdx.x] = d;
+    for_rows_of_y<M>(rows, part, [&](int32_t r) {
+        const int32_t k = M == YStore::Plain || row_rank ? __ldg(row_rank + r) : r; // Plain: only relabelled handles
+        return store_row<M>(y, r, __ldg(y_rel + k), alpha, beta, w);
+    });
 }
 
 // ---- transposed product y = A^T x --------------------------------------------------------------------------------
@@ -587,34 +577,25 @@ __global__ void __launch_bounds__(256) tjds_unrank_y_dot_kernel(const double *__
 // go to tr_part[tr_seg_off[g] + q] (one coalesced store per warp) and tjds_transpose_combine_kernel adds them in
 // segment order.  The table is walked straight whatever walk A x uses: a skewed table only has extra slots past the
 // end of each segment's first diagonal, and those threads find nothing to do.  row_ind is read, never row_rel.
-// EPI: every store of a column's value s becomes y = alpha * s + beta * y (axpby, common.cuh), empty columns too (s = +0.0).
+// Axpby / Dot: every store of a column's value s goes through the epilogue (store_row), empty columns too (s = +0.0).
+// Dot: a CTA of either kernel is a work unit.  A thread adds the dot terms of the columns it stores in the order it stores
+// them, and the CTA's threads are added in a pairwise tree into dot_part[unit].
 constexpr int TJDS_TR_UNROLL = 8; // entries whose loads are issued before the first of them is used
-__device__ __forceinline__ void tr_store(bool epi, double *__restrict__ y, int32_t c, double s, double alpha, double beta)
-{
-    y[c] = epi ? axpby(alpha, s, beta, beta != 0.0 ? y[c] : 0.0) : s;
-}
-// DOT (the *_dot_kernel wrappers): a CTA of either kernel is a work unit.  A thread adds the dot terms of the columns it
-// stores in the order it stores them, and the CTA's threads are added in a pairwise tree into dot_part[unit].
-template <bool EPI, bool DOT>
-__device__ __forceinline__ void tjds_transpose_body(const int2 *__restrict__ blocks, const int32_t *__restrict__ start_pos,
-                                                    const int32_t *__restrict__ row_ind, const double *__restrict__ val,
-                                                    const int32_t *__restrict__ perm, const double *__restrict__ x, double *__restrict__ y,
-                                                    double *__restrict__ part, const uint32_t *__restrict__ seg_off, int32_t ndiag,
-                                                    int32_t nslots, int32_t cols, int32_t nlong, double alpha, double beta,
-                                                    const double *__restrict__ dot_w, double *__restrict__ dot_part)
+template <YStore M>
+__global__ void __launch_bounds__(256) tjds_transpose_kernel(const int2 *__restrict__ blocks, const int32_t *__restrict__ start_pos,
+                                                             const int32_t *__restrict__ row_ind, const double *__restrict__ val,
+                                                             const int32_t *__restrict__ perm, const double *__restrict__ x,
+                                                             double *__restrict__ y, double *__restrict__ part,
+                                                             const uint32_t *__restrict__ seg_off, int32_t ndiag, int32_t nslots,
+                                                             int32_t cols, int32_t nlong, double alpha, double beta,
+                                                             const double *__restrict__ dot_w, double *__restrict__ dot_part)
 {
     static_assert(TJDS_SEG % TJDS_TR_UNROLL == 0, "s_sp holds TJDS_SEG + 1 entries");
-    static_assert(!DOT || EPI, "the dot is formed by the epilogue");
     __shared__ int32_t s_sp[TJDS_SEG + 1];
-    double d = 0.0; // DOT: this thread's dot terms
+    double d = 0.0; // Dot: this thread's dot terms
     // empty columns (slots nslots .. cols-1) get +0.0, spread over the whole grid
     for (int64_t p = (int64_t)nslots + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < cols; p += (int64_t)gridDim.x * blockDim.x)
-    {
-        if (DOT)
-            store_axpby_dot(y, __ldg(perm + p), 0.0, alpha, beta, dot_w, d);
-        else
-            tr_store(EPI, y, __ldg(perm + p), 0.0, alpha, beta);
-    }
+        d = __dadd_rn(d, store_row<M>(y, __ldg(perm + p), 0.0, alpha, beta, dot_w));
     const int2 blk = __ldg(blocks + blockIdx.x);
     const int32_t d_begin = blk.x * TJDS_SEG;
     const int32_t nd = min(TJDS_SEG, ndiag - d_begin);
@@ -624,7 +605,7 @@ __device__ __forceinline__ void tjds_transpose_body(const int2 *__restrict__ blo
     __syncthreads();
     const int32_t q = blk.y + (int32_t)threadIdx.x;
     const bool has = q < s_sp[1] - s_sp[0];
-    if (!DOT && !has)
+    if (M != YStore::Dot && !has)
         return; // the column at this slot ends before the segment (or the slot is past the table's diagonals)
     double s = 0.0;
     for (int32_t i0 = 0; has && i0 < nd; i0 += TJDS_TR_UNROLL)
@@ -648,57 +629,29 @@ __device__ __forceinline__ void tjds_transpose_body(const int2 *__restrict__ blo
                 s = __dadd_rn(s, __dmul_rn(v[u], xv[u]));
     }
     if (has && q >= nlong) // a column of at most TJDS_SEG entries lives in segment 0 alone
-    {
-        if (DOT)
-            store_axpby_dot(y, __ldg(perm + q), s, alpha, beta, dot_w, d);
-        else
-            tr_store(EPI, y, __ldg(perm + q), s, alpha, beta);
-    }
+        d = __dadd_rn(d, store_row<M>(y, __ldg(perm + q), s, alpha, beta, dot_w));
     else if (has)
         part[(int64_t)__ldg(seg_off + blk.x) + q] = s;
-    if (DOT)
+    if constexpr (M == YStore::Dot)
     {
         d = cta_tree_sum<256>(d);
         if (threadIdx.x == 0)
             dot_part[blockIdx.x] = d;
     }
 }
-template <bool EPI>
-__global__ void __launch_bounds__(256) tjds_transpose_kernel(const int2 *__restrict__ blocks, const int32_t *__restrict__ start_pos,
-                                                             const int32_t *__restrict__ row_ind, const double *__restrict__ val,
-                                                             const int32_t *__restrict__ perm, const double *__restrict__ x,
-                                                             double *__restrict__ y, double *__restrict__ part,
-                                                             const uint32_t *__restrict__ seg_off, int32_t ndiag, int32_t nslots,
-                                                             int32_t cols, int32_t nlong, double alpha, double beta)
-{
-    tjds_transpose_body<EPI, false>(blocks, start_pos, row_ind, val, perm, x, y, part, seg_off, ndiag, nslots, cols, nlong, alpha, beta,
-                                    nullptr, nullptr);
-}
-__global__ void __launch_bounds__(256) tjds_transpose_dot_kernel(const int2 *__restrict__ blocks, const int32_t *__restrict__ start_pos,
-                                                                 const int32_t *__restrict__ row_ind, const double *__restrict__ val,
-                                                                 const int32_t *__restrict__ perm, const double *__restrict__ x,
-                                                                 double *__restrict__ y, double *__restrict__ part,
-                                                                 const uint32_t *__restrict__ seg_off, int32_t ndiag, int32_t nslots,
-                                                                 int32_t cols, int32_t nlong, double alpha, double beta,
-                                                                 const double *__restrict__ w, double *__restrict__ dot_part)
-{
-    tjds_transpose_body<true, true>(blocks, start_pos, row_ind, val, perm, x, y, part, seg_off, ndiag, nslots, cols, nlong, alpha, beta,
-                                    w, dot_part);
-}
-
 // y[perm[q]] = tr_part partials of long column q added left to right from +0.0, chunk 0 first.  Slots [0, nwide) hold
 // more than TJDS_SEG chunks (a power-law column can hold ~1e6 entries, ~3e4 chunks): a warp loads 32 chunk sums per
 // round, TJDS_TR_ROUNDS rounds ahead, and every lane adds them in order from shuffles (the additions are the serial
 // part, the loads are not).  Slots [nwide, nlong) take one thread each.
 constexpr int TJDS_TR_ROUNDS = 4;
-template <bool EPI, bool DOT>
-__device__ __forceinline__ void tjds_transpose_combine_body(const double *__restrict__ part, const uint32_t *__restrict__ seg_off,
-                                                            const int32_t *__restrict__ slot_len, const int32_t *__restrict__ perm,
-                                                            int32_t nlong, int32_t nwide, double *__restrict__ y, double alpha, double beta,
-                                                            const double *__restrict__ dot_w, double *__restrict__ dot_part)
+template <YStore M>
+__global__ void __launch_bounds__(256) tjds_transpose_combine_kernel(const double *__restrict__ part, const uint32_t *__restrict__ seg_off,
+                                                                     const int32_t *__restrict__ slot_len, const int32_t *__restrict__ perm,
+                                                                     int32_t nlong, int32_t nwide, double *__restrict__ y, double alpha,
+                                                                     double beta, const double *__restrict__ dot_w,
+                                                                     double *__restrict__ dot_part)
 {
-    static_assert(!DOT || EPI, "the dot is formed by the epilogue");
-    double d = 0.0; // DOT: this thread's dot term
+    double d = 0.0; // Dot: this thread's dot term
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, wide_threads = (int64_t)nwide * 32;
     if (t < wide_threads)
     {
@@ -726,19 +679,14 @@ __device__ __forceinline__ void tjds_transpose_combine_body(const double *__rest
                 }
         }
         if (lane == 0)
-        {
-            if (DOT)
-                store_axpby_dot(y, __ldg(perm + q), s, alpha, beta, dot_w, d);
-            else
-                tr_store(EPI, y, __ldg(perm + q), s, alpha, beta);
-        }
-        if (!DOT)
+            d = __dadd_rn(d, store_row<M>(y, __ldg(perm + q), s, alpha, beta, dot_w));
+        if (M != YStore::Dot)
             return;
     }
     else
     {
         const int64_t qq = (int64_t)nwide + (t - wide_threads);
-        if (!DOT && qq >= nlong)
+        if (M != YStore::Dot && qq >= nlong)
             return;
         if (qq < nlong)
         {
@@ -748,53 +696,22 @@ __device__ __forceinline__ void tjds_transpose_combine_body(const double *__rest
 #pragma unroll 4
             for (int32_t g = 0; g < nch; g++)
                 s = __dadd_rn(s, __ldg(part + __ldg(seg_off + g) + q));
-            if (DOT)
-                store_axpby_dot(y, __ldg(perm + q), s, alpha, beta, dot_w, d);
-            else
-                tr_store(EPI, y, __ldg(perm + q), s, alpha, beta);
+            d = __dadd_rn(d, store_row<M>(y, __ldg(perm + q), s, alpha, beta, dot_w));
         }
     }
-    if (DOT)
+    if constexpr (M == YStore::Dot)
     {
         d = cta_tree_sum<256>(d);
         if (threadIdx.x == 0)
             dot_part[blockIdx.x] = d;
     }
 }
-template <bool EPI>
-__global__ void __launch_bounds__(256) tjds_transpose_combine_kernel(const double *__restrict__ part, const uint32_t *__restrict__ seg_off,
-                                                                     const int32_t *__restrict__ slot_len, const int32_t *__restrict__ perm,
-                                                                     int32_t nlong, int32_t nwide, double *__restrict__ y, double alpha,
-                                                                     double beta)
+// y = alpha * (+0.0) + beta * y: the scaled, accumulating transposed product of a handle without entries (Axpby, Dot)
+template <YStore M>
+__global__ void __launch_bounds__(256) tjds_axpby_empty_kernel(double *__restrict__ y, int32_t n, double alpha, double beta,
+                                                               const double *__restrict__ w, double *__restrict__ part)
 {
-    tjds_transpose_combine_body<EPI, false>(part, seg_off, slot_len, perm, nlong, nwide, y, alpha, beta, nullptr, nullptr);
-}
-__global__ void __launch_bounds__(256) tjds_transpose_combine_dot_kernel(const double *__restrict__ part, const uint32_t *__restrict__ seg_off,
-                                                                         const int32_t *__restrict__ slot_len,
-                                                                         const int32_t *__restrict__ perm, int32_t nlong, int32_t nwide,
-                                                                         double *__restrict__ y, double alpha, double beta,
-                                                                         const double *__restrict__ w, double *__restrict__ dot_part)
-{
-    tjds_transpose_combine_body<true, true>(part, seg_off, slot_len, perm, nlong, nwide, y, alpha, beta, w, dot_part);
-}
-
-// y = alpha * (+0.0) + beta * y: the scaled, accumulating transposed product of a handle without entries
-__global__ void __launch_bounds__(256) tjds_axpby_empty_kernel(double *__restrict__ y, int32_t n, double alpha, double beta)
-{
-    for (int32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
-        y[i] = axpby(alpha, 0.0, beta, beta != 0.0 ? y[i] : 0.0);
-}
-// its dot pass: one entry per thread, the work unit is a 256-entry block of y
-__global__ void __launch_bounds__(256) tjds_axpby_empty_dot_kernel(double *__restrict__ y, int32_t n, double alpha, double beta,
-                                                                   const double *__restrict__ w, double *__restrict__ part)
-{
-    const int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    double d = 0.0;
-    if (i < n)
-        store_axpby_dot(y, i, 0.0, alpha, beta, w, d);
-    d = cta_tree_sum<256>(d);
-    if (threadIdx.x == 0)
-        part[blockIdx.x] = d;
+    for_rows_of_y<M>(n, part, [&](int32_t i) { return store_row<M>(y, i, 0.0, alpha, beta, w); });
 }
 
 // partials segment g holds: the long columns (slots [0, nlong), nlong = length of diagonal TJDS_SEG) in segment 0, the
@@ -1015,58 +932,39 @@ static int64_t tjds_dot_units_max(const smvp_tjds *A)
     return ax > atx ? ax : atx;
 }
 
-// the transposed dot pass: the kernels of the epilogue with their dot partials in dot.part (tjds_transpose_units of them)
-static int tjds_transpose_pass_dot(smvp_tjds *A, const double *d_x, double *d_y, const Axpby &ab, const DotOut &dot, cudaStream_t s)
+// one transposed pass, asynchronous on s; tjds_transpose_prepare has run and A->cols > 0.  dot != NULL: a dot pass, its
+// partials in dot->part (tjds_transpose_units of them)
+static int tjds_transpose_pass(smvp_tjds *A, const double *d_x, double *d_y, const Axpby &ab, const DotOut *dot, cudaStream_t s)
 {
-    if (A->ndiag == 0)
-        SMVP_LAUNCH(tjds_axpby_empty_dot_kernel, (unsigned)ceil_div64(A->cols, 256), 256, 0, s, d_y, A->cols, ab.alpha, ab.beta, dot.w,
-                    dot.part);
-    else
+    const YStore mode = store_mode(dot, false, ab);
+    if (A->ndiag == 0 && mode == YStore::Plain) // no entries: every column is empty
     {
-        SMVP_LAUNCH(tjds_transpose_dot_kernel, (unsigned)A->num_seg_blocks, 256, 0, s, (const int2 *)A->seg_blocks,
-                    (const int32_t *)A->start_pos, (const int32_t *)A->row_ind, (const double *)A->val, (const int32_t *)A->perm, d_x, d_y,
-                    A->tr_part, (const uint32_t *)A->tr_seg_off, A->ndiag, A->nslots, A->cols, A->tr_nlong, ab.alpha, ab.beta, dot.w,
-                    dot.part);
-        if (A->ndiag > TJDS_SEG)
-        {
-            const int64_t threads = 32 * (int64_t)A->tr_nwide + (A->tr_nlong - A->tr_nwide);
-            SMVP_LAUNCH(tjds_transpose_combine_dot_kernel, (unsigned)ceil_div64(threads, 256), 256, 0, s, (const double *)A->tr_part,
-                        (const uint32_t *)A->tr_seg_off, (const int32_t *)A->slot_len, (const int32_t *)A->perm, A->tr_nlong, A->tr_nwide,
-                        d_y, ab.alpha, ab.beta, dot.w, dot.part + A->num_seg_blocks);
-        }
-    }
-    SMVP_CUDA(cudaGetLastError());
-    return SMVP_OK;
-}
-
-// one transposed pass, asynchronous on s; tjds_transpose_prepare has run and A->cols > 0
-static int tjds_transpose_pass(smvp_tjds *A, const double *d_x, double *d_y, const Axpby &ab, cudaStream_t s)
-{
-    const bool epi = !ab.plain();
-    if (A->ndiag == 0) // no entries: every column is empty
-    {
-        if (!epi)
-            SMVP_CUDA(cudaMemsetAsync(d_y, 0, sizeof(double) * (size_t)A->cols, s));
-        else
-        {
-            int64_t blocks = ceil_div64(A->cols, 256 * 4);
-            const int64_t cap = (int64_t)device_props().sms * 8;
-            SMVP_LAUNCH(tjds_axpby_empty_kernel, (unsigned)(blocks < cap ? blocks : cap), 256, 0, s, d_y, A->cols, ab.alpha, ab.beta);
-            SMVP_CUDA(cudaGetLastError());
-        }
+        SMVP_CUDA(cudaMemsetAsync(d_y, 0, sizeof(double) * (size_t)A->cols, s));
         return SMVP_OK;
     }
-    with_flag(epi, [&](auto E) {
-        constexpr bool EPI = decltype(E)::value;
-        SMVP_LAUNCH(tjds_transpose_kernel<EPI>, (unsigned)A->num_seg_blocks, 256, 0, s, (const int2 *)A->seg_blocks,
+    const double *w = dot ? dot->w : nullptr;
+    double *part = dot ? dot->part : nullptr;
+    with_store<YStore::Plain, YStore::Axpby, YStore::Dot>(mode, [&](auto S) {
+        constexpr YStore M = decltype(S)::value;
+        if constexpr (M != YStore::Plain)
+            if (A->ndiag == 0)
+            {
+                int64_t blocks = ceil_div64(A->cols, 256);
+                const int64_t cap = (int64_t)device_props().sms * 8;
+                if (M != YStore::Dot) // a grid-stride loop: 4 entries per thread, at most 8 CTAs per SM
+                    blocks = ceil_div64(A->cols, 256 * 4) < cap ? ceil_div64(A->cols, 256 * 4) : cap;
+                SMVP_LAUNCH(tjds_axpby_empty_kernel<M>, (unsigned)blocks, 256, 0, s, d_y, A->cols, ab.alpha, ab.beta, w, part);
+                return (int)SMVP_OK;
+            }
+        SMVP_LAUNCH(tjds_transpose_kernel<M>, (unsigned)A->num_seg_blocks, 256, 0, s, (const int2 *)A->seg_blocks,
                     (const int32_t *)A->start_pos, (const int32_t *)A->row_ind, (const double *)A->val, (const int32_t *)A->perm, d_x, d_y,
-                    A->tr_part, (const uint32_t *)A->tr_seg_off, A->ndiag, A->nslots, A->cols, A->tr_nlong, ab.alpha, ab.beta);
+                    A->tr_part, (const uint32_t *)A->tr_seg_off, A->ndiag, A->nslots, A->cols, A->tr_nlong, ab.alpha, ab.beta, w, part);
         if (A->ndiag > TJDS_SEG)
         {
             const int64_t threads = 32 * (int64_t)A->tr_nwide + (A->tr_nlong - A->tr_nwide);
-            SMVP_LAUNCH(tjds_transpose_combine_kernel<EPI>, (unsigned)ceil_div64(threads, 256), 256, 0, s, (const double *)A->tr_part,
+            SMVP_LAUNCH(tjds_transpose_combine_kernel<M>, (unsigned)ceil_div64(threads, 256), 256, 0, s, (const double *)A->tr_part,
                         (const uint32_t *)A->tr_seg_off, (const int32_t *)A->slot_len, (const int32_t *)A->perm, A->tr_nlong, A->tr_nwide,
-                        d_y, ab.alpha, ab.beta);
+                        d_y, ab.alpha, ab.beta, w, M == YStore::Dot ? part + A->num_seg_blocks : nullptr);
         }
         return (int)SMVP_OK;
     });
@@ -1086,7 +984,7 @@ extern "C" int smvp_tjds_mult_transpose_device(smvp_tjds *A, const double *d_x, 
         return SMVP_OK;
     cudaStream_t s = (cudaStream_t)stream;
     SMVP_TRY(tjds_transpose_prepare(A, s));
-    return tjds_transpose_pass(A, d_x, d_y, AXPBY_PLAIN, s);
+    return tjds_transpose_pass(A, d_x, d_y, AXPBY_PLAIN, nullptr, s);
 }
 
 extern "C" int smvp_tjds_mult_transpose_device_axpby(smvp_tjds *A, double alpha, const double *d_x, double beta, double *d_y,
@@ -1100,7 +998,7 @@ extern "C" int smvp_tjds_mult_transpose_device_axpby(smvp_tjds *A, double alpha,
         return SMVP_OK;
     cudaStream_t s = (cudaStream_t)stream;
     SMVP_TRY(tjds_transpose_prepare(A, s));
-    return tjds_transpose_pass(A, d_x, d_y, Axpby{alpha, beta}, s);
+    return tjds_transpose_pass(A, d_x, d_y, Axpby{alpha, beta}, nullptr, s);
 }
 
 extern "C" int smvp_tjds_mult_transpose_device_axpby_dot(smvp_tjds *A, double alpha, const double *d_x, double beta, double *d_y,
@@ -1117,8 +1015,9 @@ extern "C" int smvp_tjds_mult_transpose_device_axpby_dot(smvp_tjds *A, double al
         SMVP_TRY(tjds_transpose_prepare(A, s));
     const int64_t units = A->cols > 0 ? tjds_transpose_units(A) : 0;
     SMVP_TRY(dot_scratch(&A->dot_buf, &A->dot_cap, &A->device_bytes, tjds_dot_units_max(A), s));
+    const DotOut dot = {d_w, A->dot_buf};
     if (A->cols > 0)
-        SMVP_TRY(tjds_transpose_pass_dot(A, d_x, d_y, Axpby{alpha, beta}, DotOut{d_w, A->dot_buf}, s));
+        SMVP_TRY(tjds_transpose_pass(A, d_x, d_y, Axpby{alpha, beta}, &dot, s));
     return dot_reduce(A->dot_buf, A->dot_cap, units, d_dot, s);
 }
 
@@ -1135,7 +1034,7 @@ extern "C" int smvp_tjds_mult_transpose(smvp_tjds *A, const double *x_host, doub
     SMVP_TRY(tjds_transpose_prepare(A, 0));
     const bool small = (int64_t)A->rows + A->cols + A->nnz < SMVP_SMALL_LOOP_ITEMS;
     if (A->cols > 0)
-        SMVP_TRY(timed_loop(iters, ms_each, small, [&](cudaStream_t s) { return tjds_transpose_pass(A, A->d_xt, A->d_yt, AXPBY_PLAIN, s); }));
+        SMVP_TRY(timed_loop(iters, ms_each, small, [&](cudaStream_t s) { return tjds_transpose_pass(A, A->d_xt, A->d_yt, AXPBY_PLAIN, nullptr, s); }));
     else if (ms_each)
         for (int it = 0; it < iters; it++)
             ms_each[it] = 0.0;
@@ -1215,7 +1114,10 @@ static int tjds_pass(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit,
                      const DotOut *dot = nullptr)
 {
     const int32_t lim = tjds_effective_limit(A, diag_limit);
-    const bool ranked = A->relabel_state == 1, skew = A->skew == 1, epi = !ab.plain() || dot;
+    const YStore mode = store_mode(dot, false, ab);
+    const bool ranked = A->relabel_state == 1, skew = A->skew == 1, epi = mode != YStore::Plain;
+    const double *dot_w = dot ? dot->w : nullptr;
+    double *part = dot ? dot->part : nullptr;
     const unsigned blocks = (unsigned)A->num_seg_blocks;
     if (variant == SMVP_TJDS_ATOMIC || A->det_route != 1)
     {
@@ -1232,17 +1134,17 @@ static int tjds_pass(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit,
             else
                 SMVP_LAUNCH((tjds_atomic_kernel<4, false>), blocks, 256, 0, s, SMVP_TJDS_ARGS_COMMON, d_y, A->nslots, lim);
         }
-        if (dot)
-            SMVP_LAUNCH(tjds_unrank_y_dot_kernel, (unsigned)ceil_div64(A->rows, 256), 256, 0, s, (const double *)d_y,
-                        ranked ? (const int32_t *)A->row_rank : nullptr, A->rows, y_caller, ab.alpha, ab.beta, dot->w, dot->part);
-        else if (ranked || epi)
+        if (ranked || epi)
         {
-            int64_t ub = ceil_div64(A->rows, 256 * 4);
+            // Dot: one row per thread; the others: a grid-stride loop, 4 rows per thread, at most 8 CTAs per SM
+            int64_t ub = ceil_div64(A->rows, 256);
             const int64_t cap = (int64_t)device_props().sms * 8;
+            if (mode != YStore::Dot)
+                ub = ceil_div64(A->rows, 256 * 4) < cap ? ceil_div64(A->rows, 256 * 4) : cap;
             const int32_t *rank = ranked ? (const int32_t *)A->row_rank : nullptr;
-            with_flag(epi, [&](auto E) {
-                SMVP_LAUNCH(tjds_unrank_y_kernel<decltype(E)::value>, (unsigned)(ub < cap ? ub : cap), 256, 0, s, (const double *)d_y, rank,
-                            A->rows, y_caller, ab.alpha, ab.beta);
+            with_store<YStore::Plain, YStore::Axpby, YStore::Dot>(mode, [&](auto S) {
+                SMVP_LAUNCH(tjds_unrank_y_kernel<decltype(S)::value>, (unsigned)ub, 256, 0, s, (const double *)d_y, rank, A->rows, y_caller,
+                            ab.alpha, ab.beta, dot_w, part);
                 return (int)SMVP_OK;
             });
         }
@@ -1275,17 +1177,12 @@ static int tjds_pass(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit,
                 });
             });
         }
-        if (dot)
-            SMVP_LAUNCH(tjds_det_finalize_dot_kernel, (unsigned)ceil_div64(A->rows, 256), 256, 0, s, (const long long *)A->acc,
-                        (const int32_t *)A->row_exp, (const int32_t *)A->x_exp, A->rows, d_y,
-                        ranked ? (const int32_t *)A->row_rank : nullptr, words, r_lo, r_hi, ab.alpha, ab.beta, dot->w, dot->part);
-        else
-            with_flag(epi, [&](auto E) {
-                SMVP_LAUNCH(tjds_det_finalize_kernel<decltype(E)::value>, (unsigned)ceil_div64(A->rows, 256), 256, 0, s,
-                            (const long long *)A->acc, (const int32_t *)A->row_exp, (const int32_t *)A->x_exp, A->rows, d_y,
-                            ranked ? (const int32_t *)A->row_rank : nullptr, words, r_lo, r_hi, ab.alpha, ab.beta);
-                return (int)SMVP_OK;
-            });
+        with_store<YStore::Plain, YStore::Axpby, YStore::Dot>(mode, [&](auto S) {
+            SMVP_LAUNCH(tjds_det_finalize_kernel<decltype(S)::value>, (unsigned)ceil_div64(A->rows, 256), 256, 0, s,
+                        (const long long *)A->acc, (const int32_t *)A->row_exp, (const int32_t *)A->x_exp, A->rows, d_y,
+                        ranked ? (const int32_t *)A->row_rank : nullptr, words, r_lo, r_hi, ab.alpha, ab.beta, dot_w, part);
+            return (int)SMVP_OK;
+        });
     }
     SMVP_CUDA(cudaGetLastError());
     return SMVP_OK;

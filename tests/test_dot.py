@@ -151,31 +151,37 @@ def test_null_handle_and_null_dot_are_rejected(eng):
     assert L.smvp_tjds_mult_transpose_device_axpby_dot(None, 1.0, p, 0.0, p, None, p, None) == eng.E_ARG
 
 
-def test_dot_kernels_are_in_the_library_spill_free():
-    """Every *_dot_kernel instantiation and the reduction exist with no stack frame; none is paired with the fan-out."""
+def test_dot_mode_kernels_are_in_the_library_spill_free():
+    """Every Dot store-mode instantiation and the reduction exist with no stack frame, and each kernel family that stores
+    y is instantiated with exactly its store modes: a dot pass always runs the epilogue, never the fan-out."""
     if not os.path.exists(LIB) or not os.path.exists(CUOBJDUMP):
         pytest.skip("library or cuobjdump not available")
     res = subprocess.run([CUOBJDUMP, "-res-usage", LIB], capture_output=True, text=True, check=True).stdout
     found = re.findall(r"Function (\S+):\s*\n\s*REG:\d+ STACK:(\d+)", res)
+    D = util.ystore("Dot")
     wanted = {
-        "pattern": (r"csr_pattern_dot_kernelILi4ELi1ELi1ELi14ELi7EE", 1),
-        "merge, stencil configuration": (r"csr_merge_warp_dot_kernelILi4ELi14ELi8ELb[01]ELb1EE", 2),
-        "merge, skewed configuration": (r"csr_merge_warp_dot_kernelILi2ELi10ELi14ELb[01]ELb0EE", 2),
-        "fix-up": (r"merge_fixup_dot_kernel", 1),
-        "vector": (r"csr_vector_dot_kernelILi\d+EE", 5),
-        "det-finalize": (r"tjds_det_finalize_dot_kernel", 1),
-        "unrank": (r"tjds_unrank_y_dot_kernel", 1),
-        "transpose": (r"tjds_transpose_dot_kernel", 1),
-        "combine": (r"tjds_transpose_combine_dot_kernel", 1),
-        "empty transpose": (r"tjds_axpby_empty_dot_kernel", 1),
+        "pattern": (r"csr_pattern_kernelIdLi4ELi1ELi1ELi14ELi7E" + D, 1),
+        "merge, stencil configuration": (r"csr_merge_warp_kernelILi4ELi14ELi8ELb[01]ELb1E" + D, 2),
+        "merge, skewed configuration": (r"csr_merge_warp_kernelILi2ELi10ELi14ELb[01]ELb0E" + D, 2),
+        "fix-up": (r"merge_fixup_kernelI" + D, 1),
+        "vector": (r"csr_vector_kernelILi\d+E" + D, 5),
+        "det-finalize": (r"tjds_det_finalize_kernelI" + D, 1),
+        "unrank": (r"tjds_unrank_y_kernelI" + D, 1),
+        "transpose": (r"tjds_transpose_kernelI" + D, 1),
+        "combine": (r"tjds_transpose_combine_kernelI" + D, 1),
+        "empty transpose": (r"tjds_axpby_empty_kernelI" + D, 1),
         "reduction": (r"dot_reduce_kernel", 1),
     }
     for what, (pat, count) in wanted.items():
         hits = [(name, stack) for name, stack in found if re.search(pat, name)]
         assert len(hits) == count, (what, hits)
         assert all(stack == "0" for _, stack in hits), (what, hits)
-    # the dot kernels take no YFan: no fan-out instantiation can exist
-    assert not [name for name, _ in found if "dot_kernel" in name and "YFan" in name]
+    csr, tjds = {"Plain", "Fanout", "Axpby", "Dot"}, {"Plain", "Axpby", "Dot"}
+    assert util.store_modes(res) == {
+        "csr_vector_kernel": csr, "csr_merge_warp_kernel": csr, "merge_fixup_kernel": csr, "csr_pattern_kernel": csr,
+        "tjds_det_finalize_kernel": tjds, "tjds_unrank_y_kernel": tjds, "tjds_transpose_kernel": tjds,
+        "tjds_transpose_combine_kernel": tjds, "tjds_axpby_empty_kernel": {"Axpby", "Dot"},
+    }
 
 
 # ---------------------------------------------------------------------------- GPU helpers

@@ -25,12 +25,12 @@ def _dump(*args):
     return subprocess.run([CUOBJDUMP, *args, LIB], capture_output=True, text=True, check=True).stdout
 
 
-def test_narrow_pattern_kernels_widen_with_one_instruction():
+def test_pattern_kernels_at_every_width_widen_with_one_instruction():
     """Every pattern kernel exists at fp32 and fp16 (plain, epilogue, fan-out, dot), none spills, each stages with TMA
     and widens its values with F2F."""
     res = _dump("-res-usage")
-    found = re.findall(r"Function (\S*csr_pattern(?:_dot)?_kernel(?:_narrowI([ft])|I)\S*):\s*\n\s*REG:\d+ STACK:(\d+)", res)
-    by_type = {t: [n for n, tt, _ in found if tt == t] for t in ("", "f", "t")}  # "": fp64, f: fp32, t: fp16 (uint16_t)
+    found = re.findall(r"Function (\S*csr_pattern_kernelI([dft])\S*):\s*\n\s*REG:\d+ STACK:(\d+)", res)
+    by_type = {t: [n for n, tt, _ in found if tt == t] for t in ("d", "f", "t")}  # d: fp64, f: fp32, t: fp16 (uint16_t)
     assert all(len(v) == 4 for v in by_type.values()), {t: len(v) for t, v in by_type.items()}
     assert all(stack == "0" for _, _, stack in found), found
     for t, cvt in (("f", "F2F.F64.F32"), ("t", "F2F.F64.F16")):

@@ -1,5 +1,6 @@
 """Helpers shared by the tests (test infrastructure; may use oracle/)."""
 import os
+import re
 
 import numpy as np
 
@@ -95,3 +96,20 @@ def random_coo(rng, m, n, nnz):
     coo["val"] = rng.uniform(-1.0, 1.0, size=nnz)
     rng.shuffle(coo)
     return coo
+
+
+# The store modes of the kernels that store y (YStore in csrc/common.cuh), as they appear in mangled kernel names
+STORE_MODES = {"0": "Plain", "1": "Fanout", "2": "Axpby", "3": "Dot"}
+
+
+def ystore(mode):
+    """Regex fragment of a mangled template argument list that ends in store mode `mode` ("Plain", ... "Dot")."""
+    return "LNS_6YStoreE%sEE" % {v: k for k, v in STORE_MODES.items()}[mode]
+
+
+def store_modes(res_usage):
+    """{kernel family: the set of store modes it is instantiated with}, from `cuobjdump -res-usage` output"""
+    modes = {}
+    for name, mode in re.findall(r"Function _ZN4smvp\d+(\w+?)I\w*?LNS_6YStoreE(\d)EEE", res_usage):
+        modes.setdefault(name, set()).add(STORE_MODES[mode])
+    return modes
