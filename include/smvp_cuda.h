@@ -64,18 +64,31 @@ typedef struct smvp_tjds smvp_tjds; /* opaque: TJDSData (main-cli.c:70-75) resid
 
 /* TJDS multiply variants */
 #define SMVP_TJDS_ATOMIC 0        /* coalesced jagged-diagonal streaming, fp64 atomicAdd scatter into y */
-#define SMVP_TJDS_DETERMINISTIC 1 /* order-independent exact INTEGER accumulation: every product is split exactly into two
-                                     64-bit fixed-point words scaled per row by a bound known before the multiply
-                                     (row_exp + exponent of max|x|), the words are added with integer atomics, one final
-                                     rounding: y is the CORRECTLY ROUNDED row sum, bit-identical run to run (and between
-                                     the straight and the skewed walk, with and without row relabelling).            */
-#define SMVP_TJDS_DETERMINISTIC_FAST 2 /* the same with the high word only: a product is truncated toward zero at 2^-62 of
-                                     its row's bound B_r = 2^ceil(log2(max|a_rj| * max|x| * count_r)).  Just as
-                                     reproducible (integer sums), one reduction per run and half the accumulator traffic;
-                                     the error is bounded NORMWISE, |err_r| <= count_r * 2^-62 * B_r -- 2^-9 of what one
-                                     fp64 addition at magnitude B_r rounds away -- not relative to |y_r|: an x whose
-                                     entries span many orders of magnitude can cost a row with small products digits
-                                     that the exact variant keeps.                                                  */
+#define SMVP_TJDS_DETERMINISTIC 1 /* order-independent INTEGER accumulation in fixed point, scaled per row by a bound known
+                                     before the multiply, one final rounding; bit-identical run to run (and between the
+                                     straight and the skewed walk, with and without row relabelling).  Exactly:
+                                       e(v) = ilogb(v) + 1 (so |v| < 2^e(v)),
+                                       T_r  = max e(a_rj) over the nonzero entries of row r
+                                              + ceil(log2 count_r) (every stored entry, explicit zeros included)
+                                              + max e(x_c) over the nonzero x_c of the columns that hold entries
+                                              (x entries of empty columns are never read and change nothing),
+                                       p_j  = fl(a_rj * x_j),
+                                       y_r  = RN( sum_j trunc0(p_j * 2^(94 - T_r)) * 2^(T_r - 94) )
+                                     with trunc0 toward zero, the sum exact (integers) and RN ONE round-to-nearest-even
+                                     to fp64, subnormal results included; a row without a nonzero product is +0.0.
+                                     y_r is the CORRECTLY ROUNDED row sum whenever every product is a multiple of
+                                     2^(T_r - 94), e.g. |p_j| >= 2^(T_r - 42) for all j (products within 2^-42 of the
+                                     row bound).  Otherwise |y_r - sum_j p_j| <= ulp(y_r) / 2 + count_r * 2^(T_r - 94):
+                                     a row whose products sit far below its bound (cancellation, or a column of x much
+                                     larger than the ones the row reads) loses the digits under 2^(T_r - 94).        */
+#define SMVP_TJDS_DETERMINISTIC_FAST 2 /* the same with 2^(62 - T_r) in place of 2^(94 - T_r): one 64-bit word per product
+                                     instead of two.  Just as reproducible (integer sums), one reduction per run and
+                                     half the accumulator traffic; |y_r - sum_j p_j| <= ulp(y_r) / 2 +
+                                     count_r * 2^(T_r - 62), exact only for products that are multiples of 2^(T_r - 62)
+                                     (|p_j| >= 2^(T_r - 10)).  The bound is NORMWISE -- 2^-9 of what one fp64 addition at
+                                     magnitude 2^T_r rounds away -- not relative to |y_r|: an x whose entries span many
+                                     orders of magnitude can cost a row with small products digits that the two-word
+                                     variant keeps.                                                                  */
 
 /* ---- statistics of the per-iteration times: struct _time_data_ (main-cli.c:87-95), same field order */
 typedef struct smvp_time_stats_t

@@ -16,8 +16,8 @@
 //                 words (scaled per row by a bound known before the multiply) and accumulated with
 //                 INTEGER atomics.  Integer addition is associative, so the result is bit-identical
 //                 run to run whatever order the hardware schedules the adds in; a final pass converts
-//                 the 96-bit sums to fp64 (one rounding, i.e. more accurate than any fp64 summation
-//                 order).  Cost: two 8-byte reductions per entry instead of one, 16 B/row of
+//                 the 96-bit sums to fp64 (one rounding of the sum of the products truncated at
+//                 2^-94 of the row bound).  Cost: two 8-byte reductions per entry instead of one, 16 B/row of
 //                 accumulators to clear and read back.
 #include "common.cuh"
 
@@ -32,14 +32,20 @@ constexpr int32_t EXP_NONFINITE = 0x40000000; // "an Inf or NaN was seen": above
 constexpr int TJDS_W = 32;           // bits kept in the low word
 constexpr int TJDS_FRAC = 62 + TJDS_W; // value = V * 2^(T_r - TJDS_FRAC), |sum V| < 2^TJDS_FRAC
 
+// x_exp is taken over the slots p < nslots only: the columns that hold entries, which perm puts first.  An x entry
+// that A x never reads (an empty column) must not raise the row bounds of the deterministic variants (and truncate
+// every row), nor send the pass to the atomic kernel when it is Inf or NaN.
 __global__ void __launch_bounds__(256) tjds_permute_x_kernel(const double *__restrict__ x, const int32_t *__restrict__ perm,
-                                                             int32_t cols, double *__restrict__ x_perm, int32_t *__restrict__ x_exp)
+                                                             int32_t cols, int32_t nslots, double *__restrict__ x_perm,
+                                                             int32_t *__restrict__ x_exp)
 {
     int32_t e = INT32_MIN;
     for (int32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < cols; p += gridDim.x * blockDim.x)
     {
         const double v = x[perm[p]];
         x_perm[p] = v;
+        if (p >= nslots)
+            continue;
         if (!isfinite(v))
             e = EXP_NONFINITE; // the deterministic variant needs finite inputs: such an x is routed to the atomic kernel
         else if (v != 0.0)
@@ -371,8 +377,9 @@ __device__ __forceinline__ double pow2_f64(int32_t e) { return __hiloint2double(
 // FAST: the host has checked (tjds_det_route) that every row bound T lies in the range of fixed_split_fast and that
 // no visited row lacks an exponent, so the per-entry "is the product zero / which split" tests and the 60-instruction
 // general split disappear from the loop.  Both instantiations produce the same words, hence the same bits of y.
-// WORDS = 2 (SMVP_TJDS_DETERMINISTIC): exact -- every bit of every product reaches the accumulators; y is the correctly
-//            rounded row sum.
+// WORDS = 2 (SMVP_TJDS_DETERMINISTIC): a product keeps its bits down to 2^(T - 94), the accumulated words are converted
+//            with one rounding (fixed_to_double): y is the correctly rounded row sum when no product has bits below
+//            that grid, and within count * 2^(T - 94) of it otherwise (the exact contract is in smvp_cuda.h).
 // WORDS = 1 (SMVP_TJDS_DETERMINISTIC_FAST): only the high word, scaled to 2^(T - 62): a product loses the bits below 2^-62
 //            of its row's bound (2^-9 of what one fp64 addition at that magnitude rounds away); the sum of the integers
 //            is still associative, so the result is just as reproducible; one 8-byte reduction and one conversion per
@@ -508,6 +515,50 @@ __device__ __forceinline__ void for_rows_of_y(int32_t n, double *__restrict__ pa
             store(i);
 }
 
+// V * 2^E with V = hi * 2^W + lo, rounded ONCE to nearest even fp64, subnormal results included (they round at
+// 2^-1074).  Converting hi on its own and adding lo would round twice when hi has more than 53 significant bits (a row
+// sum near its bound).  Common case, E >= -1022: V = H * 2^W + L with 0 <= L < 2^W; a = fl(H) and H - a are exact
+// (|H - a| <= 2^10), so V = a * 2^W + r with r = (H - a) * 2^W + L exact in fp64 (|r| < 2^43): the one fp64 addition
+// rounds V once, and |fl(V)| >= 1 makes the scaling by 2^E exact.  Below that the result may be subnormal and is rounded
+// from V as a 128-bit integer: its leading 53 bits are kept (fewer for a subnormal result), the dropped bits round; with
+// q the kept bits and 2^k the weight of the lowest, the fp64 bit pattern is ((k + 1074) << 52) + q for normal and
+// subnormal results alike (a carry of q into bit 53 moves the exponent).  Rows with T < -928 take this path, and their
+// normal results do round here.  A subnormal result is in fact always exact: every product is a multiple of 2^-1074,
+// so a grid 2^E finer than that truncates nothing, and a coarser one has E > -1074.  Its rounding branch (and
+// shift > 96) only keep the function correct for any (hi, lo, E).  The row bound keeps the result below the overflow
+// threshold (tjds_det_route).
+__device__ __forceinline__ double fixed_to_double(long long hi, long long lo, int32_t E)
+{
+    if (E >= -1022)
+    {
+        const long long H = hi + (lo >> TJDS_W), L = lo & ((1LL << TJDS_W) - 1);
+        const double a = __ll2double_rn(H);
+        const long long r = (H - __double2ll_rz(a)) * (1LL << TJDS_W) + L;
+        return __dmul_rn(__dadd_rn(__dmul_rn(a, 4294967296.0), __ll2double_rn(r)), pow2_f64(E));
+    }
+    const __int128 v = (__int128)hi * ((__int128)1 << TJDS_W) + lo;
+    if (v == 0)
+        return 0.0;
+    const bool neg = v < 0;
+    const unsigned __int128 m = (unsigned __int128)(neg ? -v : v);
+    const unsigned long long mh = (unsigned long long)(m >> 64), ml = (unsigned long long)m;
+    const int32_t n = mh ? 128 - __clzll((long long)mh) : 64 - __clzll((long long)ml); // bits of m
+    const int32_t shift = max(n - 53, -1074 - E);                                     // low bits of m dropped
+    unsigned long long q;
+    if (shift <= 0)
+        q = ml << -shift; // m < 2^53: exact
+    else if (shift > 96)
+        q = 0; // m * 2^E < 2^-1075: rounds to zero
+    else
+    {
+        q = (unsigned long long)(m >> shift);
+        const unsigned __int128 rem = m - ((unsigned __int128)q << shift), half = (unsigned __int128)1 << (shift - 1);
+        q += (rem > half || (rem == half && (q & 1))) ? 1 : 0;
+    }
+    const unsigned long long bits = ((unsigned long long)(E + shift + 1074) << 52) + q;
+    return __longlong_as_double((long long)(neg ? bits | (1ULL << 63) : bits));
+}
+
 // row_rank != NULL: the accumulators and row_exp are in popularity-rank order (relabelled handle), y is not.
 // Returns the row's dot term (store_row).  Dot: the work unit is the CTA's 256 rows of y; their dot terms are added in a
 // pairwise tree.
@@ -521,17 +572,11 @@ __device__ __forceinline__ double tjds_det_finalize_row(int32_t row, const long 
     const int32_t r = row_rank ? row_rank[row] : row;
     if (r < r_lo || r >= r_hi)
         return store_row<M>(y, row, 0.0, alpha, beta, w);
-    longlong2 a;
-    a.x = acc[r];
-    a.y = words == 2 ? acc[(int64_t)rows + r] : 0; // one word: the value is hi * 2^(T - 62), i.e. lo = 0 below
+    const long long hi = acc[r];
+    const long long lo = words == 2 ? acc[(int64_t)rows + r] : 0; // one word: the value is hi * 2^(T - 62), i.e. lo = 0 below
     double out = 0.0;
-    if (a.x != 0 || a.y != 0)
-    {
-        // (hi * 2^W + lo) as one correctly-ordered fp64 sum, then one exact scaling by a power of two
-        const double s = __dadd_rn(__dmul_rn((double)a.x, 4294967296.0), (double)a.y);
-        const int32_t T = row_exp[r] + *x_exp;
-        out = scalbn(s, T - TJDS_FRAC);
-    }
+    if (hi != 0 || lo != 0)
+        out = fixed_to_double(hi, lo, row_exp[r] + *x_exp - TJDS_FRAC);
     return store_row<M>(y, row, out, alpha, beta, w);
 }
 template <YStore M>
@@ -1061,7 +1106,8 @@ extern "C" int smvp_tjds_set_x_device(smvp_tjds *A, const double *d_x, void *str
         const int64_t cap = (int64_t)device_props().sms * 8;
         if (blocks > cap)
             blocks = cap;
-        SMVP_LAUNCH(tjds_permute_x_kernel, (unsigned)blocks, 256, 0, s, d_x, (const int32_t *)A->perm, A->cols, A->x_perm, A->x_exp);
+        SMVP_LAUNCH(tjds_permute_x_kernel, (unsigned)blocks, 256, 0, s, d_x, (const int32_t *)A->perm, A->cols, A->nslots, A->x_perm,
+                    A->x_exp);
     }
     SMVP_CUDA(cudaMemcpyAsync(A->x_exp_host, A->x_exp, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
     SMVP_CUDA(cudaEventRecord(A->x_exp_event, s));

@@ -181,33 +181,6 @@ def test_out_of_range_and_bad_args(eng):
         A.mult(np.ones(2), iters=1, variant=9)
 
 
-def test_deterministic_tjds_is_exactly_rounded(eng):
-    """SMVP_TJDS_DETERMINISTIC: the two-word fixed-point accumulation is exact, every y_r equals the correctly rounded sum of
-    the fp64 products.  SMVP_TJDS_DETERMINISTIC_FAST (one word): within its documented normwise bound."""
-    rng = np.random.default_rng(5)
-    m, n, nnz = 400, 400, 20000
-    coo = util.random_coo(rng, m, n, nnz)
-    coo["val"] *= 10.0 ** rng.integers(-8, 8, nnz)  # wide dynamic range inside rows
-    x = rng.uniform(-1, 1, n) * 10.0 ** rng.integers(-3, 3, n)
-    A = eng.TjdsMatrix.build(coo, m, n)
-    y, _ = A.mult(x, 1, eng.TJDS_DETERMINISTIC)
-    y1, _ = A.mult(x, 1, eng.TJDS_DETERMINISTIC_FAST)
-    exact = np.zeros(m)
-    for r in range(m):
-        sel = coo["row"] == r
-        exact[r] = math.fsum((coo["val"][sel] * x[coo["col"][sel]]).tolist())
-    ulp = np.spacing(np.abs(exact))
-    assert np.all(np.abs(y - exact) <= 2 * ulp + 1e-300)
-    # the one-word variant truncates each product at 2^-62 of its row's bound B_r >= max|a_rj| * max|x| * count_r (a power
-    # of two, at most 8x that product): the documented NORMWISE bound, checked here with x spanning six decades
-    amax, cnt = np.zeros(m), np.zeros(m)
-    np.maximum.at(amax, coo["row"], np.abs(coo["val"]))
-    np.add.at(cnt, coo["row"], 1.0)
-    bound = cnt * 2.0 ** -62 * (8.0 * amax * np.abs(x).max() * np.maximum(cnt, 1.0))
-    assert np.all(np.abs(y1 - exact) <= bound + np.spacing(np.abs(exact)) + 1e-300)
-    A.free()
-
-
 def test_time_stats_match_oracle(eng):
     ms = np.array([0.31, 0.29, 0.5, 0.30, 0.33])
     td = eng.TimeData(ms)
