@@ -90,53 +90,35 @@ int timed_loop(int iters, double *ms_each, bool batched, const std::function<int
         return SMVP_E_ARG;
     if (env_int("SMVP_EXACT_ITER_TIMES", 0, INT32_MIN, INT32_MAX) == 1 || iters < 4)
         batched = false;
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    SMVP_CUDA(cudaEventCreate(&e0));
-    cudaError_t ce = cudaEventCreate(&e1);
-    if (ce != cudaSuccess)
-    {
-        cudaEventDestroy(e0);
-        return cuda_fail(ce, "cudaEventCreate", __FILE__, __LINE__);
-    }
-    int rc = SMVP_OK;
+    Event e0, e1;
+    SMVP_CUDA(cudaEventCreate(out(e0)));
+    SMVP_CUDA(cudaEventCreate(out(e1)));
     if (batched)
     {
         // one untimed pass first: the first launch of a kernel loads its module (milliseconds), which would otherwise be
         // charged to iteration 0 of a loop whose passes last microseconds.  Every pass rewrites all of y.
-        rc = pass(0);
-        if (rc == SMVP_OK && multi)
-            rc = multi(0, 1);
-        if (rc == SMVP_OK)
-        {
-            ce = cudaStreamSynchronize(0);
-            if (ce != cudaSuccess)
-                rc = cuda_fail(ce, "cudaStreamSynchronize", __FILE__, __LINE__);
-        }
+        SMVP_TRY(pass(0));
+        if (multi)
+            SMVP_TRY(multi(0, 1));
+        SMVP_CUDA(cudaStreamSynchronize(0));
     }
     // exact passes on the legacy stream, as before
     const int exact = batched ? 1 : iters;
-    for (int it = 0; it < exact && rc == SMVP_OK; it++)
+    for (int it = 0; it < exact; it++)
     {
-        cudaEventRecord(e0, 0);
-        rc = pass(0);
-        cudaEventRecord(e1, 0);
+        cudaEventRecord(e0.get(), 0);
+        const int rc = pass(0);
+        cudaEventRecord(e1.get(), 0);
         if (rc != SMVP_OK)
-            break;
-        ce = cudaEventSynchronize(e1);
-        if (ce != cudaSuccess)
-        {
-            rc = cuda_fail(ce, "cudaEventSynchronize", __FILE__, __LINE__);
-            break;
-        }
+            return rc;
+        SMVP_CUDA(cudaEventSynchronize(e1.get()));
         float ms = 0.f;
-        cudaEventElapsedTime(&ms, e0, e1);
+        cudaEventElapsedTime(&ms, e0.get(), e1.get());
         if (ms_each)
             ms_each[it] = (double)ms;
     }
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
-    if (rc != SMVP_OK || !batched)
-        return rc;
+    if (!batched)
+        return SMVP_OK;
 
     // ---- the remaining passes: graphs of `batch` passes replayed back to back on a private stream
     const int rest = iters - 1;
@@ -146,89 +128,71 @@ int timed_loop(int iters, double *ms_each, bool batched, const std::function<int
     if (batch > rest)
         batch = rest;
     const int nfull = rest / batch, tail = rest % batch;
-    cudaStream_t s = nullptr;
-    cudaGraph_t g[2] = {nullptr, nullptr};
-    cudaGraphExec_t ge[2] = {nullptr, nullptr};
     const int nev = nfull + (tail ? 1 : 0) + 1;
-    cudaEvent_t *ev = new (std::nothrow) cudaEvent_t[nev]();
+    Stream s;
+    Graph g[2];
+    GraphExec ge[2];
+    std::unique_ptr<Event[]> ev(new (std::nothrow) Event[nev]);
     long long captured[2] = {0, 0};
-    auto body = [&]() -> int {
-        if (!ev)
-            return SMVP_E_ALLOC;
-        SMVP_CUDA(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
-        for (int k = 0; k < nev; k++)
-            SMVP_CUDA(cudaEventCreate(&ev[k]));
-        for (int k = 0; k < 2; k++)
-        {
-            const int n = k == 0 ? batch : tail;
-            if (n == 0 || (k == 0 && nfull == 0) || multi)
-                continue;
-            const long long before = g_launches.load();
-            SMVP_CUDA(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-            int prc = SMVP_OK;
-            for (int b = 0; b < n && prc == SMVP_OK; b++)
-                prc = pass(s);
-            const cudaError_t ee = cudaStreamEndCapture(s, &g[k]);
-            captured[k] = g_launches.load() - before;
-            g_launches.fetch_sub(captured[k]); // nothing ran yet: replays are counted below
-            if (prc != SMVP_OK)
-                return prc;
-            SMVP_CUDA(ee);
-            SMVP_CUDA(cudaGraphInstantiate(&ge[k], g[k], 0));
-        }
-        int e = 0;
-        SMVP_CUDA(cudaEventRecord(ev[e++], s));
-        for (int k = 0; k < nfull; k++)
-        {
-            if (multi)
-                SMVP_TRY(multi(s, batch));
-            else
-            {
-                SMVP_CUDA(cudaGraphLaunch(ge[0], s));
-                g_launches.fetch_add(captured[0]);
-            }
-            SMVP_CUDA(cudaEventRecord(ev[e++], s));
-        }
-        if (tail)
-        {
-            if (multi)
-                SMVP_TRY(multi(s, tail));
-            else
-            {
-                SMVP_CUDA(cudaGraphLaunch(ge[1], s));
-                g_launches.fetch_add(captured[1]);
-            }
-            SMVP_CUDA(cudaEventRecord(ev[e++], s));
-        }
-        SMVP_CUDA(cudaStreamSynchronize(s));
-        int it = 1;
-        for (int k = 0; k + 1 < nev; k++)
-        {
-            float ms = 0.f;
-            SMVP_CUDA(cudaEventElapsedTime(&ms, ev[k], ev[k + 1]));
-            const int n = k < nfull ? batch : tail;
-            for (int b = 0; b < n; b++, it++)
-                if (ms_each)
-                    ms_each[it] = (double)ms / n;
-        }
-        return SMVP_OK;
-    };
-    rc = body();
+    if (!ev)
+        return SMVP_E_ALLOC;
+    SMVP_CUDA(cudaStreamCreateWithFlags(out(s), cudaStreamNonBlocking));
+    for (int k = 0; k < nev; k++)
+        SMVP_CUDA(cudaEventCreate(out(ev[k])));
     for (int k = 0; k < 2; k++)
     {
-        if (ge[k])
-            cudaGraphExecDestroy(ge[k]);
-        if (g[k])
-            cudaGraphDestroy(g[k]);
+        const int n = k == 0 ? batch : tail;
+        if (n == 0 || (k == 0 && nfull == 0) || multi)
+            continue;
+        const long long before = g_launches.load();
+        SMVP_CUDA(cudaStreamBeginCapture(s.get(), cudaStreamCaptureModeThreadLocal));
+        int prc = SMVP_OK;
+        for (int b = 0; b < n && prc == SMVP_OK; b++)
+            prc = pass(s.get());
+        const cudaError_t ee = cudaStreamEndCapture(s.get(), out(g[k]));
+        captured[k] = g_launches.load() - before;
+        g_launches.fetch_sub(captured[k]); // nothing ran yet: replays are counted below
+        if (prc != SMVP_OK)
+            return prc;
+        SMVP_CUDA(ee);
+        SMVP_CUDA(cudaGraphInstantiate(out(ge[k]), g[k].get(), 0));
     }
-    if (ev)
-        for (int k = 0; k < nev; k++)
-            if (ev[k])
-                cudaEventDestroy(ev[k]);
-    delete[] ev;
-    if (s)
-        cudaStreamDestroy(s);
-    return rc;
+    int e = 0;
+    SMVP_CUDA(cudaEventRecord(ev[e++].get(), s.get()));
+    for (int k = 0; k < nfull; k++)
+    {
+        if (multi)
+            SMVP_TRY(multi(s.get(), batch));
+        else
+        {
+            SMVP_CUDA(cudaGraphLaunch(ge[0].get(), s.get()));
+            g_launches.fetch_add(captured[0]);
+        }
+        SMVP_CUDA(cudaEventRecord(ev[e++].get(), s.get()));
+    }
+    if (tail)
+    {
+        if (multi)
+            SMVP_TRY(multi(s.get(), tail));
+        else
+        {
+            SMVP_CUDA(cudaGraphLaunch(ge[1].get(), s.get()));
+            g_launches.fetch_add(captured[1]);
+        }
+        SMVP_CUDA(cudaEventRecord(ev[e++].get(), s.get()));
+    }
+    SMVP_CUDA(cudaStreamSynchronize(s.get()));
+    int it = 1;
+    for (int k = 0; k + 1 < nev; k++)
+    {
+        float ms = 0.f;
+        SMVP_CUDA(cudaEventElapsedTime(&ms, ev[k].get(), ev[k + 1].get()));
+        const int n = k < nfull ? batch : tail;
+        for (int b = 0; b < n; b++, it++)
+            if (ms_each)
+                ms_each[it] = (double)ms / n;
+    }
+    return SMVP_OK;
 }
 } // namespace smvp
 

@@ -6,6 +6,7 @@
 #include <atomic>
 #include <cstdlib>
 #include <functional>
+#include <memory>
 #include <new>
 #include <type_traits>
 
@@ -45,6 +46,58 @@ int cuda_fail(cudaError_t e, const char *what, const char *file, int line);
     } while (0)
 
 static inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }
+
+// Owners of the library's CUDA resources: device memory, pinned host memory, events, streams and graphs are each held by
+// one of these, so every return path releases them.  cudaFree synchronises the device implicitly, and wherever an owner
+// may go out of scope while a stream still uses its memory, the code synchronises that stream first.
+struct DevFree
+{
+    void operator()(void *p) const { cudaFree(p); }
+};
+struct PinnedFree
+{
+    void operator()(void *p) const { cudaFreeHost(p); }
+};
+struct CudaDestroy
+{
+    void operator()(cudaEvent_t e) const { cudaEventDestroy(e); }
+    void operator()(cudaStream_t s) const { cudaStreamDestroy(s); }
+    void operator()(cudaGraph_t g) const { cudaGraphDestroy(g); }
+    void operator()(cudaGraphExec_t g) const { cudaGraphExecDestroy(g); }
+};
+template <typename T>
+using DevPtr = std::unique_ptr<T, DevFree>;
+template <typename T>
+using PinnedPtr = std::unique_ptr<T, PinnedFree>;
+using Event = std::unique_ptr<std::remove_pointer_t<cudaEvent_t>, CudaDestroy>;
+using Stream = std::unique_ptr<std::remove_pointer_t<cudaStream_t>, CudaDestroy>;
+using Graph = std::unique_ptr<std::remove_pointer_t<cudaGraph_t>, CudaDestroy>;
+using GraphExec = std::unique_ptr<std::remove_pointer_t<cudaGraphExec_t>, CudaDestroy>;
+
+// out(owner): the handle pointer a creating call writes to (cudaEventCreate(out(ev))); the owner takes the new handle
+// at the end of the full expression, before SMVP_CUDA looks at the result
+template <typename P>
+struct OutPtr
+{
+    P &owner;
+    typename P::pointer raw = nullptr;
+    ~OutPtr() { owner.reset(raw); }
+    operator typename P::pointer *() { return &raw; }
+};
+template <typename P>
+static inline OutPtr<P> out(P &owner)
+{
+    return OutPtr<P>{owner};
+}
+
+// device allocation padded so that 16-byte vector / bulk copies may over-read the tail
+template <typename T>
+static inline cudaError_t dev_alloc(DevPtr<T> &p, int64_t n)
+{
+    size_t bytes = (size_t)(n > 0 ? n : 0) * sizeof(T);
+    bytes = ((bytes + 255) & ~(size_t)255) + 256;
+    return cudaMalloc((void **)(T **)out(p), bytes);
+}
 
 // Lifts a run-time flag into a template argument: f(std::true_type()) or f(std::false_type()), so that a launcher names
 // each kernel instantiation once.
@@ -172,7 +225,7 @@ __device__ __forceinline__ double cta_tree_sum(double v)
 }
 // Per-handle scratch of a dot pass (dot.cu): the partials of `units` work units, the reduction's CTA sums and its counter.
 // Grows *buf (counted in *device_bytes) when the plan needs more room; may synchronise then.
-int dot_scratch(double **buf, int64_t *cap, int64_t *device_bytes, int64_t units, cudaStream_t s);
+int dot_scratch(DevPtr<double> *buf, int64_t *cap, int64_t *device_bytes, int64_t units, cudaStream_t s);
 // one launch: *out = the partials buf[0, units) summed in the fixed tree (DESIGN.md §5.7)
 int dot_reduce(double *buf, int64_t cap, int64_t units, double *out, cudaStream_t s);
 
@@ -182,37 +235,6 @@ const char *env_str(const char *name);                   // the value; NULL when
 bool env_set(const char *name);                          // set at all, even to ""
 int env_int(const char *name, int dflt, int lo, int hi); // decimal integer clamped to [lo, hi]; dflt when unset or empty
 int env_tristate(const char *name);                      // 1 for "1...", -1 for "0...", 0 otherwise
-
-// device allocation padded so that 16-byte vector / bulk copies may over-read the tail
-template <typename T>
-static inline cudaError_t dev_alloc(T **p, int64_t n)
-{
-    size_t bytes = (size_t)(n > 0 ? n : 0) * sizeof(T);
-    bytes = ((bytes + 255) & ~(size_t)255) + 256;
-    return cudaMalloc((void **)p, bytes);
-}
-
-// a device temporary that is released on every exit path (error returns included)
-struct DevTmp
-{
-    void *p = nullptr;
-    DevTmp() = default;
-    DevTmp(const DevTmp &) = delete;
-    DevTmp &operator=(const DevTmp &) = delete;
-    ~DevTmp() { cudaFree(p); }
-    template <typename T>
-    cudaError_t alloc(int64_t n)
-    {
-        cudaFree(p);
-        p = nullptr;
-        T *q = nullptr;
-        const cudaError_t e = dev_alloc(&q, n);
-        p = q;
-        return e;
-    }
-    template <typename T>
-    T *as() const { return static_cast<T *>(p); }
-};
 
 // The `-n` loop of the host entry points (main-cli.c:402-420 / :1004-1024): `iters` passes, per-iteration
 // milliseconds into ms_each (may be NULL).  `pass(stream)` enqueues ONE pass.
@@ -260,10 +282,10 @@ int coo_inspect(const int32_t *d_row, const int32_t *d_col, int64_t nnz, int32_t
 // AoS (smvp_coo, 16 B) -> SoA
 int coo_unzip(const smvp_coo *d_aos, int64_t nnz, int32_t *d_row, int32_t *d_col, double *d_val, cudaStream_t s);
 // sorting permutation of the COO: major/minor lexicographic, using the arrival order to skip work.
-// On return *d_idx (device, nnz uint32, owned by caller via cudaFree) lists source positions in sorted
-// order, or is NULL when the input already is in the requested order.
+// On return *d_idx (device, nnz uint32) lists source positions in sorted order, or is empty when the input already
+// is in the requested order.
 int coo_sort_index(const int32_t *d_major, const int32_t *d_minor, int64_t nnz, int32_t n_major, int32_t n_minor,
-                   bool already_sorted, bool sorted_transposed, uint32_t **d_idx, cudaStream_t s);
+                   bool already_sorted, bool sorted_transposed, DevPtr<uint32_t> *d_idx, cudaStream_t s);
 static inline int bits_for(uint32_t n) // bits needed to represent values in [0, n)
 {
     int b = 0;
@@ -305,16 +327,30 @@ __device__ __forceinline__ V narrow_value(double v)
     return n;
 }
 
+// streams and events of the pipelined host-vector pass (csr_mult.cu), created on its first use.  One stream per direction:
+// pieces on two or three streams per direction only share the link and finish later (10.15 ms per call with one, 11.9
+// with two, 13.2 with three; profiles/r01_logs/e2e_sweep.log).
+constexpr int PIPE_MAX_RANGES = 64;
+constexpr int PIPE_MAX_XCHUNKS = 64;
+struct PipeResources
+{
+    Stream up, down, compute;
+    Event begin, x_ready[PIPE_MAX_XCHUNKS], done[PIPE_MAX_RANGES], down_done[PIPE_MAX_RANGES], t0[PIPE_MAX_RANGES],
+        t1[PIPE_MAX_RANGES];
+};
+
 } // namespace smvp
 
 // ---------------------------------------------------------------- handles
+// Created value-initialised (new (std::nothrow) smvp_csr()), so every scalar starts at zero; the owners free everything
+// the handle holds when it is deleted.
 struct smvp_csr
 {
     int32_t rows, cols;
     int64_t nnz;
-    int32_t *row_ptr; // [rows+1]
-    int32_t *col_ind; // [nnz]
-    double *val;      // [nnz]
+    smvp::DevPtr<int32_t> row_ptr; // [rows+1]
+    smvp::DevPtr<int32_t> col_ind; // [nnz]
+    smvp::DevPtr<double> val;      // [nnz]
     int32_t max_row_nnz;
     int32_t input_order;
     int32_t auto_variant;
@@ -323,45 +359,42 @@ struct smvp_csr
     int32_t merge_headroom; // CTAs per SM the persistent merge-path grid leaves free for a co-running kernel (default 0)
     int32_t merge_cfg;      // which template instantiation the plan was made for (-1 none)
     int32_t merge_tiles;
-    int32_t *tile_row;      // [merge_tiles+1] rows consumed before each tile
-    double *head_val;       // [merge_tiles] partial of the first row that ends in the tile
-    double *carry_val;      // [merge_tiles] partial of the row that continues past the tile
+    smvp::DevPtr<int32_t> tile_row; // [merge_tiles+1] rows consumed before each tile
+    smvp::DevPtr<double> head_val;  // [merge_tiles] partial of the first row that ends in the tile
+    smvp::DevPtr<double> carry_val; // [merge_tiles] partial of the row that continues past the tile
     // scratch for the host-vector entry point
-    double *d_x, *d_y;
+    smvp::DevPtr<double> d_x, d_y;
     // plan of the pipelined host-vector pass (csr_mult.cu): tile ranges, the rows each completes and how much of x
     // (a leading part, x arrives front to back) each reads.  Host-side copies; pipe_cfg = tile size they were cut for.
     int32_t pipe_cfg, pipe_ranges, pipe_xlo; // pipe_xlo: first entry of x any nonzero reads (rounded down to 64)
-    int32_t pipe_tile[65], pipe_row[65], pipe_xneed[64];
-    void *pipe_res; // streams and events of that pass, created on first use (csr_mult.cu)
+    int32_t pipe_tile[smvp::PIPE_MAX_RANGES + 1], pipe_row[smvp::PIPE_MAX_RANGES + 1], pipe_xneed[smvp::PIPE_MAX_RANGES];
+    std::unique_ptr<smvp::PipeResources> pipe_res;
     // popularity relabelling of the column space (relabel.cu): 0 undecided, 1 in use, -1 not worth it
     int32_t relabel_state;
-    int32_t *col_rel;    // [nnz]  rank of col_ind[j]; what the kernels read instead of col_ind when in use
-    int32_t *x_order;    // [cols] column with rank p
-    double *x_rel;       // [cols] x in rank order
-    const double *x_set; // the x last given to smvp_csr_set_x_device (caller-owned)
+    smvp::DevPtr<int32_t> col_rel; // [nnz]  rank of col_ind[j]; what the kernels read instead of col_ind when in use
+    smvp::DevPtr<int32_t> x_order; // [cols] column with rank p
+    smvp::DevPtr<double> x_rel;    // [cols] x in rank order
+    const double *x_set;           // the x last given to smvp_csr_set_x_device (caller-owned)
     // row-pattern plan (pattern.cu): 0 undecided, 1 in use, -1 not used.  Row r's k-th nonzero sits in column
     // r + pat_off[pat_id[r] * PAT_LMAX + k]; the multiply reads pat_id instead of col_ind.
     int32_t pattern_state;
     int32_t pattern_count, pattern_maxlen; // distinct patterns, longest pattern
-    uint8_t *pat_id;                       // [rows]
-    int32_t *pat_off;                      // [pattern_count * PAT_LMAX]
-    int32_t *pat_len;                      // [pattern_count]
+    smvp::DevPtr<uint8_t> pat_id;          // [rows]
+    smvp::DevPtr<int32_t> pat_off;         // [pattern_count * PAT_LMAX]
+    smvp::DevPtr<int32_t> pat_len;         // [pattern_count]
     // the values the pattern kernel streams: val itself (pat_vbytes 8) or, when every value converts to fp32 / fp16 and
     // back with the same 64 bits, a copy at that width (pat_vbytes 4 / 2).  0 = not decided.  val stays for every other path.
     int32_t pat_vbytes;
-    void *pat_val; // [nnz] narrow copy (NULL at width 8)
+    smvp::DevPtr<char> pat_val; // [nnz * pat_vbytes] narrow copy (empty at width 8)
     // scratch of the fused inner product (*_axpby_dot, dot.cu): unit partials, reduction sums and counter; built at first use
-    double *dot_buf;
+    smvp::DevPtr<double> dot_buf;
     int64_t dot_cap;
 };
 namespace smvp
 {
-void csr_pipe_release(smvp_csr *A);                                // csr_mult.cu
 int csr_relabel_plan(smvp_csr *A, cudaStream_t s);                 // relabel.cu
 int csr_relabel_x(smvp_csr *A, const double *d_x, cudaStream_t s); // relabel.cu
-void csr_relabel_release(smvp_csr *A);                             // relabel.cu
 int csr_pattern_plan(smvp_csr *A, cudaStream_t s);                // pattern.cu: decides the relabelling first
-void csr_pattern_release(smvp_csr *A);                             // pattern.cu
 } // namespace smvp
 
 struct smvp_tjds
@@ -371,50 +404,49 @@ struct smvp_tjds
     int32_t ndiag;
     int32_t ref_diag_limit;
     int32_t input_order;
-    int32_t nslots;      // columns with at least one entry (= length of diagonal 0)
-    int32_t last_diag_len; // entries in the last jagged diagonal
-    int32_t *perm;       // [cols]   slot -> original column
-    int32_t *slot_len;   // [cols]   entries in the column at slot p (descending)
-    int32_t *start_pos;  // [ndiag+1]
-    int32_t *row_ind;    // [nnz]
-    double *val;         // [nnz]
-    double *x_perm;      // [cols]
-    int2 *seg_blocks;    // [num_seg_blocks] {segment, first slot}: work plan of the multiply (tjds_mult.cu)
+    int32_t nslots;                  // columns with at least one entry (= length of diagonal 0)
+    int32_t last_diag_len;           // entries in the last jagged diagonal
+    smvp::DevPtr<int32_t> perm;      // [cols]   slot -> original column
+    smvp::DevPtr<int32_t> slot_len;  // [cols]   entries in the column at slot p (descending)
+    smvp::DevPtr<int32_t> start_pos; // [ndiag+1]
+    smvp::DevPtr<int32_t> row_ind;   // [nnz]
+    smvp::DevPtr<double> val;        // [nnz]
+    smvp::DevPtr<double> x_perm;     // [cols]
+    smvp::DevPtr<int2> seg_blocks;   // [num_seg_blocks] {segment, first slot}: work plan of the multiply (tjds_mult.cu)
     int32_t num_seg_blocks;
     int64_t device_bytes;
     // deterministic variant: exact fixed-point accumulation (tjds_mult.cu)
-    int32_t *row_exp;        // [rows] ea_r + cb_r: |a_rj| < 2^ea_r, row holds <= 2^cb_r entries (aux, built lazily)
-    long long *acc;          // [2*rows] hi/lo integer accumulators
-    int32_t *x_exp;          // [1] exponent bound of max |x|
-    double *d_x, *d_y;
+    smvp::DevPtr<int32_t> row_exp; // [rows] ea_r + cb_r: |a_rj| < 2^ea_r, row holds <= 2^cb_r entries (aux, built lazily)
+    smvp::DevPtr<long long> acc;   // [2*rows] hi/lo integer accumulators
+    smvp::DevPtr<int32_t> x_exp;   // [1] exponent bound of max |x|
+    smvp::DevPtr<double> d_x, d_y;
     // popularity relabelling of the ROW space (relabel.cu): 0 undecided, 1 in use, -1 not worth it
     int32_t skew;            // walk of the multiply kernels: 0 undecided, 1 skewed (runs of equal rows), -1 straight
     int32_t det_flags[5];    // host copy: [0] bit 0 = the matrix holds Inf/NaN, bit 1 = a row has entries but only zeros;
                              // [1] / [2] = largest / smallest row_exp (EXP_NONE / EXP_LOW_NONE if none);
                              // [3] / [4] = first / last row (of the index space the kernels use) that holds an entry
-    int32_t *x_exp_host;     // pinned: x_exp as of the last smvp_tjds_set_x_device, valid once x_exp_event has passed
-    cudaEvent_t x_exp_event;
+    smvp::PinnedPtr<int32_t> x_exp_host; // x_exp as of the last smvp_tjds_set_x_device, valid once x_exp_event has passed
+    smvp::Event x_exp_event;
     int32_t x_exp_pending;   // 1: x_exp_host has not been looked at since the last set_x
     int32_t det_fast;        // for the current x: 1 every row bound is in the range of the short split loop, -1 not
     int32_t det_route;       // for the current x: 1 exact integer kernel, -1 atomic kernel (non-finite / overflowing input)
     int32_t relabel_state;
-    int32_t *row_rel;        // [nnz]  rank of row_ind[j]; what the kernels scatter through when in use
-    int32_t *row_rank;       // [rows] rank of row r
-    double *y_rel;           // [rows] y in rank order (atomic variant)
-    double *y_sum;           // [rows] atomic sums of a natural-order handle under the epilogue (*_axpby), built at first use
+    smvp::DevPtr<int32_t> row_rel;  // [nnz]  rank of row_ind[j]; what the kernels scatter through when in use
+    smvp::DevPtr<int32_t> row_rank; // [rows] rank of row r
+    smvp::DevPtr<double> y_rel;     // [rows] y in rank order (atomic variant)
+    smvp::DevPtr<double> y_sum;     // [rows] atomic sums of a natural-order handle under the epilogue (*_axpby), built at first use
     // transposed product y = A^T x (tjds_mult.cu), scratch built at its first call.  Columns longer than TJDS_SEG
     // (slots [0, tr_nlong)) are summed per segment into tr_part, then combined; tr_nwide of them are longer than
     // TJDS_SEG^2 entries and are combined by a whole warp.
     int32_t tr_ready;        // 1 once the scratch below exists
     int32_t tr_nlong, tr_nwide;
-    uint32_t *tr_seg_off;    // [nseg] first partial of segment g; slot q of segment g writes tr_part[tr_seg_off[g] + q]
-    double *tr_part;         // one partial per (segment, slot) pair of the long columns
-    double *d_xt, *d_yt;     // [rows] / [cols]: scratch of the host-vector entry point
-    double *dot_buf;         // scratch of the fused inner product (*_axpby_dot, dot.cu), built at first use
+    smvp::DevPtr<uint32_t> tr_seg_off; // [nseg] first partial of segment g; slot q of segment g writes tr_part[tr_seg_off[g] + q]
+    smvp::DevPtr<double> tr_part;      // one partial per (segment, slot) pair of the long columns
+    smvp::DevPtr<double> d_xt, d_yt;   // [rows] / [cols]: scratch of the host-vector entry point
+    smvp::DevPtr<double> dot_buf;      // scratch of the fused inner product (*_axpby_dot, dot.cu), built at first use
     int64_t dot_cap;
 };
 namespace smvp
 {
 int tjds_relabel_plan(smvp_tjds *A, cudaStream_t s); // relabel.cu
-void tjds_relabel_release(smvp_tjds *A);             // relabel.cu
 } // namespace smvp

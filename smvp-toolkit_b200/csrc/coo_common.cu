@@ -42,17 +42,16 @@ int coo_inspect(const int32_t *d_row, const int32_t *d_col, int64_t nnz, int32_t
     *order = ORDER_ROW_COL;
     if (nnz == 0)
         return SMVP_OK;
-    DevTmp flags; // released on every return path
-    SMVP_CUDA(flags.alloc<int>(4));
-    int *d_flags = flags.as<int>();
-    SMVP_CUDA(cudaMemsetAsync(d_flags, 0, 4 * sizeof(int), s));
+    DevPtr<int> flags;
+    SMVP_CUDA(dev_alloc(flags, 4));
+    SMVP_CUDA(cudaMemsetAsync(flags.get(), 0, 4 * sizeof(int), s));
     int64_t blocks = ceil_div64(nnz, 256 * 4);
     const int64_t cap = (int64_t)device_props().sms * 16;
     if (blocks > cap)
         blocks = cap;
-    SMVP_LAUNCH(coo_inspect_kernel, (unsigned)blocks, 256, 0, s, d_row, d_col, nnz, rows, cols, d_flags);
+    SMVP_LAUNCH(coo_inspect_kernel, (unsigned)blocks, 256, 0, s, d_row, d_col, nnz, rows, cols, flags.get());
     int h[4] = {0, 0, 0, 0};
-    SMVP_CUDA(cudaMemcpyAsync(h, d_flags, sizeof(h), cudaMemcpyDeviceToHost, s));
+    SMVP_CUDA(cudaMemcpyAsync(h, flags.get(), sizeof(h), cudaMemcpyDeviceToHost, s));
     SMVP_CUDA(cudaStreamSynchronize(s));
     if (h[0])
         return SMVP_E_RANGE;
@@ -112,9 +111,8 @@ __global__ void __launch_bounds__(256) make_key64_kernel(const int32_t *__restri
 //   sorted_transposed   : the list arrived sorted by (minor, major)       -> stable sort on `major` alone
 //   otherwise           : stable sort on the packed key major * 2^minor_bits + minor
 int coo_sort_index(const int32_t *d_major, const int32_t *d_minor, int64_t nnz, int32_t n_major, int32_t n_minor,
-                   bool already_sorted, bool sorted_transposed, uint32_t **d_idx, cudaStream_t s)
+                   bool already_sorted, bool sorted_transposed, DevPtr<uint32_t> *d_idx, cudaStream_t s)
 {
-    *d_idx = nullptr;
     if (already_sorted || nnz <= 1)
         return SMVP_OK;
     int64_t blocks = ceil_div64(nnz, 256 * 4);
@@ -122,35 +120,33 @@ int coo_sort_index(const int32_t *d_major, const int32_t *d_minor, int64_t nnz, 
     if (blocks > cap)
         blocks = cap;
     const int major_bits = bits_for((uint32_t)n_major), minor_bits = bits_for((uint32_t)n_minor);
-    // every temporary sits in a guard: an allocation or launch failure half-way (a 16 GB build that runs out of memory)
-    // releases what was taken so far; the surviving index buffer is detached from its guard at the end
-    DevTmp g_idx_a, g_idx_b, g_key_a, g_key_b;
+    DevPtr<uint32_t> idx_a, idx_b;
     uint32_t *res_idx = nullptr;
-    SMVP_CUDA(g_idx_a.alloc<uint32_t>(nnz));
-    SMVP_CUDA(g_idx_b.alloc<uint32_t>(nnz));
-    uint32_t *idx_a = g_idx_a.as<uint32_t>(), *idx_b = g_idx_b.as<uint32_t>();
+    SMVP_CUDA(dev_alloc(idx_a, nnz));
+    SMVP_CUDA(dev_alloc(idx_b, nnz));
     if (sorted_transposed)
     {
+        DevPtr<uint32_t> key_a, key_b;
         uint32_t *res_key = nullptr;
-        SMVP_CUDA(g_key_a.alloc<uint32_t>(nnz));
-        SMVP_CUDA(g_key_b.alloc<uint32_t>(nnz));
-        SMVP_LAUNCH(make_key32_kernel, (unsigned)blocks, 256, 0, s, d_major, nnz, g_key_a.as<uint32_t>(), idx_a);
+        SMVP_CUDA(dev_alloc(key_a, nnz));
+        SMVP_CUDA(dev_alloc(key_b, nnz));
+        SMVP_LAUNCH(make_key32_kernel, (unsigned)blocks, 256, 0, s, d_major, nnz, key_a.get(), idx_a.get());
         const int lo = 0, hi = major_bits;
-        SMVP_TRY(radix_sort_pairs<uint32_t>(g_key_a.as<uint32_t>(), idx_a, g_key_b.as<uint32_t>(), idx_b, nnz, &lo, &hi, 1, &res_key,
-                                            &res_idx, s));
+        SMVP_TRY(radix_sort_pairs<uint32_t>(key_a.get(), idx_a.get(), key_b.get(), idx_b.get(), nnz, &lo, &hi, 1, &res_key, &res_idx,
+                                            s));
     }
     else
     {
+        DevPtr<uint64_t> key_a, key_b;
         uint64_t *res_key = nullptr;
-        SMVP_CUDA(g_key_a.alloc<uint64_t>(nnz));
-        SMVP_CUDA(g_key_b.alloc<uint64_t>(nnz));
-        SMVP_LAUNCH(make_key64_kernel, (unsigned)blocks, 256, 0, s, d_major, d_minor, nnz, minor_bits, g_key_a.as<uint64_t>(), idx_a);
+        SMVP_CUDA(dev_alloc(key_a, nnz));
+        SMVP_CUDA(dev_alloc(key_b, nnz));
+        SMVP_LAUNCH(make_key64_kernel, (unsigned)blocks, 256, 0, s, d_major, d_minor, nnz, minor_bits, key_a.get(), idx_a.get());
         const int lo = 0, hi = major_bits + minor_bits;
-        SMVP_TRY(radix_sort_pairs<uint64_t>(g_key_a.as<uint64_t>(), idx_a, g_key_b.as<uint64_t>(), idx_b, nnz, &lo, &hi, 1, &res_key,
-                                            &res_idx, s));
+        SMVP_TRY(radix_sort_pairs<uint64_t>(key_a.get(), idx_a.get(), key_b.get(), idx_b.get(), nnz, &lo, &hi, 1, &res_key, &res_idx,
+                                            s));
     }
-    (res_idx == idx_a ? g_idx_a : g_idx_b).p = nullptr; // handed to the caller
-    *d_idx = res_idx;
+    *d_idx = std::move(res_idx == idx_a.get() ? idx_a : idx_b); // the sorted positions go to the caller
     return SMVP_OK;
 }
 

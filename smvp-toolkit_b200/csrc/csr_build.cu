@@ -62,62 +62,49 @@ static int csr_expand_rows(const int32_t *row_ptr, int32_t rows, int64_t nnz, in
     return SMVP_OK;
 }
 
-static void csr_release(smvp_csr *A)
-{
-    if (!A)
-        return;
-    cudaFree(A->row_ptr);
-    cudaFree(A->col_ind);
-    cudaFree(A->val);
-    cudaFree(A->tile_row);
-    cudaFree(A->head_val);
-    cudaFree(A->carry_val);
-    cudaFree(A->d_x);
-    cudaFree(A->d_y);
-    cudaFree(A->dot_buf);
-    csr_pipe_release(A);
-    csr_relabel_release(A);
-    csr_pattern_release(A);
-    delete A;
-}
-
+// a new handle of rows x cols with nnz entries, built from COO arrays on the device; handed to *out on success
 static int csr_build_impl(const int32_t *d_row, const int32_t *d_col, const double *d_val, int32_t rows, int32_t cols,
-                          int64_t nnz, smvp_csr *A, cudaStream_t s)
+                          int64_t nnz, smvp_csr **out, cudaStream_t s)
 {
+    std::unique_ptr<smvp_csr> A(new (std::nothrow) smvp_csr());
+    if (!A)
+        return SMVP_E_ALLOC;
+    A->rows = rows;
+    A->cols = cols;
+    A->nnz = nnz;
+    A->merge_cfg = -1;
     int order = ORDER_ROW_COL;
     SMVP_TRY(coo_inspect(d_row, d_col, nnz, rows, cols, &order, s));
     A->input_order = order;
 
-    SMVP_CUDA(dev_alloc(&A->row_ptr, (int64_t)rows + 1));
-    SMVP_CUDA(dev_alloc(&A->col_ind, nnz));
-    SMVP_CUDA(dev_alloc(&A->val, nnz));
+    SMVP_CUDA(dev_alloc(A->row_ptr, (int64_t)rows + 1));
+    SMVP_CUDA(dev_alloc(A->col_ind, nnz));
+    SMVP_CUDA(dev_alloc(A->val, nnz));
     A->device_bytes = 4 * ((int64_t)rows + 1) + 12 * nnz;
+    uint32_t *row_ptr = (uint32_t *)A->row_ptr.get();
 
     // row counts -> row_ptr by exclusive scan; row_ptr[rows] = nnz
-    SMVP_TRY(histogram_i32(d_row, nnz, (uint32_t *)A->row_ptr, (int64_t)rows + 1, s));
+    SMVP_TRY(histogram_i32(d_row, nnz, row_ptr, (int64_t)rows + 1, s));
     {
-        DevTmp g_max;
-        SMVP_CUDA(g_max.alloc<uint32_t>(1));
-        uint32_t *d_max = g_max.as<uint32_t>();
-        SMVP_TRY(max_u32((const uint32_t *)A->row_ptr, rows, d_max, s));
+        DevPtr<uint32_t> d_max;
+        SMVP_CUDA(dev_alloc(d_max, 1));
+        SMVP_TRY(max_u32(row_ptr, rows, d_max.get(), s));
         uint32_t h = 0;
-        SMVP_CUDA(cudaMemcpyAsync(&h, d_max, sizeof(h), cudaMemcpyDeviceToHost, s));
+        SMVP_CUDA(cudaMemcpyAsync(&h, d_max.get(), sizeof(h), cudaMemcpyDeviceToHost, s));
         SMVP_CUDA(cudaStreamSynchronize(s));
         A->max_row_nnz = (int32_t)h;
     }
-    SMVP_TRY(exclusive_scan_u32((const uint32_t *)A->row_ptr, (uint32_t *)A->row_ptr, rows, nullptr, s));
-    SMVP_LAUNCH(set_last_kernel, 1, 1, 0, s, A->row_ptr, rows, (int32_t)nnz);
+    SMVP_TRY(exclusive_scan_u32(row_ptr, row_ptr, rows, nullptr, s));
+    SMVP_LAUNCH(set_last_kernel, 1, 1, 0, s, A->row_ptr.get(), rows, (int32_t)nnz);
 
-    uint32_t *d_idx = nullptr;
+    DevPtr<uint32_t> d_idx;
     SMVP_TRY(coo_sort_index(d_row, d_col, nnz, rows, cols, order == ORDER_ROW_COL, order == ORDER_COL_ROW, &d_idx, s));
-    DevTmp g_idx;
-    g_idx.p = d_idx; // released on every return path below
-    if (d_idx == nullptr)
+    if (!d_idx)
     {
         if (nnz > 0)
         {
-            SMVP_CUDA(cudaMemcpyAsync(A->col_ind, d_col, sizeof(int32_t) * (size_t)nnz, cudaMemcpyDeviceToDevice, s));
-            SMVP_CUDA(cudaMemcpyAsync(A->val, d_val, sizeof(double) * (size_t)nnz, cudaMemcpyDeviceToDevice, s));
+            SMVP_CUDA(cudaMemcpyAsync(A->col_ind.get(), d_col, sizeof(int32_t) * (size_t)nnz, cudaMemcpyDeviceToDevice, s));
+            SMVP_CUDA(cudaMemcpyAsync(A->val.get(), d_val, sizeof(double) * (size_t)nnz, cudaMemcpyDeviceToDevice, s));
         }
     }
     else
@@ -126,8 +113,8 @@ static int csr_build_impl(const int32_t *d_row, const int32_t *d_col, const doub
         const int64_t cap = (int64_t)device_props().sms * 16;
         if (blocks > cap)
             blocks = cap;
-        SMVP_LAUNCH(gather_csr_kernel, (unsigned)blocks, 256, 0, s, (const uint32_t *)d_idx, d_col, d_val, nnz, A->col_ind,
-                    A->val);
+        SMVP_LAUNCH(gather_csr_kernel, (unsigned)blocks, 256, 0, s, (const uint32_t *)d_idx.get(), d_col, d_val, nnz, A->col_ind.get(),
+                    A->val.get());
         SMVP_CUDA(cudaStreamSynchronize(s));
     }
     SMVP_CUDA(cudaStreamSynchronize(s));
@@ -143,6 +130,7 @@ static int csr_build_impl(const int32_t *d_row, const int32_t *d_col, const doub
     // 8 TB/s), merge 2.59 ms (rows that span several warp tiles chain through the fix-up).  The crossover is put at 256.
     const bool regular_long = mean >= 256.0 && A->max_row_nnz <= 4.0 * mean + 32.0;
     A->auto_variant = ((tiny && !skewed) || regular_long) ? SMVP_CSR_VECTOR : SMVP_CSR_MERGE;
+    *out = A.release();
     return SMVP_OK;
 }
 
@@ -160,21 +148,7 @@ extern "C" int smvp_csr_build_device(const int32_t *d_row, const int32_t *d_col,
         return SMVP_E_ARG;
     if (nnz > 0x7fffffffLL - 8)
         return SMVP_E_TOOBIG;
-    smvp_csr *A = new (std::nothrow) smvp_csr();
-    if (!A)
-        return SMVP_E_ALLOC;
-    A->rows = rows;
-    A->cols = cols;
-    A->nnz = nnz;
-    A->merge_cfg = -1;
-    int rc = csr_build_impl(d_row, d_col, d_val, rows, cols, nnz, A, 0);
-    if (rc != SMVP_OK)
-    {
-        csr_release(A);
-        return rc;
-    }
-    *out = A;
-    return SMVP_OK;
+    return csr_build_impl(d_row, d_col, d_val, rows, cols, nnz, out, 0);
 }
 
 extern "C" int smvp_csr_build(const smvp_coo *coo, int32_t rows, int32_t cols, int64_t nnz, smvp_csr **out)
@@ -186,28 +160,18 @@ extern "C" int smvp_csr_build(const smvp_coo *coo, int32_t rows, int32_t cols, i
         return SMVP_E_ARG;
     if (nnz > 0x7fffffffLL - 8)
         return SMVP_E_TOOBIG;
-    smvp_coo *d_aos = nullptr;
-    int32_t *d_row = nullptr, *d_col = nullptr;
-    double *d_val = nullptr;
-    int rc = SMVP_OK;
-    auto body = [&]() -> int {
-        SMVP_CUDA(dev_alloc(&d_aos, nnz));
-        SMVP_CUDA(dev_alloc(&d_row, nnz));
-        SMVP_CUDA(dev_alloc(&d_col, nnz));
-        SMVP_CUDA(dev_alloc(&d_val, nnz));
-        if (nnz > 0)
-            SMVP_CUDA(cudaMemcpy(d_aos, coo, sizeof(smvp_coo) * (size_t)nnz, cudaMemcpyHostToDevice));
-        SMVP_TRY(coo_unzip(d_aos, nnz, d_row, d_col, d_val, 0));
-        SMVP_CUDA(cudaFree(d_aos));
-        d_aos = nullptr;
-        return smvp_csr_build_device(d_row, d_col, d_val, rows, cols, nnz, out);
-    };
-    rc = body();
-    cudaFree(d_aos);
-    cudaFree(d_row);
-    cudaFree(d_col);
-    cudaFree(d_val);
-    return rc;
+    DevPtr<smvp_coo> d_aos;
+    DevPtr<int32_t> d_row, d_col;
+    DevPtr<double> d_val;
+    SMVP_CUDA(dev_alloc(d_aos, nnz));
+    SMVP_CUDA(dev_alloc(d_row, nnz));
+    SMVP_CUDA(dev_alloc(d_col, nnz));
+    SMVP_CUDA(dev_alloc(d_val, nnz));
+    if (nnz > 0)
+        SMVP_CUDA(cudaMemcpy(d_aos.get(), coo, sizeof(smvp_coo) * (size_t)nnz, cudaMemcpyHostToDevice));
+    SMVP_TRY(coo_unzip(d_aos.get(), nnz, d_row.get(), d_col.get(), d_val.get(), 0));
+    d_aos.reset(); // before the build: lowers the peak
+    return smvp_csr_build_device(d_row.get(), d_col.get(), d_val.get(), rows, cols, nnz, out);
 }
 
 // A^T from A's arrays: the entries of A, read in its (row, col) order, are the entries of A^T in (col, row) order, so
@@ -220,41 +184,24 @@ extern "C" int smvp_csr_transpose(const smvp_csr *A, smvp_csr **out)
     *out = nullptr;
     if (!A)
         return SMVP_E_ARG;
-    smvp_csr *T = new (std::nothrow) smvp_csr();
-    if (!T)
-        return SMVP_E_ALLOC;
-    T->rows = A->cols;
-    T->cols = A->rows;
-    T->nnz = A->nnz;
-    T->merge_cfg = -1;
-    auto body = [&]() -> int {
-        DevTmp row_of;
-        SMVP_CUDA(row_of.alloc<int32_t>(A->nnz));
-        SMVP_TRY(csr_expand_rows(A->row_ptr, A->rows, A->nnz, row_of.as<int32_t>(), 0));
-        return csr_build_impl(A->col_ind, row_of.as<int32_t>(), A->val, T->rows, T->cols, T->nnz, T, 0);
-    };
-    const int rc = body();
-    if (rc != SMVP_OK)
-    {
-        csr_release(T);
-        return rc;
-    }
-    *out = T;
-    return SMVP_OK;
+    DevPtr<int32_t> row_of;
+    SMVP_CUDA(dev_alloc(row_of, A->nnz));
+    SMVP_TRY(csr_expand_rows(A->row_ptr.get(), A->rows, A->nnz, row_of.get(), 0));
+    return csr_build_impl(A->col_ind.get(), row_of.get(), A->val.get(), A->cols, A->rows, A->nnz, out, 0);
 }
 
-extern "C" void smvp_csr_free(smvp_csr *A) { smvp::csr_release(A); }
+extern "C" void smvp_csr_free(smvp_csr *A) { delete A; }
 
 extern "C" int smvp_csr_export(const smvp_csr *A, int32_t *row_ptr, int32_t *col_ind, double *val)
 {
     if (!A)
         return SMVP_E_ARG;
     if (row_ptr)
-        SMVP_CUDA(cudaMemcpy(row_ptr, A->row_ptr, sizeof(int32_t) * ((size_t)A->rows + 1), cudaMemcpyDeviceToHost));
+        SMVP_CUDA(cudaMemcpy(row_ptr, A->row_ptr.get(), sizeof(int32_t) * ((size_t)A->rows + 1), cudaMemcpyDeviceToHost));
     if (col_ind && A->nnz > 0)
-        SMVP_CUDA(cudaMemcpy(col_ind, A->col_ind, sizeof(int32_t) * (size_t)A->nnz, cudaMemcpyDeviceToHost));
+        SMVP_CUDA(cudaMemcpy(col_ind, A->col_ind.get(), sizeof(int32_t) * (size_t)A->nnz, cudaMemcpyDeviceToHost));
     if (val && A->nnz > 0)
-        SMVP_CUDA(cudaMemcpy(val, A->val, sizeof(double) * (size_t)A->nnz, cudaMemcpyDeviceToHost));
+        SMVP_CUDA(cudaMemcpy(val, A->val.get(), sizeof(double) * (size_t)A->nnz, cudaMemcpyDeviceToHost));
     return SMVP_OK;
 }
 
@@ -264,10 +211,10 @@ extern "C" int smvp_csr_arrays_device(const smvp_csr *A, const int32_t **d_row_p
     if (!A)
         return SMVP_E_ARG;
     if (d_row_ptr)
-        *d_row_ptr = A->row_ptr;
+        *d_row_ptr = A->row_ptr.get();
     if (d_col_ind)
-        *d_col_ind = A->col_ind;
+        *d_col_ind = A->col_ind.get();
     if (d_val)
-        *d_val = A->val;
+        *d_val = A->val.get();
     return SMVP_OK;
 }

@@ -271,7 +271,7 @@ __global__ void __launch_bounds__(TINY_THREADS) csr_tiny_loop_kernel(const int32
 }
 
 // the column indices the multiply kernels read: the relabelled copy when that plan is in use (relabel.cu)
-static inline const int32_t *mult_cols(const smvp_csr *A) { return A->relabel_state == 1 ? A->col_rel : A->col_ind; }
+static inline const int32_t *mult_cols(const smvp_csr *A) { return A->relabel_state == 1 ? A->col_rel.get() : A->col_ind.get(); }
 
 // lanes per row of the vector kernel, from the mean row length
 static int vector_lpr(const smvp_csr *A)
@@ -291,8 +291,9 @@ static int launch_vector(const smvp_csr *A, const double *d_x, double *d_y, cons
     if (blocks == 0)
         return SMVP_OK;
     return with_store<YStore::Plain, YStore::Fanout, YStore::Axpby, YStore::Dot>(store_mode(dot, fan, ab), [&](auto S) {
-        SMVP_LAUNCH((csr_vector_kernel<LPR, decltype(S)::value>), (unsigned)blocks, 256, 0, s, A->row_ptr, mult_cols(A), A->val, d_x,
-                    d_y, A->rows, fan ? *fan : YFan(), ab.alpha, ab.beta, dot ? dot->w : nullptr, dot ? dot->part : nullptr);
+        SMVP_LAUNCH((csr_vector_kernel<LPR, decltype(S)::value>), (unsigned)blocks, 256, 0, s, A->row_ptr.get(), mult_cols(A),
+                    A->val.get(), d_x, d_y, A->rows, fan ? *fan : YFan(), ab.alpha, ab.beta, dot ? dot->w : nullptr,
+                    dot ? dot->part : nullptr);
         return (int)SMVP_OK;
     });
 }
@@ -780,23 +781,22 @@ static int merge_plan(smvp_csr *A, cudaStream_t s)
     const int32_t tile_items = 32 * (merge_skewed(A) ? MergeSkewed::IPT : MergeStencil::IPT);
     if (A->merge_cfg == tile_items)
         return SMVP_OK;
-    cudaFree(A->tile_row);
-    cudaFree(A->head_val);
-    cudaFree(A->carry_val);
-    A->tile_row = nullptr;
-    A->head_val = A->carry_val = nullptr;
-    A->merge_cfg = -1;
     const int64_t total = (int64_t)A->rows + A->nnz;
     const int64_t tiles = ceil_div64(total, tile_items);
     if (tiles > 0x7ffffff0LL)
         return SMVP_E_TOOBIG;
-    A->merge_tiles = (int32_t)tiles;
-    SMVP_CUDA(dev_alloc(&A->tile_row, tiles + 1));
-    SMVP_CUDA(dev_alloc(&A->head_val, tiles));
-    SMVP_CUDA(dev_alloc(&A->carry_val, tiles));
-    SMVP_LAUNCH(merge_plan_kernel, (unsigned)ceil_div64(tiles + 1, 256), 256, 0, s, A->row_ptr, A->rows, A->nnz, tile_items,
-                (int32_t)tiles, A->tile_row);
+    DevPtr<int32_t> tile_row;
+    DevPtr<double> head_val, carry_val;
+    SMVP_CUDA(dev_alloc(tile_row, tiles + 1));
+    SMVP_CUDA(dev_alloc(head_val, tiles));
+    SMVP_CUDA(dev_alloc(carry_val, tiles));
+    SMVP_LAUNCH(merge_plan_kernel, (unsigned)ceil_div64(tiles + 1, 256), 256, 0, s, A->row_ptr.get(), A->rows, A->nnz, tile_items,
+                (int32_t)tiles, tile_row.get());
     SMVP_CUDA(cudaGetLastError());
+    A->tile_row = std::move(tile_row);
+    A->head_val = std::move(head_val);
+    A->carry_val = std::move(carry_val);
+    A->merge_tiles = (int32_t)tiles;
     A->merge_cfg = tile_items; // the plan depends on the tile size only
     return SMVP_OK;
 }
@@ -885,11 +885,12 @@ static int launch_wmerge(const smvp_csr *A, const double *d_x, double *d_y, cons
     if (grid > 0)
     {
         const bool early = merge_fixup_early(ntiles);
-        SMVP_LAUNCH(kern, (unsigned)grid, C::WARPS * 32, SMEM, s, A->row_ptr, mult_cols(A), A->val, d_x, d_y, A->tile_row, A->rows,
-                    A->nnz, tile_begin, tile_end, A->head_val, A->carry_val, fan, hot_l1, hot_l2, early ? 1 : 0, ab.alpha, ab.beta, w,
-                    part);
-        SMVP_TRY(launch_fixup(early, ntiles, s, merge_fixup_kernel<M>, (const int32_t *)A->tile_row, (const double *)A->head_val,
-                              (const double *)A->carry_val, tile_begin, tile_end, d_y, fan, ab.alpha, ab.beta, w, part));
+        SMVP_LAUNCH(kern, (unsigned)grid, C::WARPS * 32, SMEM, s, A->row_ptr.get(), mult_cols(A), A->val.get(), d_x, d_y,
+                    A->tile_row.get(), A->rows, A->nnz, tile_begin, tile_end, A->head_val.get(), A->carry_val.get(), fan, hot_l1,
+                    hot_l2, early ? 1 : 0, ab.alpha, ab.beta, w, part);
+        SMVP_TRY(launch_fixup(early, ntiles, s, merge_fixup_kernel<M>, (const int32_t *)A->tile_row.get(),
+                              (const double *)A->head_val.get(), (const double *)A->carry_val.get(), tile_begin, tile_end, d_y, fan,
+                              ab.alpha, ab.beta, w, part));
     }
     return SMVP_OK;
 }
@@ -1159,9 +1160,9 @@ static int launch_pattern(const smvp_csr *A, const V *val, const double *d_x, do
         int64_t grid = 0;
         SMVP_TRY(persistent_grid(kern, C::WARPS * 32, smem, A->merge_headroom, need, res, &grid));
         if (grid > 0)
-            SMVP_LAUNCH(kern, (unsigned)grid, C::WARPS * 32, smem, s, A->row_ptr, val, A->pat_id, A->pat_off, A->pat_len,
-                        A->pattern_count, maxlen, d_x, d_y, row_begin, row_end, (uint32_t)stage, fan ? *fan : YFan(), ab.alpha,
-                        ab.beta, dot ? dot->w : nullptr, dot ? dot->part : nullptr);
+            SMVP_LAUNCH(kern, (unsigned)grid, C::WARPS * 32, smem, s, A->row_ptr.get(), val, A->pat_id.get(), A->pat_off.get(),
+                        A->pat_len.get(), A->pattern_count, maxlen, d_x, d_y, row_begin, row_end, (uint32_t)stage, fan ? *fan : YFan(),
+                        ab.alpha, ab.beta, dot ? dot->w : nullptr, dot ? dot->part : nullptr);
         return (int)SMVP_OK;
     });
 }
@@ -1171,10 +1172,10 @@ static int csr_mult_pattern(const smvp_csr *A, const double *d_x, double *d_y, c
                             int32_t row_begin, int32_t row_end, const DotOut *dot = nullptr)
 {
     if (A->pat_vbytes == 2)
-        return launch_pattern(A, (const uint16_t *)A->pat_val, d_x, d_y, fan, ab, s, row_begin, row_end, dot);
+        return launch_pattern(A, (const uint16_t *)A->pat_val.get(), d_x, d_y, fan, ab, s, row_begin, row_end, dot);
     if (A->pat_vbytes == 4)
-        return launch_pattern(A, (const float *)A->pat_val, d_x, d_y, fan, ab, s, row_begin, row_end, dot);
-    return launch_pattern(A, (const double *)A->val, d_x, d_y, fan, ab, s, row_begin, row_end, dot);
+        return launch_pattern(A, (const float *)A->pat_val.get(), d_x, d_y, fan, ab, s, row_begin, row_end, dot);
+    return launch_pattern(A, (const double *)A->val.get(), d_x, d_y, fan, ab, s, row_begin, row_end, dot);
 }
 
 constexpr Axpby AXPBY_PLAIN = {1.0, 0.0};
@@ -1273,7 +1274,7 @@ static int csr_mult_any(smvp_csr *A, const double *d_x, double *d_y, const YFan 
         if (!d_dot)
             return SMVP_OK;
         SMVP_TRY(dot_scratch(&A->dot_buf, &A->dot_cap, &A->device_bytes, csr_dot_units_max(A), s));
-        return dot_reduce(A->dot_buf, A->dot_cap, 0, d_dot, s); // no rows: +0.0
+        return dot_reduce(A->dot_buf.get(), A->dot_cap, 0, d_dot, s); // no rows: +0.0
     }
     SMVP_TRY(csr_pattern_plan(A, s)); // decides the relabelling first
     const double *x = d_x; // NULL: the x last given to smvp_csr_set_x_device
@@ -1283,7 +1284,7 @@ static int csr_mult_any(smvp_csr *A, const double *d_x, double *d_y, const YFan 
             SMVP_TRY(csr_relabel_x(A, d_x, s));
         else if (!A->x_set)
             return SMVP_E_ARG;
-        x = A->x_rel;
+        x = A->x_rel.get();
     }
     else if (!d_x)
     {
@@ -1296,9 +1297,9 @@ static int csr_mult_any(smvp_csr *A, const double *d_x, double *d_y, const YFan 
     int64_t units = 0;
     SMVP_TRY(csr_dot_units(A, csr_resolve_variant(A, variant), s, &units));
     SMVP_TRY(dot_scratch(&A->dot_buf, &A->dot_cap, &A->device_bytes, csr_dot_units_max(A), s));
-    const DotOut dot = {d_w, A->dot_buf};
+    const DotOut dot = {d_w, A->dot_buf.get()};
     SMVP_TRY(csr_mult_launch(A, x, d_y, nullptr, ab, variant, s, &dot));
-    return dot_reduce(A->dot_buf, A->dot_cap, units, d_dot, s);
+    return dot_reduce(A->dot_buf.get(), A->dot_cap, units, d_dot, s);
 }
 
 extern "C" int smvp_csr_set_x_device(smvp_csr *A, const double *d_x, void *stream)
@@ -1377,9 +1378,6 @@ extern "C" int smvp_csr_mult_device_fanout(smvp_csr *A, const double *d_x, doubl
 // With iters == 1 both happen in the same pass and the call costs about ONE vector transfer (PCIe is full
 // duplex) instead of upload + multiply + download back to back.  ms_each still reports the multiply alone: the
 // sum of the ranges' own event brackets, each opened after the range's wait for x.
-constexpr int PIPE_MAX_RANGES = 64;  // == capacity of smvp_csr::pipe_tile / pipe_row / pipe_xneed (common.cuh)
-constexpr int PIPE_MAX_XCHUNKS = 64;
-
 // Piece sizes from the sweep on B200 (DESIGN.md §6, profiles/).  Piece SIZE, not piece count, is fixed, so the fixed cost
 // of a call shrinks with the block a rank owns (round 1: e2e did not scale with N).  6 MB in both directions: on the
 // 402 MB vectors of the 369^3 stencil that is 64 ranges x 64 upload pieces, the best of every sweep (round 2: 9.8 ms per
@@ -1453,29 +1451,29 @@ static int pipe_plan(smvp_csr *A)
     pipe_profile(NR, rf);
     const int32_t T = pat ? 0 : A->merge_tiles;
     const int64_t tile_items = pat ? 0 : A->merge_cfg;
-    int32_t *d_max = nullptr; // per range: {largest, smallest} column index
+    DevPtr<int32_t> d_max; // per range: {largest, smallest} column index
     int32_t h_max[2 * PIPE_MAX_RANGES];
     for (int c = 0; c < PIPE_MAX_RANGES; c++)
     {
         h_max[2 * c] = -1; // the range reads no x at all
         h_max[2 * c + 1] = 0x7fffffff;
     }
-    SMVP_CUDA(dev_alloc(&d_max, 2 * PIPE_MAX_RANGES));
-    cudaError_t e = cudaMemcpy(d_max, h_max, sizeof(h_max), cudaMemcpyHostToDevice);
+    SMVP_CUDA(dev_alloc(d_max, 2 * PIPE_MAX_RANGES));
+    SMVP_CUDA(cudaMemcpy(d_max.get(), h_max, sizeof(h_max), cudaMemcpyHostToDevice));
     int32_t pat_nz[PIPE_MAX_RANGES + 1]; // pattern plan: first nonzero of each range (row_ptr at its first row)
-    for (int c = 0; c <= NR && e == cudaSuccess; c++)
+    for (int c = 0; c <= NR; c++)
     {
         if (pat)
         {
             A->pipe_tile[c] = A->pipe_row[c] = c == NR ? A->rows : (int32_t)((double)A->rows * rf[c]);
-            e = cudaMemcpy(&pat_nz[c], A->row_ptr + A->pipe_row[c], sizeof(int32_t), cudaMemcpyDeviceToHost);
+            SMVP_CUDA(cudaMemcpy(&pat_nz[c], A->row_ptr.get() + A->pipe_row[c], sizeof(int32_t), cudaMemcpyDeviceToHost));
             continue;
         }
         A->pipe_tile[c] = c == NR ? T : (int32_t)((double)T * rf[c]);
         // rows consumed before each boundary tile (tile_row[T] = rows)
-        e = cudaMemcpy(&A->pipe_row[c], A->tile_row + A->pipe_tile[c], sizeof(int32_t), cudaMemcpyDeviceToHost);
+        SMVP_CUDA(cudaMemcpy(&A->pipe_row[c], A->tile_row.get() + A->pipe_tile[c], sizeof(int32_t), cudaMemcpyDeviceToHost));
     }
-    for (int c = 0; c < NR && e == cudaSuccess; c++)
+    for (int c = 0; c < NR; c++)
     {
         // nonzeros of the range: merge items before the boundary minus the row ends among them
         int64_t n0 = pat ? pat_nz[c] : (int64_t)A->pipe_tile[c] * tile_items - A->pipe_row[c];
@@ -1486,15 +1484,11 @@ static int pipe_plan(smvp_csr *A)
         {
             int64_t grid = ceil_div64(n1 - n0, 256 * 16);
             const int64_t cap = (int64_t)device_props().sms * 8;
-            SMVP_LAUNCH(col_range_kernel, (unsigned)(grid < cap ? grid : cap), 256, 0, 0, (const int32_t *)A->col_ind, n0, n1,
-                        d_max + 2 * c);
+            SMVP_LAUNCH(col_range_kernel, (unsigned)(grid < cap ? grid : cap), 256, 0, 0, (const int32_t *)A->col_ind.get(), n0, n1,
+                        d_max.get() + 2 * c);
         }
     }
-    if (e == cudaSuccess)
-        e = cudaMemcpy(h_max, d_max, sizeof(h_max), cudaMemcpyDeviceToHost);
-    cudaFree(d_max);
-    if (e != cudaSuccess)
-        return cuda_fail(e, "pipe_plan", __FILE__, __LINE__);
+    SMVP_CUDA(cudaMemcpy(h_max, d_max.get(), sizeof(h_max), cudaMemcpyDeviceToHost));
     int32_t need = 0, lowest = 0x7fffffff; // x arrives front to back: a range needs everything up to the largest column so far
     for (int c = 0; c < NR; c++)
     {
@@ -1510,93 +1504,34 @@ static int pipe_plan(smvp_csr *A)
     return SMVP_OK;
 }
 
-// One stream per direction: pieces on two or three streams per direction only share the link and finish later (10.15 ms
-// per call with one, 11.9 with two, 13.2 with three; profiles/r01_logs/e2e_sweep.log).
-struct PipeResources
-{
-    cudaStream_t up = nullptr, down = nullptr, compute = nullptr;
-    cudaEvent_t x_ready[PIPE_MAX_XCHUNKS] = {}, done[PIPE_MAX_RANGES] = {}, t0[PIPE_MAX_RANGES] = {}, t1[PIPE_MAX_RANGES] = {};
-    cudaEvent_t begin = nullptr, down_done[PIPE_MAX_RANGES] = {};
-    cudaError_t create()
-    {
-        // the pass runs on its own non-blocking stream: the legacy stream would serialise it against every other
-        // blocking stream of the process
-        cudaError_t e = cudaStreamCreateWithFlags(&compute, cudaStreamNonBlocking);
-        if (e == cudaSuccess)
-            e = cudaEventCreate(&begin);
-        if (e == cudaSuccess)
-            e = cudaStreamCreateWithFlags(&up, cudaStreamNonBlocking);
-        if (e == cudaSuccess)
-            e = cudaStreamCreateWithFlags(&down, cudaStreamNonBlocking);
-        for (int c = 0; c < PIPE_MAX_XCHUNKS && e == cudaSuccess; c++)
-            e = cudaEventCreate(&x_ready[c]);
-        for (int c = 0; c < PIPE_MAX_RANGES && e == cudaSuccess; c++)
-        {
-            e = cudaEventCreate(&done[c]);
-            if (e == cudaSuccess)
-                e = cudaEventCreate(&down_done[c]);
-            if (e == cudaSuccess)
-                e = cudaEventCreate(&t0[c]);
-            if (e == cudaSuccess)
-                e = cudaEventCreate(&t1[c]);
-        }
-        return e;
-    }
-    ~PipeResources()
-    {
-        if (begin)
-            cudaEventDestroy(begin);
-        if (compute)
-            cudaStreamDestroy(compute);
-        for (int c = 0; c < PIPE_MAX_XCHUNKS; c++)
-            if (x_ready[c])
-                cudaEventDestroy(x_ready[c]);
-        for (int c = 0; c < PIPE_MAX_RANGES; c++)
-        {
-            if (done[c])
-                cudaEventDestroy(done[c]);
-            if (down_done[c])
-                cudaEventDestroy(down_done[c]);
-            if (t0[c])
-                cudaEventDestroy(t0[c]);
-            if (t1[c])
-                cudaEventDestroy(t1[c]);
-        }
-        if (up)
-            cudaStreamDestroy(up);
-        if (down)
-            cudaStreamDestroy(down);
-    }
-};
-
-namespace smvp
-{
-void csr_pipe_release(smvp_csr *A)
-{
-    delete static_cast<PipeResources *>(A->pipe_res);
-    A->pipe_res = nullptr;
-}
-} // namespace smvp
-
 // one pass in ranges; x_host != NULL: upload x under the pass; y_host != NULL: download y under the pass
 static int csr_mult_pipelined(smvp_csr *A, const double *x_host, double *y_host, float *ms)
 {
     SMVP_TRY(pipe_plan(A));
-    cudaError_t e = cudaSuccess;
     if (!A->pipe_res) // streams and events live with the handle: creating ~160 events per call costs more than a range
     {
-        PipeResources *fresh = new (std::nothrow) PipeResources();
+        std::unique_ptr<PipeResources> fresh(new (std::nothrow) PipeResources());
         if (!fresh)
             return SMVP_E_ALLOC;
-        e = fresh->create();
-        if (e != cudaSuccess)
+        // the pass runs on its own non-blocking stream: the legacy stream would serialise it against every other
+        // blocking stream of the process
+        SMVP_CUDA(cudaStreamCreateWithFlags(out(fresh->compute), cudaStreamNonBlocking));
+        SMVP_CUDA(cudaEventCreate(out(fresh->begin)));
+        SMVP_CUDA(cudaStreamCreateWithFlags(out(fresh->up), cudaStreamNonBlocking));
+        SMVP_CUDA(cudaStreamCreateWithFlags(out(fresh->down), cudaStreamNonBlocking));
+        for (Event &ev : fresh->x_ready)
+            SMVP_CUDA(cudaEventCreate(out(ev)));
+        for (int c = 0; c < PIPE_MAX_RANGES; c++)
         {
-            delete fresh;
-            return cuda_fail(e, "pipeline resources", __FILE__, __LINE__);
+            SMVP_CUDA(cudaEventCreate(out(fresh->done[c])));
+            SMVP_CUDA(cudaEventCreate(out(fresh->down_done[c])));
+            SMVP_CUDA(cudaEventCreate(out(fresh->t0[c])));
+            SMVP_CUDA(cudaEventCreate(out(fresh->t1[c])));
         }
-        A->pipe_res = fresh;
+        A->pipe_res = std::move(fresh);
     }
-    PipeResources &R = *static_cast<PipeResources *>(A->pipe_res);
+    const PipeResources &R = *A->pipe_res;
+    cudaError_t e = cudaSuccess;
     // the part of x this matrix reads: [xlo, xhi).  Entries outside it are never gathered, so they are not uploaded
     const int NR = A->pipe_ranges;
     const int64_t xlo = A->pipe_xlo, xhi = NR > 0 ? A->pipe_xneed[NR - 1] : 0;
@@ -1610,7 +1545,7 @@ static int csr_mult_pipelined(smvp_csr *A, const double *x_host, double *y_host,
         int64_t at = xlo + (((int64_t)((double)xlen * xf[k]) + 63) / 64) * 64;
         xb[k] = (k == NX || at > xhi) ? xhi : at;
     }
-    cudaStream_t cs = R.compute;
+    cudaStream_t cs = R.compute.get();
     // first failing runtime call of the pass; later calls are skipped, the streams are still drained below
 #define PIPE_CK(expr)            \
     do                           \
@@ -1619,22 +1554,23 @@ static int csr_mult_pipelined(smvp_csr *A, const double *x_host, double *y_host,
             e = (expr);          \
     } while (0)
     // everything queued on the legacy stream before the call (the zero-fill of y, an earlier pass) comes first
-    PIPE_CK(cudaEventRecord(R.begin, 0));
-    PIPE_CK(cudaStreamWaitEvent(cs, R.begin, 0));
-    PIPE_CK(cudaStreamWaitEvent(R.up, R.begin, 0));
-    PIPE_CK(cudaStreamWaitEvent(R.down, R.begin, 0));
+    PIPE_CK(cudaEventRecord(R.begin.get(), 0));
+    PIPE_CK(cudaStreamWaitEvent(cs, R.begin.get(), 0));
+    PIPE_CK(cudaStreamWaitEvent(R.up.get(), R.begin.get(), 0));
+    PIPE_CK(cudaStreamWaitEvent(R.down.get(), R.begin.get(), 0));
     if (x_host)
     {
         for (int k = 0; k < NX; k++)
         {
             const int64_t a = xb[k], b = xb[k + 1];
             if (b > a)
-                PIPE_CK(cudaMemcpyAsync(A->d_x + a, x_host + a, sizeof(double) * (size_t)(b - a), cudaMemcpyHostToDevice, R.up));
-            PIPE_CK(cudaEventRecord(R.x_ready[k], R.up));
+                PIPE_CK(cudaMemcpyAsync(A->d_x.get() + a, x_host + a, sizeof(double) * (size_t)(b - a), cudaMemcpyHostToDevice,
+                                        R.up.get()));
+            PIPE_CK(cudaEventRecord(R.x_ready[k].get(), R.up.get()));
         }
     }
     int rc = SMVP_OK;
-    const double *xm = A->relabel_state == 1 ? A->x_rel : A->d_x; // callers upload under the pass only without relabelling
+    const double *xm = A->relabel_state == 1 ? A->x_rel.get() : A->d_x.get(); // callers upload under the pass only without relabelling
     int waited = -1; // last upload piece the compute stream already waits for
     for (int c = 0; c < NR && rc == SMVP_OK && e == cudaSuccess; c++)
     {
@@ -1645,30 +1581,31 @@ static int csr_mult_pipelined(smvp_csr *A, const double *x_host, double *y_host,
                 k++;
             if (k > waited) // the pieces complete in order on one stream: piece k's event covers every earlier one
             {
-                PIPE_CK(cudaStreamWaitEvent(cs, R.x_ready[k], 0));
+                PIPE_CK(cudaStreamWaitEvent(cs, R.x_ready[k].get(), 0));
                 waited = k;
             }
         }
-        PIPE_CK(cudaEventRecord(R.t0[c], cs));
+        PIPE_CK(cudaEventRecord(R.t0[c].get(), cs));
         if (A->pipe_tile[c + 1] > A->pipe_tile[c] && e == cudaSuccess)
             rc = A->pattern_state == 1
-                     ? csr_mult_pattern(A, xm, A->d_y, nullptr, AXPBY_PLAIN, cs, A->pipe_row[c], A->pipe_row[c + 1])
-                     : csr_mult_merge(A, xm, A->d_y, nullptr, AXPBY_PLAIN, cs, A->pipe_tile[c], A->pipe_tile[c + 1]);
-        PIPE_CK(cudaEventRecord(R.t1[c], cs));
+                     ? csr_mult_pattern(A, xm, A->d_y.get(), nullptr, AXPBY_PLAIN, cs, A->pipe_row[c], A->pipe_row[c + 1])
+                     : csr_mult_merge(A, xm, A->d_y.get(), nullptr, AXPBY_PLAIN, cs, A->pipe_tile[c], A->pipe_tile[c + 1]);
+        PIPE_CK(cudaEventRecord(R.t1[c].get(), cs));
         if (y_host)
         {
-            PIPE_CK(cudaEventRecord(R.done[c], cs));
-            PIPE_CK(cudaStreamWaitEvent(R.down, R.done[c], 0));
+            PIPE_CK(cudaEventRecord(R.done[c].get(), cs));
+            PIPE_CK(cudaStreamWaitEvent(R.down.get(), R.done[c].get(), 0));
             const int32_t r0 = A->pipe_row[c], r1 = A->pipe_row[c + 1];
             if (r1 > r0)
-                PIPE_CK(cudaMemcpyAsync(y_host + r0, A->d_y + r0, sizeof(double) * (size_t)(r1 - r0), cudaMemcpyDeviceToHost, R.down));
-            PIPE_CK(cudaEventRecord(R.down_done[c], R.down));
+                PIPE_CK(cudaMemcpyAsync(y_host + r0, A->d_y.get() + r0, sizeof(double) * (size_t)(r1 - r0), cudaMemcpyDeviceToHost,
+                                        R.down.get()));
+            PIPE_CK(cudaEventRecord(R.down_done[c].get(), R.down.get()));
         }
     }
     // drain every stream of the pass, also after a failure (nothing may still touch the caller's buffers on return)
     cudaError_t es = cudaStreamSynchronize(cs);
     // the upload stream too: a matrix may read less than all of x
-    const cudaError_t eu = cudaStreamSynchronize(R.up), ed = cudaStreamSynchronize(R.down);
+    const cudaError_t eu = cudaStreamSynchronize(R.up.get()), ed = cudaStreamSynchronize(R.down.get());
     if (es == cudaSuccess)
         es = eu != cudaSuccess ? eu : ed;
 #undef PIPE_CK
@@ -1682,7 +1619,7 @@ static int csr_mult_pipelined(smvp_csr *A, const double *x_host, double *y_host,
     for (int c = 0; c < NR; c++)
     {
         float t = 0.f;
-        cudaEventElapsedTime(&t, R.t0[c], R.t1[c]);
+        cudaEventElapsedTime(&t, R.t0[c].get(), R.t1[c].get());
         total += t;
     }
     *ms = total;
@@ -1690,16 +1627,17 @@ static int csr_mult_pipelined(smvp_csr *A, const double *x_host, double *y_host,
     {
         auto at = [&](cudaEvent_t ev) {
             float t = 0.f;
-            cudaEventElapsedTime(&t, R.begin, ev);
+            cudaEventElapsedTime(&t, R.begin.get(), ev);
             return t;
         };
         fprintf(stderr, "[pipe] %d ranges, %d x pieces (first %lld, largest %lld entries): ", NR, NX, (long long)(xb[1] - xb[0]),
                 (long long)(NX > 4 ? xb[NX / 2 + 1] - xb[NX / 2] : xb[1] - xb[0]));
         if (x_host)
-            fprintf(stderr, "x piece 0 at %.3f, last x piece at %.3f | ", at(R.x_ready[0]), at(R.x_ready[NX - 1]));
-        fprintf(stderr, "range 0 computed at %.3f, last range at %.3f", at(R.t1[0]), at(R.t1[NR - 1]));
+            fprintf(stderr, "x piece 0 at %.3f, last x piece at %.3f | ", at(R.x_ready[0].get()), at(R.x_ready[NX - 1].get()));
+        fprintf(stderr, "range 0 computed at %.3f, last range at %.3f", at(R.t1[0].get()), at(R.t1[NR - 1].get()));
         if (y_host)
-            fprintf(stderr, " | first rows down at %.3f, last rows down at %.3f", at(R.down_done[0]), at(R.down_done[NR - 1]));
+            fprintf(stderr, " | first rows down at %.3f, last rows down at %.3f", at(R.down_done[0].get()),
+                    at(R.down_done[NR - 1].get()));
         fprintf(stderr, " ms\n");
     }
     SMVP_CUDA(cudaGetLastError());
@@ -1713,9 +1651,9 @@ extern "C" int smvp_csr_mult(smvp_csr *A, const double *x_host, double *y_host, 
     if (variant != SMVP_CSR_AUTO && variant != SMVP_CSR_VECTOR && variant != SMVP_CSR_MERGE)
         return SMVP_E_ARG;
     if (!A->d_x)
-        SMVP_CUDA(dev_alloc(&A->d_x, A->cols));
+        SMVP_CUDA(dev_alloc(A->d_x, A->cols));
     if (!A->d_y)
-        SMVP_CUDA(dev_alloc(&A->d_y, A->rows));
+        SMVP_CUDA(dev_alloc(A->d_y, A->rows));
     const bool merge = csr_resolve_variant(A, variant) == SMVP_CSR_MERGE && A->rows > 0;
     // big vectors: pipeline their PCIe transfers with the first / last pass (SMVP_NO_OVERLAP=1: plain copies).
     // Only from page-locked buffers (smvp_host_alloc, cudaHostAlloc, torch pin_memory): an asynchronous copy from or to
@@ -1746,15 +1684,15 @@ extern "C" int smvp_csr_mult(smvp_csr *A, const double *x_host, double *y_host, 
     const bool relabeled = A->relabel_state == 1;
     const bool upload_under_pass = pipelined && !relabeled; // a relabelled x has to be complete before it is permuted
     if (A->cols > 0 && !upload_under_pass)
-        SMVP_CUDA(cudaMemcpy(A->d_x, x_host, sizeof(double) * (size_t)A->cols, cudaMemcpyHostToDevice));
+        SMVP_CUDA(cudaMemcpy(A->d_x.get(), x_host, sizeof(double) * (size_t)A->cols, cudaMemcpyHostToDevice));
     if (relabeled) // once, before the loop, as the reference permutes x for TJDS (main-cli.c:907-923)
-        SMVP_TRY(csr_relabel_x(A, A->d_x, 0));
-    const double *xm = relabeled ? A->x_rel : A->d_x;
+        SMVP_TRY(csr_relabel_x(A, A->d_x.get(), 0));
+    const double *xm = relabeled ? A->x_rel.get() : A->d_x.get();
     bool y_copied = false;
     // y is zero-filled outside the timed passes (main-cli.c:405); both kernels write every row, the fill only keeps
     // the reference's structure observable
     if (A->rows > 0)
-        SMVP_CUDA(cudaMemsetAsync(A->d_y, 0, sizeof(double) * (size_t)A->rows, 0));
+        SMVP_CUDA(cudaMemsetAsync(A->d_y.get(), 0, sizeof(double) * (size_t)A->rows, 0));
     if (!pipelined)
     {
         // small matrices: a pass is shorter than a launch + synchronisation, so the loop runs batched in CUDA graphs
@@ -1767,8 +1705,8 @@ extern "C" int smvp_csr_mult(smvp_csr *A, const double *x_host, double *y_host, 
             multi = [&](cudaStream_t s, int n) {
                 const double mean = A->rows > 0 ? (double)A->nnz / A->rows : 0.0;
 #define SMVP_TINY(L)                                                                                                              \
-    SMVP_LAUNCH(csr_tiny_loop_kernel<L>, 1, TINY_THREADS, 0, s, (const int32_t *)A->row_ptr, mult_cols(A), (const double *)A->val, xm, \
-                A->d_y, A->rows, n)
+    SMVP_LAUNCH(csr_tiny_loop_kernel<L>, 1, TINY_THREADS, 0, s, (const int32_t *)A->row_ptr.get(), mult_cols(A),                   \
+                (const double *)A->val.get(), xm, A->d_y.get(), A->rows, n)
                 if (mean <= 4.5)
                     SMVP_TINY(4);
                 else if (mean <= 9.0)
@@ -1782,56 +1720,43 @@ extern "C" int smvp_csr_mult(smvp_csr *A, const double *x_host, double *y_host, 
                 return (int)SMVP_OK;
             };
         if (A->rows > 0)
-            rc = timed_loop(iters, ms_each, small, [&](cudaStream_t s) { return csr_mult_launch(A, xm, A->d_y, nullptr, AXPBY_PLAIN, variant, s); },
-                            multi);
+            rc = timed_loop(
+                iters, ms_each, small,
+                [&](cudaStream_t s) { return csr_mult_launch(A, xm, A->d_y.get(), nullptr, AXPBY_PLAIN, variant, s); }, multi);
         else if (ms_each)
             for (int it = 0; it < iters; it++)
                 ms_each[it] = 0.0;
     }
     else
     {
-        cudaEvent_t e0, e1;
-        SMVP_CUDA(cudaEventCreate(&e0));
-        cudaError_t ce = cudaEventCreate(&e1);
-        if (ce != cudaSuccess)
-        {
-            cudaEventDestroy(e0);
-            return cuda_fail(ce, "cudaEventCreate", __FILE__, __LINE__);
-        }
-        for (int it = 0; it < iters && rc == SMVP_OK; it++)
+        Event e0, e1;
+        SMVP_CUDA(cudaEventCreate(out(e0)));
+        SMVP_CUDA(cudaEventCreate(out(e1)));
+        for (int it = 0; it < iters; it++)
         {
             float ms = 0.f;
             const bool first = it == 0, last = it == iters - 1;
             if ((first && upload_under_pass) || last)
             {
-                rc = csr_mult_pipelined(A, (first && upload_under_pass) ? x_host : nullptr, last ? y_host : nullptr, &ms);
-                y_copied = last && rc == SMVP_OK;
+                SMVP_TRY(csr_mult_pipelined(A, (first && upload_under_pass) ? x_host : nullptr, last ? y_host : nullptr, &ms));
+                y_copied = last;
             }
             else
             {
-                cudaEventRecord(e0, 0);
-                rc = csr_mult_launch(A, xm, A->d_y, nullptr, AXPBY_PLAIN, variant, 0);
-                cudaEventRecord(e1, 0);
-                if (rc != SMVP_OK)
-                    break;
-                const cudaError_t e = cudaEventSynchronize(e1);
-                if (e != cudaSuccess)
-                {
-                    rc = cuda_fail(e, "cudaEventSynchronize", __FILE__, __LINE__);
-                    break;
-                }
-                cudaEventElapsedTime(&ms, e0, e1);
+                cudaEventRecord(e0.get(), 0);
+                SMVP_TRY(csr_mult_launch(A, xm, A->d_y.get(), nullptr, AXPBY_PLAIN, variant, 0));
+                cudaEventRecord(e1.get(), 0);
+                SMVP_CUDA(cudaEventSynchronize(e1.get()));
+                cudaEventElapsedTime(&ms, e0.get(), e1.get());
             }
-            if (ms_each && rc == SMVP_OK)
+            if (ms_each)
                 ms_each[it] = (double)ms;
         }
-        cudaEventDestroy(e0);
-        cudaEventDestroy(e1);
     }
     if (rc != SMVP_OK)
         return rc;
     if (A->rows > 0 && !y_copied)
-        SMVP_CUDA(cudaMemcpy(y_host, A->d_y, sizeof(double) * (size_t)A->rows, cudaMemcpyDeviceToHost));
+        SMVP_CUDA(cudaMemcpy(y_host, A->d_y.get(), sizeof(double) * (size_t)A->rows, cudaMemcpyDeviceToHost));
     return SMVP_OK;
 }
 

@@ -56,20 +56,18 @@ __global__ void __launch_bounds__(DOT_THREADS) dot_reduce_kernel(const double *_
 }
 
 // layout: [0, units) partials | [units, units + ctas) CTA sums | counter in the last double
-int dot_scratch(double **buf, int64_t *cap, int64_t *device_bytes, int64_t units, cudaStream_t s)
+int dot_scratch(DevPtr<double> *buf, int64_t *cap, int64_t *device_bytes, int64_t units, cudaStream_t s)
 {
     const int64_t need = units + dot_ctas(units) + 1;
     if (*buf && *cap >= need)
         return SMVP_OK;
     SMVP_CUDA(cudaStreamSynchronize(s)); // an earlier dot pass on this handle may still use the old scratch
-    cudaFree(*buf);
-    *buf = nullptr;
-    *device_bytes -= 8 * *cap;
-    *cap = 0;
-    SMVP_CUDA(dev_alloc(buf, need));
-    SMVP_CUDA(cudaMemsetAsync(*buf, 0, sizeof(double) * (size_t)need, s));
+    DevPtr<double> grown;
+    SMVP_CUDA(dev_alloc(grown, need));
+    SMVP_CUDA(cudaMemsetAsync(grown.get(), 0, sizeof(double) * (size_t)need, s));
+    *buf = std::move(grown);
+    *device_bytes += 8 * (need - *cap);
     *cap = need;
-    *device_bytes += 8 * need;
     return SMVP_OK;
 }
 

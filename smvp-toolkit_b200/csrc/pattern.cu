@@ -171,50 +171,35 @@ __global__ void __launch_bounds__(256) pattern_narrow_kernel(const double *__res
         out[j] = narrow_value<V>(val[j]);
 }
 
-// the narrowest width (2, 4 or 8 bytes) that holds every value exactly, and the copy of val at that width
-static int pattern_values(smvp_csr *A, unsigned grid, cudaStream_t s)
+// the narrowest width (2, 4 or 8 bytes) that holds every value exactly, and the copy of val at that width (none at 8)
+static int pattern_values(const smvp_csr *A, unsigned grid, cudaStream_t s, int32_t *vbytes, DevPtr<char> *narrow)
 {
-    DevTmp g_flags;
-    SMVP_CUDA(g_flags.alloc<int32_t>(1));
-    int32_t *flags = g_flags.as<int32_t>(), h_flags = 0;
-    SMVP_CUDA(cudaMemsetAsync(flags, 0, sizeof(int32_t), s));
+    DevPtr<int32_t> flags;
+    SMVP_CUDA(dev_alloc(flags, 1));
+    int32_t h_flags = 0;
+    SMVP_CUDA(cudaMemsetAsync(flags.get(), 0, sizeof(int32_t), s));
     if (A->nnz > 0)
-        SMVP_LAUNCH(pattern_width_kernel, grid, 256, 0, s, (const double *)A->val, A->nnz, flags);
+        SMVP_LAUNCH(pattern_width_kernel, grid, 256, 0, s, (const double *)A->val.get(), A->nnz, flags.get());
     SMVP_CUDA(cudaGetLastError());
-    SMVP_CUDA(cudaMemcpyAsync(&h_flags, flags, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    SMVP_CUDA(cudaMemcpyAsync(&h_flags, flags.get(), sizeof(int32_t), cudaMemcpyDeviceToHost, s));
     SMVP_CUDA(cudaStreamSynchronize(s));
-    const int32_t vbytes = !(h_flags & 1) ? 2 : !(h_flags & 2) ? 4 : 8;
-    if (vbytes == 2)
-    {
-        SMVP_CUDA(dev_alloc((uint16_t **)&A->pat_val, A->nnz));
-        if (A->nnz > 0)
-            SMVP_LAUNCH(pattern_narrow_kernel<uint16_t>, grid, 256, 0, s, (const double *)A->val, A->nnz, (uint16_t *)A->pat_val);
-    }
-    else if (vbytes == 4)
-    {
-        SMVP_CUDA(dev_alloc((float **)&A->pat_val, A->nnz));
-        if (A->nnz > 0)
-            SMVP_LAUNCH(pattern_narrow_kernel<float>, grid, 256, 0, s, (const double *)A->val, A->nnz, (float *)A->pat_val);
-    }
+    const int32_t vb = !(h_flags & 1) ? 2 : !(h_flags & 2) ? 4 : 8;
+    DevPtr<char> copy;
+    if (vb < 8)
+        SMVP_CUDA(dev_alloc(copy, vb * A->nnz));
+    if (vb == 2 && A->nnz > 0)
+        SMVP_LAUNCH(pattern_narrow_kernel<uint16_t>, grid, 256, 0, s, (const double *)A->val.get(), A->nnz, (uint16_t *)copy.get());
+    else if (vb == 4 && A->nnz > 0)
+        SMVP_LAUNCH(pattern_narrow_kernel<float>, grid, 256, 0, s, (const double *)A->val.get(), A->nnz, (float *)copy.get());
     SMVP_CUDA(cudaGetLastError());
     SMVP_CUDA(cudaStreamSynchronize(s));
-    A->pat_vbytes = vbytes;
+    *vbytes = vb;
+    *narrow = std::move(copy);
     return SMVP_OK;
 }
 
-void csr_pattern_release(smvp_csr *A)
-{
-    cudaFree(A->pat_id);
-    cudaFree(A->pat_off);
-    cudaFree(A->pat_len);
-    cudaFree(A->pat_val);
-    A->pat_id = nullptr;
-    A->pat_off = A->pat_len = nullptr;
-    A->pat_val = nullptr;
-    A->pat_vbytes = 0;
-}
-
 // decides (once per handle) and, when every row matches one of at most PAT_MAX patterns, builds the plan.  Synchronous.
+// A failure leaves the plan undecided: the next pass tries again.
 int csr_pattern_plan(smvp_csr *A, cudaStream_t s)
 {
     SMVP_TRY(csr_relabel_plan(A, s)); // a relabelled handle reads col_rel: that plan decides first
@@ -225,27 +210,27 @@ int csr_pattern_plan(smvp_csr *A, cudaStream_t s)
         A->pattern_state = -1;
         return SMVP_OK;
     }
-    DevTmp g_keys, g_rep, g_flags, g_slot_id, g_reps;
-    SMVP_CUDA(g_keys.alloc<unsigned long long>(PAT_SLOTS));
-    SMVP_CUDA(g_rep.alloc<int32_t>(PAT_SLOTS));
-    SMVP_CUDA(g_flags.alloc<int32_t>(2)); // [0] flags, [1] patterns inserted
-    SMVP_CUDA(g_slot_id.alloc<int32_t>(PAT_SLOTS));
-    SMVP_CUDA(g_reps.alloc<int32_t>(PAT_MAX));
-    unsigned long long *keys = g_keys.as<unsigned long long>();
-    int32_t *rep = g_rep.as<int32_t>(), *flags = g_flags.as<int32_t>();
-    SMVP_CUDA(cudaMemsetAsync(keys, 0, sizeof(unsigned long long) * PAT_SLOTS, s));
-    SMVP_CUDA(cudaMemsetAsync(rep, 0x7f, sizeof(int32_t) * PAT_SLOTS, s));
-    SMVP_CUDA(cudaMemsetAsync(flags, 0, 2 * sizeof(int32_t), s));
+    DevPtr<unsigned long long> keys;
+    DevPtr<int32_t> rep, flags, slot_id, reps;
+    SMVP_CUDA(dev_alloc(keys, PAT_SLOTS));
+    SMVP_CUDA(dev_alloc(rep, PAT_SLOTS));
+    SMVP_CUDA(dev_alloc(flags, 2)); // [0] flags, [1] patterns inserted
+    SMVP_CUDA(dev_alloc(slot_id, PAT_SLOTS));
+    SMVP_CUDA(dev_alloc(reps, PAT_MAX));
+    SMVP_CUDA(cudaMemsetAsync(keys.get(), 0, sizeof(unsigned long long) * PAT_SLOTS, s));
+    SMVP_CUDA(cudaMemsetAsync(rep.get(), 0x7f, sizeof(int32_t) * PAT_SLOTS, s));
+    SMVP_CUDA(cudaMemsetAsync(flags.get(), 0, 2 * sizeof(int32_t), s));
     const int64_t blocks = ceil_div64(A->rows, 256), cap = (int64_t)device_props().sms * 8;
     const unsigned grid = (unsigned)(blocks < cap ? blocks : cap);
-    SMVP_LAUNCH(pattern_hash_kernel, grid, 256, 0, s, A->row_ptr, A->col_ind, A->rows, keys, rep, flags + 1, flags);
+    SMVP_LAUNCH(pattern_hash_kernel, grid, 256, 0, s, A->row_ptr.get(), A->col_ind.get(), A->rows, keys.get(), rep.get(),
+                flags.get() + 1, flags.get());
     SMVP_CUDA(cudaGetLastError());
     std::vector<unsigned long long> h_keys(PAT_SLOTS);
     std::vector<int32_t> h_rep(PAT_SLOTS);
     int32_t h_flags[2] = {0, 0};
-    SMVP_CUDA(cudaMemcpyAsync(h_flags, flags, sizeof(h_flags), cudaMemcpyDeviceToHost, s));
-    SMVP_CUDA(cudaMemcpyAsync(h_keys.data(), keys, sizeof(unsigned long long) * PAT_SLOTS, cudaMemcpyDeviceToHost, s));
-    SMVP_CUDA(cudaMemcpyAsync(h_rep.data(), rep, sizeof(int32_t) * PAT_SLOTS, cudaMemcpyDeviceToHost, s));
+    SMVP_CUDA(cudaMemcpyAsync(h_flags, flags.get(), sizeof(h_flags), cudaMemcpyDeviceToHost, s));
+    SMVP_CUDA(cudaMemcpyAsync(h_keys.data(), keys.get(), sizeof(unsigned long long) * PAT_SLOTS, cudaMemcpyDeviceToHost, s));
+    SMVP_CUDA(cudaMemcpyAsync(h_rep.data(), rep.get(), sizeof(int32_t) * PAT_SLOTS, cudaMemcpyDeviceToHost, s));
     SMVP_CUDA(cudaStreamSynchronize(s));
     if (h_flags[0])
     {
@@ -265,39 +250,38 @@ int csr_pattern_plan(smvp_csr *A, cudaStream_t s)
         h_slot_id[by_rep[p].second] = p;
         h_reps[p] = by_rep[p].first;
     }
-    auto body = [&]() -> int {
-        SMVP_CUDA(dev_alloc(&A->pat_id, A->rows));
-        SMVP_CUDA(dev_alloc(&A->pat_off, (int64_t)npat * PAT_LMAX));
-        SMVP_CUDA(dev_alloc(&A->pat_len, npat));
-        SMVP_CUDA(cudaMemcpyAsync(g_slot_id.p, h_slot_id.data(), sizeof(int32_t) * PAT_SLOTS, cudaMemcpyHostToDevice, s));
-        SMVP_CUDA(cudaMemcpyAsync(g_reps.p, h_reps.data(), sizeof(int32_t) * npat, cudaMemcpyHostToDevice, s));
-        SMVP_LAUNCH(pattern_table_kernel, (unsigned)npat, PAT_LMAX, 0, s, A->row_ptr, A->col_ind, g_reps.as<int32_t>(), npat,
-                    A->pat_off, A->pat_len);
-        SMVP_LAUNCH(pattern_assign_kernel, grid, 256, 0, s, A->row_ptr, A->col_ind, A->rows, keys, g_slot_id.as<int32_t>(),
-                    A->pat_off, A->pat_len, A->pat_id, flags);
-        SMVP_CUDA(cudaGetLastError());
-        std::vector<int32_t> h_len(npat);
-        SMVP_CUDA(cudaMemcpyAsync(h_flags, flags, sizeof(h_flags), cudaMemcpyDeviceToHost, s));
-        SMVP_CUDA(cudaMemcpyAsync(h_len.data(), A->pat_len, sizeof(int32_t) * npat, cudaMemcpyDeviceToHost, s));
-        SMVP_CUDA(cudaStreamSynchronize(s));
-        A->pattern_maxlen = npat > 0 ? *std::max_element(h_len.begin(), h_len.end()) : 0;
+    DevPtr<uint8_t> pat_id;
+    DevPtr<int32_t> pat_off, pat_len;
+    SMVP_CUDA(dev_alloc(pat_id, A->rows));
+    SMVP_CUDA(dev_alloc(pat_off, (int64_t)npat * PAT_LMAX));
+    SMVP_CUDA(dev_alloc(pat_len, npat));
+    SMVP_CUDA(cudaMemcpyAsync(slot_id.get(), h_slot_id.data(), sizeof(int32_t) * PAT_SLOTS, cudaMemcpyHostToDevice, s));
+    SMVP_CUDA(cudaMemcpyAsync(reps.get(), h_reps.data(), sizeof(int32_t) * npat, cudaMemcpyHostToDevice, s));
+    SMVP_LAUNCH(pattern_table_kernel, (unsigned)npat, PAT_LMAX, 0, s, A->row_ptr.get(), A->col_ind.get(), reps.get(), npat,
+                pat_off.get(), pat_len.get());
+    SMVP_LAUNCH(pattern_assign_kernel, grid, 256, 0, s, A->row_ptr.get(), A->col_ind.get(), A->rows, keys.get(), slot_id.get(),
+                pat_off.get(), pat_len.get(), pat_id.get(), flags.get());
+    SMVP_CUDA(cudaGetLastError());
+    std::vector<int32_t> h_len(npat);
+    SMVP_CUDA(cudaMemcpyAsync(h_flags, flags.get(), sizeof(h_flags), cudaMemcpyDeviceToHost, s));
+    SMVP_CUDA(cudaMemcpyAsync(h_len.data(), pat_len.get(), sizeof(int32_t) * npat, cudaMemcpyDeviceToHost, s));
+    SMVP_CUDA(cudaStreamSynchronize(s));
+    if (h_flags[0])
+    {
+        A->pattern_state = -1;
         return SMVP_OK;
-    };
-    const int rc = body();
-    if (rc != SMVP_OK || h_flags[0])
-    {
-        csr_pattern_release(A);
-        A->pattern_state = rc == SMVP_OK ? -1 : 0;
-        return rc;
     }
-    const int rv = pattern_values(A, grid, s);
-    if (rv != SMVP_OK)
-    {
-        csr_pattern_release(A);
-        return rv; // undecided: the next pass tries again
-    }
+    int32_t vbytes = 0;
+    DevPtr<char> narrow;
+    SMVP_TRY(pattern_values(A, grid, s, &vbytes, &narrow));
+    A->pat_id = std::move(pat_id);
+    A->pat_off = std::move(pat_off);
+    A->pat_len = std::move(pat_len);
+    A->pat_val = std::move(narrow);
+    A->pat_vbytes = vbytes;
     A->pattern_count = npat;
-    A->device_bytes += (int64_t)A->rows + 4 * (int64_t)npat * (PAT_LMAX + 1) + (A->pat_vbytes < 8 ? A->pat_vbytes * A->nnz : 0);
+    A->pattern_maxlen = npat > 0 ? *std::max_element(h_len.begin(), h_len.end()) : 0;
+    A->device_bytes += (int64_t)A->rows + 4 * (int64_t)npat * (PAT_LMAX + 1) + (vbytes < 8 ? vbytes * A->nnz : 0);
     A->pattern_state = 1;
     return SMVP_OK;
 }

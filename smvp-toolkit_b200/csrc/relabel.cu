@@ -111,90 +111,66 @@ __global__ void __launch_bounds__(256) relabel_permute_x_kernel(const double *__
 
 // Popularity order of an index space: d_idx[nnz] holds indices in [0, n).  forced > 0 builds the order whatever the
 // distribution; forced == 0 builds it only when the index space is large and skewed enough (see the header).
-// On success with *use = 1: (*d_order)[p] = index with rank p, (*d_rank)[i] = rank of index i (caller frees both).
+// When it is built: (*d_order)[p] = index with rank p, (*d_rank)[i] = rank of index i; both stay empty otherwise.
 // Synchronous.
-int popularity_plan(const int32_t *d_idx, int64_t nnz, int32_t n, int forced, double min_ratio, int32_t **d_order, int32_t **d_rank,
-                    int *use, cudaStream_t s)
+int popularity_plan(const int32_t *d_idx, int64_t nnz, int32_t n, int forced, double min_ratio, DevPtr<int32_t> *d_order,
+                    DevPtr<int32_t> *d_rank, cudaStream_t s)
 {
-    *use = 0;
-    *d_order = *d_rank = nullptr;
     if (forced < 0 || nnz == 0 || n == 0 || (forced == 0 && n < relabel_min_cols()))
         return SMVP_OK;
-    uint32_t *count = nullptr, *d_max = nullptr, *key_a = nullptr, *key_b = nullptr, *idx_a = nullptr, *idx_b = nullptr;
-    unsigned long long *d_cover = nullptr;
-    int32_t *order = nullptr, *rank = nullptr;
-    auto cleanup = [&]() {
-        cudaFree(count);
-        cudaFree(d_max);
-        cudaFree(key_a);
-        cudaFree(key_b);
-        cudaFree(idx_a);
-        cudaFree(idx_b);
-        cudaFree(d_cover);
-    };
-    auto body = [&]() -> int {
-        const unsigned cblocks = (unsigned)ceil_div64(n, 256);
-        SMVP_CUDA(dev_alloc(&count, (int64_t)n + 1));
-        SMVP_CUDA(dev_alloc(&d_max, 1));
-        SMVP_CUDA(dev_alloc(&d_cover, 1));
-        SMVP_CUDA(dev_alloc(&key_a, n));
-        SMVP_CUDA(dev_alloc(&key_b, n));
-        SMVP_CUDA(dev_alloc(&idx_a, n));
-        SMVP_CUDA(dev_alloc(&idx_b, n));
-        SMVP_TRY(histogram_i32(d_idx, nnz, count, (int64_t)n + 1, s));
-        SMVP_TRY(max_u32(count, n, d_max, s));
-        uint32_t maxc = 0;
-        SMVP_CUDA(cudaMemcpyAsync(&maxc, d_max, sizeof(maxc), cudaMemcpyDeviceToHost, s));
-        SMVP_CUDA(cudaStreamSynchronize(s));
-        SMVP_LAUNCH(relabel_key_kernel, cblocks, 256, 0, s, (const uint32_t *)count, n, maxc, key_a, idx_a);
-        uint32_t *rk = nullptr, *ri = nullptr;
-        const int lo = 0, hi = bits_for(maxc + 1u);
-        SMVP_TRY(radix_sort_pairs<uint32_t>(key_a, idx_a, key_b, idx_b, n, &lo, &hi, 1, &rk, &ri, s));
-        if (forced == 0)
-        {
-            // The test runs over the indices the handle actually TOUCHES, not over the whole index space: a row block
-            // of a banded matrix (the shard of one GPU out of 8) reads a 1/8 window of x, and measured against all n
-            // columns that window looked like a hot set holding every nonzero (round-1 misfire at 8 GPUs).
-            int32_t touched = 0;
-            SMVP_LAUNCH(relabel_touched_kernel, 1, 1, 0, s, (const uint32_t *)rk, n, maxc, (int32_t *)d_max);
-            SMVP_CUDA(cudaMemcpyAsync(&touched, d_max, sizeof(touched), cudaMemcpyDeviceToHost, s));
-            SMVP_CUDA(cudaStreamSynchronize(s));
-            if (touched < relabel_min_cols())
-                return SMVP_OK; // what is gathered fits L2 next to the streams
-            const int32_t k = (int32_t)(touched < relabel_hot_cols() ? touched : relabel_hot_cols());
-            SMVP_CUDA(cudaMemsetAsync(d_cover, 0, sizeof(unsigned long long), s));
-            SMVP_LAUNCH(relabel_cover_kernel, (unsigned)device_props().sms * 8, 256, 0, s, (const uint32_t *)rk, k, maxc, d_cover);
-            unsigned long long cover = 0;
-            SMVP_CUDA(cudaMemcpyAsync(&cover, d_cover, sizeof(cover), cudaMemcpyDeviceToHost, s));
-            SMVP_CUDA(cudaStreamSynchronize(s));
-            const double share = (double)cover / (double)nnz, fair = (double)k / (double)touched;
-            // skewed enough: the hot set holds most of the gathers AND at least twice what a flat distribution over the
-            // touched columns would give it (a banded block is exactly flat: share == fair)
-            // (min_ratio: 2 for the CSR gathers; 4 for the TJDS scatter, where the plan gains 5 % on the whole R-MAT
-            // matrix and LOSES 20 % on the column block of one GPU out of 8 -- profiles/r02_logs/r02_bench_n8_final.json
-            // before / after -- so only a pronounced skew selects it)
-            if (!(share >= 0.5 && share >= min_ratio * fair))
-                return SMVP_OK;
-        }
-        SMVP_CUDA(dev_alloc(&order, n));
-        SMVP_CUDA(dev_alloc(&rank, n));
-        SMVP_LAUNCH(relabel_rank_kernel, cblocks, 256, 0, s, (const uint32_t *)ri, n, order, rank);
-        SMVP_CUDA(cudaStreamSynchronize(s));
-        SMVP_CUDA(cudaGetLastError());
-        *use = 1;
-        return SMVP_OK;
-    };
-    const int rc = body();
-    cleanup();
-    if (rc != SMVP_OK || !*use)
+    const unsigned cblocks = (unsigned)ceil_div64(n, 256);
+    DevPtr<uint32_t> count, d_max, key_a, key_b, idx_a, idx_b;
+    DevPtr<unsigned long long> d_cover;
+    SMVP_CUDA(dev_alloc(count, (int64_t)n + 1));
+    SMVP_CUDA(dev_alloc(d_max, 1));
+    SMVP_CUDA(dev_alloc(d_cover, 1));
+    SMVP_CUDA(dev_alloc(key_a, n));
+    SMVP_CUDA(dev_alloc(key_b, n));
+    SMVP_CUDA(dev_alloc(idx_a, n));
+    SMVP_CUDA(dev_alloc(idx_b, n));
+    SMVP_TRY(histogram_i32(d_idx, nnz, count.get(), (int64_t)n + 1, s));
+    SMVP_TRY(max_u32(count.get(), n, d_max.get(), s));
+    uint32_t maxc = 0;
+    SMVP_CUDA(cudaMemcpyAsync(&maxc, d_max.get(), sizeof(maxc), cudaMemcpyDeviceToHost, s));
+    SMVP_CUDA(cudaStreamSynchronize(s));
+    SMVP_LAUNCH(relabel_key_kernel, cblocks, 256, 0, s, (const uint32_t *)count.get(), n, maxc, key_a.get(), idx_a.get());
+    uint32_t *rk = nullptr, *ri = nullptr;
+    const int lo = 0, hi = bits_for(maxc + 1u);
+    SMVP_TRY(radix_sort_pairs<uint32_t>(key_a.get(), idx_a.get(), key_b.get(), idx_b.get(), n, &lo, &hi, 1, &rk, &ri, s));
+    if (forced == 0)
     {
-        cudaFree(order);
-        cudaFree(rank);
-        *use = 0;
-        return rc;
+        // The test runs over the indices the handle actually TOUCHES, not over the whole index space: a row block
+        // of a banded matrix (the shard of one GPU out of 8) reads a 1/8 window of x, and measured against all n
+        // columns that window looked like a hot set holding every nonzero (round-1 misfire at 8 GPUs).
+        int32_t touched = 0;
+        SMVP_LAUNCH(relabel_touched_kernel, 1, 1, 0, s, (const uint32_t *)rk, n, maxc, (int32_t *)d_max.get());
+        SMVP_CUDA(cudaMemcpyAsync(&touched, d_max.get(), sizeof(touched), cudaMemcpyDeviceToHost, s));
+        SMVP_CUDA(cudaStreamSynchronize(s));
+        if (touched < relabel_min_cols())
+            return SMVP_OK; // what is gathered fits L2 next to the streams
+        const int32_t k = (int32_t)(touched < relabel_hot_cols() ? touched : relabel_hot_cols());
+        SMVP_CUDA(cudaMemsetAsync(d_cover.get(), 0, sizeof(unsigned long long), s));
+        SMVP_LAUNCH(relabel_cover_kernel, (unsigned)device_props().sms * 8, 256, 0, s, (const uint32_t *)rk, k, maxc, d_cover.get());
+        unsigned long long cover = 0;
+        SMVP_CUDA(cudaMemcpyAsync(&cover, d_cover.get(), sizeof(cover), cudaMemcpyDeviceToHost, s));
+        SMVP_CUDA(cudaStreamSynchronize(s));
+        const double share = (double)cover / (double)nnz, fair = (double)k / (double)touched;
+        // skewed enough: the hot set holds most of the gathers AND at least twice what a flat distribution over the
+        // touched columns would give it (a banded block is exactly flat: share == fair)
+        // (min_ratio: 2 for the CSR gathers; 4 for the TJDS scatter, where the plan gains 5 % on the whole R-MAT
+        // matrix and LOSES 20 % on the column block of one GPU out of 8 -- profiles/r02_logs/r02_bench_n8_final.json
+        // before / after -- so only a pronounced skew selects it)
+        if (!(share >= 0.5 && share >= min_ratio * fair))
+            return SMVP_OK;
     }
-    *d_order = order;
-    *d_rank = rank;
+    DevPtr<int32_t> order, rank;
+    SMVP_CUDA(dev_alloc(order, n));
+    SMVP_CUDA(dev_alloc(rank, n));
+    SMVP_LAUNCH(relabel_rank_kernel, cblocks, 256, 0, s, (const uint32_t *)ri, n, order.get(), rank.get());
+    SMVP_CUDA(cudaStreamSynchronize(s));
+    SMVP_CUDA(cudaGetLastError());
+    *d_order = std::move(order);
+    *d_rank = std::move(rank);
     return SMVP_OK;
 }
 
@@ -216,29 +192,21 @@ int csr_relabel_plan(smvp_csr *A, cudaStream_t s)
 {
     if (A->relabel_state != 0)
         return SMVP_OK;
-    int use = 0;
-    int32_t *order = nullptr, *rank = nullptr;
-    SMVP_TRY(popularity_plan(A->col_ind, A->nnz, A->cols, env_tristate("SMVP_CSR_RELABEL"), 2.0, &order, &rank, &use, s));
-    if (!use)
+    DevPtr<int32_t> order, rank, col_rel;
+    DevPtr<double> x_rel;
+    SMVP_TRY(popularity_plan(A->col_ind.get(), A->nnz, A->cols, env_tristate("SMVP_CSR_RELABEL"), 2.0, &order, &rank, s));
+    if (!rank)
     {
         A->relabel_state = -1;
         return SMVP_OK;
     }
-    A->x_order = order;
-    auto body = [&]() -> int {
-        SMVP_CUDA(dev_alloc(&A->x_rel, A->cols));
-        SMVP_CUDA(dev_alloc(&A->col_rel, A->nnz));
-        SMVP_TRY(relabel_indices(A->col_ind, A->nnz, rank, A->col_rel, s));
-        SMVP_CUDA(cudaStreamSynchronize(s));
-        return SMVP_OK;
-    };
-    const int rc = body();
-    cudaFree(rank);
-    if (rc != SMVP_OK)
-    {
-        csr_relabel_release(A);
-        return rc;
-    }
+    SMVP_CUDA(dev_alloc(x_rel, A->cols));
+    SMVP_CUDA(dev_alloc(col_rel, A->nnz));
+    SMVP_TRY(relabel_indices(A->col_ind.get(), A->nnz, rank.get(), col_rel.get(), s));
+    SMVP_CUDA(cudaStreamSynchronize(s));
+    A->x_order = std::move(order);
+    A->x_rel = std::move(x_rel);
+    A->col_rel = std::move(col_rel);
     A->device_bytes += 4 * A->nnz + 12 * (int64_t)A->cols;
     A->relabel_state = 1;
     return SMVP_OK;
@@ -251,41 +219,25 @@ int tjds_relabel_plan(smvp_tjds *A, cudaStream_t s)
 {
     if (A->relabel_state != 0)
         return SMVP_OK;
-    int use = 0;
-    int32_t *order = nullptr, *rank = nullptr;
-    SMVP_TRY(popularity_plan(A->row_ind, A->nnz, A->rows, env_tristate("SMVP_TJDS_RELABEL"), 4.0, &order, &rank, &use, s));
-    if (!use)
+    DevPtr<int32_t> order, rank, row_rel;
+    DevPtr<double> y_rel;
+    SMVP_TRY(popularity_plan(A->row_ind.get(), A->nnz, A->rows, env_tristate("SMVP_TJDS_RELABEL"), 4.0, &order, &rank, s));
+    if (!rank)
     {
         A->relabel_state = -1;
         return SMVP_OK;
     }
-    cudaFree(order);
-    A->row_rank = rank;
-    auto body = [&]() -> int {
-        SMVP_CUDA(dev_alloc(&A->y_rel, A->rows));
-        SMVP_CUDA(dev_alloc(&A->row_rel, A->nnz));
-        SMVP_TRY(relabel_indices(A->row_ind, A->nnz, rank, A->row_rel, s));
-        SMVP_CUDA(cudaStreamSynchronize(s));
-        return SMVP_OK;
-    };
-    const int rc = body();
-    if (rc != SMVP_OK)
-    {
-        tjds_relabel_release(A);
-        return rc;
-    }
+    order.reset(); // only the ranks are kept
+    SMVP_CUDA(dev_alloc(y_rel, A->rows));
+    SMVP_CUDA(dev_alloc(row_rel, A->nnz));
+    SMVP_TRY(relabel_indices(A->row_ind.get(), A->nnz, rank.get(), row_rel.get(), s));
+    SMVP_CUDA(cudaStreamSynchronize(s));
+    A->row_rank = std::move(rank);
+    A->y_rel = std::move(y_rel);
+    A->row_rel = std::move(row_rel);
     A->device_bytes += 4 * A->nnz + 12 * (int64_t)A->rows;
     A->relabel_state = 1;
     return SMVP_OK;
-}
-
-void tjds_relabel_release(smvp_tjds *A)
-{
-    cudaFree(A->row_rank);
-    cudaFree(A->row_rel);
-    cudaFree(A->y_rel);
-    A->row_rank = A->row_rel = nullptr;
-    A->y_rel = nullptr;
 }
 
 // x_rel = x in rank order (asynchronous on s)
@@ -293,19 +245,10 @@ int csr_relabel_x(smvp_csr *A, const double *d_x, cudaStream_t s)
 {
     int64_t blocks = ceil_div64(A->cols, 256 * 4);
     const int64_t cap = (int64_t)device_props().sms * 8;
-    SMVP_LAUNCH(relabel_permute_x_kernel, (unsigned)(blocks < cap ? blocks : cap), 256, 0, s, d_x, (const int32_t *)A->x_order, A->cols,
-                A->x_rel);
+    SMVP_LAUNCH(relabel_permute_x_kernel, (unsigned)(blocks < cap ? blocks : cap), 256, 0, s, d_x, (const int32_t *)A->x_order.get(),
+                A->cols, A->x_rel.get());
     SMVP_CUDA(cudaGetLastError());
     return SMVP_OK;
-}
-
-void csr_relabel_release(smvp_csr *A)
-{
-    cudaFree(A->x_order);
-    cudaFree(A->x_rel);
-    cudaFree(A->col_rel);
-    A->x_order = A->col_rel = nullptr;
-    A->x_rel = nullptr;
 }
 
 } // namespace smvp

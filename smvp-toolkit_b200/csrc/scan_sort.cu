@@ -141,13 +141,12 @@ int exclusive_scan_u32(const uint32_t *d_in, uint32_t *d_out, int64_t n, uint32_
             SMVP_CUDA(cudaMemsetAsync(d_total, 0, sizeof(uint32_t), s));
         return SMVP_OK;
     }
-    // the grand total needs in[n-1] before an in-place scan overwrites it.  Temporaries live in guards (cudaFree in the
-    // destructor waits for the work that uses them), so a failure half-way leaks nothing.
-    DevTmp last, sums;
+    // the grand total needs in[n-1] before an in-place scan overwrites it
+    DevPtr<uint32_t> last, sums;
     if (d_total)
     {
-        SMVP_CUDA(last.alloc<uint32_t>(1));
-        SMVP_CUDA(cudaMemcpyAsync(last.p, d_in + (n - 1), sizeof(uint32_t), cudaMemcpyDeviceToDevice, s));
+        SMVP_CUDA(dev_alloc(last, 1));
+        SMVP_CUDA(cudaMemcpyAsync(last.get(), d_in + (n - 1), sizeof(uint32_t), cudaMemcpyDeviceToDevice, s));
     }
     const int64_t blocks = ceil_div64(n, SCAN_TILE);
     if (blocks == 1)
@@ -156,14 +155,14 @@ int exclusive_scan_u32(const uint32_t *d_in, uint32_t *d_out, int64_t n, uint32_
     }
     else
     {
-        SMVP_CUDA(sums.alloc<uint32_t>(blocks));
-        uint32_t *d_sums = sums.as<uint32_t>();
+        SMVP_CUDA(dev_alloc(sums, blocks));
+        uint32_t *d_sums = sums.get();
         SMVP_LAUNCH(scan_reduce_kernel, (unsigned)blocks, SCAN_THREADS, 0, s, d_in, n, d_sums);
         SMVP_TRY(exclusive_scan_u32(d_sums, d_sums, blocks, nullptr, s));
         SMVP_LAUNCH(scan_apply_kernel, (unsigned)blocks, SCAN_THREADS, 0, s, d_in, d_out, n, (const uint32_t *)d_sums);
     }
     if (d_total)
-        SMVP_LAUNCH(scan_total_kernel, 1, 1, 0, s, (const uint32_t *)last.as<uint32_t>(), (const uint32_t *)(d_out + (n - 1)), d_total);
+        SMVP_LAUNCH(scan_total_kernel, 1, 1, 0, s, (const uint32_t *)last.get(), (const uint32_t *)(d_out + (n - 1)), d_total);
     SMVP_CUDA(cudaStreamSynchronize(s));
     SMVP_CUDA(cudaGetLastError());
     return SMVP_OK;
@@ -335,9 +334,9 @@ int radix_sort_pairs(KeyT *keys_a, uint32_t *vals_a, KeyT *keys_b, uint32_t *val
     if (n >= ((int64_t)1 << 32))
         return SMVP_E_TOOBIG;
     const uint32_t blocks = (uint32_t)ceil_div64(n, RS_TILE);
-    DevTmp g_hist;
-    SMVP_CUDA(g_hist.alloc<uint32_t>((int64_t)blocks * RS_RADIX));
-    uint32_t *d_hist = g_hist.as<uint32_t>();
+    DevPtr<uint32_t> hist;
+    SMVP_CUDA(dev_alloc(hist, (int64_t)blocks * RS_RADIX));
+    uint32_t *d_hist = hist.get();
     KeyT *kin = keys_a, *kout = keys_b;
     uint32_t *vin = vals_a, *vout = vals_b;
     int rc = SMVP_OK;

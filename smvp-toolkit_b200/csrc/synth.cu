@@ -399,26 +399,26 @@ extern "C" int smvp_synth_stencil27(int32_t nx, int32_t ny, int32_t nz, int64_t 
     *nnz = n;
     *d_row = *d_col = nullptr;
     *d_val = nullptr;
-    DevTmp g_offs, g_row, g_col, g_val; // the outputs are detached from their guards only on success
-    SMVP_CUDA(g_offs.alloc<uint32_t>(nrows));
-    SMVP_CUDA(g_row.alloc<int32_t>(n));
-    SMVP_CUDA(g_col.alloc<int32_t>(n));
-    SMVP_CUDA(g_val.alloc<double>(n));
-    uint32_t *offs = g_offs.as<uint32_t>();
+    DevPtr<uint32_t> offs;
+    DevPtr<int32_t> row, col;
+    DevPtr<double> val;
+    SMVP_CUDA(dev_alloc(offs, nrows));
+    SMVP_CUDA(dev_alloc(row, n));
+    SMVP_CUDA(dev_alloc(col, n));
+    SMVP_CUDA(dev_alloc(val, n));
     if (nrows > 0)
     {
         const unsigned blocks = (unsigned)ceil_div64(nrows, 256);
-        SMVP_LAUNCH(stencil_count_kernel, blocks, 256, 0, 0, nx, ny, nz, row_begin, nrows, offs);
-        SMVP_TRY(exclusive_scan_u32(offs, offs, nrows, nullptr, 0));
-        SMVP_LAUNCH(stencil_fill_kernel, blocks, 256, 0, 0, nx, ny, nz, row_begin, nrows, (const uint32_t *)offs, value_mode, seed,
-                    g_row.as<int32_t>(), g_col.as<int32_t>(), g_val.as<double>());
+        SMVP_LAUNCH(stencil_count_kernel, blocks, 256, 0, 0, nx, ny, nz, row_begin, nrows, offs.get());
+        SMVP_TRY(exclusive_scan_u32(offs.get(), offs.get(), nrows, nullptr, 0));
+        SMVP_LAUNCH(stencil_fill_kernel, blocks, 256, 0, 0, nx, ny, nz, row_begin, nrows, (const uint32_t *)offs.get(), value_mode,
+                    seed, row.get(), col.get(), val.get());
     }
     SMVP_CUDA(cudaDeviceSynchronize());
     SMVP_CUDA(cudaGetLastError());
-    *d_row = g_row.as<int32_t>();
-    *d_col = g_col.as<int32_t>();
-    *d_val = g_val.as<double>();
-    g_row.p = g_col.p = g_val.p = nullptr;
+    *d_row = row.release();
+    *d_col = col.release();
+    *d_val = val.release();
     return SMVP_OK;
 }
 
@@ -430,40 +430,39 @@ extern "C" int smvp_synth_rmat(int scale, int64_t nedges, double a, double b, do
     *d_row = *d_col = nullptr;
     *d_val = nullptr;
     *nnz = 0;
-    uint64_t *key_a = nullptr, *key_b = nullptr, *rk = nullptr;
-    uint32_t *idx_a = nullptr, *idx_b = nullptr, *ri = nullptr, *d_total = nullptr;
-    auto body = [&]() -> int {
-        SMVP_CUDA(dev_alloc(&key_a, nedges));
-        SMVP_CUDA(dev_alloc(&key_b, nedges));
-        SMVP_CUDA(dev_alloc(&idx_a, nedges));
-        SMVP_CUDA(dev_alloc(&idx_b, nedges));
-        SMVP_CUDA(dev_alloc(&d_total, 1));
-        if (nedges == 0)
-            return SMVP_OK;
-        SMVP_LAUNCH(rmat_edges_kernel, grid_for(nedges), 256, 0, 0, scale, nedges, a, a + b, a + b + c, seed, key_a, idx_a);
-        const int lo = 0, hi = 2 * scale;
-        SMVP_TRY(radix_sort_pairs<uint64_t>(key_a, idx_a, key_b, idx_b, nedges, &lo, &hi, 1, &rk, &ri, 0));
-        uint32_t *flag = (ri == idx_a) ? idx_b : idx_a; // the payload is not needed: reuse its spare buffer for the flags
-        SMVP_LAUNCH(unique_flag_kernel, grid_for(nedges), 256, 0, 0, (const uint64_t *)rk, nedges, flag);
-        SMVP_TRY(exclusive_scan_u32(flag, flag, nedges, d_total, 0));
-        uint32_t total = 0;
-        SMVP_CUDA(cudaMemcpy(&total, d_total, sizeof(total), cudaMemcpyDeviceToHost));
-        *nnz = (int64_t)total;
-        SMVP_CUDA(dev_alloc(d_row, total));
-        SMVP_CUDA(dev_alloc(d_col, total));
-        SMVP_CUDA(dev_alloc(d_val, total));
-        SMVP_LAUNCH(rmat_compact_kernel, grid_for(nedges), 256, 0, 0, (const uint64_t *)rk, (const uint32_t *)flag, nedges, scale,
-                    value_mode, seed, *d_row, *d_col, *d_val);
-        SMVP_CUDA(cudaDeviceSynchronize());
+    DevPtr<uint64_t> key_a, key_b;
+    DevPtr<uint32_t> idx_a, idx_b, d_total;
+    SMVP_CUDA(dev_alloc(key_a, nedges));
+    SMVP_CUDA(dev_alloc(key_b, nedges));
+    SMVP_CUDA(dev_alloc(idx_a, nedges));
+    SMVP_CUDA(dev_alloc(idx_b, nedges));
+    SMVP_CUDA(dev_alloc(d_total, 1));
+    if (nedges == 0)
         return SMVP_OK;
-    };
-    const int rc = body();
-    cudaFree(key_a);
-    cudaFree(key_b);
-    cudaFree(idx_a);
-    cudaFree(idx_b);
-    cudaFree(d_total);
-    return rc;
+    SMVP_LAUNCH(rmat_edges_kernel, grid_for(nedges), 256, 0, 0, scale, nedges, a, a + b, a + b + c, seed, key_a.get(), idx_a.get());
+    uint64_t *rk = nullptr;
+    uint32_t *ri = nullptr;
+    const int lo = 0, hi = 2 * scale;
+    SMVP_TRY(radix_sort_pairs<uint64_t>(key_a.get(), idx_a.get(), key_b.get(), idx_b.get(), nedges, &lo, &hi, 1, &rk, &ri, 0));
+    // the payload is not needed: reuse its spare buffer for the flags
+    uint32_t *flag = (ri == idx_a.get()) ? idx_b.get() : idx_a.get();
+    SMVP_LAUNCH(unique_flag_kernel, grid_for(nedges), 256, 0, 0, (const uint64_t *)rk, nedges, flag);
+    SMVP_TRY(exclusive_scan_u32(flag, flag, nedges, d_total.get(), 0));
+    uint32_t total = 0;
+    SMVP_CUDA(cudaMemcpy(&total, d_total.get(), sizeof(total), cudaMemcpyDeviceToHost));
+    *nnz = (int64_t)total;
+    DevPtr<int32_t> row, col;
+    DevPtr<double> val;
+    SMVP_CUDA(dev_alloc(row, total));
+    SMVP_CUDA(dev_alloc(col, total));
+    SMVP_CUDA(dev_alloc(val, total));
+    SMVP_LAUNCH(rmat_compact_kernel, grid_for(nedges), 256, 0, 0, (const uint64_t *)rk, (const uint32_t *)flag, nedges, scale,
+                value_mode, seed, row.get(), col.get(), val.get());
+    SMVP_CUDA(cudaDeviceSynchronize());
+    *d_row = row.release();
+    *d_col = col.release();
+    *d_val = val.release();
+    return SMVP_OK;
 }
 
 extern "C" int smvp_synth_vector(double *d_x, int64_t n, uint64_t seed, void *stream)
@@ -485,31 +484,30 @@ extern "C" int smvp_coo_filter_device(const int32_t *d_row, const int32_t *d_col
     *o_row = *o_col = nullptr;
     *o_val = nullptr;
     *o_nnz = 0;
-    uint32_t *pos = nullptr, *d_total = nullptr;
-    auto body = [&]() -> int {
-        SMVP_CUDA(dev_alloc(&pos, nnz));
-        SMVP_CUDA(dev_alloc(&d_total, 1));
-        uint32_t total = 0;
-        if (nnz > 0)
-        {
-            SMVP_LAUNCH(filter_flag_kernel, grid_for(nnz), 256, 0, 0, d_row, d_col, nnz, row_lo, row_hi, col_lo, col_hi, pos);
-            SMVP_TRY(exclusive_scan_u32(pos, pos, nnz, d_total, 0));
-            SMVP_CUDA(cudaMemcpy(&total, d_total, sizeof(total), cudaMemcpyDeviceToHost));
-        }
-        *o_nnz = (int64_t)total;
-        SMVP_CUDA(dev_alloc(o_row, total));
-        SMVP_CUDA(dev_alloc(o_col, total));
-        SMVP_CUDA(dev_alloc(o_val, total));
-        if (nnz > 0)
-            SMVP_LAUNCH(filter_scatter_kernel, grid_for(nnz), 256, 0, 0, d_row, d_col, d_val, nnz, row_lo, row_hi, col_lo, col_hi,
-                        row_shift, col_shift, (const uint32_t *)pos, *o_row, *o_col, *o_val);
-        SMVP_CUDA(cudaDeviceSynchronize());
-        return SMVP_OK;
-    };
-    const int rc = body();
-    cudaFree(pos);
-    cudaFree(d_total);
-    return rc;
+    DevPtr<uint32_t> pos, d_total;
+    SMVP_CUDA(dev_alloc(pos, nnz));
+    SMVP_CUDA(dev_alloc(d_total, 1));
+    uint32_t total = 0;
+    if (nnz > 0)
+    {
+        SMVP_LAUNCH(filter_flag_kernel, grid_for(nnz), 256, 0, 0, d_row, d_col, nnz, row_lo, row_hi, col_lo, col_hi, pos.get());
+        SMVP_TRY(exclusive_scan_u32(pos.get(), pos.get(), nnz, d_total.get(), 0));
+        SMVP_CUDA(cudaMemcpy(&total, d_total.get(), sizeof(total), cudaMemcpyDeviceToHost));
+    }
+    *o_nnz = (int64_t)total;
+    DevPtr<int32_t> row, col;
+    DevPtr<double> val;
+    SMVP_CUDA(dev_alloc(row, total));
+    SMVP_CUDA(dev_alloc(col, total));
+    SMVP_CUDA(dev_alloc(val, total));
+    if (nnz > 0)
+        SMVP_LAUNCH(filter_scatter_kernel, grid_for(nnz), 256, 0, 0, d_row, d_col, d_val, nnz, row_lo, row_hi, col_lo, col_hi,
+                    row_shift, col_shift, (const uint32_t *)pos.get(), row.get(), col.get(), val.get());
+    SMVP_CUDA(cudaDeviceSynchronize());
+    *o_row = row.release();
+    *o_col = col.release();
+    *o_val = val.release();
+    return SMVP_OK;
 }
 
 extern "C" int smvp_coo_histogram_device(const int32_t *d_row, const int32_t *d_col, int64_t nnz, int by_col, int32_t nkeys,

@@ -82,136 +82,100 @@ __global__ void __launch_bounds__(256) tjds_scatter_kernel(const uint32_t *__res
     }
 }
 
-void tjds_release(smvp_tjds *A)
-{
-    if (!A)
-        return;
-    cudaFree(A->perm);
-    cudaFree(A->slot_len);
-    cudaFree(A->start_pos);
-    cudaFree(A->row_ind);
-    cudaFree(A->val);
-    cudaFree(A->x_perm);
-    cudaFree(A->seg_blocks);
-    cudaFree(A->row_exp);
-    cudaFree(A->acc);
-    cudaFree(A->x_exp);
-    if (A->x_exp_host)
-        cudaFreeHost(A->x_exp_host);
-    if (A->x_exp_event)
-        cudaEventDestroy(A->x_exp_event);
-    cudaFree(A->d_x);
-    cudaFree(A->d_y);
-    cudaFree(A->tr_seg_off);
-    cudaFree(A->tr_part);
-    cudaFree(A->d_xt);
-    cudaFree(A->d_yt);
-    cudaFree(A->y_sum);
-    cudaFree(A->dot_buf);
-    tjds_relabel_release(A);
-    delete A;
-}
-
+// a new handle of rows x cols with nnz entries, built from COO arrays on the device; handed to *out on success
 static int tjds_build_impl(const int32_t *d_row, const int32_t *d_col, const double *d_val, int32_t rows, int32_t cols,
-                           int64_t nnz, smvp_tjds *A, cudaStream_t s)
+                           int64_t nnz, smvp_tjds **out, cudaStream_t s)
 {
+    std::unique_ptr<smvp_tjds> A(new (std::nothrow) smvp_tjds());
+    if (!A)
+        return SMVP_E_ALLOC;
+    A->rows = rows;
+    A->cols = cols;
+    A->nnz = nnz;
     int order = ORDER_ROW_COL;
     SMVP_TRY(coo_inspect(d_row, d_col, nnz, rows, cols, &order, s));
     A->input_order = order;
 
-    uint32_t *count = nullptr, *col_start = nullptr, *d_max = nullptr;
-    uint32_t *key_a = nullptr, *key_b = nullptr, *idx_a = nullptr, *idx_b = nullptr;
-    int32_t *slot_of = nullptr;
-    uint32_t *d_idx = nullptr;
-    auto cleanup = [&]() {
-        cudaFree(count);
-        cudaFree(col_start);
-        cudaFree(d_max);
-        cudaFree(key_a);
-        cudaFree(key_b);
-        cudaFree(idx_a);
-        cudaFree(idx_b);
-        cudaFree(slot_of);
-        cudaFree(d_idx);
-    };
-    auto body = [&]() -> int {
-        const unsigned cblocks = (unsigned)ceil_div64(cols > 0 ? cols : 1, 256);
-        // ---- column histogram, largest column = number of jagged diagonals
-        SMVP_CUDA(dev_alloc(&count, (int64_t)cols + 1));
-        SMVP_CUDA(dev_alloc(&col_start, (int64_t)cols + 1));
-        SMVP_CUDA(dev_alloc(&d_max, 1));
-        SMVP_TRY(histogram_i32(d_col, nnz, count, (int64_t)cols + 1, s));
-        SMVP_TRY(max_u32(count, cols, d_max, s));
-        uint32_t maxc = 0, count0 = 0;
-        SMVP_CUDA(cudaMemcpyAsync(&maxc, d_max, sizeof(maxc), cudaMemcpyDeviceToHost, s));
-        if (cols > 0)
-            SMVP_CUDA(cudaMemcpyAsync(&count0, count, sizeof(count0), cudaMemcpyDeviceToHost, s));
+    const unsigned cblocks = (unsigned)ceil_div64(cols > 0 ? cols : 1, 256);
+    // ---- column histogram, largest column = number of jagged diagonals
+    DevPtr<uint32_t> count, col_start, d_max;
+    SMVP_CUDA(dev_alloc(count, (int64_t)cols + 1));
+    SMVP_CUDA(dev_alloc(col_start, (int64_t)cols + 1));
+    SMVP_CUDA(dev_alloc(d_max, 1));
+    SMVP_TRY(histogram_i32(d_col, nnz, count.get(), (int64_t)cols + 1, s));
+    SMVP_TRY(max_u32(count.get(), cols, d_max.get(), s));
+    uint32_t maxc = 0, count0 = 0;
+    SMVP_CUDA(cudaMemcpyAsync(&maxc, d_max.get(), sizeof(maxc), cudaMemcpyDeviceToHost, s));
+    if (cols > 0)
+        SMVP_CUDA(cudaMemcpyAsync(&count0, count.get(), sizeof(count0), cudaMemcpyDeviceToHost, s));
+    SMVP_CUDA(cudaStreamSynchronize(s));
+    A->ndiag = (int32_t)maxc;
+    A->ref_diag_limit = (int32_t)count0 + 1; // main-cli.c:865 (before the sort) + the `+ 1` of :1013
+
+    // ---- perm: columns by count descending, column ascending on ties
+    DevPtr<int32_t> slot_of;
+    DevPtr<uint32_t> key_a, key_b, idx_a, idx_b;
+    SMVP_CUDA(dev_alloc(A->perm, cols));
+    SMVP_CUDA(dev_alloc(A->slot_len, cols));
+    SMVP_CUDA(dev_alloc(A->x_perm, cols));
+    SMVP_CUDA(dev_alloc(slot_of, cols));
+    SMVP_CUDA(dev_alloc(key_a, cols));
+    SMVP_CUDA(dev_alloc(key_b, cols));
+    SMVP_CUDA(dev_alloc(idx_a, cols));
+    SMVP_CUDA(dev_alloc(idx_b, cols));
+    if (cols > 0)
+    {
+        SMVP_LAUNCH(tjds_colkey_kernel, cblocks, 256, 0, s, (const uint32_t *)count.get(), cols, maxc, key_a.get(), idx_a.get());
+        uint32_t *rk = nullptr, *ri = nullptr;
+        const int lo = 0, hi = bits_for(maxc + 1u);
+        SMVP_TRY(radix_sort_pairs<uint32_t>(key_a.get(), idx_a.get(), key_b.get(), idx_b.get(), cols, &lo, &hi, 1, &rk, &ri, s));
+        SMVP_LAUNCH(tjds_perm_kernel, cblocks, 256, 0, s, (const uint32_t *)rk, (const uint32_t *)ri, cols, maxc, A->perm.get(),
+                    A->slot_len.get(), slot_of.get());
+    }
+
+    // ---- start_pos
+    SMVP_CUDA(dev_alloc(A->start_pos, (int64_t)A->ndiag + 1));
+    if (A->ndiag > 0)
+    {
+        uint32_t *start_pos = (uint32_t *)A->start_pos.get();
+        SMVP_LAUNCH(tjds_diag_len_kernel, (unsigned)ceil_div64(A->ndiag, 256), 256, 0, s, (const int32_t *)A->slot_len.get(), cols,
+                    A->ndiag, start_pos);
+        SMVP_CUDA(cudaMemcpyAsync(&A->nslots, start_pos, sizeof(int32_t), cudaMemcpyDeviceToHost, s)); // L[0]
         SMVP_CUDA(cudaStreamSynchronize(s));
-        A->ndiag = (int32_t)maxc;
-        A->ref_diag_limit = (int32_t)count0 + 1; // main-cli.c:865 (before the sort) + the `+ 1` of :1013
-
-        // ---- perm: columns by count descending, column ascending on ties
-        SMVP_CUDA(dev_alloc(&A->perm, cols));
-        SMVP_CUDA(dev_alloc(&A->slot_len, cols));
-        SMVP_CUDA(dev_alloc(&A->x_perm, cols));
-        SMVP_CUDA(dev_alloc(&slot_of, cols));
-        SMVP_CUDA(dev_alloc(&key_a, cols));
-        SMVP_CUDA(dev_alloc(&key_b, cols));
-        SMVP_CUDA(dev_alloc(&idx_a, cols));
-        SMVP_CUDA(dev_alloc(&idx_b, cols));
-        if (cols > 0)
-        {
-            SMVP_LAUNCH(tjds_colkey_kernel, cblocks, 256, 0, s, (const uint32_t *)count, cols, maxc, key_a, idx_a);
-            uint32_t *rk = nullptr, *ri = nullptr;
-            const int lo = 0, hi = bits_for(maxc + 1u);
-            SMVP_TRY(radix_sort_pairs<uint32_t>(key_a, idx_a, key_b, idx_b, cols, &lo, &hi, 1, &rk, &ri, s));
-            SMVP_LAUNCH(tjds_perm_kernel, cblocks, 256, 0, s, (const uint32_t *)rk, (const uint32_t *)ri, cols, maxc, A->perm,
-                        A->slot_len, slot_of);
-        }
-
-        // ---- start_pos
-        SMVP_CUDA(dev_alloc(&A->start_pos, (int64_t)A->ndiag + 1));
-        if (A->ndiag > 0)
-        {
-            SMVP_LAUNCH(tjds_diag_len_kernel, (unsigned)ceil_div64(A->ndiag, 256), 256, 0, s, (const int32_t *)A->slot_len, cols,
-                        A->ndiag, (uint32_t *)A->start_pos);
-            SMVP_CUDA(cudaMemcpyAsync(&A->nslots, A->start_pos, sizeof(int32_t), cudaMemcpyDeviceToHost, s)); // L[0]
-            SMVP_CUDA(cudaStreamSynchronize(s));
-            SMVP_TRY(exclusive_scan_u32((const uint32_t *)A->start_pos, (uint32_t *)A->start_pos, A->ndiag, nullptr, s));
-            int32_t last_start = 0;
-            SMVP_CUDA(cudaMemcpyAsync(&last_start, A->start_pos + (A->ndiag - 1), sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-            SMVP_CUDA(cudaStreamSynchronize(s));
-            A->last_diag_len = (int32_t)(nnz - last_start);
-        }
-        else
-        {
-            A->nslots = 0;
-            A->last_diag_len = 0;
-        }
-        SMVP_LAUNCH(tjds_set_last_kernel, 1, 1, 0, s, A->start_pos, A->ndiag, (int32_t)nnz);
-
-        // ---- rank inside the column needs column-major order
-        SMVP_TRY(exclusive_scan_u32(count, col_start, cols, nullptr, s));
-        SMVP_TRY(coo_sort_index(d_col, d_row, nnz, cols, rows, order == ORDER_COL_ROW, order == ORDER_ROW_COL, &d_idx, s));
-        SMVP_CUDA(dev_alloc(&A->row_ind, nnz));
-        SMVP_CUDA(dev_alloc(&A->val, nnz));
-        if (nnz > 0)
-        {
-            int64_t blocks = ceil_div64(nnz, 256 * 4);
-            const int64_t cap = (int64_t)device_props().sms * 16;
-            if (blocks > cap)
-                blocks = cap;
-            SMVP_LAUNCH(tjds_scatter_kernel, (unsigned)blocks, 256, 0, s, (const uint32_t *)d_idx, d_row, d_col, d_val, nnz,
-                        (const uint32_t *)col_start, (const int32_t *)slot_of, (const int32_t *)A->start_pos, A->row_ind, A->val);
-        }
+        SMVP_TRY(exclusive_scan_u32(start_pos, start_pos, A->ndiag, nullptr, s));
+        int32_t last_start = 0;
+        SMVP_CUDA(cudaMemcpyAsync(&last_start, start_pos + (A->ndiag - 1), sizeof(int32_t), cudaMemcpyDeviceToHost, s));
         SMVP_CUDA(cudaStreamSynchronize(s));
-        SMVP_CUDA(cudaGetLastError());
-        A->device_bytes = 12 * nnz + 4 * ((int64_t)A->ndiag + 1) + 16 * (int64_t)cols;
-        return SMVP_OK;
-    };
-    const int rc = body();
-    cleanup();
-    return rc;
+        A->last_diag_len = (int32_t)(nnz - last_start);
+    }
+    else
+    {
+        A->nslots = 0;
+        A->last_diag_len = 0;
+    }
+    SMVP_LAUNCH(tjds_set_last_kernel, 1, 1, 0, s, A->start_pos.get(), A->ndiag, (int32_t)nnz);
+
+    // ---- rank inside the column needs column-major order
+    DevPtr<uint32_t> d_idx;
+    SMVP_TRY(exclusive_scan_u32(count.get(), col_start.get(), cols, nullptr, s));
+    SMVP_TRY(coo_sort_index(d_col, d_row, nnz, cols, rows, order == ORDER_COL_ROW, order == ORDER_ROW_COL, &d_idx, s));
+    SMVP_CUDA(dev_alloc(A->row_ind, nnz));
+    SMVP_CUDA(dev_alloc(A->val, nnz));
+    if (nnz > 0)
+    {
+        int64_t blocks = ceil_div64(nnz, 256 * 4);
+        const int64_t cap = (int64_t)device_props().sms * 16;
+        if (blocks > cap)
+            blocks = cap;
+        SMVP_LAUNCH(tjds_scatter_kernel, (unsigned)blocks, 256, 0, s, (const uint32_t *)d_idx.get(), d_row, d_col, d_val, nnz,
+                    (const uint32_t *)col_start.get(), (const int32_t *)slot_of.get(), (const int32_t *)A->start_pos.get(),
+                    A->row_ind.get(), A->val.get());
+    }
+    SMVP_CUDA(cudaStreamSynchronize(s));
+    SMVP_CUDA(cudaGetLastError());
+    A->device_bytes = 12 * nnz + 4 * ((int64_t)A->ndiag + 1) + 16 * (int64_t)cols;
+    *out = A.release();
+    return SMVP_OK;
 }
 
 } // namespace smvp
@@ -228,20 +192,7 @@ extern "C" int smvp_tjds_build_device(const int32_t *d_row, const int32_t *d_col
         return SMVP_E_ARG;
     if (nnz > 0x7fffffffLL - 1024)
         return SMVP_E_TOOBIG;
-    smvp_tjds *A = new (std::nothrow) smvp_tjds();
-    if (!A)
-        return SMVP_E_ALLOC;
-    A->rows = rows;
-    A->cols = cols;
-    A->nnz = nnz;
-    int rc = tjds_build_impl(d_row, d_col, d_val, rows, cols, nnz, A, 0);
-    if (rc != SMVP_OK)
-    {
-        tjds_release(A);
-        return rc;
-    }
-    *out = A;
-    return SMVP_OK;
+    return tjds_build_impl(d_row, d_col, d_val, rows, cols, nnz, out, 0);
 }
 
 extern "C" int smvp_tjds_build(const smvp_coo *coo, int32_t rows, int32_t cols, int64_t nnz, smvp_tjds **out)
@@ -253,42 +204,33 @@ extern "C" int smvp_tjds_build(const smvp_coo *coo, int32_t rows, int32_t cols, 
         return SMVP_E_ARG;
     if (nnz > 0x7fffffffLL - 1024)
         return SMVP_E_TOOBIG;
-    smvp_coo *d_aos = nullptr;
-    int32_t *d_row = nullptr, *d_col = nullptr;
-    double *d_val = nullptr;
-    auto body = [&]() -> int {
-        SMVP_CUDA(dev_alloc(&d_aos, nnz));
-        SMVP_CUDA(dev_alloc(&d_row, nnz));
-        SMVP_CUDA(dev_alloc(&d_col, nnz));
-        SMVP_CUDA(dev_alloc(&d_val, nnz));
-        if (nnz > 0)
-            SMVP_CUDA(cudaMemcpy(d_aos, coo, sizeof(smvp_coo) * (size_t)nnz, cudaMemcpyHostToDevice));
-        SMVP_TRY(coo_unzip(d_aos, nnz, d_row, d_col, d_val, 0));
-        SMVP_CUDA(cudaFree(d_aos));
-        d_aos = nullptr;
-        return smvp_tjds_build_device(d_row, d_col, d_val, rows, cols, nnz, out);
-    };
-    const int rc = body();
-    cudaFree(d_aos);
-    cudaFree(d_row);
-    cudaFree(d_col);
-    cudaFree(d_val);
-    return rc;
+    DevPtr<smvp_coo> d_aos;
+    DevPtr<int32_t> d_row, d_col;
+    DevPtr<double> d_val;
+    SMVP_CUDA(dev_alloc(d_aos, nnz));
+    SMVP_CUDA(dev_alloc(d_row, nnz));
+    SMVP_CUDA(dev_alloc(d_col, nnz));
+    SMVP_CUDA(dev_alloc(d_val, nnz));
+    if (nnz > 0)
+        SMVP_CUDA(cudaMemcpy(d_aos.get(), coo, sizeof(smvp_coo) * (size_t)nnz, cudaMemcpyHostToDevice));
+    SMVP_TRY(coo_unzip(d_aos.get(), nnz, d_row.get(), d_col.get(), d_val.get(), 0));
+    d_aos.reset(); // before the build: lowers the peak
+    return smvp_tjds_build_device(d_row.get(), d_col.get(), d_val.get(), rows, cols, nnz, out);
 }
 
-extern "C" void smvp_tjds_free(smvp_tjds *A) { smvp::tjds_release(A); }
+extern "C" void smvp_tjds_free(smvp_tjds *A) { delete A; }
 
 extern "C" int smvp_tjds_export(const smvp_tjds *A, int32_t *perm, int32_t *start_pos, int32_t *row_ind, double *val)
 {
     if (!A)
         return SMVP_E_ARG;
     if (perm && A->cols > 0)
-        SMVP_CUDA(cudaMemcpy(perm, A->perm, sizeof(int32_t) * (size_t)A->cols, cudaMemcpyDeviceToHost));
+        SMVP_CUDA(cudaMemcpy(perm, A->perm.get(), sizeof(int32_t) * (size_t)A->cols, cudaMemcpyDeviceToHost));
     if (start_pos)
-        SMVP_CUDA(cudaMemcpy(start_pos, A->start_pos, sizeof(int32_t) * ((size_t)A->ndiag + 1), cudaMemcpyDeviceToHost));
+        SMVP_CUDA(cudaMemcpy(start_pos, A->start_pos.get(), sizeof(int32_t) * ((size_t)A->ndiag + 1), cudaMemcpyDeviceToHost));
     if (row_ind && A->nnz > 0)
-        SMVP_CUDA(cudaMemcpy(row_ind, A->row_ind, sizeof(int32_t) * (size_t)A->nnz, cudaMemcpyDeviceToHost));
+        SMVP_CUDA(cudaMemcpy(row_ind, A->row_ind.get(), sizeof(int32_t) * (size_t)A->nnz, cudaMemcpyDeviceToHost));
     if (val && A->nnz > 0)
-        SMVP_CUDA(cudaMemcpy(val, A->val, sizeof(double) * (size_t)A->nnz, cudaMemcpyDeviceToHost));
+        SMVP_CUDA(cudaMemcpy(val, A->val.get(), sizeof(double) * (size_t)A->nnz, cudaMemcpyDeviceToHost));
     return SMVP_OK;
 }

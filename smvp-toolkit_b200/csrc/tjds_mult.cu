@@ -21,6 +21,8 @@
 //                 accumulators to clear and read back.
 #include "common.cuh"
 
+#include <string.h>
+
 namespace smvp
 {
 
@@ -772,60 +774,56 @@ __global__ void __launch_bounds__(256) tjds_transpose_count_kernel(const int32_t
 }
 
 // the row indices the kernels scatter through: the relabelled copy when that plan is in use (relabel.cu)
-static inline const int32_t *mult_rows(const smvp_tjds *A) { return A->relabel_state == 1 ? A->row_rel : A->row_ind; }
+static inline const int32_t *mult_rows(const smvp_tjds *A) { return A->relabel_state == 1 ? A->row_rel.get() : A->row_ind.get(); }
 
 // decides the walk (once per handle) and builds the block table for it.  Synchronous.
 static int tjds_plan(smvp_tjds *A, cudaStream_t s)
 {
     if (A->seg_blocks || A->ndiag == 0)
         return SMVP_OK;
-    if (A->skew == 0)
+    int32_t skew = A->skew;
+    if (skew == 0)
     {
-        A->skew = env_tristate("SMVP_TJDS_SKEW");
-        if (A->skew == 0 && A->ndiag >= 2)
+        skew = env_tristate("SMVP_TJDS_SKEW");
+        if (skew == 0 && A->ndiag >= 2)
         {
-            DevTmp probe;
-            SMVP_CUDA(probe.alloc<unsigned long long>(2));
-            SMVP_CUDA(cudaMemsetAsync(probe.p, 0, 2 * sizeof(unsigned long long), s));
+            DevPtr<unsigned long long> probe;
+            SMVP_CUDA(dev_alloc(probe, 2));
+            SMVP_CUDA(cudaMemsetAsync(probe.get(), 0, 2 * sizeof(unsigned long long), s));
             const int pairs = A->ndiag - 1 < 8 ? A->ndiag - 1 : 8;
-            SMVP_LAUNCH(tjds_skew_probe_kernel, dim3(64, pairs), 256, 0, s, (const int32_t *)A->start_pos, (const int32_t *)A->row_ind,
-                        A->ndiag, probe.as<unsigned long long>());
+            SMVP_LAUNCH(tjds_skew_probe_kernel, dim3(64, pairs), 256, 0, s, (const int32_t *)A->start_pos.get(),
+                        (const int32_t *)A->row_ind.get(), A->ndiag, probe.get());
             unsigned long long h[2] = {0, 0};
-            SMVP_CUDA(cudaMemcpyAsync(h, probe.p, sizeof(h), cudaMemcpyDeviceToHost, s));
+            SMVP_CUDA(cudaMemcpyAsync(h, probe.get(), sizeof(h), cudaMemcpyDeviceToHost, s));
             SMVP_CUDA(cudaStreamSynchronize(s));
             // worth it when at least a quarter of the looked-at entries continue a run (the x_perm load per step has
             // to be paid for by saved reductions)
-            A->skew = (h[0] >= 1024 && 4 * h[1] >= h[0]) ? 1 : -1;
+            skew = (h[0] >= 1024 && 4 * h[1] >= h[0]) ? 1 : -1;
         }
-        else if (A->skew == 0)
-            A->skew = -1;
+        else if (skew == 0)
+            skew = -1;
     }
-    const int32_t extra = A->skew == 1 ? TJDS_SEG - 1 : 0; // the skewed walk of the last block leans TJDS_SEG-1 slots back
+    const int32_t extra = skew == 1 ? TJDS_SEG - 1 : 0; // the skewed walk of the last block leans TJDS_SEG-1 slots back
     const int32_t nseg = (A->ndiag + TJDS_SEG - 1) / TJDS_SEG;
-    DevTmp seg_nb, d_total;
-    SMVP_CUDA(seg_nb.alloc<uint32_t>(nseg));
-    SMVP_CUDA(d_total.alloc<uint32_t>(1));
-    SMVP_LAUNCH(tjds_seg_count_kernel, (unsigned)ceil_div64(nseg, 256), 256, 0, s, (const int32_t *)A->start_pos, A->ndiag, nseg, extra,
-                seg_nb.as<uint32_t>());
-    SMVP_TRY(exclusive_scan_u32(seg_nb.as<uint32_t>(), seg_nb.as<uint32_t>(), nseg, d_total.as<uint32_t>(), s));
+    DevPtr<uint32_t> seg_nb, d_total;
+    SMVP_CUDA(dev_alloc(seg_nb, nseg));
+    SMVP_CUDA(dev_alloc(d_total, 1));
+    SMVP_LAUNCH(tjds_seg_count_kernel, (unsigned)ceil_div64(nseg, 256), 256, 0, s, (const int32_t *)A->start_pos.get(), A->ndiag, nseg,
+                extra, seg_nb.get());
+    SMVP_TRY(exclusive_scan_u32(seg_nb.get(), seg_nb.get(), nseg, d_total.get(), s));
     uint32_t total = 0;
-    SMVP_CUDA(cudaMemcpyAsync(&total, d_total.p, sizeof(total), cudaMemcpyDeviceToHost, s));
+    SMVP_CUDA(cudaMemcpyAsync(&total, d_total.get(), sizeof(total), cudaMemcpyDeviceToHost, s));
     SMVP_CUDA(cudaStreamSynchronize(s));
     if (total > 0x7fffffffu)
         return SMVP_E_TOOBIG;
-    int2 *blocks = nullptr;
-    SMVP_CUDA(dev_alloc(&blocks, total));
-    SMVP_LAUNCH(tjds_seg_fill_kernel, (unsigned)nseg, 256, 0, s, (const uint32_t *)seg_nb.as<uint32_t>(), (const int32_t *)A->start_pos,
-                nseg, extra, blocks);
-    cudaError_t e = cudaStreamSynchronize(s);
-    if (e == cudaSuccess)
-        e = cudaGetLastError();
-    if (e != cudaSuccess)
-    {
-        cudaFree(blocks);
-        return cuda_fail(e, "tjds_plan", __FILE__, __LINE__);
-    }
-    A->seg_blocks = blocks;
+    DevPtr<int2> blocks;
+    SMVP_CUDA(dev_alloc(blocks, total));
+    SMVP_LAUNCH(tjds_seg_fill_kernel, (unsigned)nseg, 256, 0, s, (const uint32_t *)seg_nb.get(), (const int32_t *)A->start_pos.get(),
+                nseg, extra, blocks.get());
+    SMVP_CUDA(cudaStreamSynchronize(s));
+    SMVP_CUDA(cudaGetLastError());
+    A->skew = skew;
+    A->seg_blocks = std::move(blocks);
     A->num_seg_blocks = (int32_t)total;
     return SMVP_OK;
 }
@@ -834,46 +832,39 @@ static int tjds_prepare_det(smvp_tjds *A, cudaStream_t s)
 {
     if (A->row_exp)
         return SMVP_OK;
-    DevTmp cnt, flags;
-    int32_t *row_exp = nullptr;
-    long long *acc = nullptr;
-    auto body = [&]() -> int {
-        SMVP_CUDA(dev_alloc(&row_exp, A->rows));
-        SMVP_CUDA(dev_alloc(&acc, 2 * (int64_t)A->rows));
-        SMVP_CUDA(cnt.alloc<uint32_t>(A->rows));
-        SMVP_CUDA(flags.alloc<int32_t>(5));
-        const int32_t h0[5] = {0, EXP_NONE, EXP_LOW_NONE, 0x7fffffff, -1};
-        SMVP_CUDA(cudaMemcpyAsync(flags.p, h0, sizeof(h0), cudaMemcpyHostToDevice, s));
-        SMVP_CUDA(cudaMemsetAsync(cnt.p, 0, sizeof(uint32_t) * (size_t)A->rows, s));
-        // EXP_NONE = 0x80808080 is a byte pattern, so a memset fills it
-        SMVP_CUDA(cudaMemsetAsync(row_exp, 0x80, sizeof(int32_t) * (size_t)A->rows, s));
-        if (A->nnz > 0)
-        {
-            int64_t blocks = ceil_div64(A->nnz, 256 * 4);
-            const int64_t cap = (int64_t)device_props().sms * 16;
-            if (blocks > cap)
-                blocks = cap;
-            SMVP_LAUNCH(tjds_row_bound_kernel, (unsigned)blocks, 256, 0, s, mult_rows(A), (const double *)A->val, A->nnz, row_exp,
-                        cnt.as<uint32_t>(), flags.as<int32_t>()); // after the relabel decision: row_exp lives in the index space the kernels use
-        }
-        if (A->rows > 0)
-            SMVP_LAUNCH(tjds_row_exp_kernel, (unsigned)ceil_div64(A->rows, 256), 256, 0, s, row_exp, (const uint32_t *)cnt.as<uint32_t>(),
-                        A->rows, flags.as<int32_t>());
-        SMVP_CUDA(cudaMemcpyAsync(A->det_flags, flags.p, sizeof(A->det_flags), cudaMemcpyDeviceToHost, s));
-        static_assert(sizeof(A->det_flags) == 5 * sizeof(int32_t), "flags layout");
-        SMVP_CUDA(cudaStreamSynchronize(s));
-        SMVP_CUDA(cudaGetLastError());
-        return SMVP_OK;
-    };
-    const int rc = body();
-    if (rc != SMVP_OK)
+    DevPtr<int32_t> row_exp, flags;
+    DevPtr<long long> acc;
+    DevPtr<uint32_t> cnt;
+    SMVP_CUDA(dev_alloc(row_exp, A->rows));
+    SMVP_CUDA(dev_alloc(acc, 2 * (int64_t)A->rows));
+    SMVP_CUDA(dev_alloc(cnt, A->rows));
+    SMVP_CUDA(dev_alloc(flags, 5));
+    const int32_t h0[5] = {0, EXP_NONE, EXP_LOW_NONE, 0x7fffffff, -1};
+    SMVP_CUDA(cudaMemcpyAsync(flags.get(), h0, sizeof(h0), cudaMemcpyHostToDevice, s));
+    SMVP_CUDA(cudaMemsetAsync(cnt.get(), 0, sizeof(uint32_t) * (size_t)A->rows, s));
+    // EXP_NONE = 0x80808080 is a byte pattern, so a memset fills it
+    SMVP_CUDA(cudaMemsetAsync(row_exp.get(), 0x80, sizeof(int32_t) * (size_t)A->rows, s));
+    if (A->nnz > 0)
     {
-        cudaFree(row_exp);
-        cudaFree(acc);
-        return rc;
+        int64_t blocks = ceil_div64(A->nnz, 256 * 4);
+        const int64_t cap = (int64_t)device_props().sms * 16;
+        if (blocks > cap)
+            blocks = cap;
+        // after the relabel decision: row_exp lives in the index space the kernels use
+        SMVP_LAUNCH(tjds_row_bound_kernel, (unsigned)blocks, 256, 0, s, mult_rows(A), (const double *)A->val.get(), A->nnz,
+                    row_exp.get(), cnt.get(), flags.get());
     }
-    A->row_exp = row_exp;
-    A->acc = acc;
+    if (A->rows > 0)
+        SMVP_LAUNCH(tjds_row_exp_kernel, (unsigned)ceil_div64(A->rows, 256), 256, 0, s, row_exp.get(), (const uint32_t *)cnt.get(),
+                    A->rows, flags.get());
+    int32_t det_flags[5];
+    static_assert(sizeof(det_flags) == sizeof(A->det_flags), "flags layout");
+    SMVP_CUDA(cudaMemcpyAsync(det_flags, flags.get(), sizeof(det_flags), cudaMemcpyDeviceToHost, s));
+    SMVP_CUDA(cudaStreamSynchronize(s));
+    SMVP_CUDA(cudaGetLastError());
+    memcpy(A->det_flags, det_flags, sizeof(det_flags));
+    A->row_exp = std::move(row_exp);
+    A->acc = std::move(acc);
     A->det_route = 0; // depends on the matrix flags just computed
     return SMVP_OK;
 }
@@ -887,7 +878,7 @@ static int tjds_det_route(smvp_tjds *A)
 {
     if (A->x_exp_pending)
     {
-        SMVP_CUDA(cudaEventSynchronize(A->x_exp_event));
+        SMVP_CUDA(cudaEventSynchronize(A->x_exp_event.get()));
         A->x_exp_pending = 0;
         A->det_route = 0;
     }
@@ -921,34 +912,23 @@ static int tjds_transpose_prepare(smvp_tjds *A, cudaStream_t s)
         const int32_t nseg = (A->ndiag + TJDS_SEG - 1) / TJDS_SEG;
         const int32_t wide = TJDS_SEG * TJDS_SEG; // columns longer than this have more than TJDS_SEG chunks
         int32_t h[4] = {0, 0, 0, 0};
-        SMVP_CUDA(cudaMemcpyAsync(h, A->start_pos + TJDS_SEG, 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+        SMVP_CUDA(cudaMemcpyAsync(h, A->start_pos.get() + TJDS_SEG, 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
         if (A->ndiag > wide)
-            SMVP_CUDA(cudaMemcpyAsync(h + 2, A->start_pos + wide, 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-        uint32_t *seg_off = nullptr;
-        double *part = nullptr;
+            SMVP_CUDA(cudaMemcpyAsync(h + 2, A->start_pos.get() + wide, 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+        DevPtr<uint32_t> d_total, seg_off;
+        DevPtr<double> part;
+        SMVP_CUDA(dev_alloc(d_total, 1));
+        SMVP_CUDA(dev_alloc(seg_off, nseg));
+        SMVP_LAUNCH(tjds_transpose_count_kernel, (unsigned)ceil_div64(nseg, 256), 256, 0, s, (const int32_t *)A->start_pos.get(), nseg,
+                    seg_off.get());
+        SMVP_TRY(exclusive_scan_u32(seg_off.get(), seg_off.get(), nseg, d_total.get(), s));
         uint32_t total = 0;
-        auto body = [&]() -> int {
-            DevTmp d_total;
-            SMVP_CUDA(d_total.alloc<uint32_t>(1));
-            SMVP_CUDA(dev_alloc(&seg_off, nseg));
-            SMVP_LAUNCH(tjds_transpose_count_kernel, (unsigned)ceil_div64(nseg, 256), 256, 0, s, (const int32_t *)A->start_pos, nseg,
-                        seg_off);
-            SMVP_TRY(exclusive_scan_u32(seg_off, seg_off, nseg, d_total.as<uint32_t>(), s));
-            SMVP_CUDA(cudaMemcpyAsync(&total, d_total.p, sizeof(total), cudaMemcpyDeviceToHost, s));
-            SMVP_CUDA(cudaStreamSynchronize(s));
-            SMVP_CUDA(cudaGetLastError());
-            SMVP_CUDA(dev_alloc(&part, total));
-            return SMVP_OK;
-        };
-        const int rc = body();
-        if (rc != SMVP_OK)
-        {
-            cudaFree(seg_off);
-            cudaFree(part);
-            return rc;
-        }
-        A->tr_seg_off = seg_off;
-        A->tr_part = part;
+        SMVP_CUDA(cudaMemcpyAsync(&total, d_total.get(), sizeof(total), cudaMemcpyDeviceToHost, s));
+        SMVP_CUDA(cudaStreamSynchronize(s));
+        SMVP_CUDA(cudaGetLastError());
+        SMVP_CUDA(dev_alloc(part, total));
+        A->tr_seg_off = std::move(seg_off);
+        A->tr_part = std::move(part);
         A->tr_nlong = h[1] - h[0];
         A->tr_nwide = h[3] - h[2];
         A->device_bytes += 4 * (int64_t)nseg + 8 * (int64_t)total;
@@ -1001,14 +981,16 @@ static int tjds_transpose_pass(smvp_tjds *A, const double *d_x, double *d_y, con
                 SMVP_LAUNCH(tjds_axpby_empty_kernel<M>, (unsigned)blocks, 256, 0, s, d_y, A->cols, ab.alpha, ab.beta, w, part);
                 return (int)SMVP_OK;
             }
-        SMVP_LAUNCH(tjds_transpose_kernel<M>, (unsigned)A->num_seg_blocks, 256, 0, s, (const int2 *)A->seg_blocks,
-                    (const int32_t *)A->start_pos, (const int32_t *)A->row_ind, (const double *)A->val, (const int32_t *)A->perm, d_x, d_y,
-                    A->tr_part, (const uint32_t *)A->tr_seg_off, A->ndiag, A->nslots, A->cols, A->tr_nlong, ab.alpha, ab.beta, w, part);
+        SMVP_LAUNCH(tjds_transpose_kernel<M>, (unsigned)A->num_seg_blocks, 256, 0, s, (const int2 *)A->seg_blocks.get(),
+                    (const int32_t *)A->start_pos.get(), (const int32_t *)A->row_ind.get(), (const double *)A->val.get(),
+                    (const int32_t *)A->perm.get(), d_x, d_y, A->tr_part.get(), (const uint32_t *)A->tr_seg_off.get(), A->ndiag,
+                    A->nslots, A->cols, A->tr_nlong, ab.alpha, ab.beta, w, part);
         if (A->ndiag > TJDS_SEG)
         {
             const int64_t threads = 32 * (int64_t)A->tr_nwide + (A->tr_nlong - A->tr_nwide);
-            SMVP_LAUNCH(tjds_transpose_combine_kernel<M>, (unsigned)ceil_div64(threads, 256), 256, 0, s, (const double *)A->tr_part,
-                        (const uint32_t *)A->tr_seg_off, (const int32_t *)A->slot_len, (const int32_t *)A->perm, A->tr_nlong, A->tr_nwide,
+            SMVP_LAUNCH(tjds_transpose_combine_kernel<M>, (unsigned)ceil_div64(threads, 256), 256, 0, s,
+                        (const double *)A->tr_part.get(), (const uint32_t *)A->tr_seg_off.get(), (const int32_t *)A->slot_len.get(),
+                        (const int32_t *)A->perm.get(), A->tr_nlong, A->tr_nwide,
                         d_y, ab.alpha, ab.beta, w, M == YStore::Dot ? part + A->num_seg_blocks : nullptr);
         }
         return (int)SMVP_OK;
@@ -1060,10 +1042,10 @@ extern "C" int smvp_tjds_mult_transpose_device_axpby_dot(smvp_tjds *A, double al
         SMVP_TRY(tjds_transpose_prepare(A, s));
     const int64_t units = A->cols > 0 ? tjds_transpose_units(A) : 0;
     SMVP_TRY(dot_scratch(&A->dot_buf, &A->dot_cap, &A->device_bytes, tjds_dot_units_max(A), s));
-    const DotOut dot = {d_w, A->dot_buf};
+    const DotOut dot = {d_w, A->dot_buf.get()};
     if (A->cols > 0)
         SMVP_TRY(tjds_transpose_pass(A, d_x, d_y, Axpby{alpha, beta}, &dot, s));
-    return dot_reduce(A->dot_buf, A->dot_cap, units, d_dot, s);
+    return dot_reduce(A->dot_buf.get(), A->dot_cap, units, d_dot, s);
 }
 
 extern "C" int smvp_tjds_mult_transpose(smvp_tjds *A, const double *x_host, double *y_host, int iters, double *ms_each)
@@ -1071,20 +1053,22 @@ extern "C" int smvp_tjds_mult_transpose(smvp_tjds *A, const double *x_host, doub
     if (!A || iters < 1 || (A->rows > 0 && !x_host) || (A->cols > 0 && !y_host))
         return SMVP_E_ARG;
     if (!A->d_xt)
-        SMVP_CUDA(dev_alloc(&A->d_xt, A->rows));
+        SMVP_CUDA(dev_alloc(A->d_xt, A->rows));
     if (!A->d_yt)
-        SMVP_CUDA(dev_alloc(&A->d_yt, A->cols));
+        SMVP_CUDA(dev_alloc(A->d_yt, A->cols));
     if (A->rows > 0)
-        SMVP_CUDA(cudaMemcpy(A->d_xt, x_host, sizeof(double) * (size_t)A->rows, cudaMemcpyHostToDevice));
+        SMVP_CUDA(cudaMemcpy(A->d_xt.get(), x_host, sizeof(double) * (size_t)A->rows, cudaMemcpyHostToDevice));
     SMVP_TRY(tjds_transpose_prepare(A, 0));
     const bool small = (int64_t)A->rows + A->cols + A->nnz < SMVP_SMALL_LOOP_ITEMS;
     if (A->cols > 0)
-        SMVP_TRY(timed_loop(iters, ms_each, small, [&](cudaStream_t s) { return tjds_transpose_pass(A, A->d_xt, A->d_yt, AXPBY_PLAIN, nullptr, s); }));
+        SMVP_TRY(timed_loop(iters, ms_each, small, [&](cudaStream_t s) {
+            return tjds_transpose_pass(A, A->d_xt.get(), A->d_yt.get(), AXPBY_PLAIN, nullptr, s);
+        }));
     else if (ms_each)
         for (int it = 0; it < iters; it++)
             ms_each[it] = 0.0;
     if (A->cols > 0)
-        SMVP_CUDA(cudaMemcpy(y_host, A->d_yt, sizeof(double) * (size_t)A->cols, cudaMemcpyDeviceToHost));
+        SMVP_CUDA(cudaMemcpy(y_host, A->d_yt.get(), sizeof(double) * (size_t)A->cols, cudaMemcpyDeviceToHost));
     return SMVP_OK;
 }
 
@@ -1094,23 +1078,23 @@ extern "C" int smvp_tjds_set_x_device(smvp_tjds *A, const double *d_x, void *str
         return SMVP_E_ARG;
     cudaStream_t s = (cudaStream_t)stream;
     if (!A->x_exp)
-        SMVP_CUDA(dev_alloc(&A->x_exp, 1));
+        SMVP_CUDA(dev_alloc(A->x_exp, 1));
     if (!A->x_exp_host)
-        SMVP_CUDA(cudaHostAlloc((void **)&A->x_exp_host, sizeof(int32_t), cudaHostAllocDefault));
+        SMVP_CUDA(cudaHostAlloc((void **)(int32_t **)out(A->x_exp_host), sizeof(int32_t), cudaHostAllocDefault));
     if (!A->x_exp_event)
-        SMVP_CUDA(cudaEventCreateWithFlags(&A->x_exp_event, cudaEventDisableTiming));
-    SMVP_CUDA(cudaMemsetAsync(A->x_exp, 0x80, sizeof(int32_t), s)); // 0x80808080: below every real exponent
+        SMVP_CUDA(cudaEventCreateWithFlags(out(A->x_exp_event), cudaEventDisableTiming));
+    SMVP_CUDA(cudaMemsetAsync(A->x_exp.get(), 0x80, sizeof(int32_t), s)); // 0x80808080: below every real exponent
     if (A->cols > 0)
     {
         int64_t blocks = ceil_div64(A->cols, 256);
         const int64_t cap = (int64_t)device_props().sms * 8;
         if (blocks > cap)
             blocks = cap;
-        SMVP_LAUNCH(tjds_permute_x_kernel, (unsigned)blocks, 256, 0, s, d_x, (const int32_t *)A->perm, A->cols, A->nslots, A->x_perm,
-                    A->x_exp);
+        SMVP_LAUNCH(tjds_permute_x_kernel, (unsigned)blocks, 256, 0, s, d_x, (const int32_t *)A->perm.get(), A->cols, A->nslots,
+                    A->x_perm.get(), A->x_exp.get());
     }
-    SMVP_CUDA(cudaMemcpyAsync(A->x_exp_host, A->x_exp, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-    SMVP_CUDA(cudaEventRecord(A->x_exp_event, s));
+    SMVP_CUDA(cudaMemcpyAsync(A->x_exp_host.get(), A->x_exp.get(), sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    SMVP_CUDA(cudaEventRecord(A->x_exp_event.get(), s));
     A->x_exp_pending = 1;
     SMVP_CUDA(cudaGetLastError());
     return SMVP_OK;
@@ -1146,13 +1130,15 @@ static int tjds_prepare(smvp_tjds *A, int variant, const Axpby &ab, cudaStream_t
     // a dot pass always runs the epilogue
     if ((!ab.plain() || dot) && A->relabel_state != 1 && (variant == SMVP_TJDS_ATOMIC || A->det_route != 1) && !A->y_sum)
     {
-        SMVP_CUDA(dev_alloc(&A->y_sum, A->rows));
+        SMVP_CUDA(dev_alloc(A->y_sum, A->rows));
         A->device_bytes += 8 * (int64_t)A->rows;
     }
     return SMVP_OK;
 }
 
-#define SMVP_TJDS_ARGS_COMMON (const int2 *)A->seg_blocks, (const int32_t *)A->start_pos, mult_rows(A), (const double *)A->val, (const double *)A->x_perm
+#define SMVP_TJDS_ARGS_COMMON                                                                                    \
+    (const int2 *)A->seg_blocks.get(), (const int32_t *)A->start_pos.get(), mult_rows(A), (const double *)A->val.get(), \
+        (const double *)A->x_perm.get()
 
 // one pass, asynchronous on s; tjds_prepare has run (with the same ab and dot).  dot != NULL: the per-row kernel that
 // stores y (unrank or det-finalize) also leaves the dot partials of its 256-row blocks in dot->part.
@@ -1169,9 +1155,9 @@ static int tjds_pass(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit,
     {
         double *y_caller = d_y;
         if (ranked)
-            d_y = A->y_rel; // sums land in rank order; tjds_unrank_y_kernel puts them back
+            d_y = A->y_rel.get(); // sums land in rank order; tjds_unrank_y_kernel puts them back
         else if (epi)
-            d_y = A->y_sum; // sums land beside y; tjds_unrank_y_kernel (identity rank) applies the epilogue
+            d_y = A->y_sum.get(); // sums land beside y; tjds_unrank_y_kernel (identity rank) applies the epilogue
         SMVP_CUDA(cudaMemsetAsync(d_y, 0, sizeof(double) * (size_t)A->rows, s));
         if (blocks > 0 && lim > 0)
         {
@@ -1187,7 +1173,7 @@ static int tjds_pass(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit,
             const int64_t cap = (int64_t)device_props().sms * 8;
             if (mode != YStore::Dot)
                 ub = ceil_div64(A->rows, 256 * 4) < cap ? ceil_div64(A->rows, 256 * 4) : cap;
-            const int32_t *rank = ranked ? (const int32_t *)A->row_rank : nullptr;
+            const int32_t *rank = ranked ? (const int32_t *)A->row_rank.get() : nullptr;
             with_store<YStore::Plain, YStore::Axpby, YStore::Dot>(mode, [&](auto S) {
                 SMVP_LAUNCH(tjds_unrank_y_kernel<decltype(S)::value>, (unsigned)ub, 256, 0, s, (const double *)d_y, rank, A->rows, y_caller,
                             ab.alpha, ab.beta, dot_w, part);
@@ -1201,7 +1187,8 @@ static int tjds_pass(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit,
         // only the rows that hold entries have accumulators to clear and convert (tjds_prepare_det found the range)
         const int32_t r_lo = A->det_flags[4] >= 0 ? A->det_flags[3] : 0, r_hi = A->det_flags[4] + 1;
         for (int w = 0; w < words && r_hi > r_lo; w++)
-            SMVP_CUDA(cudaMemsetAsync(A->acc + (size_t)w * (size_t)A->rows + r_lo, 0, sizeof(long long) * (size_t)(r_hi - r_lo), s));
+            SMVP_CUDA(cudaMemsetAsync(A->acc.get() + (size_t)w * (size_t)A->rows + r_lo, 0, sizeof(long long) * (size_t)(r_hi - r_lo),
+                                      s));
         if (blocks > 0 && lim > 0)
         {
             // CTAs per SM: 6 for the two-word kernel (40 registers).  The one-word kernel of the skewed fast walk runs at 8
@@ -1213,20 +1200,20 @@ static int tjds_pass(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit,
                     constexpr bool SKEW = decltype(SK)::value, FAST = decltype(FA)::value;
                     if (words == 2)
                         SMVP_LAUNCH((tjds_det_kernel<4, SKEW, FAST, 6, 2>), blocks, 256, 0, s, SMVP_TJDS_ARGS_COMMON,
-                                    (const int32_t *)A->row_exp, (const int32_t *)A->x_exp, (unsigned long long *)A->acc, A->rows,
-                                    A->nslots, lim);
+                                    (const int32_t *)A->row_exp.get(), (const int32_t *)A->x_exp.get(),
+                                    (unsigned long long *)A->acc.get(), A->rows, A->nslots, lim);
                     else
                         SMVP_LAUNCH((tjds_det_kernel<4, SKEW, FAST, SKEW && FAST ? 8 : 6, 1>), blocks, 256, 0, s,
-                                    SMVP_TJDS_ARGS_COMMON, (const int32_t *)A->row_exp, (const int32_t *)A->x_exp,
-                                    (unsigned long long *)A->acc, A->rows, A->nslots, lim);
+                                    SMVP_TJDS_ARGS_COMMON, (const int32_t *)A->row_exp.get(), (const int32_t *)A->x_exp.get(),
+                                    (unsigned long long *)A->acc.get(), A->rows, A->nslots, lim);
                     return (int)SMVP_OK;
                 });
             });
         }
         with_store<YStore::Plain, YStore::Axpby, YStore::Dot>(mode, [&](auto S) {
             SMVP_LAUNCH(tjds_det_finalize_kernel<decltype(S)::value>, (unsigned)ceil_div64(A->rows, 256), 256, 0, s,
-                        (const long long *)A->acc, (const int32_t *)A->row_exp, (const int32_t *)A->x_exp, A->rows, d_y,
-                        ranked ? (const int32_t *)A->row_rank : nullptr, words, r_lo, r_hi, ab.alpha, ab.beta, dot_w, part);
+                        (const long long *)A->acc.get(), (const int32_t *)A->row_exp.get(), (const int32_t *)A->x_exp.get(), A->rows,
+                        d_y, ranked ? (const int32_t *)A->row_rank.get() : nullptr, words, r_lo, r_hi, ab.alpha, ab.beta, dot_w, part);
             return (int)SMVP_OK;
         });
     }
@@ -1255,10 +1242,10 @@ static int tjds_mult_any(smvp_tjds *A, const Axpby &ab, double *d_y, int variant
     SMVP_TRY(dot_scratch(&A->dot_buf, &A->dot_cap, &A->device_bytes, tjds_dot_units_max(A), s));
     if (A->rows > 0)
     {
-        const DotOut dot = {d_w, A->dot_buf};
+        const DotOut dot = {d_w, A->dot_buf.get()};
         SMVP_TRY(tjds_pass(A, d_y, variant, diag_limit, ab, s, &dot));
     }
-    return dot_reduce(A->dot_buf, A->dot_cap, units, d_dot, s);
+    return dot_reduce(A->dot_buf.get(), A->dot_cap, units, d_dot, s);
 }
 
 extern "C" int smvp_tjds_mult_device(smvp_tjds *A, double *d_y, int variant, int32_t diag_limit, void *stream)
@@ -1288,13 +1275,13 @@ extern "C" int smvp_tjds_mult(smvp_tjds *A, const double *x_host, double *y_host
     if (variant != SMVP_TJDS_ATOMIC && variant != SMVP_TJDS_DETERMINISTIC && variant != SMVP_TJDS_DETERMINISTIC_FAST)
         return SMVP_E_ARG;
     if (!A->d_x)
-        SMVP_CUDA(dev_alloc(&A->d_x, A->cols));
+        SMVP_CUDA(dev_alloc(A->d_x, A->cols));
     if (!A->d_y)
-        SMVP_CUDA(dev_alloc(&A->d_y, A->rows));
+        SMVP_CUDA(dev_alloc(A->d_y, A->rows));
     if (A->cols > 0)
-        SMVP_CUDA(cudaMemcpy(A->d_x, x_host, sizeof(double) * (size_t)A->cols, cudaMemcpyHostToDevice));
+        SMVP_CUDA(cudaMemcpy(A->d_x.get(), x_host, sizeof(double) * (size_t)A->cols, cudaMemcpyHostToDevice));
     // x is permuted once, before the loop, as the reference does at build time (main-cli.c:907-923)
-    SMVP_TRY(smvp_tjds_set_x_device(A, A->d_x, nullptr));
+    SMVP_TRY(smvp_tjds_set_x_device(A, A->d_x.get(), nullptr));
     SMVP_TRY(tjds_prepare(A, variant, AXPBY_PLAIN, 0));
     // the zero-fill of y / of the accumulators is part of the pass and therefore INSIDE the timed bracket (the
     // reference keeps its vectorInit outside, main-cli.c:1008): conservative.
@@ -1304,19 +1291,21 @@ extern "C" int smvp_tjds_mult(smvp_tjds *A, const double *x_host, double *y_host
     std::function<int(cudaStream_t, int)> multi;
     if (tiny)
         multi = [&](cudaStream_t s, int n) {
-            SMVP_LAUNCH(tjds_tiny_loop_kernel, 1, TJDS_TINY_THREADS, 0, s, (const int32_t *)A->start_pos, (const int32_t *)A->slot_len,
-                        (const int32_t *)A->row_ind, (const double *)A->val, (const double *)A->x_perm, A->d_y, A->rows, A->nslots,
-                        tjds_effective_limit(A, diag_limit), n);
+            SMVP_LAUNCH(tjds_tiny_loop_kernel, 1, TJDS_TINY_THREADS, 0, s, (const int32_t *)A->start_pos.get(),
+                        (const int32_t *)A->slot_len.get(), (const int32_t *)A->row_ind.get(), (const double *)A->val.get(),
+                        (const double *)A->x_perm.get(), A->d_y.get(), A->rows, A->nslots, tjds_effective_limit(A, diag_limit), n);
             SMVP_CUDA(cudaGetLastError());
             return (int)SMVP_OK;
         };
     if (A->rows > 0)
-        SMVP_TRY(timed_loop(iters, ms_each, small, [&](cudaStream_t s) { return tjds_pass(A, A->d_y, variant, diag_limit, AXPBY_PLAIN, s); }, multi));
+        SMVP_TRY(timed_loop(
+            iters, ms_each, small, [&](cudaStream_t s) { return tjds_pass(A, A->d_y.get(), variant, diag_limit, AXPBY_PLAIN, s); },
+            multi));
     else if (ms_each)
         for (int it = 0; it < iters; it++)
             ms_each[it] = 0.0;
     if (A->rows > 0)
-        SMVP_CUDA(cudaMemcpy(y_host, A->d_y, sizeof(double) * (size_t)A->rows, cudaMemcpyDeviceToHost));
+        SMVP_CUDA(cudaMemcpy(y_host, A->d_y.get(), sizeof(double) * (size_t)A->rows, cudaMemcpyDeviceToHost));
     return SMVP_OK;
 }
 
