@@ -45,6 +45,7 @@ extern "C" {
 #define SMVP_E_CUDA (-3)        /* CUDA runtime error (no device, launch failure, ...)       */
 #define SMVP_E_RANGE (-4)       /* a coordinate lies outside [0,rows) x [0,cols)             */
 #define SMVP_E_TOOBIG (-5)      /* nnz does not fit the format's int32 offsets               */
+#define SMVP_E_PATTERN (-6)     /* a (row, col) pair the handle does not store               */
 
 /* == MMRawData (main-cli.c:42-47): 16 bytes, no padding.  0-based coordinates. */
 typedef struct smvp_coo
@@ -257,6 +258,50 @@ int smvp_tjds_mult_device_axpby_dot(smvp_tjds *A, double alpha, double beta, dou
                                     double *d_dot, int variant, int32_t diag_limit, void *stream);
 int smvp_tjds_mult_transpose_device_axpby_dot(smvp_tjds *A, double alpha, const double *d_x, double beta, double *d_y,
                                               const double *d_w, double *d_dot, void *stream);
+
+/* ---- new values on the stored entries (Newton steps, implicit time steps, continuation, shifted systems A - sigma I: the
+ * sparsity stays, the values change) without a new build.
+ *
+ * Input: a COO list of n entries in the form the builders take -- the host variant an smvp_coo array (copied to the
+ *    device as smvp_csr_build does), the device variant structure-of-arrays device pointers.  Every (row, col) of the list
+ *    must be an entry the handle stores; its value is replaced.  Entries not in the list keep their values.  Any order,
+ *    any subset (only the diagonal, for A - sigma I, is fine).  n = 0 is a no-op.  A pair listed twice: one of its values
+ *    lands, which one is unspecified (the handle stays consistent: its plans are decided from the values that landed).
+ * Structure never changes: a value set to 0 stays stored as an explicit zero (TJDS's count_r still counts it).  To add or
+ *    remove entries, build a new handle.  A handle made by smvp_csr_transpose is updated with the same list with rows and
+ *    columns swapped.
+ * Errors that leave the handle untouched, bit for bit (the whole list is checked before anything is written):
+ *    SMVP_E_ARG a NULL handle, n < 0, or NULL arrays with n > 0; SMVP_E_RANGE a coordinate outside [0,rows) x [0,cols);
+ *    SMVP_E_PATTERN a pair the handle does not store (any pair, on a handle without entries).
+ * Errors after the write (SMVP_E_CUDA, SMVP_E_ALLOC): the handle holds the new values; its value-dependent plans are back
+ *    to "not decided" and the next pass decides them as on a new handle.
+ * Result: the handle behaves exactly like smvp_*_build run on the updated matrix once both have decided the same plans --
+ *    the same smvp_*_export arrays, the same y bits from every pass (plain, *_axpby, *_axpby_dot and its dot, transposed,
+ *    host -n loop, fan-out; SMVP_TJDS_ATOMIC as reproducible as between two runs), the same smvp_*_info except
+ *    input_order (how the handle was built) and device_bytes (the scratch allocated so far).
+ * Kept, not recomputed: row_ptr / col_ind, TJDS perm / start_pos / row_ind; the merge tiles, the row patterns, the
+ *    relabelling, the TJDS walk and segment table, the pipelined host plan, the transposed and dot scratch, the co-runner
+ *    headroom, and the x declared with smvp_*_set_x_device (it stays in effect).  val is rewritten in place: the pointers
+ *    of smvp_csr_arrays_device stay valid.
+ * Decided again for the new values: CSR with row_patterns > 0 -- value_bytes and its narrow copy (device_bytes follows
+ *    the width); TJDS once a deterministic pass has run -- the row bounds and matrix flags, and det_route goes back to 0
+ *    so that the next pass routes the current x again (Inf / NaN, the short split loop).  A plan still undecided stays so.
+ * Synchronous, like the builders: ordered on `stream` after the work enqueued there, returns when the update is complete.
+ *    No pass on the handle may be in flight on another stream (the rule of smvp_*_free).  A CUDA graph captured before an
+ *    update must be captured again: kernel choices baked into it (value width, TJDS short split) may no longer hold.
+ * Cost: no sort, no structural plan work; a fixed number of launches whatever n and nnz (CSR: 2, plus 2 with the row
+ *    patterns; TJDS: 3, plus 2 with the deterministic state; the host variants 1 more to unzip the list).  One thread per
+ *    entry binary-searches its row (CSR) or its column (TJDS), twice: once to check the whole list, once to write.
+ *    Temporaries: O(rows + cols) (TJDS: the slot of every column, and the row counts of the bound pass), never O(nnz) or
+ *    O(n); the host variants stage the list on the device as the builders do (32 bytes per entry).
+ *    Measured (DESIGN.md §5.8): faster than a rebuild for a CSR list in row order and for short lists (the diagonal); a
+ *    full list in random order, and a full TJDS list in any order, cost about a rebuild or more.                      */
+int smvp_csr_update_values(smvp_csr *A, const smvp_coo *coo, int64_t n);
+int smvp_csr_update_values_device(smvp_csr *A, const int32_t *d_row, const int32_t *d_col, const double *d_val, int64_t n,
+                                  void *stream);
+int smvp_tjds_update_values(smvp_tjds *A, const smvp_coo *coo, int64_t n);
+int smvp_tjds_update_values_device(smvp_tjds *A, const int32_t *d_row, const int32_t *d_col, const double *d_val, int64_t n,
+                                   void *stream);
 
 /* ---- introspection ---- */
 typedef struct smvp_csr_info_t

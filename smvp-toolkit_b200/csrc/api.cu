@@ -22,6 +22,8 @@ extern "C" const char *smvp_strerror(int code)
         return "matrix coordinate out of range";
     case SMVP_E_TOOBIG:
         return "problem too large for int32 offsets";
+    case SMVP_E_PATTERN:
+        return "entry not stored in the matrix (a value update cannot add entries)";
     default:
         return "unknown error";
     }

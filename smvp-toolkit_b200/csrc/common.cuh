@@ -395,6 +395,7 @@ namespace smvp
 int csr_relabel_plan(smvp_csr *A, cudaStream_t s);                 // relabel.cu
 int csr_relabel_x(smvp_csr *A, const double *d_x, cudaStream_t s); // relabel.cu
 int csr_pattern_plan(smvp_csr *A, cudaStream_t s);                // pattern.cu: decides the relabelling first
+int csr_pattern_values(smvp_csr *A, cudaStream_t s);              // pattern.cu: the value width of an accepted plan
 } // namespace smvp
 
 struct smvp_tjds
@@ -449,4 +450,5 @@ struct smvp_tjds
 namespace smvp
 {
 int tjds_relabel_plan(smvp_tjds *A, cudaStream_t s); // relabel.cu
+int tjds_update_det(smvp_tjds *A, cudaStream_t s);   // tjds_mult.cu: the row bounds again after a value update
 } // namespace smvp

@@ -171,9 +171,19 @@ __global__ void __launch_bounds__(256) pattern_narrow_kernel(const double *__res
         out[j] = narrow_value<V>(val[j]);
 }
 
-// the narrowest width (2, 4 or 8 bytes) that holds every value exactly, and the copy of val at that width (none at 8)
-static int pattern_values(const smvp_csr *A, unsigned grid, cudaStream_t s, int32_t *vbytes, DevPtr<char> *narrow)
+// The value width of an accepted plan: the narrowest width (2, 4 or 8 bytes) that holds every value of val exactly, and the
+// copy of val at that width (none at 8) -- narrowed in place when the handle already holds a copy at that width (a value
+// update that keeps the width).  Used by the plan and by smvp_csr_update_values (update.cu), so that both decide the
+// width with the same code.  Synchronous.  On failure the width is left undecided (pat_vbytes 0, no copy): the next pass
+// decides it again.
+int csr_pattern_values(smvp_csr *A, cudaStream_t s)
 {
+    const int32_t held = A->pat_vbytes;
+    DevPtr<char> copy = std::move(A->pat_val);
+    A->device_bytes -= held > 0 && held < 8 ? held * A->nnz : 0;
+    A->pat_vbytes = 0;
+    const int64_t blocks = ceil_div64(A->rows, 256), cap = (int64_t)device_props().sms * 8;
+    const unsigned grid = (unsigned)(blocks < cap ? blocks : cap);
     DevPtr<int32_t> flags;
     SMVP_CUDA(dev_alloc(flags, 1));
     int32_t h_flags = 0;
@@ -184,8 +194,9 @@ static int pattern_values(const smvp_csr *A, unsigned grid, cudaStream_t s, int3
     SMVP_CUDA(cudaMemcpyAsync(&h_flags, flags.get(), sizeof(int32_t), cudaMemcpyDeviceToHost, s));
     SMVP_CUDA(cudaStreamSynchronize(s));
     const int32_t vb = !(h_flags & 1) ? 2 : !(h_flags & 2) ? 4 : 8;
-    DevPtr<char> copy;
-    if (vb < 8)
+    if (vb != held)
+        copy.reset();
+    if (vb < 8 && !copy)
         SMVP_CUDA(dev_alloc(copy, vb * A->nnz));
     if (vb == 2 && A->nnz > 0)
         SMVP_LAUNCH(pattern_narrow_kernel<uint16_t>, grid, 256, 0, s, (const double *)A->val.get(), A->nnz, (uint16_t *)copy.get());
@@ -193,8 +204,9 @@ static int pattern_values(const smvp_csr *A, unsigned grid, cudaStream_t s, int3
         SMVP_LAUNCH(pattern_narrow_kernel<float>, grid, 256, 0, s, (const double *)A->val.get(), A->nnz, (float *)copy.get());
     SMVP_CUDA(cudaGetLastError());
     SMVP_CUDA(cudaStreamSynchronize(s));
-    *vbytes = vb;
-    *narrow = std::move(copy);
+    A->pat_val = std::move(copy);
+    A->pat_vbytes = vb;
+    A->device_bytes += vb < 8 ? vb * A->nnz : 0;
     return SMVP_OK;
 }
 
@@ -203,6 +215,8 @@ static int pattern_values(const smvp_csr *A, unsigned grid, cudaStream_t s, int3
 int csr_pattern_plan(smvp_csr *A, cudaStream_t s)
 {
     SMVP_TRY(csr_relabel_plan(A, s)); // a relabelled handle reads col_rel: that plan decides first
+    if (A->pattern_state == 1 && A->pat_vbytes == 0)
+        return csr_pattern_values(A, s); // a value update failed after its write: the width is decided again
     if (A->pattern_state != 0)
         return SMVP_OK;
     if (A->relabel_state == 1 || A->rows == 0 || env_tristate("SMVP_CSR_PATTERN") == -1)
@@ -271,17 +285,13 @@ int csr_pattern_plan(smvp_csr *A, cudaStream_t s)
         A->pattern_state = -1;
         return SMVP_OK;
     }
-    int32_t vbytes = 0;
-    DevPtr<char> narrow;
-    SMVP_TRY(pattern_values(A, grid, s, &vbytes, &narrow));
+    SMVP_TRY(csr_pattern_values(A, s));
     A->pat_id = std::move(pat_id);
     A->pat_off = std::move(pat_off);
     A->pat_len = std::move(pat_len);
-    A->pat_val = std::move(narrow);
-    A->pat_vbytes = vbytes;
     A->pattern_count = npat;
     A->pattern_maxlen = npat > 0 ? *std::max_element(h_len.begin(), h_len.end()) : 0;
-    A->device_bytes += (int64_t)A->rows + 4 * (int64_t)npat * (PAT_LMAX + 1) + (vbytes < 8 ? vbytes * A->nnz : 0);
+    A->device_bytes += (int64_t)A->rows + 4 * (int64_t)npat * (PAT_LMAX + 1);
     A->pattern_state = 1;
     return SMVP_OK;
 }

@@ -828,22 +828,19 @@ static int tjds_plan(smvp_tjds *A, cudaStream_t s)
     return SMVP_OK;
 }
 
-static int tjds_prepare_det(smvp_tjds *A, cudaStream_t s)
+// The row bounds of the deterministic variants, from the current values: row_exp[rows] and the matrix flags
+// (smvp_tjds::det_flags) into det_flags.  Synchronous.
+static int tjds_row_bounds(const smvp_tjds *A, int32_t *row_exp, int32_t det_flags[5], cudaStream_t s)
 {
-    if (A->row_exp)
-        return SMVP_OK;
-    DevPtr<int32_t> row_exp, flags;
-    DevPtr<long long> acc;
+    DevPtr<int32_t> flags;
     DevPtr<uint32_t> cnt;
-    SMVP_CUDA(dev_alloc(row_exp, A->rows));
-    SMVP_CUDA(dev_alloc(acc, 2 * (int64_t)A->rows));
     SMVP_CUDA(dev_alloc(cnt, A->rows));
     SMVP_CUDA(dev_alloc(flags, 5));
     const int32_t h0[5] = {0, EXP_NONE, EXP_LOW_NONE, 0x7fffffff, -1};
     SMVP_CUDA(cudaMemcpyAsync(flags.get(), h0, sizeof(h0), cudaMemcpyHostToDevice, s));
     SMVP_CUDA(cudaMemsetAsync(cnt.get(), 0, sizeof(uint32_t) * (size_t)A->rows, s));
     // EXP_NONE = 0x80808080 is a byte pattern, so a memset fills it
-    SMVP_CUDA(cudaMemsetAsync(row_exp.get(), 0x80, sizeof(int32_t) * (size_t)A->rows, s));
+    SMVP_CUDA(cudaMemsetAsync(row_exp, 0x80, sizeof(int32_t) * (size_t)A->rows, s));
     if (A->nnz > 0)
     {
         int64_t blocks = ceil_div64(A->nnz, 256 * 4);
@@ -852,20 +849,52 @@ static int tjds_prepare_det(smvp_tjds *A, cudaStream_t s)
             blocks = cap;
         // after the relabel decision: row_exp lives in the index space the kernels use
         SMVP_LAUNCH(tjds_row_bound_kernel, (unsigned)blocks, 256, 0, s, mult_rows(A), (const double *)A->val.get(), A->nnz,
-                    row_exp.get(), cnt.get(), flags.get());
+                    row_exp, cnt.get(), flags.get());
     }
     if (A->rows > 0)
-        SMVP_LAUNCH(tjds_row_exp_kernel, (unsigned)ceil_div64(A->rows, 256), 256, 0, s, row_exp.get(), (const uint32_t *)cnt.get(),
+        SMVP_LAUNCH(tjds_row_exp_kernel, (unsigned)ceil_div64(A->rows, 256), 256, 0, s, row_exp, (const uint32_t *)cnt.get(),
                     A->rows, flags.get());
-    int32_t det_flags[5];
-    static_assert(sizeof(det_flags) == sizeof(A->det_flags), "flags layout");
-    SMVP_CUDA(cudaMemcpyAsync(det_flags, flags.get(), sizeof(det_flags), cudaMemcpyDeviceToHost, s));
+    SMVP_CUDA(cudaMemcpyAsync(det_flags, flags.get(), 5 * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
     SMVP_CUDA(cudaStreamSynchronize(s));
     SMVP_CUDA(cudaGetLastError());
+    return SMVP_OK;
+}
+
+static int tjds_prepare_det(smvp_tjds *A, cudaStream_t s)
+{
+    if (A->row_exp)
+        return SMVP_OK;
+    DevPtr<int32_t> row_exp;
+    DevPtr<long long> acc;
+    SMVP_CUDA(dev_alloc(row_exp, A->rows));
+    SMVP_CUDA(dev_alloc(acc, 2 * (int64_t)A->rows));
+    int32_t det_flags[5];
+    static_assert(sizeof(det_flags) == sizeof(A->det_flags), "flags layout");
+    SMVP_TRY(tjds_row_bounds(A, row_exp.get(), det_flags, s));
     memcpy(A->det_flags, det_flags, sizeof(det_flags));
     A->row_exp = std::move(row_exp);
     A->acc = std::move(acc);
     A->det_route = 0; // depends on the matrix flags just computed
+    return SMVP_OK;
+}
+
+// After smvp_tjds_update_values has written new values: the row bounds and matrix flags again, into the handle's own
+// row_exp, and the route of the current x decided again at the next pass.  Nothing to do while the deterministic state
+// does not exist yet.  On failure that state is dropped, so the next deterministic pass builds it as on a new handle.
+int tjds_update_det(smvp_tjds *A, cudaStream_t s)
+{
+    if (!A->row_exp)
+        return SMVP_OK;
+    A->det_route = 0;
+    int32_t det_flags[5];
+    const int rc = tjds_row_bounds(A, A->row_exp.get(), det_flags, s);
+    if (rc != SMVP_OK)
+    {
+        A->row_exp.reset();
+        A->acc.reset();
+        return rc;
+    }
+    memcpy(A->det_flags, det_flags, sizeof(det_flags));
     return SMVP_OK;
 }
 

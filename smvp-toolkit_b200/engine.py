@@ -28,7 +28,7 @@ CSR_AUTO, CSR_VECTOR, CSR_MERGE = 0, 1, 2
 TJDS_ATOMIC, TJDS_DETERMINISTIC, TJDS_DETERMINISTIC_FAST = 0, 1, 2
 VAL_STENCIL, VAL_HASH, VAL_ONES = 0, 1, 2
 
-OK, E_ARG, E_ALLOC, E_CUDA, E_RANGE, E_TOOBIG = 0, -1, -2, -3, -4, -5
+OK, E_ARG, E_ALLOC, E_CUDA, E_RANGE, E_TOOBIG, E_PATTERN = 0, -1, -2, -3, -4, -5, -6
 
 
 class SmvpError(RuntimeError):
@@ -88,6 +88,10 @@ SIGNATURES = {
     "smvp_csr_mult_device_axpby_dot": (_int, [_vp, _dbl, _vp, _dbl, _vp, _vp, _vp, _int, _vp]),
     "smvp_tjds_mult_device_axpby_dot": (_int, [_vp, _dbl, _dbl, _vp, _vp, _vp, _int, _i32, _vp]),
     "smvp_tjds_mult_transpose_device_axpby_dot": (_int, [_vp, _dbl, _vp, _dbl, _vp, _vp, _vp, _vp]),
+    "smvp_csr_update_values": (_int, [_vp, _vp, _i64]),
+    "smvp_csr_update_values_device": (_int, [_vp, _vp, _vp, _vp, _i64, _vp]),
+    "smvp_tjds_update_values": (_int, [_vp, _vp, _i64]),
+    "smvp_tjds_update_values_device": (_int, [_vp, _vp, _vp, _vp, _i64, _vp]),
     "smvp_csr_info": (_int, [_vp, ctypes.POINTER(_CsrInfo)]),
     "smvp_tjds_info": (_int, [_vp, ctypes.POINTER(_TjdsInfo)]),
     "smvp_csr_export": (_int, [_vp, _vp, _vp, _vp]),
@@ -313,6 +317,18 @@ class CsrMatrix:
         _check(lib().smvp_csr_mult_device_fanout(self._h, _ptr(d_x), arr, len(y_ptrs), variant, _stream(stream)),
                "smvp_csr_mult_device_fanout")
 
+    def update_values(self, coo):
+        """New values on stored entries from a host COO list (any order, any subset; smvp_csr_update_values): every
+        (row, col) must be stored (SmvpError E_PATTERN otherwise, E_RANGE outside the matrix; the matrix is then
+        unchanged).  Plans that depend only on the structure and the declared x stay; the value width is decided again."""
+        coo = _as_coo(coo)
+        _check(lib().smvp_csr_update_values(self._h, _ptr(coo), len(coo)), "smvp_csr_update_values")
+
+    def update_values_device(self, d_row, d_col, d_val, n, stream=None):
+        """update_values from a structure-of-arrays device COO of n entries, ordered on `stream`; returns when done."""
+        _check(lib().smvp_csr_update_values_device(self._h, _ptr(d_row), _ptr(d_col), _ptr(d_val), n, _stream(stream)),
+               "smvp_csr_update_values_device")
+
     def export(self):
         row_ptr = np.zeros(self.rows + 1, np.int32)
         col_ind = np.zeros(self.nnz, np.int32)
@@ -434,6 +450,17 @@ class TjdsMatrix:
         """mult_device_axpby with d_dot[0] = sum of w[r] * y_new[r] formed in the same pass (d_w=None: w = y_new)."""
         _check(lib().smvp_tjds_mult_device_axpby_dot(self._h, alpha, beta, _ptr(d_y), _ptr(d_w), _ptr(d_dot), variant, diag_limit,
                                                      _stream(stream)), "smvp_tjds_mult_device_axpby_dot")
+
+    def update_values(self, coo):
+        """New values on stored entries from a host COO list (smvp_tjds_update_values; the contract of
+        CsrMatrix.update_values).  The deterministic row bounds are decided again; the declared x stays."""
+        coo = _as_coo(coo)
+        _check(lib().smvp_tjds_update_values(self._h, _ptr(coo), len(coo)), "smvp_tjds_update_values")
+
+    def update_values_device(self, d_row, d_col, d_val, n, stream=None):
+        """update_values from a structure-of-arrays device COO of n entries, ordered on `stream`; returns when done."""
+        _check(lib().smvp_tjds_update_values_device(self._h, _ptr(d_row), _ptr(d_col), _ptr(d_val), n, _stream(stream)),
+               "smvp_tjds_update_values_device")
 
     def export(self):
         perm = np.zeros(self.cols, np.int32)
